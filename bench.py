@@ -21,6 +21,9 @@ Weak scaling by default (Q queries per GPU); `--scaling strong` shards `--querie
 config 4 as written: 4096 queries over 1/2/4/8 GPUs); at N > 1 the weak run also reports the strong figure.
 
 `--impl reference` times only the CPU leg (all host cores) and prints the same JSON shape.
+
+`--dump-outputs DIR` writes what the device-resident leg returned in its last timed step (rank 0's queries) as
+DIR/<name>.npy, so that two builds can be compared output for output: the inputs depend only on the arguments.
 """
 from __future__ import annotations
 
@@ -44,6 +47,7 @@ UNIT = "evals/s"
 FLOP_PER_EVAL = 5.0      # 2 SUB + 1 MUL + 1 FMA (SURVEY.md section 8d)
 N_PEDS, T_OBS = 50, 51
 TARGET_SPEED = 6.0
+DUMP_LIMIT = 60 << 20    # array bytes --dump-outputs may write: with the file headers, under 64 MB however counted
 
 
 # ------------------------------------------------------------------------------------------
@@ -70,6 +74,25 @@ def make_queries(first: int, count: int):
         ego, dyn[i, 0] = ego_and_field(first + i)
         frenet[i] = ego_to_frenet(CoordinateConverter(spline), EgoVehicleState(*ego), 0.0)
     return spline, frenet, dyn
+
+
+def dump_outputs(out_dir, out, query_ids):
+    """The winner block `out` of queries `query_ids` as out_dir/<name>.npy in float64: best_idx, best_cost, stats,
+    winner_len, winner [n, 15, n_t_max] and query_id.  Every value is finite: a query without a path (best_idx -1)
+    has its infinite best_cost stored as 0, and winner samples at or past winner_len, which the kernel never writes,
+    are stored as 0.  Above DUMP_LIMIT bytes a fixed, seeded sample of the queries is written."""
+    host = {k: v.cpu().numpy().astype(np.float64) for k, v in out.items()}
+    host["best_cost"] = np.where(host["best_idx"] >= 0, host["best_cost"], 0.0)
+    host["winner"] = np.where(np.arange(host["winner"].shape[2]) < host["winner_len"][:, None, None], host["winner"], 0.0)
+    host["query_id"] = np.asarray(query_ids, dtype=np.float64)
+    n = len(query_ids)
+    row_bytes = sum(v[0].nbytes for v in host.values())
+    keep = np.arange(n)
+    if n * row_bytes > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v[keep])
 
 
 # ------------------------------------------------------------------------------------------
@@ -299,6 +322,8 @@ def main():
     ap.add_argument("--gather-priority", type=int, default=0, help="tuning: CUDA priority of the gather stream (0 default, -1 high)")
     ap.add_argument("--brief", action="store_true", help="resident + e2e legs only (scaling experiments)")
     ap.add_argument("--wc-input", action="store_true", help="experiment: e2e input in write-combined pinned memory (cudaHostAllocWriteCombined)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the resident leg's last-step winners (rank 0's queries) "
+                                                          "as DIR/<name>.npy, float64, at most 64 MB")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -528,6 +553,8 @@ def main():
     evals_local = leg.batch.dense_evals()
     evals_total = float(sum(all_list(evals_local)))
     ms_step, stage, clocks = leg.run(args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, leg.batch.out, np.arange(q_lo, q_hi))
     gather_ok = leg.verify_gather()
     sweep_ms = float(stage[:, 1].mean())
     value = evals_total / (ms_step * 1e-3)

@@ -100,7 +100,7 @@ def make_standard():
 
 def make_closed_loop(max_calls=96):
     """Config 1: scenario_01_cv closed loop; the reference planner drives the simulation and every
-    plan() call is recorded (a spread of `max_calls` of them is stored, always including the calls
+    plan() call is recorded (a spread of up to `max_calls` of them is stored, always including the calls
     made with constraint overrides, i.e. the CAUTION / EMERGENCY retries)."""
     import yaml
     from src.config import SimulationConfig, validate_config
@@ -164,6 +164,9 @@ def make_closed_loop(max_calls=96):
     forced = [i for i, c in enumerate(calls) if not np.all(np.isnan(c["ovr"]))]
     spread = list(np.linspace(0, n - 1, max(2, max_calls - min(len(forced), max_calls // 2))).astype(int))
     keep = sorted(set(forced[: max_calls // 2]) | set(spread))
+    # every third kept call without overrides is left out, which keeps the file under 1 MB; every retry stays
+    plain = [i for i in keep if i not in set(forced)]
+    keep = sorted(set(keep) - set(plain[2::3]))
     store = {"n_calls_total": np.int64(n), "kept": np.array(keep, dtype=np.int64),
              "waypoints_x": np.array(cfg.reference_waypoints_x, dtype=np.float64),
              "waypoints_y": np.array(cfg.reference_waypoints_y, dtype=np.float64)}
