@@ -27,10 +27,11 @@
 extern "C" {
 #endif
 
-#define FOT_ABI_VERSION 6   /* 2: + prediction post-processing and safety metrics; 3: + fot_plan_batch_device_to_host;
+#define FOT_ABI_VERSION 7   /* 2: + prediction post-processing and safety metrics; 3: + fot_plan_batch_device_to_host;
                                4: + fot_result_t.winner_samples, fot_fetch_winners, fot_reload_options;
                                5: + fot_set_result_mirror, fot_peer_* (gather of a sharded sweep over peer memory);
-                               6: + fot_last_sweep_kind, fot_last_pair_features (fot_sweep_pairs is the default sweep kernel) */
+                               6: + fot_last_sweep_kind, fot_last_pair_features (fot_sweep_pairs is the default sweep kernel);
+                               7: + fot_nearest_s_device (nearest point on the path, certified against the host) */
 #define FOT_MAX_CIRCLES 8
 #define FOT_N_STATS 8    /* ok, max_speed, max_accel, max_curvature, max_lat_accel, road_bound, collision, stop_distance */
 #define FOT_N_SERIES 15  /* t s s_d s_dd s_ddd d d_d d_dd d_ddd x y yaw c v a  (data_structures.py:149-181) */
@@ -277,6 +278,15 @@ int fot_prepend_current_device(int device, void* stream, int n_q, int S, int P, 
 int fot_safety_metrics_device(int device, void* stream, int n_q, int P, const double* ego, const double* ped_pos,
                               const double* ped_vel, const int32_t* n_peds, double combined_radius,
                               const double* offsets, int n_circ, double* out);
+
+/* ---- ego state -> Frenet: the nearest-point search on the device (DESIGN.md section 4e) -------------------------
+ * best_s of find_nearest_point_on_path for n points (coordinate_converter.py:202-283) on the handle's path.
+ * x, y, prev_s (NaN = no cache) [n], s_out [n], status [n]: DEVICE pointers; status 0 = s_out is the reference's
+ * value, 1 = the caller must recompute that point on the host.  Asynchronous on `stream`, the stream on which the
+ * inputs are written (NULL: the handle's stream, ordered after the work queued so far on the legacy default stream,
+ * and synchronised).  prev_s is only read: the caller updates its caches. */
+int fot_nearest_s_device(fot_handle_t* h, void* stream, int n, const double* x, const double* y,
+                         const double* prev_s, double* s_out, int32_t* status);
 
 #ifdef __cplusplus
 }

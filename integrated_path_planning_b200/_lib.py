@@ -11,7 +11,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libfot.so")
 
-FOT_ABI_VERSION = 6
+FOT_ABI_VERSION = 7
 FOT_MAX_CIRCLES = 8
 FOT_N_STATS = 8
 FOT_N_SERIES = 15
@@ -101,6 +101,8 @@ SYMBOLS = (
                                              C.c_void_p, C.c_void_p, C.c_int, C.c_void_p)),
     ("fot_safety_metrics_device", C.c_int, (C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_double, c_double_p, C.c_int, C.c_void_p)),
+    ("fot_nearest_s_device", C.c_int, (C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p)),
 )
 
 _lib = None

@@ -12,6 +12,7 @@ import numpy as np
 
 from . import _lib
 from .engine import SweepEngine, SweepResult, speed_grid_batch
+from .frenet_host import BatchCoordinateConverter, ego_to_frenet_many
 from .planner import FrenetPlanner
 
 
@@ -23,7 +24,8 @@ def shard_bounds(n_q: int, world_size: int, rank: int):
 
 
 class BatchFrenetPlanner(FrenetPlanner):
-    """FrenetPlanner plus `plan_batch` (host arrays) and `plan_batch_device` (torch buffers)."""
+    """FrenetPlanner plus `plan_batch` (host arrays, Frenet states), `plan_batch_from_ego` (host arrays, ego states)
+    and `plan_batch_device` (torch buffers)."""
 
     def plan_batch(self, frenet_states, target_speed, dynamic_obstacles=None, distribution=None,
                    static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None,
@@ -46,6 +48,25 @@ class BatchFrenetPlanner(FrenetPlanner):
         return self.engine.run_host(fs, target_speed, limits, max_stop_distance, static_obstacles, dyn, mode,
                                     static_per_query=per_query, want_candidates=want_candidates,
                                     winner_samples=winner_samples)
+
+    def plan_batch_from_ego(self, ego, target_speed, last_kappa=0.0, converter: Optional[BatchCoordinateConverter] = None,
+                            **kwargs):
+        """plan() for n_q ego states at once: ego [n_q,5] (x, y, yaw, v, a), last_kappa scalar or [n_q] (the ego
+        curvature plan() keeps between calls), `converter` the n_q nearest-point caches to use and update (row q for
+        ego q; None: fresh ones on this planner's device, as a first plan() call has).  The nearest-point search runs
+        on the device (DESIGN.md section 4e), the rest of the Frenet conversion on the host, then `plan_batch` with
+        **kwargs.  Returns (SweepResult, ok): where ok is False the conversion failed and plan() would return None --
+        best_idx -1, best_cost inf, stats zero, winner_len 0."""
+        ego = np.asarray(ego, dtype=np.float64).reshape(-1, 5)
+        n_q = ego.shape[0]
+        if converter is None:
+            converter = BatchCoordinateConverter(self.csp, n_q, engine=self.engine)
+        kappa = np.broadcast_to(np.asarray(last_kappa, dtype=np.float64), (n_q,))
+        frenet, ok = ego_to_frenet_many(converter, np.arange(n_q), ego, kappa)
+        res = self.plan_batch(frenet, target_speed, **kwargs)
+        bad = ~ok
+        res.best_idx[bad], res.best_cost[bad], res.stats[bad], res.winner_len[bad] = -1, np.inf, 0, 0
+        return res, ok
 
 
 class DeviceBatch:

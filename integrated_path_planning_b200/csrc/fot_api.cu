@@ -16,6 +16,7 @@
 #include "fot_sweep_warp.cuh"
 #include "fot_sweep_pairs.cuh"
 #include "fot_predict.cuh"
+#include "fot_frenet.cuh"
 
 using namespace fot;
 
@@ -1457,6 +1458,25 @@ extern "C" int fot_safety_metrics_device(int device, void* stream, int n_q, int 
   fot_safety_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ego, ped_pos, ped_vel, n_peds, out, n_q, P,
                                                                                          combined_radius, off, n_circ);
   return pred_end(stream);
+}
+
+// ---- nearest point on the reference path (DESIGN.md section 4e) -----------------------------------------
+extern "C" int fot_nearest_s_device(fot_handle_t* h, void* stream, int n, const double* x, const double* y,
+                                    const double* prev_s, double* s_out, int32_t* status) {
+  if (!h || n < 0 || (n > 0 && (!x || !y || !prev_s || !s_out || !status)))
+    return fail(FOT_ERR_ARG, "fot_nearest_s_device: bad argument");
+  if (n == 0) return FOT_OK;
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  if (!stream) {                 // the handle's stream does not synchronise with the legacy default stream on its own:
+    CK(cudaEventRecord(h->ev_join, cudaStreamLegacy));   // inputs written there (plain or pinned async copies) come first
+    CK(cudaStreamWaitEvent(st, h->ev_join, 0));
+  }
+  const int threads = 256, per_block = threads / 32;
+  fot_nearest_s<<<(unsigned)((n + per_block - 1) / per_block), threads, 0, st>>>(h->plan, n, x, y, prev_s, s_out, status);
+  CK(cudaGetLastError());
+  if (!stream) CK(cudaStreamSynchronize(st));
+  return FOT_OK;
 }
 
 #ifdef FOT_PHASE_CLOCKS

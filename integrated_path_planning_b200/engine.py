@@ -169,6 +169,8 @@ class SweepEngine:
         self.n_steps, self.n_steps_b, self.n_total = self._keep["n_steps"], self._keep["n_steps_b"], n_total
         self._pinned = {}
         self._grid_cache = None
+        self._near_bufs = None                             # nearest_s: pinned / device staging, grown on demand
+        self._near_stream = None                           # nearest_s: its stream
         self._h = C.c_void_p()
         _lib.check(self.lib.fot_create(C.byref(cfg), C.byref(tb), self.device, C.byref(self._h)), "fot_create")
         self.n_t_max = self.lib.fot_n_t_max(self._h)
@@ -282,6 +284,42 @@ class SweepEngine:
         _lib.check(self.lib.fot_plan_batch_device(self._h, C.byref(batch), C.byref(result),
                                                   C.c_void_p(stream) if stream else None),
                    "fot_plan_batch_device")
+
+    def nearest_s(self, x, y, prev_s):
+        """fot_nearest_s_device for m points on this engine's path: returns (s [m], status [m] int32), status 0 where
+        s is the reference's best_s, 1 where the host has to recompute it.  One upload of x | y | prev_s, one
+        download of s | status, one synchronise; prev_s (NaN = no cache) is not modified."""
+        import torch
+        m = len(x)
+        if m == 0:
+            return np.zeros(0), np.zeros(0, dtype=np.int32)
+        bufs = self._near_bufs
+        if bufs is None or bufs[0].numel() < 3 * m:
+            cap = max(3 * m, 3 * 256)
+            dev = torch.device("cuda", self.device)
+            bufs = self._near_bufs = (torch.empty(cap, dtype=torch.float64, pin_memory=True),
+                                      torch.empty(cap, dtype=torch.float64, device=dev),
+                                      torch.empty(12 * (cap // 3), dtype=torch.uint8, pin_memory=True),
+                                      torch.empty(12 * (cap // 3), dtype=torch.uint8, device=dev))
+        h_in, d_in, h_out, d_out = bufs
+        a = h_in.numpy()
+        a[:m], a[m:2 * m], a[2 * m:3 * m] = x, y, prev_s
+        # upload, kernel and download on one stream of this engine's own: the kernel is ordered after the upload
+        # whatever stream the caller has made current (torch's default stream would reach the C call as NULL)
+        if self._near_stream is None:
+            self._near_stream = torch.cuda.Stream(self.device)
+        stream = self._near_stream
+        with torch.cuda.stream(stream):
+            d_in[:3 * m].copy_(h_in[:3 * m], non_blocking=True)
+            p_in, p_out = d_in.data_ptr(), d_out.data_ptr()
+            _lib.check(self.lib.fot_nearest_s_device(self._h, C.c_void_p(stream.cuda_stream), m, C.c_void_p(p_in),
+                                                     C.c_void_p(p_in + 8 * m), C.c_void_p(p_in + 16 * m),
+                                                     C.c_void_p(p_out), C.c_void_p(p_out + 8 * m)),
+                       "fot_nearest_s_device")
+            h_out[:12 * m].copy_(d_out[:12 * m], non_blocking=True)
+        stream.synchronize()
+        raw = h_out.numpy()
+        return raw[:8 * m].view(np.float64).copy(), raw[8 * m:12 * m].view(np.int32).copy()
 
     def launch_stage_ms(self, back: int = 0):
         """(prepass, sweep, winner) device ms of the `back`-th most recent launch."""

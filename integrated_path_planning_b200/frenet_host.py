@@ -224,11 +224,18 @@ class BatchCoordinateConverter:
 
     NEAR = 16.0 * np.finfo(np.float64).eps
 
-    def __init__(self, reference_path, n: int):
+    def __init__(self, reference_path, n: int, engine=None):
+        """engine: a SweepEngine built on the same path.  With it, `nearest_s` runs the search on the device
+        (fot_nearest_s_device) and recomputes here only the rows whose every decision the device could not certify
+        (DESIGN.md section 4e); the results and caches are the same either way.  `device_rows` / `host_rows` count
+        the rows each side answered."""
         self.one = CoordinateConverter(reference_path)
         self.path_end = float(reference_path.s[-1])
         self.prev_s = np.full(n, np.nan)
         self._global = None
+        self.engine = engine
+        self.device_rows = 0
+        self.host_rows = 0
 
     # positions as [rows, cols] arrays
     def _xy_grid(self, s):
@@ -249,6 +256,22 @@ class BatchCoordinateConverter:
     def nearest_s(self, idx, x, y):
         """best_s of find_nearest_point_on_path (coordinate_converter.py:202-283) for converters `idx` at
         the points (x, y); updates their caches."""
+        if self.engine is None:
+            return self._nearest_s_host(idx, x, y)
+        idx = np.asarray(idx, dtype=np.int64)
+        x = np.asarray(x, dtype=np.float64)
+        y = np.asarray(y, dtype=np.float64)
+        best, status = self.engine.nearest_s(x, y, self.prev_s[idx])
+        sure = status == 0
+        self.prev_s[idx[sure]] = best[sure]
+        redo = np.nonzero(~sure)[0]
+        if len(redo):                                     # their caches still hold the values from before this call
+            best[redo] = self._nearest_s_host(idx[redo], x[redo], y[redo])
+        self.device_rows += len(idx) - len(redo)
+        self.host_rows += len(redo)
+        return best
+
+    def _nearest_s_host(self, idx, x, y):
         idx = np.asarray(idx, dtype=np.int64)
         x = np.asarray(x, dtype=np.float64)
         y = np.asarray(y, dtype=np.float64)

@@ -230,8 +230,8 @@ class BatchedClosedLoop:
         # per-simulation planner state: ego curvature cache and the two nearest-point caches (the planner's
         # converter and the simulator's own goal-check converter are separate objects in the reference)
         self.last_kappa = np.zeros(self.n)
-        self.plan_conv = BatchCoordinateConverter(self.spline, self.n)
-        self.goal_conv = BatchCoordinateConverter(self.spline, self.n)
+        self.plan_conv = BatchCoordinateConverter(self.spline, self.n, engine=self.planner.engine)
+        self.goal_conv = BatchCoordinateConverter(self.spline, self.n, engine=self.planner.engine)
         # replayed pedestrians (replay_source.py:31-111): forward-difference velocities, shared clock
         vel = np.zeros_like(self.tracks)
         if self.n_frames >= 2:
