@@ -210,8 +210,8 @@ int fot_reload_options(fot_handle_t* h);
 float fot_last_kernel_ms(const fot_handle_t* h);
 
 /* Which sweep kernel the last launch on this handle used: 4 fot_sweep_pairs (one longitudinal profile per warp; the
- * default), 1 fot_sweep_items (sample-major with block barriers; shapes beyond the limits of fot_sweep_pairs), 3
- * fot_sweep_warp (FOT_SWEEP=warp), 2 fot_sweep (candidate-major; very long time grids), 0 none yet. */
+ * default), 1 fot_sweep_items (sample-major with block barriers; shapes beyond the limits of fot_sweep_pairs), 2
+ * fot_sweep (candidate-major; very long time grids), 0 none yet. */
 int fot_last_sweep_kind(const fot_handle_t* h);
 
 /* fot_sweep_pairs is compiled per set of optional modes (1 static obstacles, 2 footprint circles, 4 violation budget,

@@ -13,7 +13,6 @@
 
 #include "fot_kernels.cuh"
 #include "fot_sweep_items.cuh"
-#include "fot_sweep_warp.cuh"
 #include "fot_sweep_pairs.cuh"
 #include "fot_predict.cuh"
 #include "fot_frenet.cuh"
@@ -65,50 +64,35 @@ struct Buf {
 // point reads the environment on the planning path -- and again only on an explicit fot_reload_options() (the tests
 // and tuning scripts switch variants on a live handle that way).  Defaults are the product behaviour.
 struct Options {
-  int item_threads = 0;        // FOT_ITEM_THREADS   0: kItemThreads
   int bpc = 0;                 // FOT_BPC            blocks per CTA (0: rule of item_geometry)
   int qcap = 1024;             // FOT_QCAP           collision queue entries (tests force the queue-full path)
   int fused_box = 0;           // FOT_FUSED_BOX      1: trajectory boxes in the sweep even for a resident tensor
   int stage_dyn = 1;           // FOT_STAGE_DYN      0: never stage the obstacle block in shared memory
   int sweep = 0;               // FOT_SWEEP          0 auto (fot_sweep_pairs, else fot_sweep_items, else the candidate-major kernel), 1 "items" (fail if
-                               //                    unsupported), 2 "generic" (candidate-major kernel), 3 "warp" (fot_sweep_warp: two
-                               //                    barriers per block + barrier-free collision queue; measured equal to "items",
-                               //                    DESIGN.md section 4c; fail if unsupported)
-                               //                    4 "pairs" (fot_sweep_pairs: one longitudinal profile per warp, no block
-                               //                    barriers; fail if unsupported)
+                               //                    unsupported), 2 "generic" (candidate-major kernel), 4 "pairs" (fot_sweep_pairs:
+                               //                    one longitudinal profile per warp, no block barriers; fail if unsupported)
   int pair_cpq = 0;            // FOT_PAIR_CPQ       CTAs per query of fot_sweep_pairs (0: rule of pair_geometry)
   int pair_simple = 1;         // FOT_PAIR_SIMPLE    0: always the instantiation of fot_sweep_pairs with every mode compiled in (tests)
   int pair_feat = 0;           // FOT_PAIR_FEAT      mode bits (PAIR_*) added to what the batch needs (tests, tuning)
   int host_chunks = 0;         // FOT_HOST_CHUNKS    equal chunks of the host-pointer call (0: rule)
-  std::string chunk_waves;     // FOT_CHUNK_WAVES    chunk sizes in sweep waves, "1,2,3" (+ the rest)
-  int host_streams = 2;        // FOT_HOST_STREAMS   1: chunks on one compute stream
   int gated = 1;               // FOT_GATED          0: chunked launches instead of gated ones
   int gate_uploads = 16;       // FOT_GATE_UPLOADS   upload slices of a gated call
-  int gate_copy_streams = 1;   // FOT_GATE_COPY_STREAMS
-  int gate_flag_stream = 0;    // FOT_GATE_FLAG_STREAM  1: slice flags written by a second stream
-  int gate_tail_bpc = 0;       // FOT_GATE_TAIL_BPC  blocks per CTA of the last gated range
   int gate_memcpy = 0;         // FOT_GATE_MEMCPY    1: flags by 4-byte copies instead of stream writes
   int debug_timing = 0;        // FOT_DEBUG_TIMING   1: print the timeline of every host-pointer call
   void resolve() {
     *this = Options{};
     auto geti = [](const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; };
-    item_threads = geti("FOT_ITEM_THREADS", 0);
     bpc = geti("FOT_BPC", 0);
     qcap = std::max(1, std::min(1 << 15, geti("FOT_QCAP", 1024)));
     fused_box = geti("FOT_FUSED_BOX", 0) != 0;
     stage_dyn = geti("FOT_STAGE_DYN", 1) != 0;
-    if (const char* e = getenv("FOT_SWEEP")) sweep = !strcmp(e, "generic") ? 2 : !strcmp(e, "items") ? 1 : !strcmp(e, "warp") ? 3 : !strcmp(e, "pairs") ? 4 : 0;
+    if (const char* e = getenv("FOT_SWEEP")) sweep = !strcmp(e, "generic") ? 2 : !strcmp(e, "items") ? 1 : !strcmp(e, "pairs") ? 4 : 0;
     pair_cpq = geti("FOT_PAIR_CPQ", 0);
     pair_simple = geti("FOT_PAIR_SIMPLE", 1) != 0;
     pair_feat = geti("FOT_PAIR_FEAT", 0) & 31;
     host_chunks = geti("FOT_HOST_CHUNKS", 0);
-    if (const char* e = getenv("FOT_CHUNK_WAVES")) chunk_waves = e;
-    host_streams = geti("FOT_HOST_STREAMS", 2);
     gated = geti("FOT_GATED", 1) != 0;
     gate_uploads = geti("FOT_GATE_UPLOADS", 16);
-    gate_copy_streams = geti("FOT_GATE_COPY_STREAMS", 1) >= 2 ? 2 : 1;
-    gate_flag_stream = geti("FOT_GATE_FLAG_STREAM", 0) != 0;
-    gate_tail_bpc = geti("FOT_GATE_TAIL_BPC", 0);
     gate_memcpy = getenv("FOT_GATE_MEMCPY") != nullptr;
     debug_timing = getenv("FOT_DEBUG_TIMING") != nullptr;
   }
@@ -141,11 +125,10 @@ struct fot_handle {
   int device = 0;
   Plan plan{};
   void* tables_dev = nullptr;
-  cudaStream_t stream = nullptr, stream2 = nullptr, copy_stream = nullptr, copy_stream2 = nullptr, d2h_stream = nullptr;
+  cudaStream_t stream = nullptr, stream2 = nullptr, copy_stream = nullptr, d2h_stream = nullptr;
   static constexpr int kMaxChunks = 16;
   cudaEvent_t ev_copy[kMaxChunks] = {}, ev_done[kMaxChunks] = {};
   cudaEvent_t ev_join = nullptr, ev_blob = nullptr;
-  cudaEvent_t ev_slice[64] = {};     // gated uploads: one event per slice (kGateSlices)
   cudaStream_t pstream[4] = {};      // gated launches: one stream per range of queries, earlier ranges at higher priority
   Buf gate_d, gate_h;                // gated launches: device progress / error words, pinned source words
   uint32_t gate_epoch = 0;
@@ -158,7 +141,7 @@ struct fot_handle {
   int sms = 148;                     // SM count of the device (block-per-CTA grouping, host chunk sizes)
   Buf obs_tm, obs_max2, stat_tm, stat_max2, part_cost, part_idx, dyn_box, cost_tab;   // device scratch
   int last_pair_feat = -1;           // mode set (PAIR_*) of the fot_sweep_pairs instantiation of the last launch
-  int last_sweep_kind = 0;           // 4: fot_sweep_pairs, 1: fot_sweep_items, 3: fot_sweep_warp, 2: fot_sweep (generic)
+  int last_sweep_kind = 0;           // 4: fot_sweep_pairs, 1: fot_sweep_items, 2: fot_sweep (generic)
   fot_result_t mirror{};             // fot_set_result_mirror: second destination of the winner block (all null: none)
   unsigned* mirror_flag = nullptr;   // word published behind each mirrored launch (fot_set_result_mirror), or null
   unsigned mirror_seq = 0;
@@ -237,7 +220,6 @@ extern "C" int fot_create(const fot_config_t* cfg, const fot_tables_t* tb, int d
   CK(cudaStreamCreateWithFlags(&h->stream2, cudaStreamNonBlocking));
   CK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
   CK(cudaEventCreateWithFlags(&h->ev_blob, cudaEventDisableTiming));
-  for (auto& ev : h->ev_slice) CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
   {
     int least = 0, greatest = 0;
     CK(cudaDeviceGetStreamPriorityRange(&least, &greatest));     // numerically lower = higher priority
@@ -245,7 +227,6 @@ extern "C" int fot_create(const fot_config_t* cfg, const fot_tables_t* tb, int d
       CK(cudaStreamCreateWithPriority(&h->pstream[i], cudaStreamNonBlocking, std::min(least, greatest + i)));
   }
   CK(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-  CK(cudaStreamCreateWithFlags(&h->copy_stream2, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&h->d2h_stream, cudaStreamNonBlocking));
   for (auto& ev : h->ev_copy) CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
   for (auto& ev : h->ev_done) CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
@@ -259,8 +240,6 @@ extern "C" int fot_create(const fot_config_t* cfg, const fot_tables_t* tb, int d
   CK(cudaFuncSetAttribute(fot_sweep, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
   CK(cudaFuncSetAttribute(fot_sweep_items<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
   CK(cudaFuncSetAttribute(fot_sweep_items<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
-  CK(cudaFuncSetAttribute(fot_sweep_warp<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
-  CK(cudaFuncSetAttribute(fot_sweep_warp<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
   for (int i = 0; i < kPairInstanceCount; ++i)
     for (int f = 0; f < 2; ++f)
       CK(cudaFuncSetAttribute(pair_kernel(f != 0, kPairInstances[i]), cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
@@ -293,12 +272,10 @@ extern "C" int fot_destroy(fot_handle_t* h) {
   for (auto ev : h->ev_done) if (ev) cudaEventDestroy(ev);
   if (h->ev_join) cudaEventDestroy(h->ev_join);
   if (h->ev_blob) cudaEventDestroy(h->ev_blob);
-  for (auto ev : h->ev_slice) if (ev) cudaEventDestroy(ev);
   for (auto ps : h->pstream) if (ps) cudaStreamDestroy(ps);
   if (h->stream2) cudaStreamDestroy(h->stream2);
   if (h->d2h_stream) cudaStreamDestroy(h->d2h_stream);
   if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-  if (h->copy_stream2) cudaStreamDestroy(h->copy_stream2);
   if (h->stream) cudaStreamDestroy(h->stream);
   delete h;
   return FOT_OK;
@@ -383,15 +360,13 @@ static int sweep_geometry(const fot_handle* h, const fot_batch_t* b, SweepGeom* 
 // outside what that kernel covers (very long time grids, huge per-step obstacle counts); the
 // candidate-major fot_sweep then runs.
 static bool item_geometry(const fot_handle* h, const fot_batch_t* b, ItemGeom* g, size_t* smem_bytes,
-                          bool want_fused_box = false, int bpc_override = 0) {
+                          bool want_fused_box = false) {
   const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = h->plan.cfg.nx;
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
   const long long SPl = has_dyn ? (long long)b->S * b->P : 0;
   if (NT > 128 || nd > 8192 || SPl > 32768 || b->n_static > 32768) return false;   // 128: one NumPy pairwise block
   const int SP = (int)SPl;
-  int max_threads = kItemThreads;
-  if (h->opt.item_threads > 0) max_threads = std::max(NT, std::min(kItemThreads, h->opt.item_threads));
-  const int ppc_max = max_threads / NT;
+  const int ppc_max = kItemThreads / NT;
   ItemGeom G{};
   G.chunks = (b->n_v_max + ppc_max - 1) / ppc_max;
   G.ppc = (b->n_v_max + G.chunks - 1) / G.chunks;
@@ -406,7 +381,6 @@ static bool item_geometry(const fot_handle* h, const fot_batch_t* b, ItemGeom* g
     const long long total = (long long)b->n_q * G.blocks_per_query;
     long long bpc = total / ((long long)sms * 2 * 4);
     bpc = std::max<long long>(1, std::min<long long>(bpc, G.blocks_per_query));
-    if (bpc_override > 0) bpc = std::max(1, std::min(bpc_override, (int)G.blocks_per_query));
     if (h->opt.bpc > 0) bpc = std::max(1, std::min(h->opt.bpc, (int)G.blocks_per_query));
     G.ctas_per_query = (int)((G.blocks_per_query + bpc - 1) / bpc);
     G.bpc = (G.blocks_per_query + G.ctas_per_query - 1) / G.ctas_per_query;
@@ -460,93 +434,11 @@ static bool item_geometry(const fot_handle* h, const fot_batch_t* b, ItemGeom* g
   return true;
 }
 
-// Geometry of the warp-local kernel (fot_sweep_warp): the block decomposition of fot_sweep_items, per-warp obstacle
-// lists and survivor queues, and the per-block state in two copies.  False when the shape is outside its range
-// (more than kWarpListCap obstacle entries per query, long time grids): fot_sweep_items then runs.
-static bool warp_geometry(const fot_handle* h, const fot_batch_t* b, WarpGeom* g, size_t* smem_bytes,
-                          bool want_fused_box = false, int bpc_override = 0) {
-  const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = h->plan.cfg.nx;
-  const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
-  const long long SPl = has_dyn ? (long long)b->S * b->P : 0;
-  if (NT > 128 || nd > 8192 || SPl + b->n_static > kWarpListCap) return false;
-  const int SP = (int)SPl;
-  int max_threads = kItemThreads;
-  if (h->opt.item_threads > 0) max_threads = std::max(NT, std::min(kItemThreads, h->opt.item_threads));
-  const int ppc_max = max_threads / NT;
-  WarpGeom G{};
-  G.chunks = (b->n_v_max + ppc_max - 1) / ppc_max;
-  G.ppc = (b->n_v_max + G.chunks - 1) / G.chunks;
-  G.grid_blocks = h->plan.cfg.n_T * G.chunks;
-  G.ppb = nB > 0 ? std::min(nB, ppc_max) : 0;
-  G.brake_blocks = nB > 0 ? (nB + G.ppb - 1) / G.ppb : 0;
-  G.blocks_per_query = G.grid_blocks + G.brake_blocks;
-  {
-    const long long total = (long long)b->n_q * G.blocks_per_query;
-    long long bpc = total / ((long long)h->sms * 2 * 4);
-    bpc = std::max<long long>(1, std::min<long long>(bpc, G.blocks_per_query));
-    if (bpc_override > 0) bpc = std::max(1, std::min(bpc_override, (int)G.blocks_per_query));
-    if (h->opt.bpc > 0) bpc = std::max(1, std::min(h->opt.bpc, (int)G.blocks_per_query));
-    G.ctas_per_query = (int)((G.blocks_per_query + bpc - 1) / bpc);
-    G.bpc = (G.blocks_per_query + G.ctas_per_query - 1) / G.ctas_per_query;
-  }
-  G.pcap = std::max(G.ppc, std::max(G.ppb, 1));
-  G.threads = (G.pcap * NT + 31) / 32 * 32;
-  G.ct_lcap = std::max(nd, std::max(G.ppb, 1));
-  G.nw4 = (nd + 3) / 4;
-  G.nwc = (nd + 31) / 32;
-  const int max_viol = b->dyn_mode == FOT_DYN_DISTRIBUTION ? (int)std::floor(h->plan.cfg.chance_epsilon * (double)b->S) : 0;
-  G.vwords = max_viol > 0 ? (b->S + 31) / 32 : 0;
-  G.lcap = std::max(1, SP + b->n_static);
-  G.spline_smem = nx <= 128 ? 1 : 0;
-  const size_t dyn_bytes = (size_t)SP * b->T_obs * 16;
-  const bool fuse = want_fused_box || h->opt.fused_box;
-  auto layout = [&](bool stage) {
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 15) / 16 * 16; return (int32_t)o; };
-    G.o_row = take((size_t)G.pcap * NT * kRowW * 8);
-    G.o_dgrid = take((size_t)nd * 8);
-    G.o_spl = take(G.spline_smem ? (size_t)9 * nx * 8 : 0);
-    G.o_dyn = take(stage ? dyn_bytes : 0);
-    G.o_box = take((size_t)SP * 16);                      // trajectory boxes: built here (fused) or copied from fot_prepass
-    G.o_wlist = take((size_t)(G.threads / 32) * G.lcap * 4);
-    G.o_wq = take((size_t)(G.threads / 32) * kWarpQueue * 4);
-    G.o_bq = take((size_t)kBlockQueue * 4);
-    G.o_buf = take(0);
-    size_t bo = 0;
-    auto btake = [&](size_t bytes) { size_t o = bo; bo = (bo + bytes + 15) / 16 * 16; return (int32_t)o; };
-    G.b_fnr = btake((size_t)G.pcap * 4);
-    G.b_flags = btake((size_t)G.pcap * G.nw4 * 4);
-    G.b_hit = btake((size_t)G.pcap * G.nwc * 4);
-    G.b_viol = btake((size_t)G.pcap * nd * G.vwords * 4);
-    G.b_dirty = btake((size_t)G.pcap * G.nwc * 4);
-    G.b_qctl = btake(16);
-    G.n_zero = (int32_t)((bo - (size_t)G.b_fnr) / 4);
-    G.b_sdl = btake((size_t)G.pcap * 8);
-    G.b_ct = btake((size_t)(G.pcap + 2 * G.ct_lcap) * 8);
-    G.b_vlast = btake((size_t)G.pcap * nd * 8);
-    G.b_span = btake((size_t)G.pcap * 8);
-    G.buf_bytes = (int32_t)bo;
-    off += 2 * bo;
-    G.stage_dyn = stage ? 1 : 0;
-    G.fused_box = stage && fuse ? 1 : 0;
-    return off;
-  };
-  bool stage = has_dyn && dyn_bytes > 0 && dyn_bytes <= 64 * 1024 && ((uintptr_t)b->dyn & 15) == 0;
-  stage = stage && h->opt.stage_dyn;
-  size_t bytes = layout(stage);
-  if (stage && bytes > 110 * 1024) { stage = false; bytes = layout(false); }
-  if (bytes > (size_t)h->smem_optin) return false;
-  *g = G;
-  *smem_bytes = bytes;
-  return true;
-}
-
-
 // Geometry of the pair-per-warp kernel (fot_sweep_pairs): one CTA per query (several for small batches), every warp
 // with a private slice of shared memory for the pair it is working on.  False when the shape is outside its range
 // (time grids beyond 64 samples, lateral grids beyond 96 targets, tables that do not fit): fot_sweep_items then runs.
 static bool pair_geometry(const fot_handle* h, const fot_batch_t* b, PairGeom* g, size_t* smem_bytes,
-                          bool want_fused_box = false, int cpq_override = 0) {
+                          bool want_fused_box = false) {
   const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = h->plan.cfg.nx;
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
   const long long SPl = has_dyn ? (long long)b->S * b->P : 0;
@@ -585,7 +477,6 @@ static bool pair_geometry(const fot_handle* h, const fot_batch_t* b, PairGeom* g
     const int n_units = h->plan.cfg.n_T * b->n_v_max + nB;
     long long cpq = ((long long)h->sms * 2 * 4 + b->n_q - 1) / b->n_q;
     cpq = std::max<long long>(1, std::min<long long>(cpq, (n_units + kPairWarps - 1) / kPairWarps));
-    if (cpq_override > 0) cpq = std::max(1, std::min(cpq_override, n_units));
     if (h->opt.pair_cpq > 0) cpq = std::max(1, std::min(h->opt.pair_cpq, n_units));
     G.ctas_per_query = (int)cpq;
   }
@@ -639,27 +530,15 @@ struct Gate {
 };
 
 static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r, cudaStream_t st, size_t q_off = 0,
-                      size_t q_total = 0, Gate gate = Gate{}, int bpc_override = 0, bool record_span = true) {
+                      size_t q_total = 0, Gate gate = Gate{}, bool record_span = true) {
   if (q_total == 0) q_total = (size_t)b->n_q;
-  // kernel choice: the sample-major fot_sweep_items unless the shape is outside its range (or
-  // FOT_SWEEP=generic asks for the candidate-major kernel, which the tests use as a cross-check)
+  // kernel choice: the pair-per-warp fot_sweep_pairs wherever its shape limits allow, else the sample-major
+  // fot_sweep_items, else the candidate-major fot_sweep.  FOT_SWEEP=pairs / items / generic insists on one of them
+  // (the tests cross-check the three).
   ItemGeom ig{};
   size_t ismem = 0;
-  bool use_items = item_geometry(h, b, &ig, &ismem, gate.word != nullptr, bpc_override);
+  bool use_items = item_geometry(h, b, &ig, &ismem, gate.word != nullptr);
   if (h->opt.sweep == 2) use_items = false;
-  // the two-barrier kernel on request (FOT_SWEEP=warp)
-  WarpGeom wg{};
-  size_t wsmem = 0;
-  bool use_warp = h->opt.sweep == 3 && warp_geometry(h, b, &wg, &wsmem, gate.word != nullptr, bpc_override);
-  if (use_warp && gate.word && !wg.fused_box) use_warp = false;
-  if (h->opt.sweep == 3 && !use_warp && !gate.word) return fail(FOT_ERR_ARG, "FOT_SWEEP=warp: shape not supported by fot_sweep_warp");
-  if (use_warp) {
-    // same block decomposition and scratch as fot_sweep_items: the code below sizes everything from `ig`
-    use_items = true;
-    ig.blocks_per_query = wg.blocks_per_query; ig.ctas_per_query = wg.ctas_per_query; ig.threads = wg.threads;
-    ig.fused_box = wg.fused_box;
-  }
-  // the pair-per-warp kernel: the default wherever its shape limits allow (FOT_SWEEP=pairs insists on it)
   PairGeom pg{};
   size_t psmem = 0;
   bool use_pairs = (h->opt.sweep == 0 || h->opt.sweep == 4) && use_items && pair_geometry(h, b, &pg, &psmem, gate.word != nullptr);
@@ -667,18 +546,13 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
   if (h->opt.sweep == 4 && !use_pairs && !gate.word) return fail(FOT_ERR_ARG, "FOT_SWEEP=pairs: shape not supported by fot_sweep_pairs");
   if (use_pairs) {
     // same scratch (cost tables, trajectory boxes, one arg-min partial per CTA) as fot_sweep_items
-    use_items = true;
-    use_warp = false;
     ig.blocks_per_query = h->plan.cfg.n_T * b->n_v_max + h->plan.cfg.n_B;      // upper bound of ctas_per_query (scratch stride)
     ig.ctas_per_query = pg.ctas_per_query; ig.threads = kPairThreads;
     ig.fused_box = pg.fused_box;
     if (gate.word) { pg.gate = gate.word; pg.gate_epoch = gate.epoch; pg.gate_per = gate.per; pg.gate_q0 = (int32_t)q_off; }
   }
   if (gate.word && !(use_items && ig.fused_box)) return fail(FOT_ERR_ARG, "gated launch needs a sample-major sweep with a staged obstacle block");
-  if (gate.word) {
-    ig.gate = gate.word; ig.gate_epoch = gate.epoch; ig.gate_per = gate.per; ig.gate_q0 = (int32_t)q_off;
-    wg.gate = gate.word; wg.gate_epoch = gate.epoch; wg.gate_per = gate.per; wg.gate_q0 = (int32_t)q_off;
-  }
+  if (gate.word) { ig.gate = gate.word; ig.gate_epoch = gate.epoch; ig.gate_per = gate.per; ig.gate_q0 = (int32_t)q_off; }
   if (h->opt.sweep == 1 && !use_items) return fail(FOT_ERR_ARG, "FOT_SWEEP=items: shape not supported by fot_sweep_items");
   SweepGeom g{};
   size_t smem = 0;
@@ -793,12 +667,10 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
       if ((kPairInstances[i] & need) == need) { feat = kPairInstances[i]; break; }
     pair_kernel(pg.fused_box != 0, feat)<<<(unsigned)n_part, kPairThreads, psmem, st>>>(h->plan, B, O, pg);
     h->last_pair_feat = feat;
-  } else if (use_warp && wg.fused_box) fot_sweep_warp<true><<<(unsigned)n_part, wg.threads, wsmem, st>>>(h->plan, B, O, wg);
-  else if (use_warp) fot_sweep_warp<false><<<(unsigned)n_part, wg.threads, wsmem, st>>>(h->plan, B, O, wg);
-  else if (use_items && ig.fused_box) fot_sweep_items<true><<<(unsigned)n_part, ig.threads, ismem, st>>>(h->plan, B, O, ig);
+  } else if (use_items && ig.fused_box) fot_sweep_items<true><<<(unsigned)n_part, ig.threads, ismem, st>>>(h->plan, B, O, ig);
   else if (use_items) fot_sweep_items<false><<<(unsigned)n_part, ig.threads, ismem, st>>>(h->plan, B, O, ig);
   else fot_sweep<<<(unsigned)n_part, kSweepThreads, smem, st>>>(h->plan, B, O, g);
-  h->last_sweep_kind = use_pairs ? 4 : use_warp ? 3 : use_items ? 1 : 2;
+  h->last_sweep_kind = use_pairs ? 4 : use_items ? 1 : 2;
   CK(cudaEventRecord(ring[2], st));
   fot_winner<<<b->n_q, 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, O, g);
   if (O.m_winner && h->mirror_flag) fot_publish_kernel<<<1, 1, 0, st>>>(h->mirror_flag, ++h->mirror_seq);
@@ -870,8 +742,8 @@ static void drain_after_failure(fot_handle* h) {
     std::vector<uint32_t> w(kGateSlices, h->gate_epoch);
     cudaMemcpy(h->gate_d.p, w.data(), kGateSlices * sizeof(uint32_t), cudaMemcpyHostToDevice);
   }
-  for (cudaStream_t s : {h->copy_stream, h->copy_stream2, h->stream, h->stream2, h->pstream[0], h->pstream[1], h->pstream[2],
-                         h->pstream[3], h->d2h_stream})
+  for (cudaStream_t s : {h->copy_stream, h->stream, h->stream2, h->pstream[0], h->pstream[1], h->pstream[2], h->pstream[3],
+                         h->d2h_stream})
     if (s) cudaStreamSynchronize(s);
   if (h->gate_d.p) cudaMemset((uint32_t*)h->gate_d.p + kGateSlices, 0, sizeof(uint32_t));
   cudaGetLastError();
@@ -982,24 +854,9 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
     const int per_ = (nq + n_chunks - 1) / n_chunks;
     for (int c = 0; c <= n_chunks; ++c) bounds[c] = std::min(nq, c * per_);
   }
-  if (!h->opt.chunk_waves.empty()) {                       // tuning: chunk sizes in sweep waves, "1,2,3,4,3" (+ the rest)
-    const char* env = h->opt.chunk_waves.c_str();
-    const int wave = 2 * h->sms;
-    n_chunks = 0;
-    int at = 0;
-    for (const char* p = env; *p && n_chunks < kMaxChunks - 1 && at < nq;) {
-      at = std::min(nq, at + std::max(1, atoi(p)) * wave);
-      bounds[++n_chunks] = at;
-      while (*p && *p != ',') ++p;
-      if (*p == ',') ++p;
-    }
-    if (at < nq) bounds[++n_chunks] = nq;
-    for (int c = n_chunks + 1; c <= kMaxChunks; ++c) bounds[c] = nq;
-  }
   // chunks alternate between two compute streams, so that the next chunk's CTAs fill the SMs the tail wave of
   // the previous chunk leaves idle (the chunks touch disjoint scratch, see launch_all)
   bool two_streams = n_chunks > 1;
-  two_streams = two_streams && h->opt.host_streams >= 2;
   if (two_streams) {
     ItemGeom ig{};
     size_t ismem = 0;
@@ -1036,7 +893,7 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
     // launch ranges: about 1/2, 5/16, 3/16 of the queries, in whole waves
     const int wave = 2 * h->sms;
     auto waves = [&](int frac16) { const int w = std::max(1, (int)((long long)nq * frac16 / 16 / wave)); return w * wave; };
-    if (h->opt.host_chunks <= 0 && h->opt.chunk_waves.empty()) {
+    if (h->opt.host_chunks <= 0) {
       const int cuts[] = {waves(8), waves(13), nq};
       n_chunks = 3;
       for (int c = 0; c < n_chunks; ++c) bounds[c + 1] = std::min(nq, std::max(cuts[c], bounds[c]));
@@ -1054,36 +911,20 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
   CK(cudaEventRecord(h->ev_blob, h->copy_stream));
   // every obstacle upload is queued first (they depend on nothing), one event per chunk
   if (gated) {
-    // each slice is followed, in its stream, by the write of its flag (two alternating upload streams are a
-    // tuning knob; measured slower than one)
+    // each slice is followed on the upload stream by the write of its flag, which stream order keeps behind the slice
     uint32_t* words = (uint32_t*)h->gate_h.p;
-    const int n_cs = h->opt.gate_copy_streams;
-    const bool flag_stream = h->opt.gate_flag_stream && n_cs == 1;
-    CK(cudaStreamWaitEvent(h->copy_stream2, h->ev_blob, 0));      // nothing of this call before the previous call's flags are history
     for (int u = 0; u < n_up; ++u) {
       const int q0 = ub[u], cq = ub[u + 1] - q0;
       if (cq <= 0) continue;
-      cudaStream_t cs = (n_cs == 2 && (u & 1)) ? h->copy_stream2 : h->copy_stream;
       char* dst = (char*)h->dyn_d.p + (size_t)q0 * dyn_q_bytes;
       const char* src = (const char*)b->dyn + (size_t)q0 * dyn_q_bytes;
-      CK(cudaMemcpyAsync(dst, src, (size_t)cq * dyn_q_bytes, cudaMemcpyHostToDevice, cs));
+      CK(cudaMemcpyAsync(dst, src, (size_t)cq * dyn_q_bytes, cudaMemcpyHostToDevice, h->copy_stream));
       words[u] = gate.epoch;
-      // FOT_GATE_FLAG_STREAM=1: the flag is written by a second stream behind an event of the slice, so that the
-      // upload stream carries nothing but copies and event records (a stream write between two slices costs the
-      // upload ~15 us of DMA idle time: uploads done at 3.3 ms instead of 3.1).  Faster in isolation (3.75 against
-      // 3.86 ms per call), no better inside bench.py, and it depends on the two streams not sharing a hardware
-      // queue; the default keeps the flag in line, where its order behind the slice needs nothing else.
-      cudaStream_t fs = cs;
-      if (flag_stream) {
-        CK(cudaEventRecord(h->ev_slice[u], cs));
-        CK(cudaStreamWaitEvent(h->copy_stream2, h->ev_slice[u], 0));
-        fs = h->copy_stream2;
-      }
       if (StreamWrite32 wr = h->opt.gate_memcpy ? nullptr : stream_write32()) {
-        if (wr(fs, (unsigned long long)(uintptr_t)(gate.word + u), gate.epoch, 0u) != 0)
+        if (wr(h->copy_stream, (unsigned long long)(uintptr_t)(gate.word + u), gate.epoch, 0u) != 0)
           return fail(FOT_ERR_CUDA, "cuStreamWriteValue32");
       } else {
-        CK(cudaMemcpyAsync(gate.word + u, words + u, sizeof(uint32_t), cudaMemcpyHostToDevice, fs));
+        CK(cudaMemcpyAsync(gate.word + u, words + u, sizeof(uint32_t), cudaMemcpyHostToDevice, h->copy_stream));
       }
     }
   } else if (has_dyn)
@@ -1097,7 +938,6 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
       if (dbg) cudaEventRecord(tl[c][0], h->copy_stream);
     }
   if (dbg) {
-    if (gated) { cudaEventRecord(h->ev_join, h->copy_stream2); cudaStreamWaitEvent(h->copy_stream, h->ev_join, 0); }
     cudaEventRecord(d1, h->copy_stream);
     cudaPointerAttributes pa{};
     cudaError_t pe = cudaPointerGetAttributes(&pa, b->dyn);
@@ -1136,11 +976,7 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
     dr.winner = (double*)(od + r_w) + (size_t)q0 * FOT_N_SERIES * NT;
     dr.cand_cat = r->cand_cat ? (uint8_t*)(od + r_cc) + (size_t)q0 * r->cand_stride : nullptr;
     dr.cand_cost = r->cand_cost ? (double*)(od + r_cs) + (size_t)q0 * r->cand_stride : nullptr;
-    // (tuning knob: blocks per CTA of the last gated range; shorter CTAs there measured no better than the
-    // rule of item_geometry)
-    int tail_bpc = 0;
-    if (gated && bounds[c + 1] >= nq) tail_bpc = h->opt.gate_tail_bpc;
-    rc = launch_all(h, &db, &dr, st, (size_t)q0, (size_t)nq, gate, tail_bpc, /*record_span=*/false);
+    rc = launch_all(h, &db, &dr, st, (size_t)q0, (size_t)nq, gate, /*record_span=*/false);
     if (rc != FOT_OK) return rc;
     // winners of this chunk straight into the caller's arrays, on their own stream so the next
     // chunk's kernels never queue behind a copy engine that is busy with the uploads
@@ -1162,7 +998,6 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
   if (gated) {
     for (auto ps : h->pstream) CK(cudaStreamSynchronize(ps));
     CK(cudaStreamSynchronize(h->copy_stream));
-    CK(cudaStreamSynchronize(h->copy_stream2));
   }
   if (gated && std::chrono::steady_clock::now() - t_wall0 > std::chrono::nanoseconds(kGateTimeoutNs)) {
     unsigned gave_up = 0;
@@ -1249,7 +1084,7 @@ static int plan_batch_device_to_host_impl(fot_handle_t* h, const fot_batch_t* b,
     dr.cand_cat = r->cand_cat ? (uint8_t*)(od + r_cc) + (size_t)q0 * r->cand_stride : nullptr;
     dr.cand_cost = r->cand_cost ? (double*)(od + r_cs) + (size_t)q0 * r->cand_stride : nullptr;
     if (c == 0) CK(cudaEventRecord(h->ev0, st));
-    rc = launch_all(h, &db, &dr, st, (size_t)q0, (size_t)nq, Gate{}, 0, /*record_span=*/false);
+    rc = launch_all(h, &db, &dr, st, (size_t)q0, (size_t)nq, Gate{}, /*record_span=*/false);
     if (rc != FOT_OK) return rc;
     rc = read_back(h, r, dr, (double*)(od + r_wh) + (size_t)q0 * FOT_N_SERIES * k_head, q0, cq, NT, st, h->d2h_stream, h->ev_done[c]);
     if (rc != FOT_OK) return rc;

@@ -4,7 +4,8 @@
 // flags, collision verdict, category and cost come out bit-identical.  What changes is who waits for whom.
 // fot_sweep_items cuts a query into blocks of six longitudinal profiles and walks its 320 threads through six
 // block-wide barriers per block; ncu charges 3.1 stall cycles per issued instruction to those barriers, and
-// fot_sweep_warp (fewer barriers, a shared producer/consumer queue) only moved the wait into the queue.  Here the
+// a two-barrier variant (fewer barriers, a shared producer/consumer queue; DESIGN.md section 4c) only moved the wait
+// into the queue.  Here the
 // unit of work is ONE PAIR = one longitudinal profile (horizon T_j, terminal speed v_k) or one brake horizon,
 // and a pair belongs to ONE WARP from its first instruction to its last:
 //

@@ -92,8 +92,6 @@ def test_full_collision_queue_degrades_to_in_place_tests():
     pl = _planner()
     run = lambda: pl.plan_batch(frenet, 6.0, dynamic_obstacles=dyn, static_obstacles=wall, want_candidates=True)
     base = run()
-    with _env(FOT_SWEEP="warp"):                           # the two-barrier kernel (73 entries per query)
-        warp = run()
     with _env(FOT_SWEEP="items"):                          # the sample-major kernel (the default is fot_sweep_pairs)
         items = run()
     with _env(FOT_SWEEP="items", FOT_QCAP=4):
@@ -102,11 +100,9 @@ def test_full_collision_queue_degrades_to_in_place_tests():
         unstaged = run()
     with _env(FOT_STAGE_DYN=0, FOT_PAIR_CPQ=8):
         unstaged_pairs = run()
-    with _env(FOT_SWEEP="warp", FOT_STAGE_DYN=0, FOT_BPC=1):
-        unstaged_warp = run()
     with _env(FOT_SWEEP="generic"):
         generic = run()
-    for other in (warp, items, capped, unstaged, unstaged_pairs, unstaged_warp, generic):
+    for other in (items, capped, unstaged, unstaged_pairs, generic):
         assert np.array_equal(base.cand_cat, other.cand_cat)
         assert np.array_equal(base.best_idx, other.best_idx) and np.array_equal(base.stats, other.stats)
         assert np.array_equal(base.best_cost.view(np.uint64), other.best_cost.view(np.uint64))
@@ -159,7 +155,7 @@ def test_host_chunking_and_cta_grouping_do_not_change_results():
 def test_gated_upload_pipeline_matches_the_single_launch():
     """The host-pointer call launches the sweep while the obstacle tensor is still being uploaded: CTAs wait for
     the slice of their query and box the predicted trajectories themselves.  Every variant of that pipeline
-    (gated, chunked on two streams, chunked on one, odd slice counts, flags by copy instead of stream write)
+    (gated, chunked on two streams, odd slice and range counts, flags by copy instead of stream write)
     has to return what one plain launch over the resident tensor returns -- including queries with a NaN
     trajectory, whose box is NaN (fp.py:1211-1222), and a shared static wall."""
     import bench
@@ -175,10 +171,10 @@ def test_gated_upload_pipeline_matches_the_single_launch():
         ref = run()
         ref = {k: getattr(ref, k).copy() for k in keys}
     assert len(set(ref["best_idx"].tolist())) > 20
-    variants = [dict(), dict(FOT_SWEEP="items"), dict(FOT_SWEEP="items", FOT_GATED=0), dict(FOT_SWEEP="warp"), dict(FOT_SWEEP="warp", FOT_GATED=0), dict(FOT_GATED=0), dict(FOT_GATED=0, FOT_HOST_STREAMS=1), dict(FOT_GATE_UPLOADS=7),
-                dict(FOT_GATE_UPLOADS=64, FOT_GATE_COPY_STREAMS=2), dict(FOT_GATE_MEMCPY=1, FOT_CHUNK_WAVES="1,1"),
-                dict(FOT_GATE_TAIL_BPC=1), dict(FOT_GATE_FLAG_STREAM=1), dict(FOT_STAGE_DYN=0), dict(FOT_STAGE_DYN=0, FOT_HOST_STREAMS=1), dict(FOT_GATED=0, FOT_HOST_CHUNKS=1, FOT_FUSED_BOX=1),
-                dict(FOT_SWEEP="warp", FOT_GATED=0, FOT_HOST_CHUNKS=1, FOT_FUSED_BOX=1)]
+    variants = [dict(), dict(FOT_SWEEP="items"), dict(FOT_SWEEP="items", FOT_GATED=0), dict(FOT_GATED=0), dict(FOT_GATE_UPLOADS=7),
+                dict(FOT_GATE_UPLOADS=64), dict(FOT_GATE_MEMCPY=1, FOT_HOST_CHUNKS=5),
+                dict(FOT_STAGE_DYN=0), dict(FOT_GATED=0, FOT_HOST_CHUNKS=1, FOT_FUSED_BOX=1),
+                dict(FOT_SWEEP="items", FOT_GATED=0, FOT_HOST_CHUNKS=1, FOT_FUSED_BOX=1)]
     for env in variants:
         with _env(**env):
             got = run()

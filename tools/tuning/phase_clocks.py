@@ -5,6 +5,7 @@ with -DFOT_PHASE_CLOCKS and prints the share of warp-cycles spent between the ke
        -DFOT_PHASE_CLOCKS -I include -o tools/tuning/libfot_clk.so integrated_path_planning_b200/csrc/fot_api.cu
 """
 import ctypes as C, os, sys
+os.environ["FOT_SWEEP"] = "items"     # the only kernel with phase marks; the default fot_sweep_pairs has none
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))  # repo root
 sys.path.insert(0, ROOT)
 from integrated_path_planning_b200 import _lib
@@ -25,22 +26,13 @@ lib.fot_debug_phase_clocks(buf)
 batch.launch(None)
 lib.fot_debug_phase_clocks(buf)
 v = list(buf)
-import os
-if os.environ.get("FOT_SWEEP", "warp") in ("warp", ""):
-    names = ["B work (items)", "barrier (i)", "CD item consts + screens", "CD validity loop", "CD slow units, vlast", "CD warp list build",
-             "CD cull (produce)", "CD exact tests (consume, incl. waiting for entries)", "barrier (ii)", "E work", "-", "-"]
-else:
-    names = ["A work", "A barrier", "B work (items, jerk)", "B barrier", "C work (lists, validity loop)", "C barrier",
-             "D cull", "D cull barrier", "D process+slow", "D process barrier", "E work", "E barrier"]
+names = ["A work", "A barrier", "B work (items, jerk)", "B barrier", "C work (lists, validity loop)", "C barrier",
+         "D cull", "D cull barrier", "D process+slow", "D process barrier", "E work", "E barrier"]
 tot = sum(v[:12])
 for n, x in zip(names, v[:12]):
     print(f"{n:32s} {x / tot * 100:6.2f} %   {x / (nq * 12 * 10):9.0f} cycles per warp per block")
 print("total cycles per warp per block", tot / (nq * 12 * 10))
 
-if os.environ.get("FOT_SWEEP", "warp") in ("warp", ""):
-    print(f"warp lists: {v[13]:.3e} warp-blocks with a list, mean length {v[12] / max(v[13], 1):.1f}; queue entries per block "
-          f"{v[14] / (nq * 12):.1f}; slow items per block {v[15] / (nq * 12):.1f}")
-    sys.exit(0)
 print(f"validity screen: valid items {v[12]:.3e}, dirty items {v[13]:.3e} ({v[13] / max(v[12], 1) * 100:.1f} %), warps with valid items "
       f"{v[14] & 0xffffffff:.3e}, of them skipped {v[15]:.3e} ({v[15] / max(v[14] & 0xffffffff, 1) * 100:.1f} %), full-chain warps "
       f"{v[14] >> 32:.3e} ({(v[14] >> 32) / max(v[14] & 0xffffffff, 1) * 100:.1f} %)")
