@@ -1237,6 +1237,8 @@ extern "C" int fot_predict_cv_device(int device, void* stream, int n_q, int P, c
   const int T_out = n_steps + (cur_pos ? 1 : 0);
   const size_t smem = (size_t)P * 2 * sizeof(double);
   if (smem > 48 * 1024) return fail(FOT_ERR_TOO_LARGE, "fot_predict_cv_device: too many pedestrians per query");
+  // the kernel's static shared memory comes on top: near 48 KB of dynamic shared memory the launch needs the opt-in
+  if (smem > 32 * 1024) CK(cudaFuncSetAttribute(fot_cv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   fot_cv_kernel<<<n_q, 256, smem, (cudaStream_t)stream>>>(p_curr, p_prev, staleness, time_target, cur_pos, out, P, n_steps,
                                                           T_out, sgan_dt, obs_float32);
   return pred_end(stream);

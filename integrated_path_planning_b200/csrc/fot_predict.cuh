@@ -138,7 +138,9 @@ __global__ void fot_resample_kernel(const double* __restrict__ pred, const doubl
     if (!constant && L >= 2) {                                         // :305-311
       const int lookback = min(3, L);
       v_tail = (ys[L - 1] - ys[L - lookback]) / ((double)(lookback - 1) * sgan_dt);
-      v_tail = fmax(fmin(v_tail, 2.5), -2.5);
+      // Python's max(min(v_tail, 2.5), -2.5): a NaN passes through (fmin / fmax would drop it)
+      v_tail = (2.5 < v_tail) ? 2.5 : v_tail;
+      v_tail = (-2.5 > v_tail) ? -2.5 : v_tail;
     }
     double* row = o + (size_t)p * n_steps * 2 + ax;
     for (int i = 0; i < n_steps; ++i) {
@@ -183,6 +185,40 @@ __global__ void fot_prepend_kernel(const double* __restrict__ in, const int32_t*
   }
 }
 
+// np_pairwise_sum (fot_device.cuh) without the recursion: NumPy's split tree walked with an explicit stack.
+// The recursive form takes a 200-byte stack frame per level here, and P * T of a few thousand overflows the
+// default 1 KB thread stack.  Same additions in the same order, so the same value.
+template <class F>
+__device__ double np_pairwise_sum_flat(const F& f, int n) {
+  if (n <= 128) return np_block_sum(f, 0, n);
+  int s_lo[32], s_n[32], s_state[32];                   // depth <= log2(n / 128) + 1 < 32
+  double s_left[32];
+  int sp = 0;
+  s_lo[0] = 0; s_n[0] = n; s_state[0] = 0;
+  double ret = 0.0;
+  for (;;) {
+    const int lo = s_lo[sp], m = s_n[sp];
+    int m2 = m / 2;
+    m2 -= m2 % 8;
+    if (m <= 128) {
+      ret = np_block_sum(f, lo, m);
+      --sp;
+    } else if (s_state[sp] == 0) {                      // descend left
+      s_state[sp] = 1;
+      ++sp; s_lo[sp] = lo; s_n[sp] = m2; s_state[sp] = 0;
+      continue;
+    } else if (s_state[sp] == 1) {                      // left done: descend right
+      s_left[sp] = ret; s_state[sp] = 2;
+      ++sp; s_lo[sp] = lo + m2; s_n[sp] = m - m2; s_state[sp] = 0;
+      continue;
+    } else {                                            // both done: left + right
+      ret = s_left[sp] + ret;
+      --sp;
+    }
+    if (sp < 0) return ret;
+  }
+}
+
 // Closest-to-mean sample (trajectory_predictor.py:346-351): mean over the samples (sequential add over S,
 // then / S, as np.mean reduces an outer axis), per-point 2-norm, np.sum over (pedestrians, steps) in NumPy's
 // pairwise order, first arg-min.  fot_best_dist_kernel: one thread per (query, sample) distance;
@@ -200,7 +236,7 @@ __global__ void fot_best_dist_kernel(const double* __restrict__ samples, double*
     const double dx = mine[(size_t)e * 2] - mx, dy = mine[(size_t)e * 2 + 1] - my;
     return sqrt(dx * dx + dy * dy);
   };
-  dist[g] = np_pairwise_sum(term, 0, PT);
+  dist[g] = np_pairwise_sum_flat(term, PT);
 }
 __global__ void fot_best_pick_kernel(const double* __restrict__ dist, int32_t* __restrict__ best_idx, int n_q, int S) {
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -221,9 +257,17 @@ __global__ void fot_best_pick_kernel(const double* __restrict__ dist, int32_t* _
 // of sight, the clearance and the clearance restricted to pedestrians ahead of the vehicle.  These are the
 // inputs of the fail-safe state machine, needed once per query and step in batched roll-outs.
 // One warp per query; out[q] = {min_distance, collision, ttc, clearance, clearance_ahead}.
+// The reference's dot products are BLAS calls; the kernel writes out the order OpenBLAS's x86-64 kernels use
+// (pinned on the host by tests/test_prediction_host_order.py):
+//   [1,2] @ [2] and np.dot of two 2-vectors   fma(a1, b1, a0 * b0)
+//   [k,2] @ [2], k >= 2                       fma(a0, b0, a1 * b1)
+//   np.linalg.norm of a 2-vector              sqrt(fma(a1, a1, a0 * a0))
+// np.linalg.norm(..., axis=2) over the distance matrix is an element-wise reduce: sqrt(a0 * a0 + a1 * a1).
 struct CircleOffsets {
   double v[FOT_MAX_CIRCLES];          // EgoFootprint.offsets, passed by value (a kernel parameter, no device buffer)
 };
+// np.min: a NaN anywhere makes the minimum NaN (fmin would drop it)
+__device__ __forceinline__ double nan_min(double a, double b) { return (a != a || a < b) ? a : b; }
 __global__ void fot_safety_kernel(const double* __restrict__ ego, const double* __restrict__ ped_pos,
                                   const double* __restrict__ ped_vel, const int32_t* __restrict__ n_peds,
                                   double* __restrict__ out, int n_q, int P, double combined_radius,
@@ -234,21 +278,22 @@ __global__ void fot_safety_kernel(const double* __restrict__ ego, const double* 
   const double x = e[0], y = e[1], yaw = e[2], v = e[3];
   const double hx = cos(yaw), hy = sin(yaw);                                   // :371-372 / footprint.py:44
   const double evx = v * hx, evy = v * hy;                                     // :350-351
-  const int np_ = n_peds ? n_peds[q] : P;
+  const int np_ = min(max(n_peds ? n_peds[q] : P, 0), P);
   const double inf = INFINITY;
   double dmin = inf, ttc = inf, dmin_ahead = inf;
   for (int p = lane; p < np_; p += 32) {
     const double px = ped_pos[((size_t)q * P + p) * 2], py = ped_pos[((size_t)q * P + p) * 2 + 1];
     const double vx = ped_vel[((size_t)q * P + p) * 2], vy = ped_vel[((size_t)q * P + p) * 2 + 1];
-    const bool ahead = (px - x) * hx + (py - y) * hy > 0.0;                    // :373-374
+    const double ax = px - x, ay = py - y;                                     // :373-374, one row or a [k,2] matrix
+    const bool ahead = (np_ == 1 ? fma(ay, hy, ax * hx) : fma(ax, hx, ay * hy)) > 0.0;
     for (int c = 0; c < (n_circ > 0 ? n_circ : 1); ++c) {
       const double cx = n_circ > 0 ? x + offsets.v[c] * hx : x, cy = n_circ > 0 ? y + offsets.v[c] * hy : y;   // footprint.py:45
       const double rx = px - cx, ry = py - cy;
       const double dist = sqrt(rx * rx + ry * ry);                             // :337-339
-      dmin = fmin(dmin, dist);
-      if (ahead) dmin_ahead = fmin(dmin_ahead, dist);
+      dmin = nan_min(dmin, dist);
+      if (ahead) dmin_ahead = nan_min(dmin_ahead, dist);
       const double rvx = vx - evx, rvy = vy - evy;
-      const double along = -(rx * rvx + ry * rvy) / (dist + 1e-8);             // :358
+      const double along = -fma(ry, rvy, rx * rvx) / (sqrt(fma(ry, ry, rx * rx)) + 1e-8);   // :358
       if (along > 1e-5) {
         const double t = (dist - combined_radius) / along;                     // :360
         if (t >= 0.0) ttc = fmin(ttc, t);
@@ -256,9 +301,9 @@ __global__ void fot_safety_kernel(const double* __restrict__ ego, const double* 
     }
   }
   for (int off = 16; off > 0; off >>= 1) {
-    dmin = fmin(dmin, __shfl_xor_sync(0xffffffffu, dmin, off));
-    ttc = fmin(ttc, __shfl_xor_sync(0xffffffffu, ttc, off));
-    dmin_ahead = fmin(dmin_ahead, __shfl_xor_sync(0xffffffffu, dmin_ahead, off));
+    dmin = nan_min(dmin, __shfl_xor_sync(0xffffffffu, dmin, off));
+    ttc = fmin(ttc, __shfl_xor_sync(0xffffffffu, ttc, off));                  // never NaN (t >= 0 above)
+    dmin_ahead = nan_min(dmin_ahead, __shfl_xor_sync(0xffffffffu, dmin_ahead, off));
   }
   if (lane == 0) {
     double* o = out + 5 * (size_t)q;
@@ -266,7 +311,7 @@ __global__ void fot_safety_kernel(const double* __restrict__ ego, const double* 
     o[1] = dmin < combined_radius ? 1.0 : 0.0;                                 // :345
     o[2] = ttc;
     o[3] = dmin - combined_radius;                                             // :385
-    o[4] = dmin_ahead < inf ? dmin_ahead - combined_radius : inf;              // :375-376
+    o[4] = dmin_ahead == inf ? inf : dmin_ahead - combined_radius;             // :375-376
   }
 }
 

@@ -142,8 +142,9 @@ def safety_metrics(ego, ped_pos, ped_vel, ego_radius: float, ped_radius: float, 
                    device: int = 0):
     """compute_safety_metrics_static (src/core/data_structures.py:301-388) for a batch of queries on the
     device.  ego [n_q, 5] (x, y, yaw, v, a), ped_pos / ped_vel [n_q, P, 2] (host arrays or CUDA tensors),
-    n_peds optional int32 [n_q].  Returns a dict of CUDA tensors [n_q]: min_distance, collision (bool),
-    ttc, clearance, clearance_ahead -- the inputs of FailSafeStateMachine.update / _get_planner_config."""
+    n_peds optional [n_q], each in [0, P] (ValueError otherwise).  Returns a dict of CUDA tensors [n_q]:
+    min_distance, collision (bool), ttc, clearance, clearance_ahead -- the inputs of
+    FailSafeStateMachine.update / _get_planner_config."""
     import torch
     lib = _lib.load()
     dev = torch.device("cuda", int(device))
@@ -153,7 +154,15 @@ def safety_metrics(ego, ped_pos, ped_vel, ego_radius: float, ped_radius: float, 
     n_q, P = ego_t.shape[0], pos_t.shape[1]
     if tuple(pos_t.shape) != (n_q, P, 2) or tuple(vel_t.shape) != (n_q, P, 2):
         raise ValueError("ped_pos / ped_vel must be [n_q, P, 2]")
-    np_t = None if n_peds is None else torch.as_tensor(n_peds, dtype=torch.int32).to(dev).contiguous()
+    np_t = None
+    if n_peds is not None:
+        # a count above P would read the next query's pedestrians (past the buffer for the last query)
+        n = n_peds if isinstance(n_peds, torch.Tensor) else torch.as_tensor(np.asarray(n_peds))
+        if tuple(n.shape) != (n_q,):
+            raise ValueError(f"n_peds must be [n_q] = [{n_q}], got {tuple(n.shape)}")
+        if bool(((n < 0) | (n > P)).any()):
+            raise ValueError(f"n_peds must lie in [0, P] = [0, {P}]")
+        np_t = n.to(dev, dtype=torch.int32).contiguous()
     if footprint is None:
         combined, offs, n_circ = float(ego_radius) + float(ped_radius), None, 0
     else:
