@@ -10,6 +10,7 @@
 #include <vector>
 #include <mutex>
 #include <set>
+#include <initializer_list>
 
 #include "fot_kernels.cuh"
 #include "fot_sweep_items.cuh"
@@ -485,6 +486,49 @@ static bool pair_geometry(const fot_handle* h, const fot_batch_t* b, PairGeom* g
   return true;
 }
 
+// The sweep kernel of a launch, with its geometry and dynamic shared memory.  kind takes the values of
+// fot_last_sweep_kind (and of Options::sweep).
+enum SweepKind { kItems = 1, kGeneric = 2, kPairs = 4 };
+struct Sweep {
+  int kind = 0;
+  ItemGeom ig{};      // fot_sweep_items; for fot_sweep_pairs the scratch layout it shares with it
+  PairGeom pg{};      // fot_sweep_pairs
+  SweepGeom g{};      // fot_sweep; for the other two only blocks_per_query, which fot_winner reads
+  size_t smem = 0;
+};
+
+// Kernel choice: the pair-per-warp fot_sweep_pairs wherever its shape limits allow, else the sample-major
+// fot_sweep_items, else the candidate-major fot_sweep.  FOT_SWEEP=pairs / items / generic insists on one of them (the
+// tests cross-check the three).  A gated launch needs a sample-major kernel with a staged obstacle block: the gate of
+// fot_sweep_items decides that, and fot_sweep_pairs runs gated only where it stages the block too.
+static int select_sweep(const fot_handle* h, const fot_batch_t* b, bool gated, Sweep* s) {
+  *s = Sweep{};
+  size_t ismem = 0, psmem = 0;
+  const bool items = h->opt.sweep != kGeneric && item_geometry(h, b, &s->ig, &ismem, gated);
+  if (gated && !(items && s->ig.fused_box))
+    return fail(FOT_ERR_ARG, "gated launch needs a sample-major sweep with a staged obstacle block");
+  if (h->opt.sweep == kItems && !items) return fail(FOT_ERR_ARG, "FOT_SWEEP=items: shape not supported by fot_sweep_items");
+  const bool pairs = (h->opt.sweep == 0 || h->opt.sweep == kPairs) && items && pair_geometry(h, b, &s->pg, &psmem, gated) &&
+                     (!gated || s->pg.fused_box);
+  if (h->opt.sweep == kPairs && !pairs && !gated) return fail(FOT_ERR_ARG, "FOT_SWEEP=pairs: shape not supported by fot_sweep_pairs");
+  if (pairs) {
+    // same scratch (cost tables, trajectory boxes, one arg-min partial per CTA) as fot_sweep_items
+    s->ig.blocks_per_query = h->plan.cfg.n_T * b->n_v_max + h->plan.cfg.n_B;      // upper bound of ctas_per_query (scratch stride)
+    s->ig.ctas_per_query = s->pg.ctas_per_query; s->ig.threads = kPairThreads;
+    s->ig.fused_box = s->pg.fused_box;
+    s->kind = kPairs;
+    s->smem = psmem;
+  } else if (items) {
+    s->kind = kItems;
+    s->smem = ismem;
+  } else {
+    s->kind = kGeneric;
+    return sweep_geometry(h, b, &s->g, &s->smem);
+  }
+  s->g.blocks_per_query = s->ig.ctas_per_query;     // fot_winner reads one partial per CTA
+  return FOT_OK;
+}
+
 static int check_batch(const fot_handle* h, const fot_batch_t* b, const fot_result_t* r) {
   if (!h || !b || !r) return fail(FOT_ERR_ARG, "null argument");
   if (b->n_q < 1 || b->n_v_max < 1) return fail(FOT_ERR_ARG, "n_q and n_v_max must be >= 1");
@@ -532,35 +576,16 @@ struct Gate {
 static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r, cudaStream_t st, size_t q_off = 0,
                       size_t q_total = 0, Gate gate = Gate{}, bool record_span = true) {
   if (q_total == 0) q_total = (size_t)b->n_q;
-  // kernel choice: the pair-per-warp fot_sweep_pairs wherever its shape limits allow, else the sample-major
-  // fot_sweep_items, else the candidate-major fot_sweep.  FOT_SWEEP=pairs / items / generic insists on one of them
-  // (the tests cross-check the three).
-  ItemGeom ig{};
-  size_t ismem = 0;
-  bool use_items = item_geometry(h, b, &ig, &ismem, gate.word != nullptr);
-  if (h->opt.sweep == 2) use_items = false;
-  PairGeom pg{};
-  size_t psmem = 0;
-  bool use_pairs = (h->opt.sweep == 0 || h->opt.sweep == 4) && use_items && pair_geometry(h, b, &pg, &psmem, gate.word != nullptr);
-  if (use_pairs && gate.word && !pg.fused_box) use_pairs = false;
-  if (h->opt.sweep == 4 && !use_pairs && !gate.word) return fail(FOT_ERR_ARG, "FOT_SWEEP=pairs: shape not supported by fot_sweep_pairs");
-  if (use_pairs) {
-    // same scratch (cost tables, trajectory boxes, one arg-min partial per CTA) as fot_sweep_items
-    ig.blocks_per_query = h->plan.cfg.n_T * b->n_v_max + h->plan.cfg.n_B;      // upper bound of ctas_per_query (scratch stride)
-    ig.ctas_per_query = pg.ctas_per_query; ig.threads = kPairThreads;
-    ig.fused_box = pg.fused_box;
-    if (gate.word) { pg.gate = gate.word; pg.gate_epoch = gate.epoch; pg.gate_per = gate.per; pg.gate_q0 = (int32_t)q_off; }
-  }
-  if (gate.word && !(use_items && ig.fused_box)) return fail(FOT_ERR_ARG, "gated launch needs a sample-major sweep with a staged obstacle block");
-  if (gate.word) { ig.gate = gate.word; ig.gate_epoch = gate.epoch; ig.gate_per = gate.per; ig.gate_q0 = (int32_t)q_off; }
-  if (h->opt.sweep == 1 && !use_items) return fail(FOT_ERR_ARG, "FOT_SWEEP=items: shape not supported by fot_sweep_items");
-  SweepGeom g{};
-  size_t smem = 0;
-  if (!use_items) {
-    int rc = sweep_geometry(h, b, &g, &smem);
-    if (rc != FOT_OK) return rc;
-  } else {
-    g.blocks_per_query = ig.ctas_per_query;     // fot_winner reads one partial per CTA
+  Sweep s;
+  const int rc = select_sweep(h, b, gate.word != nullptr, &s);
+  if (rc != FOT_OK) return rc;
+  const bool use_pairs = s.kind == kPairs, use_items = s.kind != kGeneric;
+  ItemGeom& ig = s.ig;
+  PairGeom& pg = s.pg;
+  const SweepGeom& g = s.g;
+  if (gate.word) {
+    ig.gate = gate.word; ig.gate_epoch = gate.epoch; ig.gate_per = gate.per; ig.gate_q0 = (int32_t)q_off;
+    pg.gate = gate.word; pg.gate_epoch = gate.epoch; pg.gate_per = gate.per; pg.gate_q0 = (int32_t)q_off;
   }
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
   const size_t n_part = (size_t)b->n_q * g.blocks_per_query;
@@ -665,12 +690,12 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
     int feat = PAIR_ALL;
     for (int i = 0; i < kPairInstanceCount; ++i)
       if ((kPairInstances[i] & need) == need) { feat = kPairInstances[i]; break; }
-    pair_kernel(pg.fused_box != 0, feat)<<<(unsigned)n_part, kPairThreads, psmem, st>>>(h->plan, B, O, pg);
+    pair_kernel(pg.fused_box != 0, feat)<<<(unsigned)n_part, kPairThreads, s.smem, st>>>(h->plan, B, O, pg);
     h->last_pair_feat = feat;
-  } else if (use_items && ig.fused_box) fot_sweep_items<true><<<(unsigned)n_part, ig.threads, ismem, st>>>(h->plan, B, O, ig);
-  else if (use_items) fot_sweep_items<false><<<(unsigned)n_part, ig.threads, ismem, st>>>(h->plan, B, O, ig);
-  else fot_sweep<<<(unsigned)n_part, kSweepThreads, smem, st>>>(h->plan, B, O, g);
-  h->last_sweep_kind = use_pairs ? 4 : use_items ? 1 : 2;
+  } else if (use_items && ig.fused_box) fot_sweep_items<true><<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
+  else if (use_items) fot_sweep_items<false><<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
+  else fot_sweep<<<(unsigned)n_part, kSweepThreads, s.smem, st>>>(h->plan, B, O, g);
+  h->last_sweep_kind = s.kind;
   CK(cudaEventRecord(ring[2], st));
   fot_winner<<<b->n_q, 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, O, g);
   if (O.m_winner && h->mirror_flag) fot_publish_kernel<<<1, 1, 0, st>>>(h->mirror_flag, ++h->mirror_seq);
@@ -762,36 +787,163 @@ static int close_span(fot_handle* h, cudaStream_t first) {
   return FOT_OK;
 }
 
-static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r);
-static int plan_batch_device_to_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r, void* stream);
+// Query ranges of a host-result call: range c is queries [bound[c], bound[c + 1]).  gated (host-pointer call only): the
+// sweep waits for slices of the obstacle upload, not for whole ranges.
+struct Ranges {
+  int n = 1;
+  int bound[fot_handle::kMaxChunks + 1] = {};
+  bool gated = false;
+};
 
-extern "C" int fot_plan_batch_host(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r) {
-  int rc = check_batch(h, b, r);
-  if (rc != FOT_OK) return rc;
-  CK(cudaSetDevice(h->device));
-  rc = plan_batch_host_impl(h, b, r);
-  if (rc != FOT_OK) drain_after_failure(h);
-  return rc;
+// Ranges ending at about frac16[i] / 16 of the nq queries, in whole waves of the sweep (one CTA per query, two CTAs per
+// SM) where possible, and a last range ending at nq.
+static void cut16(const fot_handle* h, int nq, std::initializer_list<int> frac16, Ranges* rg) {
+  const int wave = 2 * h->sms;
+  rg->n = 0;
+  rg->bound[0] = 0;
+  for (int f : frac16) {
+    const int cut = std::max(1, (int)((long long)nq * f / 16 / wave)) * wave;
+    rg->bound[rg->n + 1] = std::min(nq, std::max(cut, rg->bound[rg->n]));
+    ++rg->n;
+  }
+  rg->bound[++rg->n] = nq;
 }
 
-extern "C" int fot_plan_batch_device_to_host(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r, void* stream) {
-  int rc = check_batch(h, b, r);
-  if (rc != FOT_OK) return rc;
-  CK(cudaSetDevice(h->device));
-  rc = plan_batch_device_to_host_impl(h, b, r, stream);
-  if (rc != FOT_OK) drain_after_failure(h);
-  return rc;
+static Ranges plan_ranges(const fot_handle* h, const fot_batch_t* b, bool host) {
+  const int nq = b->n_q;
+  const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
+  Ranges rg;
+  rg.bound[1] = nq;
+  const std::string keep = g_err;      // a kernel the probes below refuse is not an error of this call
+  Sweep s;
+  if (host) {
+    // Ranges only pay when the obstacle upload is large.  The kernels are the longer leg of the pipeline (the upload runs
+    // at PCIe speed), so the first ranges are small -- the sweep starts after 1/16 of the upload -- and the rest large
+    // enough to keep the wave tail short: about 1/16, 1/8, 3/16, 5/16, 5/16 of the queries.
+    const size_t upload = has_dyn ? (size_t)nq * b->S * b->P * b->T_obs * 16 : 0;
+    if (upload > ((size_t)8 << 20) && nq >= 1024) cut16(h, nq, {1, 3, 6, 11}, &rg);
+    if (h->opt.host_chunks > 0) {
+      rg.n = std::max(1, std::min(fot_handle::kMaxChunks, h->opt.host_chunks));
+      const int per = (nq + rg.n - 1) / rg.n;
+      for (int c = 0; c <= rg.n; ++c) rg.bound[c] = std::min(nq, c * per);
+    }
+    // Gated, the sweep does not wait for whole ranges, so a few large ones do: about 1/2, 5/16, 3/16 of the queries.
+    rg.gated = h->opt.gated && rg.n > 1 && has_dyn && nq < (1 << 22) && select_sweep(h, b, true, &s) == FOT_OK;
+    if (rg.gated && h->opt.host_chunks <= 0) cut16(h, nq, {8, 13}, &rg);
+  } else if (nq >= 1024) {
+    cut16(h, nq, {8, 13}, &rg);
+  }
+  // only the sample-major kernels address their scratch by query offset: the candidate-major fot_sweep takes one range
+  if (!rg.gated && rg.n > 1 && (select_sweep(h, b, false, &s) != FOT_OK || s.kind == kGeneric)) {
+    rg.n = 1;
+    rg.bound[1] = nq;
+  }
+  g_err = keep;
+  return rg;
 }
 
-// Host-pointer entry point.  Small per-query arrays go through one pinned blob; the obstacle tensor
-// is copied straight from the caller's memory (pinned memory makes that a true async DMA).  Large
-// batches are cut into chunks of queries: chunk c+1's obstacle upload runs on the copy stream while
-// chunk c's kernels run on the compute stream, and each chunk's winners go back as soon as its
-// kernels finish, directly into the caller's result arrays.
-static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r) {
-  int rc = FOT_OK;
-  cudaStream_t st = h->stream;
+// FOT_DEBUG_TIMING=1: the device timeline of a host-pointer call on stderr, in ms from the start of the call
+// (profiles/r1/e2e_timeline.txt; tools/tuning/e2e_lib.sh reads the last lines).  A timeline that is off records nothing.
+struct Timeline {
+  enum { kStart, kCopyStart, kCopiesDone, kKernelsDone, kRange };   // then per range: upload done,
+  static constexpr int kEvents = kRange + 4 * fot_handle::kMaxChunks;  // kernels start / end, read-back done
+  cudaEvent_t ev[kEvents] = {};
+  bool marked[kEvents] = {};
+  explicit Timeline(bool on) { if (on) for (auto& e : ev) cudaEventCreate(&e); }
+  ~Timeline() { for (auto e : ev) if (e) cudaEventDestroy(e); }
+  void mark(int i, cudaStream_t s) { if (ev[i]) marked[i] = cudaEventRecord(ev[i], s) == cudaSuccess; }
+  void range(int c, int k, cudaStream_t s) { mark(kRange + 4 * c + k, s); }
+  float ms(int i) const {
+    float t = -1.0f;
+    if (marked[kStart] && marked[i] && cudaEventSynchronize(ev[kStart]) == cudaSuccess && cudaEventSynchronize(ev[i]) == cudaSuccess)
+      cudaEventElapsedTime(&t, ev[kStart], ev[i]);
+    return t;
+  }
+  void print(const Ranges& rg) const {
+    if (!ev[kStart]) return;
+    fprintf(stderr, "[fot] chunks=%d copy-stream start %.3f ms, copies done %.3f ms, first kernel may start %.3f ms, kernels done %.3f ms\n",
+            rg.n, ms(kCopyStart), ms(kCopiesDone), ms(kRange + 1), ms(kKernelsDone));   // range 0 is never empty
+    for (int c = 0; c < rg.n; ++c) {
+      const int e = kRange + 4 * c;
+      fprintf(stderr, "[fot]   chunk %2d queries %5d..%5d  upload done %.3f  kernels %.3f -> %.3f  read-back done %.3f\n", c,
+              rg.bound[c], rg.bound[c + 1], ms(e), ms(e + 1), ms(e + 2), ms(e + 3));
+    }
+  }
+};
+
+// The range loop of both host-result calls: `b` is the whole batch in device memory, `r` the caller's host arrays.  Range c
+// is swept once wait[c] (if given) has fired, and its winners go back on the d2h stream as soon as its kernels finish, so
+// only the last range's read-back is exposed.  With `prio` the ranges run on streams of descending priority: every
+// range's kernels are eligible from the start, and a CTA of a later range that got an SM slot early would only sit there
+// waiting (gated: for its slice of the upload).  Otherwise they alternate two compute streams, so that the next range's
+// CTAs fill the SMs the tail wave of the previous range leaves idle (the ranges touch disjoint scratch, see launch_all).
+static int run_ranges(fot_handle* h, const fot_batch_t* b, const fot_result_t* r, const Ranges& rg, Gate gate, bool prio,
+                      const cudaEvent_t* wait, Timeline& tl) {
   const int nq = b->n_q, NT = h->plan.n_t_max;
+  size_t ro = 0;
+  auto rtake = [&](size_t bytes) { size_t o = ro; ro = align_up(ro + bytes); return o; };
+  const size_t r_bi = rtake((size_t)nq * 4), r_bc = rtake((size_t)nq * 8), r_st = rtake((size_t)nq * FOT_N_STATS * 4),
+               r_wl = rtake((size_t)nq * 4), r_w = rtake((size_t)nq * FOT_N_SERIES * NT * 8);
+  const size_t r_cc = r->cand_cat ? rtake((size_t)nq * r->cand_stride) : 0;
+  const size_t r_cs = r->cand_cost ? rtake((size_t)nq * r->cand_stride * 8) : 0;
+  const int k_head = r->winner_samples > 0 ? std::min(r->winner_samples, NT) : 0;
+  const size_t r_wh = k_head ? rtake((size_t)nq * FOT_N_SERIES * k_head * 8) : 0;
+  CK(h->out_d.reserve(ro));
+  char* od = (char*)h->out_d.p;
+  h->last_winner_d = (const double*)(od + r_w);     // fot_fetch_winners
+  h->last_winner_nq = nq;
+  const size_t dyn_q_bytes = b->dyn_mode != FOT_DYN_NONE ? (size_t)b->S * b->P * b->T_obs * 16 : 0;
+  auto stream_of = [&](int i) { return prio ? h->pstream[i & 3] : (i & 1) ? h->stream2 : h->stream; };
+  int n_issued = 0;
+  for (int c = 0; c < rg.n; ++c) {
+    const int q0 = rg.bound[c], cq = rg.bound[c + 1] - q0;
+    if (cq <= 0) continue;
+    const int i = n_issued++;
+    cudaStream_t st = stream_of(i);
+    if (wait) CK(cudaStreamWaitEvent(st, wait[c], 0));
+    if (i == 0) CK(cudaEventRecord(h->ev0, st));
+    tl.range(c, 1, st);
+    fot_batch_t db = *b;
+    db.n_q = cq;
+    db.frenet = b->frenet + (size_t)q0 * 6;
+    db.target_speed = b->target_speed + q0;
+    db.limits = b->limits + (size_t)q0 * 4;
+    db.stop_dist = b->stop_dist + q0;
+    db.v_grid = b->v_grid + (size_t)q0 * b->n_v_max;
+    db.n_v = b->n_v + q0;
+    if (dyn_q_bytes) db.dyn = (const double*)((const char*)b->dyn + (size_t)q0 * dyn_q_bytes);
+    if (b->n_static > 0 && b->static_per_query) db.static_obs = b->static_obs + (size_t)q0 * b->n_static * 2;
+    fot_result_t dr = *r;
+    dr.best_idx = (int32_t*)(od + r_bi) + q0;
+    dr.best_cost = (double*)(od + r_bc) + q0;
+    dr.stats = (int32_t*)(od + r_st) + (size_t)q0 * FOT_N_STATS;
+    dr.winner_len = (int32_t*)(od + r_wl) + q0;
+    dr.winner = (double*)(od + r_w) + (size_t)q0 * FOT_N_SERIES * NT;
+    dr.cand_cat = r->cand_cat ? (uint8_t*)(od + r_cc) + (size_t)q0 * r->cand_stride : nullptr;
+    dr.cand_cost = r->cand_cost ? (double*)(od + r_cs) + (size_t)q0 * r->cand_stride : nullptr;
+    int rc = launch_all(h, &db, &dr, st, (size_t)q0, (size_t)nq, gate, /*record_span=*/false);
+    if (rc != FOT_OK) return rc;
+    tl.range(c, 2, st);
+    // on their own stream, so that the next range's kernels never queue behind a copy engine busy with the uploads
+    rc = read_back(h, r, dr, (double*)(od + r_wh) + (size_t)q0 * FOT_N_SERIES * k_head, q0, cq, NT, st, h->d2h_stream, h->ev_done[c]);
+    if (rc != FOT_OK) return rc;
+    tl.range(c, 3, h->d2h_stream);
+  }
+  const int rc = close_span(h, stream_of(0));
+  if (rc != FOT_OK) return rc;
+  tl.mark(Timeline::kKernelsDone, stream_of(0));
+  CK(cudaStreamSynchronize(h->d2h_stream));   // the last read-backs wait for the last kernels of every compute stream
+  for (int i = 0; i < n_issued && i < 4; ++i) CK(cudaStreamSynchronize(stream_of(i)));
+  tl.print(rg);
+  return FOT_OK;
+}
+
+// Host-pointer entry point.  Small per-query arrays go through one pinned blob; the obstacle tensor is copied straight
+// from the caller's memory (pinned memory makes that a true async DMA).  A large upload is pipelined with the sweep: the
+// sweep either waits for fine slices of it (gated) or for whole ranges of queries, so that range c+1's upload runs on
+// the copy stream while range c's kernels run.
+static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r) {
+  const int nq = b->n_q;
   // ---- small per-query arrays: one pinned blob, one H2D -------------------------------
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
@@ -810,7 +962,7 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
   // streams.  (A copy on the compute stream makes the driver service that stream's later timed event
   // records on the copy engine, where they queue behind the uploads and serialise the pipeline.)
   CK(cudaMemcpyAsync(h->stage_d.p, sh, off, cudaMemcpyHostToDevice, h->copy_stream));
-  char* sd = (char*)h->stage_d.p;
+  const char* sd = (const char*)h->stage_d.p;
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
   const size_t dyn_q_bytes = has_dyn ? (size_t)b->S * b->P * b->T_obs * 16 : 0;
   if (has_dyn) CK(h->dyn_d.reserve((size_t)nq * dyn_q_bytes));
@@ -819,66 +971,22 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
     CK(h->stat_d.reserve(bytes));
     CK(cudaMemcpyAsync(h->stat_d.p, b->static_obs, bytes, cudaMemcpyHostToDevice, h->copy_stream));
   }
-  // ---- device result blob ---------------------------------------------------------------
-  size_t ro = 0;
-  auto rtake = [&](size_t bytes) { size_t o = ro; ro = align_up(ro + bytes); return o; };
-  const size_t r_bi = rtake((size_t)nq * 4), r_bc = rtake((size_t)nq * 8), r_st = rtake((size_t)nq * FOT_N_STATS * 4),
-               r_wl = rtake((size_t)nq * 4), r_w = rtake((size_t)nq * FOT_N_SERIES * NT * 8);
-  const size_t r_cc = r->cand_cat ? rtake((size_t)nq * r->cand_stride) : 0;
-  const size_t r_cs = r->cand_cost ? rtake((size_t)nq * r->cand_stride * 8) : 0;
-  const int k_head = r->winner_samples > 0 ? std::min(r->winner_samples, NT) : 0;
-  const size_t r_wh = k_head ? rtake((size_t)nq * FOT_N_SERIES * k_head * 8) : 0;
-  CK(h->out_d.reserve(ro));
-  char* od = (char*)h->out_d.p;
-  h->last_winner_d = (const double*)(od + r_w);     // fot_fetch_winners
-  h->last_winner_nq = nq;
-
-  // chunking: only worth it when the obstacle upload is large.  The kernels are the longer leg of the
-  // pipeline (the upload runs at PCIe speed), so the first chunks are small -- the sweep starts after
-  // 1/16 of the upload -- and the rest are large enough to keep the wave tail short.
-  int n_chunks = 1;
-  constexpr int kMaxChunks = fot_handle::kMaxChunks;
-  int bounds[kMaxChunks + 1];
-  bounds[0] = 0;
-  for (int c = 1; c <= kMaxChunks; ++c) bounds[c] = nq;
-  if ((size_t)nq * dyn_q_bytes > ((size_t)8 << 20) && nq >= 1024) {
-    // chunk sizes in whole waves of the sweep (one CTA per query, two CTAs per SM) where possible
-    const int wave = 2 * h->sms;
-    auto waves = [&](int frac16) { const int w = std::max(1, (int)((long long)nq * frac16 / 16 / wave)); return w * wave; };
-    const int cuts[] = {waves(1), waves(3), waves(6), waves(11), nq};  // about 1/16, 1/8, 3/16, 5/16, 5/16 of the queries
-    n_chunks = 5;
-    for (int c = 0; c < n_chunks; ++c) bounds[c + 1] = std::min(nq, std::max(cuts[c], bounds[c]));
-  }
-  if (h->opt.host_chunks > 0) {
-    n_chunks = std::max(1, std::min(kMaxChunks, h->opt.host_chunks));
-    const int per_ = (nq + n_chunks - 1) / n_chunks;
-    for (int c = 0; c <= n_chunks; ++c) bounds[c] = std::min(nq, c * per_);
-  }
-  // chunks alternate between two compute streams, so that the next chunk's CTAs fill the SMs the tail wave of
-  // the previous chunk leaves idle (the chunks touch disjoint scratch, see launch_all)
-  bool two_streams = n_chunks > 1;
-  if (two_streams) {
-    ItemGeom ig{};
-    size_t ismem = 0;
-    fot_batch_t probe = *b;
-    probe.n_q = bounds[1] - bounds[0];
-    if (!item_geometry(h, &probe, &ig, &ismem) || h->opt.sweep == 2) two_streams = false;
-  }
-  // Gated launches (large uploads through fot_sweep_items): the sweep does not wait for whole chunks.  The upload
-  // is cut into fine slices, each followed by a 4-byte copy that publishes "queries uploaded so far"; the sweep
-  // is launched over few, large ranges of queries and every CTA waits for its own query's slice (ItemGeom::gate).
-  // The ranges only exist so that winners of the first queries go back while the last are still being swept.
-  bool gated = false;
+  // the batch as the kernels read it
+  fot_batch_t db = *b;
+  db.frenet = (const double*)(sd + o_fr);
+  db.target_speed = (const double*)(sd + o_tg);
+  db.limits = (const double*)(sd + o_lm);
+  db.stop_dist = (const double*)(sd + o_sd);
+  db.v_grid = (const double*)(sd + o_vg);
+  db.n_v = (const int32_t*)(sd + o_nv);
+  if (has_dyn) db.dyn = (const double*)h->dyn_d.p;
+  if (b->n_static > 0) db.static_obs = (const double*)h->stat_d.p;
+  const Ranges rg = plan_ranges(h, b, true);
+  // Gated: the upload is cut into fine slices, each followed by a 4-byte write that publishes "queries uploaded so
+  // far", and every CTA of the sweep waits for its own query's slice (ItemGeom::gate).
   int n_up = 0, ub[kGateSlices + 1] = {0};
   Gate gate{};
-  {
-    if (h->opt.gated && n_chunks > 1 && has_dyn && nq < (1 << 22) && h->opt.sweep != 2) {
-      ItemGeom ig{};
-      size_t ismem = 0;
-      gated = item_geometry(h, b, &ig, &ismem, true) && ig.fused_box;
-    }
-  }
-  if (gated) {
+  if (rg.gated) {
     const bool fresh = h->gate_d.p == nullptr;
     CK(h->gate_d.reserve((kGateSlices + 1) * sizeof(uint32_t)));
     CK(h->gate_h.reserve((kGateSlices + 1) * sizeof(uint32_t)));
@@ -890,27 +998,14 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
     gate.per = (nq + n_up - 1) / n_up;
     n_up = (nq + gate.per - 1) / gate.per;
     for (int u = 0; u <= n_up; ++u) ub[u] = std::min(nq, u * gate.per);
-    // launch ranges: about 1/2, 5/16, 3/16 of the queries, in whole waves
-    const int wave = 2 * h->sms;
-    auto waves = [&](int frac16) { const int w = std::max(1, (int)((long long)nq * frac16 / 16 / wave)); return w * wave; };
-    if (h->opt.host_chunks <= 0) {
-      const int cuts[] = {waves(8), waves(13), nq};
-      n_chunks = 3;
-      for (int c = 0; c < n_chunks; ++c) bounds[c + 1] = std::min(nq, std::max(cuts[c], bounds[c]));
-      for (int c = n_chunks + 1; c <= kMaxChunks; ++c) bounds[c] = nq;
-    }
-    two_streams = n_chunks > 1;
   }
   const auto t_wall0 = std::chrono::steady_clock::now();
-  const bool dbg = h->opt.debug_timing != 0;
-  cudaEvent_t d0 = nullptr, d1 = nullptr, d2 = nullptr, d3 = nullptr, d4 = nullptr;
-  cudaEvent_t tl[kMaxChunks][4] = {};                    // debug timeline per chunk: upload done, kernels start / end, read-back done
-  if (dbg) for (auto& row : tl) for (auto& ev : row) cudaEventCreate(&ev);
-  if (dbg) { cudaEventCreate(&d0); cudaEventCreate(&d1); cudaEventCreate(&d2); cudaEventCreate(&d3); cudaEventCreate(&d4);
-             cudaEventRecord(d0, st); cudaEventRecord(d4, h->copy_stream); }
+  Timeline tl(h->opt.debug_timing != 0);
+  tl.mark(Timeline::kStart, h->stream);
+  tl.mark(Timeline::kCopyStart, h->copy_stream);
   CK(cudaEventRecord(h->ev_blob, h->copy_stream));
-  // every obstacle upload is queued first (they depend on nothing), one event per chunk
-  if (gated) {
+  // every obstacle upload is queued first (they depend on nothing)
+  if (rg.gated) {
     // each slice is followed on the upload stream by the write of its flag, which stream order keeps behind the slice
     uint32_t* words = (uint32_t*)h->gate_h.p;
     for (int u = 0; u < n_up; ++u) {
@@ -928,78 +1023,28 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
       }
     }
   } else if (has_dyn)
-    for (int c = 0; c < n_chunks; ++c) {
-      const int q0 = bounds[c], cq = bounds[c + 1] - q0;
+    for (int c = 0; c < rg.n; ++c) {
+      const int q0 = rg.bound[c], cq = rg.bound[c + 1] - q0;
       if (cq <= 0) continue;
       char* dst = (char*)h->dyn_d.p + (size_t)q0 * dyn_q_bytes;
       const char* src = (const char*)b->dyn + (size_t)q0 * dyn_q_bytes;
       CK(cudaMemcpyAsync(dst, src, (size_t)cq * dyn_q_bytes, cudaMemcpyHostToDevice, h->copy_stream));
       CK(cudaEventRecord(h->ev_copy[c], h->copy_stream));
-      if (dbg) cudaEventRecord(tl[c][0], h->copy_stream);
+      tl.range(c, 0, h->copy_stream);
     }
-  if (dbg) {
-    cudaEventRecord(d1, h->copy_stream);
+  tl.mark(Timeline::kCopiesDone, h->copy_stream);
+  if (h->opt.debug_timing) {
     cudaPointerAttributes pa{};
     cudaError_t pe = cudaPointerGetAttributes(&pa, b->dyn);
     fprintf(stderr, "[fot] dyn pointer attr: err=%d type=%d (0 unregistered, 1 host, 2 device, 3 managed)\n", (int)pe, (int)pa.type);
   }
-  int n_issued = 0;
-  cudaStream_t span_first = nullptr;
-  for (int c = 0; c < n_chunks; ++c) {
-    const int q0 = bounds[c], cq = bounds[c + 1] - q0;
-    if (cq <= 0) continue;
-    // Gated ranges run on streams of descending priority: every range's kernels are eligible from the start, and a
-    // CTA of a later range that got an SM slot early would only sit there waiting for its slice of the upload.
-    cudaStream_t st = gated ? h->pstream[n_issued & 3] : (two_streams && (n_issued & 1)) ? h->stream2 : h->stream;
-    ++n_issued;
-    if (has_dyn && !gated) CK(cudaStreamWaitEvent(st, h->ev_copy[c], 0));
-    else CK(cudaStreamWaitEvent(st, h->ev_blob, 0));
-    if (!span_first) { span_first = st; CK(cudaEventRecord(h->ev0, st)); }
-    if (dbg && c == 0) cudaEventRecord(d2, st);
-    if (dbg) cudaEventRecord(tl[c][1], st);
-    fot_batch_t db = *b;
-    db.n_q = cq;
-    db.frenet = (const double*)(sd + o_fr) + (size_t)q0 * 6;
-    db.target_speed = (const double*)(sd + o_tg) + q0;
-    db.limits = (const double*)(sd + o_lm) + (size_t)q0 * 4;
-    db.stop_dist = (const double*)(sd + o_sd) + q0;
-    db.v_grid = (const double*)(sd + o_vg) + (size_t)q0 * b->n_v_max;
-    db.n_v = (const int32_t*)(sd + o_nv) + q0;
-    if (has_dyn) db.dyn = (const double*)((char*)h->dyn_d.p + (size_t)q0 * dyn_q_bytes);
-    if (b->n_static > 0)
-      db.static_obs = (const double*)h->stat_d.p + (b->static_per_query ? (size_t)q0 * b->n_static * 2 : 0);
-    fot_result_t dr = *r;
-    dr.best_idx = (int32_t*)(od + r_bi) + q0;
-    dr.best_cost = (double*)(od + r_bc) + q0;
-    dr.stats = (int32_t*)(od + r_st) + (size_t)q0 * FOT_N_STATS;
-    dr.winner_len = (int32_t*)(od + r_wl) + q0;
-    dr.winner = (double*)(od + r_w) + (size_t)q0 * FOT_N_SERIES * NT;
-    dr.cand_cat = r->cand_cat ? (uint8_t*)(od + r_cc) + (size_t)q0 * r->cand_stride : nullptr;
-    dr.cand_cost = r->cand_cost ? (double*)(od + r_cs) + (size_t)q0 * r->cand_stride : nullptr;
-    rc = launch_all(h, &db, &dr, st, (size_t)q0, (size_t)nq, gate, /*record_span=*/false);
-    if (rc != FOT_OK) return rc;
-    // winners of this chunk straight into the caller's arrays, on their own stream so the next
-    // chunk's kernels never queue behind a copy engine that is busy with the uploads
-    cudaStream_t ds = h->d2h_stream;
-    if (dbg) cudaEventRecord(tl[c][2], st);
-    rc = read_back(h, r, dr, (double*)(od + r_wh) + (size_t)q0 * FOT_N_SERIES * k_head, q0, cq, NT, st, ds, h->ev_done[c]);
-    if (rc != FOT_OK) return rc;
-    if (dbg) cudaEventRecord(tl[c][3], ds);
-  }
-  if (dbg) {
-    cudaEventRecord(h->ev_join, h->stream2); cudaStreamWaitEvent(st, h->ev_join, 0);
-    for (auto ps : h->pstream) { cudaEventRecord(h->ev_join, ps); cudaStreamWaitEvent(st, h->ev_join, 0); }
-    cudaEventRecord(d3, st);
-  }
-  if (span_first) { rc = close_span(h, span_first); if (rc != FOT_OK) return rc; }
-  CK(cudaStreamSynchronize(h->d2h_stream));   // the last read-backs wait for the last kernels of every compute stream
-  CK(cudaStreamSynchronize(st));
-  CK(cudaStreamSynchronize(h->stream2));
-  if (gated) {
-    for (auto ps : h->pstream) CK(cudaStreamSynchronize(ps));
-    CK(cudaStreamSynchronize(h->copy_stream));
-  }
-  if (gated && std::chrono::steady_clock::now() - t_wall0 > std::chrono::nanoseconds(kGateTimeoutNs)) {
+  cudaEvent_t wait[fot_handle::kMaxChunks];
+  for (int c = 0; c < rg.n; ++c) wait[c] = has_dyn && !rg.gated ? h->ev_copy[c] : h->ev_blob;
+  const int rc = run_ranges(h, &db, r, rg, gate, /*prio=*/rg.gated, wait, tl);
+  if (rc != FOT_OK) return rc;
+  if (!rg.gated) return FOT_OK;
+  CK(cudaStreamSynchronize(h->copy_stream));
+  if (std::chrono::steady_clock::now() - t_wall0 > std::chrono::nanoseconds(kGateTimeoutNs)) {
     unsigned gave_up = 0;
     CK(cudaMemcpy(&gave_up, gate.word + kGateSlices, sizeof(unsigned), cudaMemcpyDeviceToHost));
     if (gave_up) {
@@ -1007,93 +1052,34 @@ static int plan_batch_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot
       return fail(FOT_ERR_CUDA, "gated sweep: the obstacle upload did not arrive");
     }
   }
-  if (dbg) {
-    float a = 0, bb = 0, cc = 0, dd = 0;
-    cudaEventElapsedTime(&a, d0, d1); cudaEventElapsedTime(&bb, d0, d2); cudaEventElapsedTime(&cc, d0, d3); cudaEventElapsedTime(&dd, d0, d4);
-    fprintf(stderr, "[fot] chunks=%d copy-stream start %.3f ms, copies done %.3f ms, first kernel may start %.3f ms, kernels done %.3f ms\n", n_chunks, dd, a, bb, cc);
-    for (int c = 0; c < n_chunks; ++c) {
-      float t[4] = {-1, -1, -1, -1};
-      for (int k = 0; k < 4; ++k) if (k > 0 || (has_dyn && !gated)) cudaEventElapsedTime(&t[k], d0, tl[c][k]);
-      fprintf(stderr, "[fot]   chunk %2d queries %5d..%5d  upload done %.3f  kernels %.3f -> %.3f  read-back done %.3f\n", c,
-              bounds[c], bounds[c + 1], t[0], t[1], t[2], t[3]);
-    }
-    for (auto& row : tl) for (auto& ev : row) cudaEventDestroy(ev);
-    cudaEventDestroy(d0); cudaEventDestroy(d1); cudaEventDestroy(d2); cudaEventDestroy(d3); cudaEventDestroy(d4);
-  }
   return FOT_OK;
 }
 
-// Device inputs, HOST results: the call of a caller whose obstacle tensor was produced on the GPU (the prediction
-// post-processing of fot_predict.cuh) but who consumes the winners on the host.  The queries are swept in three
-// ranges on the priority streams, and each range's winners go back over PCIe while the next range is swept, so
-// only the last range's read-back is exposed.  `stream` is the stream on which the inputs become ready (NULL:
-// they are ready now).  Returns when the results are in `res`.
-static int plan_batch_device_to_host_impl(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r, void* stream) {
-  int rc = FOT_OK;
-  const int nq = b->n_q, NT = h->plan.n_t_max;
-  size_t ro = 0;
-  auto rtake = [&](size_t bytes) { size_t o = ro; ro = align_up(ro + bytes); return o; };
-  const size_t r_bi = rtake((size_t)nq * 4), r_bc = rtake((size_t)nq * 8), r_st = rtake((size_t)nq * FOT_N_STATS * 4),
-               r_wl = rtake((size_t)nq * 4), r_w = rtake((size_t)nq * FOT_N_SERIES * NT * 8);
-  const size_t r_cc = r->cand_cat ? rtake((size_t)nq * r->cand_stride) : 0;
-  const size_t r_cs = r->cand_cost ? rtake((size_t)nq * r->cand_stride * 8) : 0;
-  const int k_head = r->winner_samples > 0 ? std::min(r->winner_samples, NT) : 0;
-  const size_t r_wh = k_head ? rtake((size_t)nq * FOT_N_SERIES * k_head * 8) : 0;
-  CK(h->out_d.reserve(ro));
-  char* od = (char*)h->out_d.p;
-  h->last_winner_d = (const double*)(od + r_w);     // fot_fetch_winners
-  h->last_winner_nq = nq;
-  // ranges: about 1/2, 5/16, 3/16 of the queries in whole waves; one range for small batches or the fallback kernel
-  int n_ranges = 1, bounds[4] = {0, nq, nq, nq};
-  {
-    ItemGeom ig{};
-    size_t ismem = 0;
-    const bool items = item_geometry(h, b, &ig, &ismem) && h->opt.sweep != 2;
-    if (items && nq >= 1024) {
-      const int wave = 2 * h->sms;
-      auto waves = [&](int frac16) { const int w = std::max(1, (int)((long long)nq * frac16 / 16 / wave)); return w * wave; };
-      const int cuts[] = {waves(8), waves(13), nq};
-      n_ranges = 3;
-      for (int c = 0; c < n_ranges; ++c) bounds[c + 1] = std::min(nq, std::max(cuts[c], bounds[c]));
-    }
-  }
-  if (stream) CK(cudaEventRecord(h->ev_blob, (cudaStream_t)stream));
-  const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
-  const size_t dyn_q_bytes = has_dyn ? (size_t)b->S * b->P * b->T_obs * 16 : 0;
-  for (int c = 0; c < n_ranges; ++c) {
-    const int q0 = bounds[c], cq = bounds[c + 1] - q0;
-    if (cq <= 0) continue;
-    cudaStream_t st = h->pstream[c & 3];
-    if (stream) CK(cudaStreamWaitEvent(st, h->ev_blob, 0));
-    fot_batch_t db = *b;
-    db.n_q = cq;
-    db.frenet = b->frenet + (size_t)q0 * 6;
-    db.target_speed = b->target_speed + q0;
-    db.limits = b->limits + (size_t)q0 * 4;
-    db.stop_dist = b->stop_dist + q0;
-    db.v_grid = b->v_grid + (size_t)q0 * b->n_v_max;
-    db.n_v = b->n_v + q0;
-    if (has_dyn) db.dyn = (const double*)((const char*)b->dyn + (size_t)q0 * dyn_q_bytes);
-    if (b->n_static > 0 && b->static_per_query) db.static_obs = b->static_obs + (size_t)q0 * b->n_static * 2;
-    fot_result_t dr = *r;
-    dr.best_idx = (int32_t*)(od + r_bi) + q0;
-    dr.best_cost = (double*)(od + r_bc) + q0;
-    dr.stats = (int32_t*)(od + r_st) + (size_t)q0 * FOT_N_STATS;
-    dr.winner_len = (int32_t*)(od + r_wl) + q0;
-    dr.winner = (double*)(od + r_w) + (size_t)q0 * FOT_N_SERIES * NT;
-    dr.cand_cat = r->cand_cat ? (uint8_t*)(od + r_cc) + (size_t)q0 * r->cand_stride : nullptr;
-    dr.cand_cost = r->cand_cost ? (double*)(od + r_cs) + (size_t)q0 * r->cand_stride : nullptr;
-    if (c == 0) CK(cudaEventRecord(h->ev0, st));
-    rc = launch_all(h, &db, &dr, st, (size_t)q0, (size_t)nq, Gate{}, /*record_span=*/false);
-    if (rc != FOT_OK) return rc;
-    rc = read_back(h, r, dr, (double*)(od + r_wh) + (size_t)q0 * FOT_N_SERIES * k_head, q0, cq, NT, st, h->d2h_stream, h->ev_done[c]);
-    if (rc != FOT_OK) return rc;
-  }
-  rc = close_span(h, h->pstream[0]);
+extern "C" int fot_plan_batch_host(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r) {
+  int rc = check_batch(h, b, r);
   if (rc != FOT_OK) return rc;
-  CK(cudaStreamSynchronize(h->d2h_stream));
-  for (int c = 0; c < n_ranges; ++c) CK(cudaStreamSynchronize(h->pstream[c & 3]));
-  return FOT_OK;
+  CK(cudaSetDevice(h->device));
+  rc = plan_batch_host_impl(h, b, r);
+  if (rc != FOT_OK) drain_after_failure(h);
+  return rc;
+}
+
+// Device inputs, HOST results: the call of a caller whose obstacle tensor was produced on the GPU (the prediction
+// post-processing of fot_predict.cuh) but who consumes the winners on the host.  Large batches are swept in three
+// ranges on the priority streams, and each range's winners go back over PCIe while the next range is swept, so only
+// the last range's read-back is exposed.  `stream` is the stream on which the inputs become ready (NULL: they are
+// ready now).  Returns when the results are in `res`.
+extern "C" int fot_plan_batch_device_to_host(fot_handle_t* h, const fot_batch_t* b, const fot_result_t* r, void* stream) {
+  int rc = check_batch(h, b, r);
+  if (rc != FOT_OK) return rc;
+  CK(cudaSetDevice(h->device));
+  cudaEvent_t wait[fot_handle::kMaxChunks];
+  for (auto& e : wait) e = h->ev_blob;
+  if (stream) CK(cudaEventRecord(h->ev_blob, (cudaStream_t)stream));
+  Timeline off(false);
+  rc = run_ranges(h, b, r, plan_ranges(h, b, false), Gate{}, /*prio=*/true, stream ? wait : nullptr, off);
+  if (rc != FOT_OK) drain_after_failure(h);
+  return rc;
 }
 
 // ---- the gather of a sharded sweep over peer memory ---------------------------------------------------------------

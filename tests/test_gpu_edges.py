@@ -286,3 +286,41 @@ def test_pair_kernel_shape_limits_and_fallback():
         res = pl.plan_batch(fs, 6.0, dynamic_obstacles=np.stack([dyn] * 2), want_candidates=True)
         assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == kind, (knobs, kind)
         _check(res, [orc.plan_frenet(tuple(s), np.empty((0, 2)), dyn, 6.0) for s in fs])
+
+
+def test_candidate_major_sweep_takes_a_large_upload_in_one_range():
+    """A time grid of 129 samples is beyond fot_sweep_items and fot_sweep_pairs, so the candidate-major fot_sweep runs.
+    It addresses its scratch from query 0, so the host-result calls give it the whole batch as one range, even where
+    the upload size (1024 queries x 5 pedestrians x 129 steps, 10.6 MB) or FOT_HOST_CHUNKS would cut the batch into
+    several.  Both calls must return the bits of a plain launch over the resident tensor."""
+    import torch
+    from integrated_path_planning_b200 import DeviceBatch, _lib
+    knobs = dict(scenarios.S1_KNOBS, dt=0.05, min_t=6.0, max_t=6.4, d_road_w=0.9, d_t_s=3.0)
+    rng = np.random.default_rng(41)
+    n = 1024
+    frenet = np.stack([rng.uniform(2, 15, n), rng.uniform(1, 7, n), rng.uniform(-1, 1, n), rng.uniform(-1, 1, n),
+                       rng.normal(0, 0.2, n), rng.normal(0, 0.05, n)], axis=1)
+    dyn = np.stack([scenarios.pedestrian_field(rng, 5, n_steps=129, dt=0.05) for _ in range(n)])
+    pl = _planner(knobs)
+    assert pl.engine.n_t_max > 128
+    batch = DeviceBatch(pl, frenet, 6.0, dyn[:, None], _lib.FOT_DYN_SINGLE)
+    batch.launch(None)
+    assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == 2
+    want = {k: v.cpu().numpy() for k, v in batch.out.items()}
+    assert len(set(want["best_idx"].tolist())) > 5
+
+    def agree(got, how):
+        for k, v in want.items():
+            assert _same(k, v, np.asarray(got[k]), want["winner_len"]), (how, k)
+
+    res = pl.plan_batch(frenet, 6.0, dynamic_obstacles=dyn, want_candidates=True)
+    assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == 2
+    agree({k: getattr(res, k) for k in want}, "plan_batch")
+    orc = _oracle(knobs)
+    _check(res, [orc.plan_frenet(tuple(frenet[i]), np.empty((0, 2)), dyn[i], 6.0) for i in range(3)])
+    with _env(FOT_HOST_CHUNKS=3):
+        res = pl.plan_batch(frenet, 6.0, dynamic_obstacles=dyn)
+    agree({k: getattr(res, k) for k in want}, "FOT_HOST_CHUNKS=3")
+    host = {k: torch.full(v.shape, -7, dtype=v.dtype).pin_memory() for k, v in batch.out.items()}
+    batch.launch_to_host(host)
+    agree({k: v.numpy() for k, v in host.items()}, "launch_to_host")

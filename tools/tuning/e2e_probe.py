@@ -1,5 +1,5 @@
 """End-to-end (host-pointer C-ABI) timing of the bench workload only: python tools/tuning/e2e_probe.py [queries] [reps]
-Environment knobs (FOT_HOST_CHUNKS) are read by the library per call."""
+Environment knobs (FOT_HOST_CHUNKS, ...) are resolved per handle; PROBE_VARIANTS switches them with reload_options()."""
 import os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
