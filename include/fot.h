@@ -27,12 +27,14 @@
 extern "C" {
 #endif
 
-#define FOT_ABI_VERSION 7   /* 2: + prediction post-processing and safety metrics; 3: + fot_plan_batch_device_to_host;
+#define FOT_ABI_VERSION 8   /* 2: + prediction post-processing and safety metrics; 3: + fot_plan_batch_device_to_host;
                                4: + fot_result_t.winner_samples, fot_fetch_winners, fot_reload_options;
                                5: + fot_set_result_mirror, fot_peer_* (gather of a sharded sweep over peer memory);
                                6: + fot_last_sweep_kind, fot_last_pair_features (fot_sweep_pairs is the default sweep kernel);
-                               7: + fot_nearest_s_device (nearest point on the path, certified against the host) */
+                               7: + fot_nearest_s_device (nearest point on the path, certified against the host);
+                               8: + fot_ranked_t, fot_rank_candidates (the k best feasible candidates per query) */
 #define FOT_MAX_CIRCLES 8
+#define FOT_MAX_RANKED 32
 #define FOT_N_STATS 8    /* ok, max_speed, max_accel, max_curvature, max_lat_accel, road_bound, collision, stop_distance */
 #define FOT_N_SERIES 15  /* t s s_d s_dd s_ddd d d_d d_dd d_ddd x y yaw c v a  (data_structures.py:149-181) */
 
@@ -156,6 +158,26 @@ int fot_candidate_count(const fot_handle_t* h, int n_v, int has_brake);
  * DEVICE pointers.  Asynchronous on `stream` (a cudaStream_t, NULL = the handle's own stream,
  * which is then synchronised before returning). */
 int fot_plan_batch_device(fot_handle_t* h, const fot_batch_t* batch, const fot_result_t* res, void* stream);
+
+/* ---- ranked alternatives (DESIGN.md section 4f) --------------------------------------------------------------------
+ * For query q the ranked list holds the candidates the winner selection could pick, best first: category FOT_CAT_OK
+ * after the stop-distance filter and a cost below +inf (a NaN cost never ranks, as it never wins), ordered by lower
+ * cost first and, on exactly equal cost, lower generation index first -- the reference's tie rule (first strict
+ * minimum, frenet_planner.py:1254-1257) extended to a ranking.  Rank 0 is therefore best_idx / best_cost of the same
+ * launch.  Ranks past the last such candidate are padded: idx -1, cost +inf, len 0 (their series rows are not
+ * written).  Series rows hold samples [0, N) of the candidate's N; the first len of them are what the reference keeps. */
+typedef struct fot_ranked {
+  int32_t  k;        /* 1 .. FOT_MAX_RANKED */
+  int32_t* idx;      /* [n_q][k] generation-order index, -1 = no further feasible candidate */
+  double*  cost;     /* [n_q][k] +inf where idx == -1 */
+  int32_t* len;      /* [n_q][k] samples kept after NaN-prefix truncation, or NULL */
+  double*  series;   /* [n_q][k][FOT_N_SERIES][n_t_max], or NULL (needs len) */
+} fot_ranked_t;
+/* The k best candidates of every query from the per-candidate table a fot_plan_batch_device launch of the same batch
+   wrote (cand_cat / cand_cost / cand_stride), with their 15 series regenerated as fot_winner does.  DEVICE pointers;
+   stream-ordered after that launch on `stream` (NULL: the handle's stream, synchronised). */
+int fot_rank_candidates(fot_handle_t* h, const fot_batch_t* batch, const uint8_t* cand_cat, const double* cand_cost,
+                        int cand_stride, const fot_ranked_t* out, void* stream);
 
 /* DEVICE inputs (`batch`), HOST results (`res`): for a caller whose obstacle tensor is produced on the GPU (the
  * entry points below) and whose winners are consumed on the host -- frenet_planner.py:271-294 for n_q queries

@@ -11,8 +11,9 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libfot.so")
 
-FOT_ABI_VERSION = 7
+FOT_ABI_VERSION = 8
 FOT_MAX_CIRCLES = 8
+FOT_MAX_RANKED = 32
 FOT_N_STATS = 8
 FOT_N_SERIES = 15
 FOT_DYN_NONE, FOT_DYN_SINGLE, FOT_DYN_DISTRIBUTION = 0, 1, 2
@@ -67,6 +68,12 @@ class FotResult(C.Structure):
     ]
 
 
+class FotRanked(C.Structure):
+    _fields_ = [
+        ("k", C.c_int32), ("idx", C.c_void_p), ("cost", C.c_void_p), ("len", C.c_void_p), ("series", C.c_void_p),
+    ]
+
+
 # every symbol include/fot.h declares: (name, restype, argtypes)
 SYMBOLS = (
     ("fot_abi_version", C.c_int, ()),
@@ -76,6 +83,8 @@ SYMBOLS = (
     ("fot_n_t_max", C.c_int, (C.c_void_p,)),
     ("fot_candidate_count", C.c_int, (C.c_void_p, C.c_int, C.c_int)),
     ("fot_plan_batch_device", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotResult), C.c_void_p)),
+    ("fot_rank_candidates", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.c_void_p, C.c_void_p, C.c_int,
+                                      C.POINTER(FotRanked), C.c_void_p)),
     ("fot_plan_batch_host", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotResult))),
     ("fot_plan_batch_device_to_host", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotResult), C.c_void_p)),
     ("fot_set_result_mirror", C.c_int, (C.c_void_p, C.POINTER(FotResult), C.c_void_p)),

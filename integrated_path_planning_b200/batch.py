@@ -29,11 +29,14 @@ class BatchFrenetPlanner(FrenetPlanner):
 
     def plan_batch(self, frenet_states, target_speed, dynamic_obstacles=None, distribution=None,
                    static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None,
-                   want_candidates: bool = False, winner_samples: int = 0) -> SweepResult:
+                   want_candidates: bool = False, winner_samples: int = 0, top_k: int = 0,
+                   rank_series: bool = True) -> SweepResult:
         """frenet_states [n_q,6]; target_speed scalar or [n_q]; dynamic_obstacles [n_q,P,T,2] or
         distribution [n_q,S,P,T,2]; static_obstacles [M,2] (shared) or [n_q,M,2]; limits [n_q,4]
         overrides constraint_overrides; max_stop_distance scalar / [n_q] (NaN = none); winner_samples = k > 0
-        reads back only the first k samples of each winner series (`engine.fetch_winners` for the rest)."""
+        reads back only the first k samples of each winner series (`engine.fetch_winners` for the rest).
+        top_k > 0: also the top_k best feasible candidates of every query (`SweepResult.rank_*`, `alternatives`),
+        with their series unless rank_series is False; the batch then runs as a device-resident `DeviceBatch`."""
         fs = np.asarray(frenet_states, dtype=np.float64).reshape(-1, 6)
         n_q = fs.shape[0]
         if limits is None:
@@ -45,6 +48,11 @@ class BatchFrenetPlanner(FrenetPlanner):
             d = np.asarray(dynamic_obstacles, dtype=np.float64)
             mode, dyn = _lib.FOT_DYN_SINGLE, d.reshape(n_q, 1, *d.shape[1:])
         per_query = static_obstacles is not None and np.ndim(static_obstacles) == 3
+        if top_k > 0:
+            db = DeviceBatch(self, fs, target_speed, dyn, mode, limits=limits, max_stop_distance=max_stop_distance,
+                             static_obstacles=static_obstacles, top_k=top_k, rank_series=rank_series)
+            db.launch()
+            return db.sweep_result(want_candidates, winner_samples)
         return self.engine.run_host(fs, target_speed, limits, max_stop_distance, static_obstacles, dyn, mode,
                                     static_per_query=per_query, want_candidates=want_candidates,
                                     winner_samples=winner_samples)
@@ -66,15 +74,23 @@ class BatchFrenetPlanner(FrenetPlanner):
         res = self.plan_batch(frenet, target_speed, **kwargs)
         bad = ~ok
         res.best_idx[bad], res.best_cost[bad], res.stats[bad], res.winner_len[bad] = -1, np.inf, 0, 0
+        if res.rank_idx is not None:
+            res.rank_idx[bad], res.rank_cost[bad] = -1, np.inf
+            if res.rank_len is not None:
+                res.rank_len[bad] = 0
         return res, ok
 
 
 class DeviceBatch:
     """A batch whose inputs and outputs live in torch CUDA tensors (buffers only): the timed
-    region of `bench.py`'s device-resident leg calls `launch()` and nothing else."""
+    region of `bench.py`'s device-resident leg calls `launch()` and nothing else.
+
+    top_k > 0: every launch also writes the per-candidate table and ranks it (fot_rank_candidates) into
+    out["rank_idx"] / out["rank_cost"] [n_q, top_k] and, with rank_series, out["rank_len"] [n_q, top_k] and
+    out["rank_series"] [n_q, top_k, 15, n_t_max]."""
 
     def __init__(self, planner: FrenetPlanner, frenet_states, target_speed, dyn, dyn_mode, limits=None,
-                 max_stop_distance=None, static_obstacles=None):
+                 max_stop_distance=None, static_obstacles=None, top_k: int = 0, rank_series: bool = True):
         import torch
         eng = planner.engine
         dev = torch.device("cuda", eng.device)
@@ -113,6 +129,25 @@ class DeviceBatch:
         r.best_idx, r.best_cost, r.stats = self.out["best_idx"].data_ptr(), self.out["best_cost"].data_ptr(), self.out["stats"].data_ptr()
         r.winner_len, r.winner = self.out["winner_len"].data_ptr(), self.out["winner"].data_ptr()
         self.result = r
+        self.top_k = int(top_k)
+        if self.top_k > 0:
+            if self.top_k > _lib.FOT_MAX_RANKED:
+                raise ValueError(f"top_k must be in [1, {_lib.FOT_MAX_RANKED}]")
+            stride = eng.lib.fot_candidate_count(eng._h, int(b.n_v_max), 1)
+            self.t["cand_cat"] = torch.empty((n_q, stride), dtype=torch.uint8, device=dev)
+            self.t["cand_cost"] = torch.empty((n_q, stride), dtype=torch.float64, device=dev)
+            r.cand_cat, r.cand_cost, r.cand_stride = self.t["cand_cat"].data_ptr(), self.t["cand_cost"].data_ptr(), stride
+            k = self.top_k
+            self.out = dict(self.out, rank_idx=torch.empty((n_q, k), dtype=torch.int32, device=dev),
+                            rank_cost=torch.empty((n_q, k), dtype=torch.float64, device=dev))
+            rk = _lib.FotRanked()
+            rk.k, rk.idx, rk.cost = k, self.out["rank_idx"].data_ptr(), self.out["rank_cost"].data_ptr()
+            if rank_series:
+                self.out["rank_len"] = torch.empty((n_q, k), dtype=torch.int32, device=dev)
+                self.out["rank_series"] = torch.empty((n_q, k, _lib.FOT_N_SERIES, eng.n_t_max), dtype=torch.float64,
+                                                      device=dev)
+                rk.len, rk.series = self.out["rank_len"].data_ptr(), self.out["rank_series"].data_ptr()
+            self.ranked = rk
 
     def launch(self, stream: Optional[int] = None) -> None:
         """Enqueue prepass + sweep + winner kernels on `stream` (raw cudaStream_t).  None: torch's current stream
@@ -121,10 +156,32 @@ class DeviceBatch:
         if stream is None:
             import torch
             cur = torch.cuda.current_stream(self.out["best_idx"].device)
-            self.engine.run_device(self.batch, self.result, cur.cuda_stream or None)
+            self._enqueue(cur.cuda_stream or None)
             cur.synchronize()
             return
+        self._enqueue(stream)
+
+    def _enqueue(self, stream) -> None:
         self.engine.run_device(self.batch, self.result, stream)
+        if self.top_k > 0:
+            r = self.result
+            self.engine.rank_device(self.batch, r.cand_cat, r.cand_cost, r.cand_stride, self.ranked, stream)
+
+    def sweep_result(self, want_candidates: bool = False, winner_samples: int = 0) -> SweepResult:
+        """Host copy of the outputs of the last launch, once it has finished (launch() without a stream waits), as a
+        SweepResult: the candidate table only with want_candidates, which needs top_k > 0; winner_samples = k > 0: the
+        first k samples of each winner series."""
+        h = {k: v.cpu().numpy() for k, v in self.out.items()}
+        if winner_samples and winner_samples > 0:
+            h["winner"] = np.ascontiguousarray(h["winner"][:, :, :min(int(winner_samples), h["winner"].shape[2])])
+        res = SweepResult(best_idx=h["best_idx"], best_cost=h["best_cost"], stats=h["stats"],
+                          winner_len=h["winner_len"], winner=h["winner"], rank_idx=h.get("rank_idx"),
+                          rank_cost=h.get("rank_cost"), rank_len=h.get("rank_len"), rank_series=h.get("rank_series"))
+        if want_candidates:
+            res.cand_cat, res.cand_cost = self.t["cand_cat"].cpu().numpy(), self.t["cand_cost"].cpu().numpy()
+        res.n_cand = self.engine.candidate_counts(self.frenet_host, self.n_v_host)
+        res.kernel_ms = self.engine.last_kernel_ms()
+        return res
 
     def launch_to_host(self, host_out: dict, stream: Optional[int] = None, winner_samples: int = 0) -> None:
         """fot_plan_batch_device_to_host: sweep the (device-resident) batch and deliver the winners into the host
@@ -132,7 +189,10 @@ class DeviceBatch:
         queries run in ranges and each range's winners are copied back while the next range is swept.  `stream`:
         the raw cudaStream_t on which the batch's inputs become ready (None: they are ready).  `winner_samples = k > 0`:
         only the first k samples of every winner series come back (`host_out["winner"]` is [n_q, 15, k]) -- what a
-        closed-loop caller consumes (integrated_simulator.py:663), 240 B instead of 6.1 KB per query at k = 2."""
+        closed-loop caller consumes (integrated_simulator.py:663), 240 B instead of 6.1 KB per query at k = 2.
+        Ranked outputs do not come back through this call: a batch with top_k > 0 raises ValueError."""
+        if self.top_k > 0:
+            raise ValueError("launch_to_host does not return ranked outputs; use launch() with top_k > 0")
         import ctypes as C
         ptr = lambda a: a.data_ptr() if hasattr(a, "data_ptr") else a.ctypes.data
         r = _lib.FotResult()

@@ -17,6 +17,7 @@
 #include "fot_sweep_pairs.cuh"
 #include "fot_predict.cuh"
 #include "fot_frenet.cuh"
+#include "fot_rank.cuh"
 
 using namespace fot;
 
@@ -715,6 +716,31 @@ extern "C" int fot_plan_batch_device(fot_handle_t* h, const fot_batch_t* b, cons
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
   rc = launch_all(h, b, r, st);
   if (rc != FOT_OK) return rc;
+  if (!stream) CK(cudaStreamSynchronize(st));
+  return FOT_OK;
+}
+
+extern "C" int fot_rank_candidates(fot_handle_t* h, const fot_batch_t* b, const uint8_t* cand_cat, const double* cand_cost,
+                                   int cand_stride, const fot_ranked_t* out, void* stream) {
+  if (!h || !b || !out || !cand_cat || !cand_cost) return fail(FOT_ERR_ARG, "fot_rank_candidates: null argument");
+  if (b->n_q < 1 || b->n_v_max < 1) return fail(FOT_ERR_ARG, "fot_rank_candidates: n_q and n_v_max must be >= 1");
+  if (out->k < 1 || out->k > FOT_MAX_RANKED) return fail(FOT_ERR_ARG, "fot_rank_candidates: k must be in [1, FOT_MAX_RANKED]");
+  if (!out->idx || !out->cost) return fail(FOT_ERR_ARG, "fot_rank_candidates: null idx or cost");
+  if (out->series && !out->len) return fail(FOT_ERR_ARG, "fot_rank_candidates: series needs len");
+  if (cand_stride < fot_candidate_count(h, b->n_v_max, 1)) return fail(FOT_ERR_ARG, "fot_rank_candidates: cand_stride too small");
+  if (out->len && (!b->frenet || !b->v_grid || !b->n_v)) return fail(FOT_ERR_ARG, "fot_rank_candidates: null query array");
+  if ((size_t)b->n_q * out->k > 0x7fffffffull) return fail(FOT_ERR_ARG, "fot_rank_candidates: batch too large for one launch");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  const Ranked R{out->k, out->idx, out->cost, out->len, out->series};
+  fot_rank<<<b->n_q, kRankThreads, 0, st>>>(cand_cat, cand_cost, cand_stride, R);
+  if (out->len) {
+    Batch B{};
+    B.n_q = b->n_q; B.n_v_max = b->n_v_max;
+    B.frenet = b->frenet; B.v_grid = b->v_grid; B.n_v = b->n_v;
+    fot_rank_series<<<(unsigned)((size_t)b->n_q * out->k), 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, R);
+  }
+  CK(cudaGetLastError());
   if (!stream) CK(cudaStreamSynchronize(st));
   return FOT_OK;
 }

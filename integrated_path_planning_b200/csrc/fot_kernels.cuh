@@ -771,6 +771,59 @@ fot_sweep(const Plan P, const Batch B, const Out O, const SweepGeom G) {
 }
 
 // ----------------------------------------------------------------------------------------
+// Regeneration of one candidate by a whole block, in the reference's arithmetic order: decode the generation-order
+// index i of query q (fp.py:398-449, brake ladder appended), solve its two profiles, convert every sample to Cartesian.
+// W (and MW, when not null) receive the [FOT_N_SERIES][NT] rows, samples [0, N); kStore false: nothing is stored, only
+// the length is found.  `tt` is the block's [NT][kTT] time table; *s_first_nan must hold 0x7fffffff and be visible to the
+// block on entry.  Returns to every thread the samples kept after the NaN-prefix truncation (first NaN x, else N).
+// ----------------------------------------------------------------------------------------
+template <bool kStore = true>
+__device__ __forceinline__ int regenerate(const Plan& P, const Batch& B, int q, int i, const double* tt, double* W,
+                                          double* MW, int* s_first_nan) {
+  const int NT = P.n_t_max, tid = threadIdx.x;
+  const double* fs = B.frenet + 6 * (size_t)q;
+  const int n_v = B.n_v[q], n_d = P.cfg.n_d;
+  const int grid_total = P.cfg.n_T * n_v * n_d;
+  Lon lon;
+  Lat lat;
+  int N;
+  if (i < grid_total) {
+    const int id = i % n_d, kv = (i / n_d) % n_v, jT = i / (n_d * n_v);
+    N = P.n_steps[jT] + 1;
+    lon = lon_solve(fs, B.v_grid[(size_t)q * B.n_v_max + kv], P.T[jT], P.inv4 + 4 * jT, n_v == 1, N - 1);
+    lat = lat_solve(fs, P.d_grid[id], P.T[jT], P.inv5 + 9 * jT, n_d == 1, N - 1);
+  } else {
+    const int bi = i - grid_total;
+    N = P.cfg.n_total;
+    lon = lon_solve(fs, 0.0, P.Tb[bi], P.inv4b + 4 * bi, true, P.n_steps_b[bi]);
+    lat = lat_solve(fs, fs[3], P.Tb[bi], P.inv5b + 9 * bi, true, P.n_steps_b[bi]);
+  }
+  for (int n = tid; n < N; n += blockDim.x) {
+    const double s = lon_p0(lon, tt, n), sd = lon_p1(lon, tt, n), sdd = lon_p2(lon, tt, n);
+    const double d = lat_p0(lat, tt, n), dd = lat_p1(lat, tt, n), ddd = lat_p2(lat, tt, n);
+    const RefPt r = spline_ref(P, s);
+    double sn, cs;
+    sincos(r.rth, &sn, &cs);
+    const CartPt cp = to_cartesian(r.rx, r.ry, cs, sn, r.rth, r.rk, r.rdk, sd, sdd, d, dd, ddd);
+    if (cp.x != cp.x) atomicMin(s_first_nan, n);
+    if (!kStore) continue;
+    W[0 * NT + n] = tt[kTT * n];
+    W[1 * NT + n] = s;   W[2 * NT + n] = sd;  W[3 * NT + n] = sdd; W[4 * NT + n] = lon_p3(lon, tt, n);
+    W[5 * NT + n] = d;   W[6 * NT + n] = dd;  W[7 * NT + n] = ddd; W[8 * NT + n] = lat_p3(lat, tt, n);
+    W[9 * NT + n] = cp.x; W[10 * NT + n] = cp.y; W[11 * NT + n] = wrap_angle(cp.ang);
+    W[12 * NT + n] = cp.kappa; W[13 * NT + n] = cp.v; W[14 * NT + n] = cp.a;
+    if (MW) {
+      // the same values into the mirror: plain stores, which the memory system carries over NVLink when the mirror is
+      // a peer's memory -- the gather of the sharded sweep happens here, without a collective call
+#pragma unroll
+      for (int r = 0; r < FOT_N_SERIES; ++r) MW[r * NT + n] = W[r * NT + n];
+    }
+  }
+  __syncthreads();
+  return *s_first_nan < N ? *s_first_nan : N;
+}
+
+// ----------------------------------------------------------------------------------------
 // Winner kernel: one block per query.
 // ----------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128)
@@ -810,49 +863,12 @@ fot_winner(const Plan P, const Batch B, const Out O, const SweepGeom G) {
     }
     return;
   }
-  const double* fs = B.frenet + 6 * (size_t)q;
-  const int n_v = B.n_v[q], n_d = P.cfg.n_d;
-  const int grid_total = P.cfg.n_T * n_v * n_d;
-  Lon lon;
-  Lat lat;
-  int N;
-  if (i < grid_total) {
-    const int id = i % n_d, kv = (i / n_d) % n_v, jT = i / (n_d * n_v);
-    N = P.n_steps[jT] + 1;
-    lon = lon_solve(fs, B.v_grid[(size_t)q * B.n_v_max + kv], P.T[jT], P.inv4 + 4 * jT, n_v == 1, N - 1);
-    lat = lat_solve(fs, P.d_grid[id], P.T[jT], P.inv5 + 9 * jT, n_d == 1, N - 1);
-  } else {
-    const int bi = i - grid_total;
-    N = P.cfg.n_total;
-    lon = lon_solve(fs, 0.0, P.Tb[bi], P.inv4b + 4 * bi, true, P.n_steps_b[bi]);
-    lat = lat_solve(fs, fs[3], P.Tb[bi], P.inv5b + 9 * bi, true, P.n_steps_b[bi]);
-  }
-  for (int n = tid; n < N; n += blockDim.x) {
-    const double s = lon_p0(lon, tt, n), sd = lon_p1(lon, tt, n), sdd = lon_p2(lon, tt, n);
-    const double d = lat_p0(lat, tt, n), dd = lat_p1(lat, tt, n), ddd = lat_p2(lat, tt, n);
-    const RefPt r = spline_ref(P, s);
-    double sn, cs;
-    sincos(r.rth, &sn, &cs);
-    const CartPt cp = to_cartesian(r.rx, r.ry, cs, sn, r.rth, r.rk, r.rdk, sd, sdd, d, dd, ddd);
-    if (cp.x != cp.x) atomicMin(&s_first_nan, n);
-    W[0 * NT + n] = tt[kTT * n];
-    W[1 * NT + n] = s;   W[2 * NT + n] = sd;  W[3 * NT + n] = sdd; W[4 * NT + n] = lon_p3(lon, tt, n);
-    W[5 * NT + n] = d;   W[6 * NT + n] = dd;  W[7 * NT + n] = ddd; W[8 * NT + n] = lat_p3(lat, tt, n);
-    W[9 * NT + n] = cp.x; W[10 * NT + n] = cp.y; W[11 * NT + n] = wrap_angle(cp.ang);
-    W[12 * NT + n] = cp.kappa; W[13 * NT + n] = cp.v; W[14 * NT + n] = cp.a;
-    if (MW) {
-      // the same values into the mirror: plain stores, which the memory system carries over NVLink when the mirror is
-      // a peer's memory -- the gather of the sharded sweep happens here, without a collective call
-#pragma unroll
-      for (int r = 0; r < FOT_N_SERIES; ++r) MW[r * NT + n] = W[r * NT + n];
-    }
-  }
-  __syncthreads();
+  const int len = regenerate(P, B, q, i, tt, W, MW, &s_first_nan);
   if (tid == 0) {
     O.best_idx[q] = i;
     O.best_cost[q] = c;
-    O.winner_len[q] = s_first_nan < N ? s_first_nan : N;
-    if (O.m_best_idx) { O.m_best_idx[q] = i; O.m_best_cost[q] = c; O.m_winner_len[q] = s_first_nan < N ? s_first_nan : N; }
+    O.winner_len[q] = len;
+    if (O.m_best_idx) { O.m_best_idx[q] = i; O.m_best_cost[q] = c; O.m_winner_len[q] = len; }
   }
 }
 

@@ -96,6 +96,12 @@ class SweepResult:
     cand_cost: Optional[np.ndarray] = None   # [n_q, stride]
     n_cand: Optional[np.ndarray] = None      # [n_q] candidates generated per query
     kernel_ms: float = float("nan")
+    # ranked alternatives (top_k > 0; include/fot.h fot_ranked_t): rank 0 is the winner, -1 / inf / 0 pad the ranks
+    # past the last feasible candidate
+    rank_idx: Optional[np.ndarray] = None     # [n_q, k] int32
+    rank_cost: Optional[np.ndarray] = None    # [n_q, k]
+    rank_len: Optional[np.ndarray] = None     # [n_q, k] int32, or None without series
+    rank_series: Optional[np.ndarray] = None  # [n_q, k, 15, n_t_max], or None
 
     def series(self, q: int = 0):
         """The 15 winner sequences of query q truncated to their kept length, or None."""
@@ -103,6 +109,21 @@ class SweepResult:
             return None
         n = min(int(self.winner_len[q]), self.winner.shape[2])      # winner_samples = k: the first k samples only
         return {name: self.winner[q, j, :n].copy() for j, name in enumerate(SERIES)}
+
+    def alternatives(self, q: int = 0):
+        """The ranked alternatives of query q, best first: a list of {"index", "cost", "series"}, where series holds
+        the 15 sequences truncated to their kept length (None when the series were not requested)."""
+        out = []
+        for r in range(self.rank_idx.shape[1]):
+            i = int(self.rank_idx[q, r])
+            if i < 0:
+                break
+            series = None
+            if self.rank_series is not None:
+                n = int(self.rank_len[q, r])
+                series = {name: self.rank_series[q, r, j, :n].copy() for j, name in enumerate(SERIES)}
+            out.append({"index": i, "cost": np.float64(self.rank_cost[q, r]), "series": series})
+        return out
 
 
 class SweepEngine:
@@ -284,6 +305,14 @@ class SweepEngine:
         _lib.check(self.lib.fot_plan_batch_device(self._h, C.byref(batch), C.byref(result),
                                                   C.c_void_p(stream) if stream else None),
                    "fot_plan_batch_device")
+
+    def rank_device(self, batch: "_lib.FotBatch", cand_cat: int, cand_cost: int, cand_stride: int,
+                    ranked: "_lib.FotRanked", stream=None) -> None:
+        """fot_rank_candidates on the per-candidate table of a fot_plan_batch_device launch of `batch` (device
+        pointers), stream-ordered behind it."""
+        _lib.check(self.lib.fot_rank_candidates(self._h, C.byref(batch), C.c_void_p(cand_cat), C.c_void_p(cand_cost),
+                                                int(cand_stride), C.byref(ranked), C.c_void_p(stream) if stream else None),
+                   "fot_rank_candidates")
 
     def nearest_s(self, x, y, prev_s):
         """fot_nearest_s_device for m points on this engine's path: returns (s [m], status [m] int32), status 0 where

@@ -14,7 +14,7 @@ There is no CPU path for the sweep: without libfot.so or a CUDA device `plan()` 
 from __future__ import annotations
 
 import os
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 
 import numpy as np
 
@@ -50,6 +50,16 @@ _REF_STAT_ORDER = ("max_speed_error", "max_accel_error", "max_curvature_error", 
 
 def _default_device() -> int:
     return int(os.environ.get("LOCAL_RANK", "0"))
+
+
+def _frenet_path(series, cost) -> FrenetPath:
+    """A FrenetPath from the 15 sequences of one candidate, as the reference returns it (frenet_planner.py:294)."""
+    path = FrenetPath(cost=np.float64(cost))
+    for name in SERIES[:9]:
+        setattr(path, name, series[name])
+    for name in SERIES[9:]:
+        setattr(path, name, series[name].tolist())
+    return path
 
 
 def classify_dynamic(dynamic_obstacles, distribution):
@@ -146,33 +156,70 @@ class FrenetPlanner:
                                      constraint_overrides, dynamic_obstacles_distribution, max_stop_distance,
                                      _want_candidates)
 
+    def plan_alternatives(self, ego_state, static_obstacles, dynamic_obstacles=None,
+                          target_speed: float = TARGET_SPEED, constraint_overrides: Optional[Dict[str, float]] = None,
+                          dynamic_obstacles_distribution=None, max_stop_distance: Optional[float] = None,
+                          k: int = 5) -> List[FrenetPath]:
+        """The k best feasible trajectories from the current ego state, best first (fewer when fewer are feasible):
+        a fallback when the first choice is vetoed downstream.  Element 0 is what plan() returns, and the list is
+        empty where plan() returns None.  Side effects are plan()'s: last_check_stats, the nearest-point cache and
+        the curvature fed back from element 0.  Ranking: lower cost first, equal costs in generation order
+        (include/fot.h, fot_ranked_t)."""
+        if not 1 <= int(k) <= _lib.FOT_MAX_RANKED:
+            raise ValueError(f"k must be in [1, {_lib.FOT_MAX_RANKED}]")
+        self.last_check_stats = None
+        self.last_result = None
+        fs = self._cartesian_to_frenet_state(ego_state)
+        if fs is None:
+            return []
+        res = self._sweep(fs.to_array(), static_obstacles, dynamic_obstacles, target_speed, constraint_overrides,
+                          dynamic_obstacles_distribution, max_stop_distance, top_k=int(k))
+        paths = [_frenet_path(a["series"], a["cost"]) for a in res.alternatives(0)]
+        if paths:
+            self._feed_back_curvature(paths[0])
+        return paths
+
     def plan_from_frenet(self, frenet_state, static_obstacles, dynamic_obstacles=None,
                          target_speed: float = TARGET_SPEED, constraint_overrides=None,
                          dynamic_obstacles_distribution=None, max_stop_distance=None,
                          _want_candidates: bool = False) -> Optional[FrenetPath]:
         """frenet_planner.py:271-304 for a given Frenet state [s, s_d, s_dd, d, d_d, d_dd]."""
+        res = self._sweep(frenet_state, static_obstacles, dynamic_obstacles, target_speed, constraint_overrides,
+                          dynamic_obstacles_distribution, max_stop_distance, want_candidates=_want_candidates)
+        series = res.series(0)
+        if series is None:
+            return None
+        return self._feed_back_curvature(_frenet_path(series, res.best_cost[0]))
+
+    def _sweep(self, frenet_state, static_obstacles, dynamic_obstacles, target_speed, constraint_overrides,
+               dynamic_obstacles_distribution, max_stop_distance, want_candidates: bool = False,
+               top_k: int = 0) -> SweepResult:
+        """One query through the sweep (ranked when top_k > 0); sets last_result and last_check_stats."""
         mode, dyn = classify_dynamic(dynamic_obstacles, dynamic_obstacles_distribution)
         static = None
         if static_obstacles is not None and len(static_obstacles) > 0:
             static = np.asarray(static_obstacles, dtype=np.float64).reshape(-1, 2)
         stop = np.nan if max_stop_distance is None else float(max_stop_distance)
-        res = self.engine.run_host(
-            np.asarray(frenet_state, dtype=np.float64).reshape(1, 6), float(target_speed),
-            self.resolve_limits(constraint_overrides), stop, static, dyn, mode,
-            want_candidates=_want_candidates)
+        frenet = np.asarray(frenet_state, dtype=np.float64).reshape(1, 6)
+        limits = self.resolve_limits(constraint_overrides)
+        if top_k > 0:
+            from .batch import DeviceBatch           # batch.py builds on this module
+            db = DeviceBatch(self, frenet, float(target_speed), dyn, mode, limits=limits, max_stop_distance=stop,
+                             static_obstacles=static, top_k=top_k)
+            db.launch()
+            res = db.sweep_result(want_candidates)
+        else:
+            res = self.engine.run_host(frenet, float(target_speed), limits, stop, static, dyn, mode,
+                                       want_candidates=want_candidates)
         self.last_result = res
         stats = {key: int(res.stats[0, _lib.STAT_KEYS.index(key)]) for key in _REF_STAT_ORDER}
         if max_stop_distance is not None:
             stats["stop_distance_error"] = int(res.stats[0, _lib.STAT_KEYS.index("stop_distance_error")])
         self.last_check_stats = stats
-        series = res.series(0)
-        if series is None:
-            return None
-        path = FrenetPath(cost=np.float64(res.best_cost[0]))
-        for name in SERIES[:9]:
-            setattr(path, name, series[name])
-        for name in SERIES[9:]:
-            setattr(path, name, series[name].tolist())
+        return res
+
+    def _feed_back_curvature(self, path: FrenetPath) -> FrenetPath:
+        """The ego curvature the next call starts from (frenet_planner.py:301-302)."""
         if len(path.c) > 1:
             self._last_kappa = float(path.c[1])
         return path
