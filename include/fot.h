@@ -33,6 +33,10 @@ extern "C" {
                                6: + fot_last_sweep_kind, fot_last_pair_features (fot_sweep_pairs is the default sweep kernel);
                                7: + fot_nearest_s_device (nearest point on the path, certified against the host);
                                8: + fot_ranked_t, fot_rank_candidates (the k best feasible candidates per query) */
+#define FOT_ABI_MINOR 1     /* additions within a version that change no existing struct, entry point or behaviour, so a
+                               caller built against an earlier minor of the same version keeps working; 0 at each new
+                               version.  Version 8: 1: + fot_weighted_t, fot_select_weighted, fot_cost_terms (winners
+                               under many cost weightings, the five cost terms per candidate) */
 #define FOT_MAX_CIRCLES 8
 #define FOT_MAX_RANKED 32
 #define FOT_N_STATS 8    /* ok, max_speed, max_accel, max_curvature, max_lat_accel, road_bound, collision, stop_distance */
@@ -139,8 +143,9 @@ typedef struct fot_result {
  * caller (handles are cheap: < 1 MB plus scratch that grows with the batch). */
 typedef struct fot_handle fot_handle_t;
 
-/* ABI version of the loaded library. */
+/* ABI version of the loaded library, and its minor revision within that version (FOT_ABI_MINOR). */
 int fot_abi_version(void);
+int fot_abi_minor(void);
 /* Human-readable text of the last error on this thread. */
 const char* fot_last_error(void);
 
@@ -178,6 +183,39 @@ typedef struct fot_ranked {
    stream-ordered after that launch on `stream` (NULL: the handle's stream, synchronised). */
 int fot_rank_candidates(fot_handle_t* h, const fot_batch_t* batch, const uint8_t* cand_cat, const double* cand_cost,
                         int cand_stride, const fot_ranked_t* out, void* stream);
+
+/* ---- cost-weight sweeps (DESIGN.md section 4g) ---------------------------------------------------------------------
+ * No cost weight affects a candidate's category; the weights enter only the cost, a fixed expression of five
+ * per-candidate terms (frenet_planner.py:703-734):
+ *   lat = k_j*Jp + k_t*Jt + k_d*Jd      Jp = sum d'''^2, Jd = d_end^2
+ *   lon = k_j*Js + k_t*Jt + k_s_dot*Jv  Js = sum s'''^2, Jv = (target_speed - s_d[-1])^2, Jt = t[-1]
+ *   cost_w = k_lat*lat + k_lon*lon
+ * evaluated left to right, every product and sum rounded on its own (no contraction).  For query q and weighting
+ * w = (k_j, k_t, k_d, k_s_dot, k_lat, k_lon) the selected candidate is the one a planner created with w returns for the
+ * same inputs: among the candidates whose table category is FOT_CAT_OK, the smallest cost_w below +inf, and on exactly
+ * equal cost the lower generation index (first strict minimum, frenet_planner.py:1254-1257).  A NaN or infinite cost_w
+ * never wins, so a NaN weight gives no winner.  No winner: idx -1, cost +inf, len 0, series row not written.  For w
+ * equal to the handle's own weights the selection is best_idx / best_cost / winner of the same launch. */
+#define FOT_MAX_WEIGHT_SETS 256
+typedef struct fot_weighted {
+  int32_t n_w;              /* 1 .. FOT_MAX_WEIGHT_SETS */
+  int32_t per_query;        /* 0: one list of n_w weightings for every query; 1: a list per query */
+  const double* weights;    /* [(n_q | 1)][n_w][6]  k_j k_t k_d k_s_dot k_lat k_lon */
+  int32_t* idx;             /* [n_q][n_w]  generation-order index, -1 = no candidate */
+  double*  cost;            /* [n_q][n_w]  +inf where idx == -1 */
+  int32_t* len;             /* [n_q][n_w] samples kept after NaN-prefix truncation, or NULL */
+  double*  series;          /* [n_q][n_w][FOT_N_SERIES][n_t_max], or NULL (needs len) */
+} fot_weighted_t;
+/* The winner of every query under each of n_w weightings, from the per-candidate table (cand_cat, cand_stride) a
+   fot_plan_batch_device launch of the same batch wrote, with the winners' series regenerated as fot_winner does.
+   DEVICE pointers; stream-ordered after that launch on `stream` (NULL: the handle's stream, synchronised). */
+int fot_select_weighted(fot_handle_t* h, const fot_batch_t* batch, const uint8_t* cand_cat, int cand_stride,
+                        const fot_weighted_t* out, void* stream);
+/* The five cost terms of every generated candidate, for cost learning: terms[n_q][cand_stride][5] = (Jp, Jd, Js, Jv, Jt)
+   as above, NaN past the query's candidates (fot_candidate_count).  Every candidate has its terms whatever its category
+   (the reference computes the cost before the checks).  Needs only the batch's frenet, target_speed, v_grid and n_v;
+   no sweep.  DEVICE pointers; asynchronous on `stream` (NULL: the handle's stream, synchronised). */
+int fot_cost_terms(fot_handle_t* h, const fot_batch_t* batch, int cand_stride, double* terms, void* stream);
 
 /* DEVICE inputs (`batch`), HOST results (`res`): for a caller whose obstacle tensor is produced on the GPU (the
  * entry points below) and whose winners are consumed on the host -- frenet_planner.py:271-294 for n_q queries

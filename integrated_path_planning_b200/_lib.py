@@ -12,8 +12,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libfot.so")
 
 FOT_ABI_VERSION = 8
+FOT_ABI_MINOR = 1
 FOT_MAX_CIRCLES = 8
 FOT_MAX_RANKED = 32
+FOT_MAX_WEIGHT_SETS = 256
 FOT_N_STATS = 8
 FOT_N_SERIES = 15
 FOT_DYN_NONE, FOT_DYN_SINGLE, FOT_DYN_DISTRIBUTION = 0, 1, 2
@@ -21,6 +23,8 @@ CAT_OK, CAT_SPEED, CAT_ACCEL, CAT_CURV, CAT_LAT, CAT_ROAD, CAT_COLL, CAT_STOP, C
 # last_check_stats keys in the slot order of fot_result_t.stats (frenet_planner.py:910-918, :324)
 STAT_KEYS = ("ok", "max_speed_error", "max_accel_error", "max_curvature_error", "max_lat_accel_error",
              "road_bound_error", "collision_error", "stop_distance_error")
+# the six cost weights in the order of fot_weighted_t.weights (frenet_planner.py:187-192)
+COST_WEIGHT_KEYS = ("k_j", "k_t", "k_d", "k_s_dot", "k_lat", "k_lon")
 
 c_double_p = C.POINTER(C.c_double)
 c_int32_p = C.POINTER(C.c_int32)
@@ -74,9 +78,17 @@ class FotRanked(C.Structure):
     ]
 
 
+class FotWeighted(C.Structure):
+    _fields_ = [
+        ("n_w", C.c_int32), ("per_query", C.c_int32), ("weights", C.c_void_p), ("idx", C.c_void_p),
+        ("cost", C.c_void_p), ("len", C.c_void_p), ("series", C.c_void_p),
+    ]
+
+
 # every symbol include/fot.h declares: (name, restype, argtypes)
 SYMBOLS = (
     ("fot_abi_version", C.c_int, ()),
+    ("fot_abi_minor", C.c_int, ()),
     ("fot_last_error", C.c_char_p, ()),
     ("fot_create", C.c_int, (C.POINTER(FotConfig), C.POINTER(FotTables), C.c_int, C.POINTER(C.c_void_p))),
     ("fot_destroy", C.c_int, (C.c_void_p,)),
@@ -85,6 +97,9 @@ SYMBOLS = (
     ("fot_plan_batch_device", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotResult), C.c_void_p)),
     ("fot_rank_candidates", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.c_void_p, C.c_void_p, C.c_int,
                                       C.POINTER(FotRanked), C.c_void_p)),
+    ("fot_select_weighted", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.c_void_p, C.c_int, C.POINTER(FotWeighted),
+                                      C.c_void_p)),
+    ("fot_cost_terms", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.c_int, C.c_void_p, C.c_void_p)),
     ("fot_plan_batch_host", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotResult))),
     ("fot_plan_batch_device_to_host", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotResult), C.c_void_p)),
     ("fot_set_result_mirror", C.c_int, (C.c_void_p, C.POINTER(FotResult), C.c_void_p)),
@@ -134,10 +149,13 @@ def load() -> C.CDLL:
             "there is no CPU fallback.")
     lib = C.CDLL(LIB_PATH)
     for name, restype, argtypes in SYMBOLS:
-        fn = getattr(lib, name)
+        try:
+            fn = getattr(lib, name)
+        except AttributeError:
+            raise FotError(f"libfot.so lacks {name} (built from older sources); rebuild") from None
         fn.restype = restype
         fn.argtypes = list(argtypes)
-    if lib.fot_abi_version() != FOT_ABI_VERSION:
+    if lib.fot_abi_version() != FOT_ABI_VERSION or lib.fot_abi_minor() != FOT_ABI_MINOR:
         raise FotError("libfot.so ABI version mismatch; rebuild")
     _lib = lib
     return lib

@@ -30,13 +30,17 @@ class BatchFrenetPlanner(FrenetPlanner):
     def plan_batch(self, frenet_states, target_speed, dynamic_obstacles=None, distribution=None,
                    static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None,
                    want_candidates: bool = False, winner_samples: int = 0, top_k: int = 0,
-                   rank_series: bool = True) -> SweepResult:
+                   rank_series: bool = True, cost_weights=None, weight_series: bool = True,
+                   cost_terms: bool = False) -> SweepResult:
         """frenet_states [n_q,6]; target_speed scalar or [n_q]; dynamic_obstacles [n_q,P,T,2] or
         distribution [n_q,S,P,T,2]; static_obstacles [M,2] (shared) or [n_q,M,2]; limits [n_q,4]
         overrides constraint_overrides; max_stop_distance scalar / [n_q] (NaN = none); winner_samples = k > 0
         reads back only the first k samples of each winner series (`engine.fetch_winners` for the rest).
         top_k > 0: also the top_k best feasible candidates of every query (`SweepResult.rank_*`, `alternatives`),
-        with their series unless rank_series is False; the batch then runs as a device-resident `DeviceBatch`."""
+        with their series unless rank_series is False.  cost_weights [n_w,6] (every query) or [n_q,n_w,6] (columns
+        _lib.COST_WEIGHT_KEYS): also every query's winner under each weighting (`SweepResult.w_*`, `under_weights`),
+        with its series unless weight_series is False.  cost_terms: also the five cost terms of every candidate
+        (`SweepResult.cost_terms`).  With any of these the batch runs as a device-resident `DeviceBatch`."""
         fs = np.asarray(frenet_states, dtype=np.float64).reshape(-1, 6)
         n_q = fs.shape[0]
         if limits is None:
@@ -48,9 +52,10 @@ class BatchFrenetPlanner(FrenetPlanner):
             d = np.asarray(dynamic_obstacles, dtype=np.float64)
             mode, dyn = _lib.FOT_DYN_SINGLE, d.reshape(n_q, 1, *d.shape[1:])
         per_query = static_obstacles is not None and np.ndim(static_obstacles) == 3
-        if top_k > 0:
+        if top_k > 0 or cost_weights is not None or cost_terms:
             db = DeviceBatch(self, fs, target_speed, dyn, mode, limits=limits, max_stop_distance=max_stop_distance,
-                             static_obstacles=static_obstacles, top_k=top_k, rank_series=rank_series)
+                             static_obstacles=static_obstacles, top_k=top_k, rank_series=rank_series,
+                             cost_weights=cost_weights, weight_series=weight_series, cost_terms=cost_terms)
             db.launch()
             return db.sweep_result(want_candidates, winner_samples)
         return self.engine.run_host(fs, target_speed, limits, max_stop_distance, static_obstacles, dyn, mode,
@@ -78,6 +83,12 @@ class BatchFrenetPlanner(FrenetPlanner):
             res.rank_idx[bad], res.rank_cost[bad] = -1, np.inf
             if res.rank_len is not None:
                 res.rank_len[bad] = 0
+        if res.w_idx is not None:
+            res.w_idx[bad], res.w_cost[bad] = -1, np.inf
+            if res.w_len is not None:
+                res.w_len[bad] = 0
+        if res.cost_terms is not None:
+            res.cost_terms[bad] = np.nan
         return res, ok
 
 
@@ -87,10 +98,17 @@ class DeviceBatch:
 
     top_k > 0: every launch also writes the per-candidate table and ranks it (fot_rank_candidates) into
     out["rank_idx"] / out["rank_cost"] [n_q, top_k] and, with rank_series, out["rank_len"] [n_q, top_k] and
-    out["rank_series"] [n_q, top_k, 15, n_t_max]."""
+    out["rank_series"] [n_q, top_k, 15, n_t_max].
+
+    cost_weights [n_w, 6] (every query) or [n_q, n_w, 6] (a list per query), columns _lib.COST_WEIGHT_KEYS: every
+    launch also writes the per-candidate categories (shared with top_k) and selects each query's winner under every
+    weighting (fot_select_weighted) into out["w_idx"] / out["w_cost"] [n_q, n_w] and, with weight_series,
+    out["w_len"] [n_q, n_w] and out["w_series"] [n_q, n_w, 15, n_t_max].  cost_terms: out["cost_terms"]
+    [n_q, stride, 5] = (Jp, Jd, Js, Jv, Jt) of every candidate (fot_cost_terms)."""
 
     def __init__(self, planner: FrenetPlanner, frenet_states, target_speed, dyn, dyn_mode, limits=None,
-                 max_stop_distance=None, static_obstacles=None, top_k: int = 0, rank_series: bool = True):
+                 max_stop_distance=None, static_obstacles=None, top_k: int = 0, rank_series: bool = True,
+                 cost_weights=None, weight_series: bool = True, cost_terms: bool = False):
         import torch
         eng = planner.engine
         dev = torch.device("cuda", eng.device)
@@ -130,13 +148,17 @@ class DeviceBatch:
         r.winner_len, r.winner = self.out["winner_len"].data_ptr(), self.out["winner"].data_ptr()
         self.result = r
         self.top_k = int(top_k)
+        if self.top_k > _lib.FOT_MAX_RANKED:
+            raise ValueError(f"top_k must be in [1, {_lib.FOT_MAX_RANKED}]")
+        weights, per_query = _weight_table(cost_weights, n_q)
+        self.n_w = 0 if weights is None else weights.shape[-2]
+        self.stride = eng.lib.fot_candidate_count(eng._h, int(b.n_v_max), 1)
+        if self.top_k > 0 or self.n_w > 0:
+            self.t["cand_cat"] = torch.empty((n_q, self.stride), dtype=torch.uint8, device=dev)
+            r.cand_cat, r.cand_stride = self.t["cand_cat"].data_ptr(), self.stride
         if self.top_k > 0:
-            if self.top_k > _lib.FOT_MAX_RANKED:
-                raise ValueError(f"top_k must be in [1, {_lib.FOT_MAX_RANKED}]")
-            stride = eng.lib.fot_candidate_count(eng._h, int(b.n_v_max), 1)
-            self.t["cand_cat"] = torch.empty((n_q, stride), dtype=torch.uint8, device=dev)
-            self.t["cand_cost"] = torch.empty((n_q, stride), dtype=torch.float64, device=dev)
-            r.cand_cat, r.cand_cost, r.cand_stride = self.t["cand_cat"].data_ptr(), self.t["cand_cost"].data_ptr(), stride
+            self.t["cand_cost"] = torch.empty((n_q, self.stride), dtype=torch.float64, device=dev)
+            r.cand_cost = self.t["cand_cost"].data_ptr()
             k = self.top_k
             self.out = dict(self.out, rank_idx=torch.empty((n_q, k), dtype=torch.int32, device=dev),
                             rank_cost=torch.empty((n_q, k), dtype=torch.float64, device=dev))
@@ -148,6 +170,23 @@ class DeviceBatch:
                                                       device=dev)
                 rk.len, rk.series = self.out["rank_len"].data_ptr(), self.out["rank_series"].data_ptr()
             self.ranked = rk
+        if self.n_w > 0:
+            n_w = self.n_w
+            self.t["weights"] = up(weights)
+            self.out = dict(self.out, w_idx=torch.empty((n_q, n_w), dtype=torch.int32, device=dev),
+                            w_cost=torch.empty((n_q, n_w), dtype=torch.float64, device=dev))
+            wt = _lib.FotWeighted()
+            wt.n_w, wt.per_query, wt.weights = n_w, per_query, self.t["weights"].data_ptr()
+            wt.idx, wt.cost = self.out["w_idx"].data_ptr(), self.out["w_cost"].data_ptr()
+            if weight_series:
+                self.out["w_len"] = torch.empty((n_q, n_w), dtype=torch.int32, device=dev)
+                self.out["w_series"] = torch.empty((n_q, n_w, _lib.FOT_N_SERIES, eng.n_t_max), dtype=torch.float64,
+                                                   device=dev)
+                wt.len, wt.series = self.out["w_len"].data_ptr(), self.out["w_series"].data_ptr()
+            self.weighted = wt
+        self.cost_terms = bool(cost_terms)
+        if self.cost_terms:
+            self.out = dict(self.out, cost_terms=torch.empty((n_q, self.stride, 5), dtype=torch.float64, device=dev))
 
     def launch(self, stream: Optional[int] = None) -> None:
         """Enqueue prepass + sweep + winner kernels on `stream` (raw cudaStream_t).  None: torch's current stream
@@ -166,19 +205,26 @@ class DeviceBatch:
         if self.top_k > 0:
             r = self.result
             self.engine.rank_device(self.batch, r.cand_cat, r.cand_cost, r.cand_stride, self.ranked, stream)
+        if self.n_w > 0:
+            self.engine.select_weighted_device(self.batch, self.result.cand_cat, self.stride, self.weighted, stream)
+        if self.cost_terms:
+            self.engine.cost_terms_device(self.batch, self.stride, self.out["cost_terms"].data_ptr(), stream)
 
     def sweep_result(self, want_candidates: bool = False, winner_samples: int = 0) -> SweepResult:
         """Host copy of the outputs of the last launch, once it has finished (launch() without a stream waits), as a
-        SweepResult: the candidate table only with want_candidates, which needs top_k > 0; winner_samples = k > 0: the
-        first k samples of each winner series."""
+        SweepResult: the candidate table only with want_candidates, which needs top_k > 0 (or cost_weights, for the
+        categories alone); winner_samples = k > 0: the first k samples of each winner series."""
         h = {k: v.cpu().numpy() for k, v in self.out.items()}
         if winner_samples and winner_samples > 0:
             h["winner"] = np.ascontiguousarray(h["winner"][:, :, :min(int(winner_samples), h["winner"].shape[2])])
         res = SweepResult(best_idx=h["best_idx"], best_cost=h["best_cost"], stats=h["stats"],
                           winner_len=h["winner_len"], winner=h["winner"], rank_idx=h.get("rank_idx"),
-                          rank_cost=h.get("rank_cost"), rank_len=h.get("rank_len"), rank_series=h.get("rank_series"))
+                          rank_cost=h.get("rank_cost"), rank_len=h.get("rank_len"), rank_series=h.get("rank_series"),
+                          w_idx=h.get("w_idx"), w_cost=h.get("w_cost"), w_len=h.get("w_len"),
+                          w_series=h.get("w_series"), cost_terms=h.get("cost_terms"))
         if want_candidates:
-            res.cand_cat, res.cand_cost = self.t["cand_cat"].cpu().numpy(), self.t["cand_cost"].cpu().numpy()
+            res.cand_cat = self.t["cand_cat"].cpu().numpy()
+            res.cand_cost = self.t["cand_cost"].cpu().numpy() if "cand_cost" in self.t else None
         res.n_cand = self.engine.candidate_counts(self.frenet_host, self.n_v_host)
         res.kernel_ms = self.engine.last_kernel_ms()
         return res
@@ -190,9 +236,12 @@ class DeviceBatch:
         the raw cudaStream_t on which the batch's inputs become ready (None: they are ready).  `winner_samples = k > 0`:
         only the first k samples of every winner series come back (`host_out["winner"]` is [n_q, 15, k]) -- what a
         closed-loop caller consumes (integrated_simulator.py:663), 240 B instead of 6.1 KB per query at k = 2.
-        Ranked outputs do not come back through this call: a batch with top_k > 0 raises ValueError."""
+        Ranked and weighted outputs do not come back through this call: a batch with top_k > 0, cost_weights or
+        cost_terms raises ValueError."""
         if self.top_k > 0:
             raise ValueError("launch_to_host does not return ranked outputs; use launch() with top_k > 0")
+        if self.n_w > 0 or self.cost_terms:
+            raise ValueError("launch_to_host does not return weighted outputs or cost terms; use launch()")
         import ctypes as C
         ptr = lambda a: a.data_ptr() if hasattr(a, "data_ptr") else a.ctypes.data
         r = _lib.FotResult()
@@ -209,6 +258,25 @@ class DeviceBatch:
         n_circ = max(1, self.engine.n_circles)
         per_point = self.batch.S * self.batch.P + self.batch.n_static
         return int(pts.sum()) * n_circ * int(per_point)
+
+
+def _weight_table(cost_weights, n_q: int):
+    """cost_weights as a contiguous float64 array and its fot_weighted_t.per_query flag: [n_w, 6] -> 0 (one list for
+    every query), [n_q, n_w, 6] -> 1; None -> (None, 0).  Raises ValueError on any other shape or n_w outside
+    [1, FOT_MAX_WEIGHT_SETS]."""
+    if cost_weights is None:
+        return None, 0
+    w = np.ascontiguousarray(cost_weights, dtype=np.float64)
+    n_k = len(_lib.COST_WEIGHT_KEYS)
+    if w.ndim == 2 and w.shape[1] == n_k:
+        per_query = 0
+    elif w.ndim == 3 and w.shape[0] == n_q and w.shape[2] == n_k:
+        per_query = 1
+    else:
+        raise ValueError(f"cost_weights must be [n_w, {n_k}] or [n_q={n_q}, n_w, {n_k}], got {list(w.shape)}")
+    if not 1 <= w.shape[-2] <= _lib.FOT_MAX_WEIGHT_SETS:
+        raise ValueError(f"the number of weightings must be in [1, {_lib.FOT_MAX_WEIGHT_SETS}], got {w.shape[-2]}")
+    return w, per_query
 
 
 class WinnerBlock:

@@ -18,6 +18,7 @@
 #include "fot_predict.cuh"
 #include "fot_frenet.cuh"
 #include "fot_rank.cuh"
+#include "fot_weights.cuh"
 
 using namespace fot;
 
@@ -142,6 +143,7 @@ struct fot_handle {
   int smem_optin = 0;
   int sms = 148;                     // SM count of the device (block-per-CTA grouping, host chunk sizes)
   Buf obs_tm, obs_max2, stat_tm, stat_max2, part_cost, part_idx, dyn_box, cost_tab;   // device scratch
+  Buf w_pieces;                      // cost pieces of fot_select_weighted / fot_cost_terms (fot_weights.cuh)
   int last_pair_feat = -1;           // mode set (PAIR_*) of the fot_sweep_pairs instantiation of the last launch
   int last_sweep_kind = 0;           // 4: fot_sweep_pairs, 1: fot_sweep_items, 2: fot_sweep (generic)
   fot_result_t mirror{};             // fot_set_result_mirror: second destination of the winner block (all null: none)
@@ -154,6 +156,7 @@ struct fot_handle {
 };
 
 extern "C" int fot_abi_version(void) { return FOT_ABI_VERSION; }
+extern "C" int fot_abi_minor(void) { return FOT_ABI_MINOR; }
 extern "C" const char* fot_last_error(void) { return g_err.c_str(); }
 
 extern "C" int fot_create(const fot_config_t* cfg, const fot_tables_t* tb, int device, fot_handle_t** out) {
@@ -263,7 +266,7 @@ extern "C" int fot_destroy(fot_handle_t* h) {
   { std::lock_guard<std::mutex> lk(g_live_mu); g_live.erase(h); }
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();          // every stream of the handle (compute, priority, copy) is idle before its buffers go
-  for (Buf* b : {&h->gate_d, &h->gate_h, &h->obs_tm, &h->obs_max2, &h->stat_tm, &h->stat_max2, &h->part_cost, &h->part_idx, &h->dyn_box, &h->cost_tab, &h->stage_h, &h->stage_d, &h->out_d,
+  for (Buf* b : {&h->gate_d, &h->gate_h, &h->obs_tm, &h->obs_max2, &h->stat_tm, &h->stat_max2, &h->part_cost, &h->part_idx, &h->dyn_box, &h->cost_tab, &h->w_pieces, &h->stage_h, &h->stage_d, &h->out_d,
                  &h->dyn_d, &h->stat_d})
     b->release();
   if (h->tables_dev) cudaFree(h->tables_dev);
@@ -740,6 +743,69 @@ extern "C" int fot_rank_candidates(fot_handle_t* h, const fot_batch_t* b, const 
     B.frenet = b->frenet; B.v_grid = b->v_grid; B.n_v = b->n_v;
     fot_rank_series<<<(unsigned)((size_t)b->n_q * out->k), 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, R);
   }
+  CK(cudaGetLastError());
+  if (!stream) CK(cudaStreamSynchronize(st));
+  return FOT_OK;
+}
+
+// The query arrays the cost pieces read, as a Batch; and the pieces themselves into the handle's scratch, on `st`.
+static int weighted_pieces(fot_handle* h, const fot_batch_t* b, cudaStream_t st, Batch* B) {
+  *B = Batch{};
+  B->n_q = b->n_q; B->n_v_max = b->n_v_max;
+  B->frenet = b->frenet; B->target = b->target_speed; B->v_grid = b->v_grid; B->n_v = b->n_v;
+  const long long n_prof = (long long)b->n_q * piece_profiles(h->plan.cfg, b->n_v_max);
+  if ((n_prof + 255) / 256 > 0x7fffffffll) return fail(FOT_ERR_ARG, "batch too large for one launch");
+  CK(h->w_pieces.reserve((size_t)b->n_q * piece_stride(h->plan.cfg, b->n_v_max) * sizeof(double)));
+  fot_cost_pieces<<<(unsigned)((n_prof + 255) / 256), 256, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(
+      h->plan, *B, (double*)h->w_pieces.p);
+  return FOT_OK;
+}
+
+extern "C" int fot_select_weighted(fot_handle_t* h, const fot_batch_t* b, const uint8_t* cand_cat, int cand_stride,
+                                   const fot_weighted_t* out, void* stream) {
+  if (!h || !b || !out || !cand_cat) return fail(FOT_ERR_ARG, "fot_select_weighted: null argument");
+  if (b->n_q < 1 || b->n_v_max < 1) return fail(FOT_ERR_ARG, "fot_select_weighted: n_q and n_v_max must be >= 1");
+  if (out->n_w < 1 || out->n_w > FOT_MAX_WEIGHT_SETS)
+    return fail(FOT_ERR_ARG, "fot_select_weighted: n_w must be in [1, FOT_MAX_WEIGHT_SETS]");
+  if (out->per_query != 0 && out->per_query != 1) return fail(FOT_ERR_ARG, "fot_select_weighted: per_query must be 0 or 1");
+  if (!out->weights || !out->idx || !out->cost) return fail(FOT_ERR_ARG, "fot_select_weighted: null weights, idx or cost");
+  if (out->series && !out->len) return fail(FOT_ERR_ARG, "fot_select_weighted: series needs len");
+  if (cand_stride < fot_candidate_count(h, b->n_v_max, 1)) return fail(FOT_ERR_ARG, "fot_select_weighted: cand_stride too small");
+  if (!b->frenet || !b->target_speed || !b->v_grid || !b->n_v) return fail(FOT_ERR_ARG, "fot_select_weighted: null query array");
+  const size_t n_chunks = ((size_t)out->n_w + kWChunk - 1) / kWChunk;
+  if ((size_t)b->n_q * n_chunks > 0x7fffffffull || (size_t)b->n_q * out->n_w > 0x7fffffffull)
+    return fail(FOT_ERR_ARG, "fot_select_weighted: batch too large for one launch");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  Batch B;
+  int rc = weighted_pieces(h, b, st, &B);
+  if (rc != FOT_OK) return rc;
+  const Weighted W{out->n_w, out->per_query, out->weights, out->idx, out->cost, out->len};
+  fot_select_weighted_kernel<<<(unsigned)((size_t)b->n_q * n_chunks), kWThreads, 0, st>>>(
+      h->plan, B, cand_cat, cand_stride, (const double*)h->w_pieces.p, W);
+  if (out->len) {
+    // the selected candidates' series, regenerated as fot_winner does: a ranked list of n_w entries per query
+    const Ranked R{out->n_w, out->idx, out->cost, out->len, out->series};
+    fot_rank_series<<<(unsigned)((size_t)b->n_q * out->n_w), 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, R);
+  }
+  CK(cudaGetLastError());
+  if (!stream) CK(cudaStreamSynchronize(st));
+  return FOT_OK;
+}
+
+extern "C" int fot_cost_terms(fot_handle_t* h, const fot_batch_t* b, int cand_stride, double* terms, void* stream) {
+  if (!h || !b || !terms) return fail(FOT_ERR_ARG, "fot_cost_terms: null argument");
+  if (b->n_q < 1 || b->n_v_max < 1) return fail(FOT_ERR_ARG, "fot_cost_terms: n_q and n_v_max must be >= 1");
+  if (cand_stride < fot_candidate_count(h, b->n_v_max, 1)) return fail(FOT_ERR_ARG, "fot_cost_terms: cand_stride too small");
+  if (!b->frenet || !b->target_speed || !b->v_grid || !b->n_v) return fail(FOT_ERR_ARG, "fot_cost_terms: null query array");
+  const long long n = (long long)b->n_q * cand_stride;
+  if ((n + 255) / 256 > 0x7fffffffll) return fail(FOT_ERR_ARG, "fot_cost_terms: batch too large for one launch");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  Batch B;
+  int rc = weighted_pieces(h, b, st, &B);
+  if (rc != FOT_OK) return rc;
+  fot_cost_terms_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->plan, B, cand_stride, (const double*)h->w_pieces.p, terms);
   CK(cudaGetLastError());
   if (!stream) CK(cudaStreamSynchronize(st));
   return FOT_OK;

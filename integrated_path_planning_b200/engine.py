@@ -102,6 +102,12 @@ class SweepResult:
     rank_cost: Optional[np.ndarray] = None    # [n_q, k]
     rank_len: Optional[np.ndarray] = None     # [n_q, k] int32, or None without series
     rank_series: Optional[np.ndarray] = None  # [n_q, k, 15, n_t_max], or None
+    # winners under cost weightings (cost_weights; include/fot.h fot_weighted_t): -1 / inf / 0 where none is feasible
+    w_idx: Optional[np.ndarray] = None        # [n_q, n_w] int32
+    w_cost: Optional[np.ndarray] = None       # [n_q, n_w]
+    w_len: Optional[np.ndarray] = None        # [n_q, n_w] int32, or None without series
+    w_series: Optional[np.ndarray] = None     # [n_q, n_w, 15, n_t_max], or None
+    cost_terms: Optional[np.ndarray] = None   # [n_q, stride, 5] (Jp, Jd, Js, Jv, Jt), NaN past the candidates
 
     def series(self, q: int = 0):
         """The 15 winner sequences of query q truncated to their kept length, or None."""
@@ -123,6 +129,23 @@ class SweepResult:
                 n = int(self.rank_len[q, r])
                 series = {name: self.rank_series[q, r, j, :n].copy() for j, name in enumerate(SERIES)}
             out.append({"index": i, "cost": np.float64(self.rank_cost[q, r]), "series": series})
+        return out
+
+    def under_weights(self, q: int = 0):
+        """The winner of query q under each weighting, in weighting order: {"index", "cost", "series"} (series: the 15
+        sequences truncated to their kept length, or None when they were not requested), or None where no candidate
+        is feasible under that weighting."""
+        out = []
+        for w in range(self.w_idx.shape[1]):
+            i = int(self.w_idx[q, w])
+            if i < 0:
+                out.append(None)
+                continue
+            series = None
+            if self.w_series is not None:
+                n = int(self.w_len[q, w])
+                series = {name: self.w_series[q, w, j, :n].copy() for j, name in enumerate(SERIES)}
+            out.append({"index": i, "cost": np.float64(self.w_cost[q, w]), "series": series})
         return out
 
 
@@ -313,6 +336,19 @@ class SweepEngine:
         _lib.check(self.lib.fot_rank_candidates(self._h, C.byref(batch), C.c_void_p(cand_cat), C.c_void_p(cand_cost),
                                                 int(cand_stride), C.byref(ranked), C.c_void_p(stream) if stream else None),
                    "fot_rank_candidates")
+
+    def select_weighted_device(self, batch: "_lib.FotBatch", cand_cat: int, cand_stride: int,
+                               weighted: "_lib.FotWeighted", stream=None) -> None:
+        """fot_select_weighted on the per-candidate table of a fot_plan_batch_device launch of `batch` (device
+        pointers), stream-ordered behind it."""
+        _lib.check(self.lib.fot_select_weighted(self._h, C.byref(batch), C.c_void_p(cand_cat), int(cand_stride),
+                                                C.byref(weighted), C.c_void_p(stream) if stream else None),
+                   "fot_select_weighted")
+
+    def cost_terms_device(self, batch: "_lib.FotBatch", cand_stride: int, terms: int, stream=None) -> None:
+        """fot_cost_terms: (Jp, Jd, Js, Jv, Jt) of every candidate of `batch` into terms [n_q, cand_stride, 5]."""
+        _lib.check(self.lib.fot_cost_terms(self._h, C.byref(batch), int(cand_stride), C.c_void_p(terms),
+                                           C.c_void_p(stream) if stream else None), "fot_cost_terms")
 
     def nearest_s(self, x, y, prev_s):
         """fot_nearest_s_device for m points on this engine's path: returns (s [m], status [m] int32), status 0 where

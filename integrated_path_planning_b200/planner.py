@@ -179,6 +179,50 @@ class FrenetPlanner:
             self._feed_back_curvature(paths[0])
         return paths
 
+    def plan_under_weights(self, ego_state, static_obstacles, dynamic_obstacles=None,
+                           target_speed: float = TARGET_SPEED, constraint_overrides: Optional[Dict[str, float]] = None,
+                           dynamic_obstacles_distribution=None, max_stop_distance: Optional[float] = None,
+                           weights=None) -> List[Optional[FrenetPath]]:
+        """The trajectory a planner built with each weighting of the cost knobs would return from the current ego
+        state, one entry per weighting (None where none is feasible under it), from ONE sweep.  `weights`: an
+        [n_w, 6] array (columns _lib.COST_WEIGHT_KEYS) or a list of dicts keyed by those names, where a missing key
+        takes this planner's own value.  Side effects are plan()'s, from this planner's own winner of the same
+        launch: last_check_stats, the nearest-point cache and the curvature fed back.  Selection rule:
+        include/fot.h, fot_weighted_t."""
+        w = self.cost_weight_table(weights)
+        self.last_check_stats = None
+        self.last_result = None
+        fs = self._cartesian_to_frenet_state(ego_state)
+        if fs is None:
+            return [None] * w.shape[0]
+        res = self._sweep(fs.to_array(), static_obstacles, dynamic_obstacles, target_speed, constraint_overrides,
+                          dynamic_obstacles_distribution, max_stop_distance, cost_weights=w)
+        own = res.series(0)
+        if own is not None:
+            self._feed_back_curvature(_frenet_path(own, res.best_cost[0]))
+        return [None if e is None else _frenet_path(e["series"], e["cost"]) for e in res.under_weights(0)]
+
+    def cost_weight_table(self, weights) -> np.ndarray:
+        """[n_w, 6] float64 weightings (columns _lib.COST_WEIGHT_KEYS) from an [n_w, 6] array or a list of dicts keyed
+        by those names; a key a dict leaves out takes this planner's own value.  Raises ValueError on anything else
+        or on n_w outside [1, FOT_MAX_WEIGHT_SETS]."""
+        keys = _lib.COST_WEIGHT_KEYS
+        if isinstance(weights, dict):
+            weights = [weights]
+        if isinstance(weights, (list, tuple)) and weights and all(isinstance(d, dict) for d in weights):
+            for d in weights:
+                unknown = set(d) - set(keys)
+                if unknown:
+                    raise ValueError(f"unknown cost weight keys {sorted(unknown)}; expected a subset of {keys}")
+            w = np.array([[float(d.get(k, getattr(self, k))) for k in keys] for d in weights], dtype=np.float64)
+        else:
+            w = np.asarray(weights, dtype=np.float64) if weights is not None else np.empty((0,))
+            if w.ndim != 2 or w.shape[1] != len(keys):
+                raise ValueError(f"weights must be [n_w, {len(keys)}] or a list of dicts keyed by {keys}")
+        if not 1 <= w.shape[0] <= _lib.FOT_MAX_WEIGHT_SETS:
+            raise ValueError(f"the number of weightings must be in [1, {_lib.FOT_MAX_WEIGHT_SETS}]")
+        return w
+
     def plan_from_frenet(self, frenet_state, static_obstacles, dynamic_obstacles=None,
                          target_speed: float = TARGET_SPEED, constraint_overrides=None,
                          dynamic_obstacles_distribution=None, max_stop_distance=None,
@@ -193,8 +237,9 @@ class FrenetPlanner:
 
     def _sweep(self, frenet_state, static_obstacles, dynamic_obstacles, target_speed, constraint_overrides,
                dynamic_obstacles_distribution, max_stop_distance, want_candidates: bool = False,
-               top_k: int = 0) -> SweepResult:
-        """One query through the sweep (ranked when top_k > 0); sets last_result and last_check_stats."""
+               top_k: int = 0, cost_weights=None) -> SweepResult:
+        """One query through the sweep (ranked when top_k > 0, selected under each weighting of cost_weights [n_w, 6]
+        when given); sets last_result and last_check_stats."""
         mode, dyn = classify_dynamic(dynamic_obstacles, dynamic_obstacles_distribution)
         static = None
         if static_obstacles is not None and len(static_obstacles) > 0:
@@ -202,10 +247,10 @@ class FrenetPlanner:
         stop = np.nan if max_stop_distance is None else float(max_stop_distance)
         frenet = np.asarray(frenet_state, dtype=np.float64).reshape(1, 6)
         limits = self.resolve_limits(constraint_overrides)
-        if top_k > 0:
+        if top_k > 0 or cost_weights is not None:
             from .batch import DeviceBatch           # batch.py builds on this module
             db = DeviceBatch(self, frenet, float(target_speed), dyn, mode, limits=limits, max_stop_distance=stop,
-                             static_obstacles=static, top_k=top_k)
+                             static_obstacles=static, top_k=top_k, cost_weights=cost_weights)
             db.launch()
             res = db.sweep_result(want_candidates)
         else:

@@ -199,7 +199,7 @@ class BatchedClosedLoop:
     """
 
     def __init__(self, waypoints_x, waypoints_y, knobs: Dict[str, float], ped_tracks: np.ndarray, ego0: np.ndarray,
-                 device: int = 0, static_obstacles=None, record: bool = False, sampler=None):
+                 device: int = 0, static_obstacles=None, record: bool = False, sampler=None, cost_weights=None):
         k = {key: (None if (isinstance(v, float) and math.isnan(v)) else v) for key, v in knobs.items()}
         self.k = k
         self.dt = float(k["dt"])
@@ -221,6 +221,14 @@ class BatchedClosedLoop:
             k_s_dot=k["k_s_dot"], k_lat=k["k_lat"], k_lon=k["k_lon"], chance_epsilon=_knob(k, "chance_epsilon", 0.0),
             collision_margin_inflation=_knob(k, "collision_margin_inflation", 1.0), footprint=self.footprint, device=device)
         self.device = device
+        # [N, 6] weighting of each simulation's cost (columns _lib.COST_WEIGHT_KEYS): every planning attempt selects
+        # under it from the same sweep (fot_select_weighted) instead of under the knobs above; None: the knobs
+        self.cost_weights = None
+        if cost_weights is not None:
+            self.cost_weights = np.ascontiguousarray(cost_weights, dtype=np.float64)
+            if self.cost_weights.shape != (self.n, len(_lib.COST_WEIGHT_KEYS)):
+                raise ValueError(f"cost_weights must be [{self.n}, {len(_lib.COST_WEIGHT_KEYS)}], "
+                                 f"got {list(self.cost_weights.shape)}")
         self.post = DevicePredictionPostprocessor(pred_len=int(_knob(k, "pred_len", 12)), sgan_dt=SGAN_DT, sim_dt=self.dt,
                                                   plan_horizon=_knob(k, "max_t", 5.0), device=device)
         self.sampler = sampler
@@ -279,15 +287,21 @@ class BatchedClosedLoop:
         self.n_plan_calls += len(idx)
         t1 = time.perf_counter()
         sel = torch.as_tensor(np.asarray(idx), device=dyn_dev.device)
+        weights = None if self.cost_weights is None else self.cost_weights[np.asarray(idx)][:, None, :]
         batch = DeviceBatch(self.planner, frenet, target, dyn_dev.index_select(0, sel), mode,
                             limits=limits, max_stop_distance=msd,
-                            static_obstacles=self.static_points if len(self.static_points) else None)
+                            static_obstacles=self.static_points if len(self.static_points) else None,
+                            cost_weights=weights)
         batch.launch(None)
-        best = batch.out["best_idx"].cpu().numpy()
-        wlen = batch.out["winner_len"].cpu().numpy()
-        win = batch.out["winner"][:, 9:15, :2].cpu().numpy()          # x y yaw c v a, first two samples
+        if weights is None:
+            o_idx, o_len, o_cost, o_win = (batch.out[key] for key in ("best_idx", "winner_len", "best_cost", "winner"))
+        else:                                                          # the winner under each simulation's weighting
+            o_idx, o_len, o_cost, o_win = (batch.out[key][:, 0] for key in ("w_idx", "w_len", "w_cost", "w_series"))
+        best = o_idx.cpu().numpy()
+        wlen = o_len.cpu().numpy()
+        win = o_win[:, 9:15, :2].cpu().numpy()                         # x y yaw c v a, first two samples
         found = ok & (best >= 0)
-        self._last_full = (batch.out["winner"].cpu().numpy(), batch.out["best_cost"].cpu().numpy()) if self.record else None
+        self._last_full = (o_win.cpu().numpy(), o_cost.cpu().numpy()) if self.record else None
         self.timers["frenet_host"] += t1 - t0
         self.timers["sweep"] += time.perf_counter() - t1
         return found, wlen, win
