@@ -53,7 +53,8 @@ enum {
   FOT_ERR_ARG = -1,        /* bad argument / unsupported size */
   FOT_ERR_CUDA = -2,       /* CUDA runtime error (see fot_last_error) */
   FOT_ERR_NO_DEVICE = -3,  /* no CUDA device: there is no CPU fallback */
-  FOT_ERR_TOO_LARGE = -4   /* time grid does not fit shared memory */
+  FOT_ERR_TOO_LARGE = -4   /* batch shape beyond the sweep: time grid over 320 samples, lateral grid over 8192 targets,
+                              S*P or static points over 32768, tables beyond shared memory (fot_last_error names it) */
 };
 
 /* dynamic-obstacle modes (frenet_planner.py:1043-1047) */
@@ -270,8 +271,8 @@ int fot_reload_options(fot_handle_t* h);
 float fot_last_kernel_ms(const fot_handle_t* h);
 
 /* Which sweep kernel the last launch on this handle used: 4 fot_sweep_pairs (one longitudinal profile per warp; the
- * default), 1 fot_sweep_items (sample-major with block barriers; shapes beyond the limits of fot_sweep_pairs), 2
- * fot_sweep (candidate-major; very long time grids), 0 none yet. */
+ * default), 1 fot_sweep_items (sample-major with block barriers; shapes beyond the limits of fot_sweep_pairs), 0 none
+ * yet; 2 (the retired candidate-major kernel) is never returned. */
 int fot_last_sweep_kind(const fot_handle_t* h);
 
 /* fot_sweep_pairs is compiled per set of optional modes (1 static obstacles, 2 footprint circles, 4 violation budget,

@@ -71,8 +71,7 @@ struct Options {
   int qcap = 1024;             // FOT_QCAP           collision queue entries (tests force the queue-full path)
   int fused_box = 0;           // FOT_FUSED_BOX      1: trajectory boxes in the sweep even for a resident tensor
   int stage_dyn = 1;           // FOT_STAGE_DYN      0: never stage the obstacle block in shared memory
-  int sweep = 0;               // FOT_SWEEP          0 auto (fot_sweep_pairs, else fot_sweep_items, else the candidate-major kernel), 1 "items" (fail if
-                               //                    unsupported), 2 "generic" (candidate-major kernel), 4 "pairs" (fot_sweep_pairs:
+  int sweep = 0;               // FOT_SWEEP          0 auto (fot_sweep_pairs, else fot_sweep_items), 1 "items", 4 "pairs" (fot_sweep_pairs:
                                //                    one longitudinal profile per warp, no block barriers; fail if unsupported)
   int pair_cpq = 0;            // FOT_PAIR_CPQ       CTAs per query of fot_sweep_pairs (0: rule of pair_geometry)
   int pair_simple = 1;         // FOT_PAIR_SIMPLE    0: always the instantiation of fot_sweep_pairs with every mode compiled in (tests)
@@ -89,7 +88,7 @@ struct Options {
     qcap = std::max(1, std::min(1 << 15, geti("FOT_QCAP", 1024)));
     fused_box = geti("FOT_FUSED_BOX", 0) != 0;
     stage_dyn = geti("FOT_STAGE_DYN", 1) != 0;
-    if (const char* e = getenv("FOT_SWEEP")) sweep = !strcmp(e, "generic") ? 2 : !strcmp(e, "items") ? 1 : !strcmp(e, "pairs") ? 4 : 0;
+    if (const char* e = getenv("FOT_SWEEP")) sweep = !strcmp(e, "items") ? 1 : !strcmp(e, "pairs") ? 4 : 0;
     pair_cpq = geti("FOT_PAIR_CPQ", 0);
     pair_simple = geti("FOT_PAIR_SIMPLE", 1) != 0;
     pair_feat = geti("FOT_PAIR_FEAT", 0) & 31;
@@ -142,10 +141,10 @@ struct fot_handle {
   long long n_launch = 0;
   int smem_optin = 0;
   int sms = 148;                     // SM count of the device (block-per-CTA grouping, host chunk sizes)
-  Buf obs_tm, obs_max2, stat_tm, stat_max2, part_cost, part_idx, dyn_box, cost_tab;   // device scratch
+  Buf part_cost, part_idx, dyn_box, cost_tab;   // device scratch
   Buf w_pieces;                      // cost pieces of fot_select_weighted / fot_cost_terms (fot_weights.cuh)
   int last_pair_feat = -1;           // mode set (PAIR_*) of the fot_sweep_pairs instantiation of the last launch
-  int last_sweep_kind = 0;           // 4: fot_sweep_pairs, 1: fot_sweep_items, 2: fot_sweep (generic)
+  int last_sweep_kind = 0;           // 4: fot_sweep_pairs, 1: fot_sweep_items
   fot_result_t mirror{};             // fot_set_result_mirror: second destination of the winner block (all null: none)
   unsigned* mirror_flag = nullptr;   // word published behind each mirrored launch (fot_set_result_mirror), or null
   unsigned mirror_seq = 0;
@@ -242,7 +241,6 @@ extern "C" int fot_create(const fot_config_t* cfg, const fot_tables_t* tb, int d
   CK(cudaDeviceGetAttribute(&h->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
   CK(cudaDeviceGetAttribute(&h->sms, cudaDevAttrMultiProcessorCount, device));
   h->smem_optin -= 2048;   // leave room for the kernels' static shared memory
-  CK(cudaFuncSetAttribute(fot_sweep, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
   CK(cudaFuncSetAttribute(fot_sweep_items<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
   CK(cudaFuncSetAttribute(fot_sweep_items<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
   for (int i = 0; i < kPairInstanceCount; ++i)
@@ -266,8 +264,8 @@ extern "C" int fot_destroy(fot_handle_t* h) {
   { std::lock_guard<std::mutex> lk(g_live_mu); g_live.erase(h); }
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();          // every stream of the handle (compute, priority, copy) is idle before its buffers go
-  for (Buf* b : {&h->gate_d, &h->gate_h, &h->obs_tm, &h->obs_max2, &h->stat_tm, &h->stat_max2, &h->part_cost, &h->part_idx, &h->dyn_box, &h->cost_tab, &h->w_pieces, &h->stage_h, &h->stage_d, &h->out_d,
-                 &h->dyn_d, &h->stat_d})
+  for (Buf* b : {&h->gate_d, &h->gate_h, &h->part_cost, &h->part_idx, &h->dyn_box, &h->cost_tab, &h->w_pieces, &h->stage_h, &h->stage_d,
+                 &h->out_d, &h->dyn_d, &h->stat_d})
     b->release();
   if (h->tables_dev) cudaFree(h->tables_dev);
   for (auto ev : h->ring) if (ev) cudaEventDestroy(ev);
@@ -293,83 +291,25 @@ extern "C" int fot_candidate_count(const fot_handle_t* h, int n_v, int has_brake
   return h->plan.cfg.n_T * n_v * h->plan.cfg.n_d + (has_brake ? h->plan.cfg.n_B : 0);
 }
 
-// Block geometry: how many (speed, lateral) candidates one block takes, bounded by the shared
-// memory its per-speed reference samples need.
-static int sweep_geometry(const fot_handle* h, const fot_batch_t* b, SweepGeom* g, size_t* smem_bytes) {
-  const int n_v_max = b->n_v_max;
-  const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B;
-  const size_t budget = std::min<size_t>((size_t)h->smem_optin, 200 * 1024);
-  // obstacle ring: stage capacity in entries per plane.  Small fields: several whole time planes per
-  // stage (about 4 KB); large fields: 512-entry chunks (12 KB).
-  const int SPp = b->dyn_mode != FOT_DYN_NONE ? ((b->S * b->P + 3) & ~3) : 0;
-  const int Mp = (b->n_static + 3) & ~3;
-  int tile_cap = 0, n_stages = 0;
-  if (SPp > 0 || Mp > 0) {
-    if (SPp > 0 && SPp <= 512) tile_cap = std::min(kGmax, std::max(1, 160 / SPp)) * SPp;   // whole planes, about 4 KB per stage
-    else if (SPp > 512) tile_cap = 512;
-    else tile_cap = std::min(512, Mp);
-    n_stages = 3;
-  }
-  const bool footprint = h->plan.cfg.n_circles > 0;
-  // layout (doubles): tt | hot | js,lonc (6 kv) | jp,dend (2 jp_cap) | kin | [phase-2 region] | ints
-  auto layout = [&](int kv, int* phase2_off, int* ints_off) {
-    const size_t jp_cap = (size_t)kv * nd + (((size_t)kv * nd) & 1);
-    const size_t head = (size_t)kTT * NT + (size_t)kHot * kv * NT + 6 * (size_t)kv + 2 * jp_cap;
-    const size_t kin_sz = (size_t)kKin * kv * NT;
-    const size_t p2 = (size_t)n_stages * 3 * tile_cap + (size_t)kSweepThreads * kRec;
-    const bool alias = !footprint && p2 <= kin_sz;
-    const size_t p2_off = alias ? head : head + kin_sz;
-    const size_t ints = std::max(head + kin_sz, p2_off + p2);
-    if (phase2_off) *phase2_off = (int)p2_off;
-    if (ints_off) *ints_off = (int)ints;
-    return ints * sizeof(double) + ((size_t)4 * kv + NT + kSweepThreads + (size_t)kv * kGmax) * sizeof(int32_t) +
-           (size_t)kv * kGmax * kCullCap * sizeof(unsigned short) + 16;
-  };
-  auto bytes = [&](int kv) { return layout(kv, nullptr, nullptr); };
-  const int nT = h->plan.cfg.n_T;
-  const long long grid_total = (long long)nT * n_v_max * nd;
-  // whole pairs per block when a pair fits (no pair straddles two blocks, so its reference samples and
-  // cull lists are built once); otherwise plain 128-candidate chunks
-  int ch = nd <= kSweepThreads ? (kSweepThreads / nd) * nd : kSweepThreads;
-  ch = (int)std::min<long long>(ch, grid_total);
-  ch = std::max(ch, 1);
-  auto pairs_of = [&](int c) {
-    const int p = (c % nd == 0) ? c / nd : (c - 1) / nd + 2;
-    return (int)std::min<long long>((long long)nT * n_v_max, p);
-  };
-  int kv = std::max(pairs_of(ch), std::min(nB, 8));
-  while (bytes(kv) > std::min<size_t>(budget, 72 * 1024) && ch > nd && ch > 1) {   // keep >= 3 blocks/SM when possible
-    ch = nd <= ch / 2 ? (ch / 2 / nd) * nd : std::max(nd, ch / 2);
-    kv = std::max(pairs_of(ch), std::min(nB, 8));
-  }
-  while (bytes(kv) > budget && ch > 1) { ch = std::max(1, ch / 2); kv = std::max(pairs_of(ch), 1); }
-  if (bytes(kv) > budget) return fail(FOT_ERR_TOO_LARGE, "time grid too long for shared memory");
-  g->ch_eff = ch;
-  g->kv_cap = std::max(kv, 1);
-  g->jp_cap = g->kv_cap * nd + ((g->kv_cap * nd) & 1);   // even: keeps the following tables 16-byte aligned
-  int p2 = 0, io = 0;
-  layout(g->kv_cap, &p2, &io);
-  g->phase2_off = p2;
-  g->ints_off = io;
-  g->tile_cap = tile_cap;
-  g->n_stages = n_stages;
-  g->grid_blocks = (int)((grid_total + ch - 1) / ch);
-  g->brake_blocks = nB > 0 ? (nB + g->kv_cap - 1) / g->kv_cap : 0;
-  g->blocks_per_query = g->grid_blocks + g->brake_blocks;
-  *smem_bytes = bytes(g->kv_cap);
-  return FOT_OK;
-}
-
-
-// Geometry of the sample-major kernel (fot_sweep_items).  Returns false when the batch's shape is
-// outside what that kernel covers (very long time grids, huge per-step obstacle counts); the
-// candidate-major fot_sweep then runs.
+// Geometry of the sample-major kernel (fot_sweep_items).  Returns false, with the limit that was exceeded in
+// fot_last_error, when the batch's shape is outside what that kernel covers: then no sweep kernel takes it.
 static bool item_geometry(const fot_handle* h, const fot_batch_t* b, ItemGeom* g, size_t* smem_bytes,
                           bool want_fused_box = false) {
   const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = h->plan.cfg.nx;
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
   const long long SPl = has_dyn ? (long long)b->S * b->P : 0;
-  if (NT > 128 || nd > 8192 || SPl > 32768 || b->n_static > 32768) return false;   // 128: one NumPy pairwise block
+  char why[160];
+  if (NT > kItemThreads)
+    snprintf(why, sizeof why, "time grid of %d samples: the sweep takes at most %d", NT, kItemThreads);
+  else if (nd > 8192)
+    snprintf(why, sizeof why, "lateral grid of %d targets: the sweep takes at most 8192", nd);
+  else if (SPl > 32768)
+    snprintf(why, sizeof why, "%lld obstacle trajectories (S*P): the sweep takes at most 32768", SPl);
+  else if (b->n_static > 32768)
+    snprintf(why, sizeof why, "%d static obstacle points: the sweep takes at most 32768", b->n_static);
+  else
+    why[0] = 0;
+  if (why[0]) { fail(FOT_ERR_TOO_LARGE, why); return false; }
   const int SP = (int)SPl;
   const int ppc_max = kItemThreads / NT;
   ItemGeom G{};
@@ -433,7 +373,11 @@ static bool item_geometry(const fot_handle* h, const fot_batch_t* b, ItemGeom* g
   stage = stage && h->opt.stage_dyn;
   size_t bytes = layout(stage);
   if (stage && bytes > 110 * 1024) { stage = false; bytes = layout(false); }
-  if (bytes > (size_t)h->smem_optin) return false;
+  if (bytes > (size_t)h->smem_optin) {
+    snprintf(why, sizeof why, "sweep tables of %zu bytes: a block has %d bytes of shared memory", bytes, h->smem_optin);
+    fail(FOT_ERR_TOO_LARGE, why);
+    return false;
+  }
   *g = G;
   *smem_bytes = bytes;
   return true;
@@ -492,27 +436,25 @@ static bool pair_geometry(const fot_handle* h, const fot_batch_t* b, PairGeom* g
 
 // The sweep kernel of a launch, with its geometry and dynamic shared memory.  kind takes the values of
 // fot_last_sweep_kind (and of Options::sweep).
-enum SweepKind { kItems = 1, kGeneric = 2, kPairs = 4 };
+enum SweepKind { kItems = 1, kPairs = 4 };
 struct Sweep {
   int kind = 0;
   ItemGeom ig{};      // fot_sweep_items; for fot_sweep_pairs the scratch layout it shares with it
   PairGeom pg{};      // fot_sweep_pairs
-  SweepGeom g{};      // fot_sweep; for the other two only blocks_per_query, which fot_winner reads
   size_t smem = 0;
 };
 
 // Kernel choice: the pair-per-warp fot_sweep_pairs wherever its shape limits allow, else the sample-major
-// fot_sweep_items, else the candidate-major fot_sweep.  FOT_SWEEP=pairs / items / generic insists on one of them (the
-// tests cross-check the three).  A gated launch needs a sample-major kernel with a staged obstacle block: the gate of
-// fot_sweep_items decides that, and fot_sweep_pairs runs gated only where it stages the block too.
+// fot_sweep_items.  FOT_SWEEP=pairs / items insists on one of them (the tests cross-check the two).  A shape beyond
+// fot_sweep_items is FOT_ERR_TOO_LARGE: fot_sweep_pairs needs its scratch layout.  A gated launch needs a sweep with a
+// staged obstacle block: the gate of fot_sweep_items decides that, and fot_sweep_pairs runs gated only where it stages
+// the block too.
 static int select_sweep(const fot_handle* h, const fot_batch_t* b, bool gated, Sweep* s) {
   *s = Sweep{};
   size_t ismem = 0, psmem = 0;
-  const bool items = h->opt.sweep != kGeneric && item_geometry(h, b, &s->ig, &ismem, gated);
-  if (gated && !(items && s->ig.fused_box))
-    return fail(FOT_ERR_ARG, "gated launch needs a sample-major sweep with a staged obstacle block");
-  if (h->opt.sweep == kItems && !items) return fail(FOT_ERR_ARG, "FOT_SWEEP=items: shape not supported by fot_sweep_items");
-  const bool pairs = (h->opt.sweep == 0 || h->opt.sweep == kPairs) && items && pair_geometry(h, b, &s->pg, &psmem, gated) &&
+  if (!item_geometry(h, b, &s->ig, &ismem, gated)) return FOT_ERR_TOO_LARGE;
+  if (gated && !s->ig.fused_box) return fail(FOT_ERR_ARG, "gated launch needs a sample-major sweep with a staged obstacle block");
+  const bool pairs = (h->opt.sweep == 0 || h->opt.sweep == kPairs) && pair_geometry(h, b, &s->pg, &psmem, gated) &&
                      (!gated || s->pg.fused_box);
   if (h->opt.sweep == kPairs && !pairs && !gated) return fail(FOT_ERR_ARG, "FOT_SWEEP=pairs: shape not supported by fot_sweep_pairs");
   if (pairs) {
@@ -522,14 +464,10 @@ static int select_sweep(const fot_handle* h, const fot_batch_t* b, bool gated, S
     s->ig.fused_box = s->pg.fused_box;
     s->kind = kPairs;
     s->smem = psmem;
-  } else if (items) {
+  } else {
     s->kind = kItems;
     s->smem = ismem;
-  } else {
-    s->kind = kGeneric;
-    return sweep_geometry(h, b, &s->g, &s->smem);
   }
-  s->g.blocks_per_query = s->ig.ctas_per_query;     // fot_winner reads one partial per CTA
   return FOT_OK;
 }
 
@@ -583,53 +521,33 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
   Sweep s;
   const int rc = select_sweep(h, b, gate.word != nullptr, &s);
   if (rc != FOT_OK) return rc;
-  const bool use_pairs = s.kind == kPairs, use_items = s.kind != kGeneric;
   ItemGeom& ig = s.ig;
   PairGeom& pg = s.pg;
-  const SweepGeom& g = s.g;
   if (gate.word) {
     ig.gate = gate.word; ig.gate_epoch = gate.epoch; ig.gate_per = gate.per; ig.gate_q0 = (int32_t)q_off;
     pg.gate = gate.word; pg.gate_epoch = gate.epoch; pg.gate_per = gate.per; pg.gate_q0 = (int32_t)q_off;
   }
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
-  const size_t n_part = (size_t)b->n_q * g.blocks_per_query;
-  if ((size_t)b->n_q * (size_t)g.blocks_per_query > 0x7fffffffull) return fail(FOT_ERR_ARG, "batch too large for one launch");
+  const size_t n_part = (size_t)b->n_q * ig.ctas_per_query;
+  if (n_part > 0x7fffffffull) return fail(FOT_ERR_ARG, "batch too large for one launch");
   // partial winners: chunks of one batch may cut their queries into different numbers of CTAs; the stride that
   // addresses the scratch is the largest any chunk can use
-  const size_t part_stride = use_items ? (size_t)std::max(ig.blocks_per_query, ig.ctas_per_query) : (size_t)g.blocks_per_query;
-  if (q_off != 0 && !use_items) return fail(FOT_ERR_ARG, "chunk offsets need the fot_sweep_items path");
+  const size_t part_stride = (size_t)std::max(ig.blocks_per_query, ig.ctas_per_query);
   CK(h->part_cost.reserve(q_total * part_stride * sizeof(double)));
   CK(h->part_idx.reserve(q_total * part_stride * sizeof(int32_t)));
   const int SP = has_dyn ? b->S * b->P : 0;
-  const int SPp = (SP + 3) & ~3, Mp = (b->n_static + 3) & ~3;
-  const int nq_s = b->static_per_query ? b->n_q : 1;
-  const bool need_box = use_items && has_dyn && !ig.fused_box;
+  const bool need_box = has_dyn && !ig.fused_box;
   const size_t cost_stride = (size_t)h->plan.cfg.n_T * (b->n_v_max + 2 * h->plan.cfg.n_d) + 3 * (size_t)h->plan.cfg.n_B;
-  if (!use_items) {
-    if (has_dyn) {
-      CK(h->obs_tm.reserve((size_t)b->n_q * b->T_obs * 3 * SPp * sizeof(double)));
-      CK(h->obs_max2.reserve((size_t)b->n_q * sizeof(double)));
-    }
-    if (b->n_static > 0) {
-      CK(h->stat_tm.reserve((size_t)nq_s * 3 * Mp * sizeof(double)));
-      CK(h->stat_max2.reserve((size_t)nq_s * sizeof(double)));
-    }
-  } else {
-    if (need_box) CK(h->dyn_box.reserve(q_total * SP * sizeof(float4)));
-    CK(h->cost_tab.reserve(q_total * cost_stride * sizeof(double)));
-  }
+  if (need_box) CK(h->dyn_box.reserve(q_total * SP * sizeof(float4)));
+  CK(h->cost_tab.reserve(q_total * cost_stride * sizeof(double)));
   float4* dyn_box = need_box ? (float4*)h->dyn_box.p + q_off * SP : nullptr;
-  double* cost_tab = use_items ? (double*)h->cost_tab.p + q_off * cost_stride : nullptr;
+  double* cost_tab = (double*)h->cost_tab.p + q_off * cost_stride;
 
   Batch B{};
   B.n_q = b->n_q; B.n_v_max = b->n_v_max;
   B.frenet = b->frenet; B.target = b->target_speed; B.limits = b->limits; B.stop_dist = b->stop_dist;
   B.v_grid = b->v_grid; B.n_v = b->n_v;
-  B.static_tm = (!use_items && b->n_static > 0) ? (const double*)h->stat_tm.p : nullptr;
-  B.static_max2 = (!use_items && b->n_static > 0) ? (const double*)h->stat_max2.p : nullptr;
   B.n_static = b->n_static; B.static_per_query = b->static_per_query;
-  B.obs_tm = (!use_items && has_dyn) ? (const double*)h->obs_tm.p : nullptr;
-  B.obs_max2 = (!use_items && has_dyn) ? (const double*)h->obs_max2.p : nullptr;
   B.S = has_dyn ? b->S : 0; B.P = has_dyn ? b->P : 0; B.T_obs = has_dyn ? b->T_obs : 0; B.dyn_mode = b->dyn_mode;
   B.dyn_raw = has_dyn ? b->dyn : nullptr;
   B.static_raw = b->n_static > 0 ? b->static_obs : nullptr;
@@ -650,26 +568,10 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
     const size_t n_cat = r->cand_cat ? (size_t)b->n_q * r->cand_stride : 0;
     const size_t work = std::max<size_t>((size_t)b->n_q * FOT_N_STATS, n_cat);
     const int blocks = (int)std::min<size_t>(1024, (work + 255) / 256);
-    const bool planes = !use_items;
-    fot_init_kernel<<<blocks, 256, 0, st>>>(r->stats, b->n_q * FOT_N_STATS,
-                                            planes && has_dyn ? (double*)h->obs_max2.p : nullptr, planes && has_dyn ? b->n_q : 0,
-                                            planes && b->n_static > 0 ? (double*)h->stat_max2.p : nullptr,
-                                            planes && b->n_static > 0 ? nq_s : 0, r->cand_cat, n_cat);
+    fot_init_kernel<<<blocks, 256, 0, st>>>(r->stats, b->n_q * FOT_N_STATS, r->cand_cat, n_cat);
   }
   CK(cudaEventRecord(ring[0], st));
-  if (!use_items) {
-    if (has_dyn) {
-      const long long warps = (long long)b->n_q * SP;
-      const int blocks = (int)((warps * 32 + 255) / 256);
-      fot_obstacle_prepass<<<blocks, 256, 0, st>>>((const double2*)b->dyn, (double*)h->obs_tm.p,
-                                                   (double*)h->obs_max2.p, b->n_q, SP, b->T_obs);
-    }
-    if (b->n_static > 0) {
-      const int total = nq_s * b->n_static;
-      fot_static_prepass<<<(total + 255) / 256, 256, 0, st>>>((const double2*)b->static_obs, (double*)h->stat_tm.p,
-                                                              (double*)h->stat_max2.p, nq_s, b->n_static);
-    }
-  } else {
+  {
     // cost tables (one thread per polynomial profile) and trajectory boxes (one warp per trajectory), one launch
     const long long n_prof = (long long)h->plan.cfg.n_T * (b->n_v_max + h->plan.cfg.n_d) + 2 * h->plan.cfg.n_B;
     const long long cblocks = ((long long)b->n_q * n_prof + 255) / 256;
@@ -680,7 +582,7 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
                                                                (const double2*)b->dyn, dyn_box, n_traj, b->T_obs);
   }
   CK(cudaEventRecord(ring[1], st));
-  if (use_pairs) {
+  if (s.kind == kPairs) {
     // the modes this batch needs; the smallest instantiated superset runs (everything else is compiled out of it)
     int need = 0;
     if (b->n_static > 0) need |= PAIR_STATIC;
@@ -696,12 +598,11 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
       if ((kPairInstances[i] & need) == need) { feat = kPairInstances[i]; break; }
     pair_kernel(pg.fused_box != 0, feat)<<<(unsigned)n_part, kPairThreads, s.smem, st>>>(h->plan, B, O, pg);
     h->last_pair_feat = feat;
-  } else if (use_items && ig.fused_box) fot_sweep_items<true><<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
-  else if (use_items) fot_sweep_items<false><<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
-  else fot_sweep<<<(unsigned)n_part, kSweepThreads, s.smem, st>>>(h->plan, B, O, g);
+  } else if (ig.fused_box) fot_sweep_items<true><<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
+  else fot_sweep_items<false><<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
   h->last_sweep_kind = s.kind;
   CK(cudaEventRecord(ring[2], st));
-  fot_winner<<<b->n_q, 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, O, g);
+  fot_winner<<<b->n_q, 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, O, ig.ctas_per_query);
   if (O.m_winner && h->mirror_flag) fot_publish_kernel<<<1, 1, 0, st>>>(h->mirror_flag, ++h->mirror_seq);
   CK(cudaEventRecord(ring[3], st));
   if (record_span) CK(cudaEventRecord(h->ev1, st));
@@ -906,8 +807,7 @@ static Ranges plan_ranges(const fot_handle* h, const fot_batch_t* b, bool host) 
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
   Ranges rg;
   rg.bound[1] = nq;
-  const std::string keep = g_err;      // a kernel the probes below refuse is not an error of this call
-  Sweep s;
+  const std::string keep = g_err;      // a kernel the probe below refuses is not an error of this call
   if (host) {
     // Ranges only pay when the obstacle upload is large.  The kernels are the longer leg of the pipeline (the upload runs
     // at PCIe speed), so the first ranges are small -- the sweep starts after 1/16 of the upload -- and the rest large
@@ -920,15 +820,11 @@ static Ranges plan_ranges(const fot_handle* h, const fot_batch_t* b, bool host) 
       for (int c = 0; c <= rg.n; ++c) rg.bound[c] = std::min(nq, c * per);
     }
     // Gated, the sweep does not wait for whole ranges, so a few large ones do: about 1/2, 5/16, 3/16 of the queries.
+    Sweep s;
     rg.gated = h->opt.gated && rg.n > 1 && has_dyn && nq < (1 << 22) && select_sweep(h, b, true, &s) == FOT_OK;
     if (rg.gated && h->opt.host_chunks <= 0) cut16(h, nq, {8, 13}, &rg);
   } else if (nq >= 1024) {
     cut16(h, nq, {8, 13}, &rg);
-  }
-  // only the sample-major kernels address their scratch by query offset: the candidate-major fot_sweep takes one range
-  if (!rg.gated && rg.n > 1 && (select_sweep(h, b, false, &s) != FOT_OK || s.kind == kGeneric)) {
-    rg.n = 1;
-    rg.bound[1] = nq;
   }
   g_err = keep;
   return rg;

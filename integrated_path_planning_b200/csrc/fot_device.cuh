@@ -29,17 +29,16 @@ struct Batch {
   int32_t n_q, n_v_max;
   const double *frenet, *target, *limits, *stop_dist, *v_grid;
   const int32_t* n_v;
-  const double* static_tm;    // static obstacles as planes [n_q or 1][3][pad4(M)] of (-2x, -2y, x^2+y^2)
-  const double* static_max2;  // [n_q or 1] max x^2+y^2 (rounding band of the expanded distance form)
   int32_t n_static, static_per_query;
-  const double* obs_tm;       // dynamic obstacles, time-major planes [n_q][T_obs][3][pad4(S*P)]
-  const double* obs_max2;     // [n_q]
   int32_t S, P, T_obs, dyn_mode;
-  // fot_sweep_items reads the caller's tensors directly:
+  // the sweep kernels read the caller's tensors directly:
   const double* dyn_raw;      // [n_q][S][P][T_obs][2] (reference layout) or null
   const double* static_raw;   // [n_q or 1][M][2] or null
   const float4* dyn_box;      // [n_q][S*P] trajectory boxes (xmin, xmax, ymin, ymax) from fot_aabb_prepass
   const double* cost_tab;     // [n_q][n_T*(n_v_max + 2 n_d) + 3 n_B] jerk sums / terminal offsets from fot_cost_prepass
+  // Unused.  Out and the geometry follow Batch in the sweep kernels' parameters; without these 32 bytes ptxas schedules
+  // fot_sweep_pairs differently, and the sweep of bench.py ran 1.2 % slower (1.597 against 1.578 ms; B200, 1000 W).
+  const void* pad_[4];
 };
 
 struct Out {
@@ -181,6 +180,7 @@ __device__ __forceinline__ double lat_fast0(const Lat& L, double t) {
 // np.sum over a contiguous float64 vector: NumPy's pairwise summation (8 interleaved
 // accumulators per <=128-element block, halving above that).  The jerk costs fp.py:718,:722
 // go through it, so the cost -- and with it the arg-min -- only reproduces with this order.
+// np_block_sum is one block; np_pairwise_sum_flat is the whole sum for any n.
 template <class F>
 __device__ __forceinline__ double np_block_sum(const F& f, int lo, int n) {   // n <= 128
   if (n < 8) {
@@ -200,19 +200,38 @@ __device__ __forceinline__ double np_block_sum(const F& f, int lo, int n) {   //
   for (; i < n; ++i) res += f(lo + i);
   return res;
 }
+// Above 128 elements NumPy halves the range (the left half rounded down to a multiple of 8) and adds the two halves'
+// sums.  That split tree is walked here with an explicit stack rather than by recursion: a recursive form takes a
+// 200-byte stack frame per level, and sums of a few thousand terms overflow the default 1 KB thread stack.
 template <class F>
-__device__ __noinline__ double np_split_sum(const F& f, int lo, int n) {      // only reached for n > 128: halve, 8-aligned
-  int n2 = n / 2;
-  n2 -= n2 % 8;
-  const int n3 = n - n2;
-  const double left = n2 <= 128 ? np_block_sum(f, lo, n2) : np_split_sum(f, lo, n2);
-  const double right = n3 <= 128 ? np_block_sum(f, lo + n2, n3) : np_split_sum(f, lo + n2, n3);
-  return left + right;
-}
-template <class F>
-__device__ __forceinline__ double np_pairwise_sum(const F& f, int lo, int n) {
-  if (n <= 128) return np_block_sum(f, lo, n);
-  return np_split_sum(f, lo, n);
+__device__ double np_pairwise_sum_flat(const F& f, int n) {
+  if (n <= 128) return np_block_sum(f, 0, n);
+  int s_lo[32], s_n[32], s_state[32];                   // depth <= log2(n / 128) + 1 < 32
+  double s_left[32];
+  int sp = 0;
+  s_lo[0] = 0; s_n[0] = n; s_state[0] = 0;
+  double ret = 0.0;
+  for (;;) {
+    const int lo = s_lo[sp], m = s_n[sp];
+    int m2 = m / 2;
+    m2 -= m2 % 8;
+    if (m <= 128) {
+      ret = np_block_sum(f, lo, m);
+      --sp;
+    } else if (s_state[sp] == 0) {                      // descend left
+      s_state[sp] = 1;
+      ++sp; s_lo[sp] = lo; s_n[sp] = m2; s_state[sp] = 0;
+      continue;
+    } else if (s_state[sp] == 1) {                      // left done: descend right
+      s_left[sp] = ret; s_state[sp] = 2;
+      ++sp; s_lo[sp] = lo + m2; s_n[sp] = m - m2; s_state[sp] = 0;
+      continue;
+    } else {                                            // both done: left + right
+      ret = s_left[sp] + ret;
+      --sp;
+    }
+    if (sp < 0) return ret;
+  }
 }
 
 // Reference-line sample at arc length s (cs.py:47-166, :215-288).  NaN outside the knot range.

@@ -185,40 +185,6 @@ __global__ void fot_prepend_kernel(const double* __restrict__ in, const int32_t*
   }
 }
 
-// np_pairwise_sum (fot_device.cuh) without the recursion: NumPy's split tree walked with an explicit stack.
-// The recursive form takes a 200-byte stack frame per level here, and P * T of a few thousand overflows the
-// default 1 KB thread stack.  Same additions in the same order, so the same value.
-template <class F>
-__device__ double np_pairwise_sum_flat(const F& f, int n) {
-  if (n <= 128) return np_block_sum(f, 0, n);
-  int s_lo[32], s_n[32], s_state[32];                   // depth <= log2(n / 128) + 1 < 32
-  double s_left[32];
-  int sp = 0;
-  s_lo[0] = 0; s_n[0] = n; s_state[0] = 0;
-  double ret = 0.0;
-  for (;;) {
-    const int lo = s_lo[sp], m = s_n[sp];
-    int m2 = m / 2;
-    m2 -= m2 % 8;
-    if (m <= 128) {
-      ret = np_block_sum(f, lo, m);
-      --sp;
-    } else if (s_state[sp] == 0) {                      // descend left
-      s_state[sp] = 1;
-      ++sp; s_lo[sp] = lo; s_n[sp] = m2; s_state[sp] = 0;
-      continue;
-    } else if (s_state[sp] == 1) {                      // left done: descend right
-      s_left[sp] = ret; s_state[sp] = 2;
-      ++sp; s_lo[sp] = lo + m2; s_n[sp] = m - m2; s_state[sp] = 0;
-      continue;
-    } else {                                            // both done: left + right
-      ret = s_left[sp] + ret;
-      --sp;
-    }
-    if (sp < 0) return ret;
-  }
-}
-
 // Closest-to-mean sample (trajectory_predictor.py:346-351): mean over the samples (sequential add over S,
 // then / S, as np.mean reduces an outer axis), per-point 2-norm, np.sum over (pedestrians, steps) in NumPy's
 // pairwise order, first arg-min.  fot_best_dist_kernel: one thread per (query, sample) distance;

@@ -1,8 +1,7 @@
 // fot_sweep_items.cuh -- the sample-major sweep kernel (sm_100a, fp64).
 //
-// Same contract as fot_sweep (fot_kernels.cuh): one fused kernel for the whole candidate sweep of
-// every query, per-block arg-min partials out, no trajectory written to HBM.  The work is laid out
-// the other way round:
+// One fused kernel for the whole candidate sweep of every query, per-CTA arg-min partials out (reduced
+// by fot_winner, fot_kernels.cuh), no trajectory written to HBM.  The work is laid out sample-major:
 //
 //   block  = (query, horizon T_j, chunk of terminal speeds)  -- or the query's brake ladder;
 //            a CTA sweeps `bpc` consecutive blocks of one query (all of them in large batches), so
@@ -1028,7 +1027,7 @@ __device__ __forceinline__ void cost_prepass_body(const Plan& P, const Batch& B,
       const double j = k > hold ? 0.0 : 6.0 * a3 + 24.0 * a4 * ((double)k * dt);
       return j * j;
     };
-    out[slot] = np_block_sum(jerk2, 0, N);               // N <= 128: one pairwise block
+    out[slot] = np_pairwise_sum_flat(jerk2, N);
   } else {                                               // lateral
     Lat L;
     int N, slot_j, slot_d;
@@ -1050,7 +1049,7 @@ __device__ __forceinline__ void cost_prepass_body(const Plan& P, const Batch& B,
       const double j = k > hold ? 0.0 : 6.0 * a3 + 24.0 * a4 * t + 60.0 * a5 * (t * t);
       return j * j;
     };
-    out[slot_j] = np_block_sum(jerk2, 0, N);
+    out[slot_j] = np_pairwise_sum_flat(jerk2, N);
     const TPow te = tpow(min(N - 1, hold), dt);
     out[slot_d] = L.a0 + L.a1 * te.t + L.a2 * te.t2 + L.a3 * te.t3 + L.a4 * te.t4 + L.a5 * te.t5;     // fp.py:688, :719
   }

@@ -24,7 +24,7 @@ def reload_options():
 
 
 class fot_env:
-    """with fot_env(FOT_SWEEP="generic"): ...   -- environment change + option reload, restored on exit."""
+    """with fot_env(FOT_SWEEP="items"): ...   -- environment change + option reload, restored on exit."""
 
     def __init__(self, **kv):
         self.kv = kv

@@ -100,9 +100,7 @@ def test_full_collision_queue_degrades_to_in_place_tests():
         unstaged = run()
     with _env(FOT_STAGE_DYN=0, FOT_PAIR_CPQ=8):
         unstaged_pairs = run()
-    with _env(FOT_SWEEP="generic"):
-        generic = run()
-    for other in (items, capped, unstaged, unstaged_pairs, generic):
+    for other in (items, capped, unstaged, unstaged_pairs):
         assert np.array_equal(base.cand_cat, other.cand_cat)
         assert np.array_equal(base.best_idx, other.best_idx) and np.array_equal(base.stats, other.stats)
         assert np.array_equal(base.best_cost.view(np.uint64), other.best_cost.view(np.uint64))
@@ -288,11 +286,11 @@ def test_pair_kernel_shape_limits_and_fallback():
         _check(res, [orc.plan_frenet(tuple(s), np.empty((0, 2)), dyn, 6.0) for s in fs])
 
 
-def test_candidate_major_sweep_takes_a_large_upload_in_one_range():
-    """A time grid of 129 samples is beyond fot_sweep_items and fot_sweep_pairs, so the candidate-major fot_sweep runs.
-    It addresses its scratch from query 0, so the host-result calls give it the whole batch as one range, even where
-    the upload size (1024 queries x 5 pedestrians x 129 steps, 10.6 MB) or FOT_HOST_CHUNKS would cut the batch into
-    several.  Both calls must return the bits of a plain launch over the resident tensor."""
+def test_long_time_grid_large_upload_matches_the_resident_launch():
+    """A time grid of 129 samples is beyond fot_sweep_pairs, so fot_sweep_items runs.  The upload size (1024 queries x
+    5 pedestrians x 129 steps, 10.6 MB) and FOT_HOST_CHUNKS cut the batch into query ranges, and the host-pointer call
+    may gate the sweep on the upload.  Both host-result calls must return the bits of a plain launch over the resident
+    tensor."""
     import torch
     from integrated_path_planning_b200 import DeviceBatch, _lib
     knobs = dict(scenarios.S1_KNOBS, dt=0.05, min_t=6.0, max_t=6.4, d_road_w=0.9, d_t_s=3.0)
@@ -305,7 +303,7 @@ def test_candidate_major_sweep_takes_a_large_upload_in_one_range():
     assert pl.engine.n_t_max > 128
     batch = DeviceBatch(pl, frenet, 6.0, dyn[:, None], _lib.FOT_DYN_SINGLE)
     batch.launch(None)
-    assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == 2
+    assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == 1
     want = {k: v.cpu().numpy() for k, v in batch.out.items()}
     assert len(set(want["best_idx"].tolist())) > 5
 
@@ -314,7 +312,7 @@ def test_candidate_major_sweep_takes_a_large_upload_in_one_range():
             assert _same(k, v, np.asarray(got[k]), want["winner_len"]), (how, k)
 
     res = pl.plan_batch(frenet, 6.0, dynamic_obstacles=dyn, want_candidates=True)
-    assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == 2
+    assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == 1
     agree({k: getattr(res, k) for k in want}, "plan_batch")
     orc = _oracle(knobs)
     _check(res, [orc.plan_frenet(tuple(frenet[i]), np.empty((0, 2)), dyn[i], 6.0) for i in range(3)])

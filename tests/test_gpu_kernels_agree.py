@@ -1,7 +1,6 @@
-"""GPU: the three sweep kernels are independent implementations of the same contract -- the
-pair-per-warp `fot_sweep_pairs` (default), the sample-major `fot_sweep_items` (FOT_SWEEP=items, also
-the kernel for shapes beyond the pair kernel's limits) and the candidate-major `fot_sweep`
-(FOT_SWEEP=generic, also the fallback for very long time grids).  They must agree bit for bit on every
+"""GPU: the two sweep kernels are independent implementations of the same contract -- the
+pair-per-warp `fot_sweep_pairs` (default) and the sample-major `fot_sweep_items` (FOT_SWEEP=items, also
+the kernel for shapes beyond the pair kernel's limits).  They must agree bit for bit on every
 candidate's category and cost, on the winner and on the histogram, at sizes the NumPy oracle cannot reach."""
 import os
 
@@ -41,8 +40,7 @@ def test_config4_batch_both_kernels():
     _, frenet, dyn = bench.make_queries(1000, 512)
     pl = _planner(scenarios.S1_KNOBS, scenarios.STRAIGHT_60)
     run = lambda: pl.plan_batch(frenet, 6.0, dynamic_obstacles=dyn[:, 0], want_candidates=True)
-    b, c, d = _run("items", run), _run("generic", run), _run("pairs", run)
-    _assert_same(b, c)
+    b, d = _run("items", run), _run("pairs", run)
     _assert_same(b, d)
     assert (b.stats[:, 6] > 0).any() and (b.best_idx >= 0).any()
 
@@ -67,8 +65,7 @@ def test_curved_path_state_machine_knobs_both_kernels():
     pl = _planner(k, wp)
     run = lambda: pl.plan_batch(frenet, target, dynamic_obstacles=dyn, static_obstacles=wall, limits=limits,
                                 max_stop_distance=msd, want_candidates=True)
-    b, c, d = _run("items", run), _run("generic", run), _run("pairs", run)
-    _assert_same(b, c)
+    b, d = _run("items", run), _run("pairs", run)
     _assert_same(b, d)
 
 
@@ -83,8 +80,7 @@ def test_dense_grid_distribution_both_kernels():
     pl = _planner(knobs, wp)
     fs = np.array([[5.0, 5.0, 0.0, 0.0, 0.0, 0.0]])
     run = lambda: pl.plan_batch(fs, 6.2, distribution=dist[None], want_candidates=True)
-    a, b, d = _run("items", run), _run("generic", run), _run("pairs", run)
-    _assert_same(a, b)
+    a, d = _run("items", run), _run("pairs", run)
     _assert_same(a, d)
     assert int(a.n_cand[0]) > 60000
 
@@ -107,8 +103,7 @@ def test_budgeted_distribution_and_footprint_both_kernels():
     from tests import runners
     pl = BatchFrenetPlanner(CubicSpline2D(*wp), footprint=runners.make_footprint((4.5, 2.0, 3)), **knobs)
     run = lambda: pl.plan_batch(frenet, 6.0, distribution=dist, want_candidates=True)
-    b, c, d = _run("items", run), _run("generic", run), _run("pairs", run)
-    _assert_same(b, c)
+    b, d = _run("items", run), _run("pairs", run)
     _assert_same(b, d)
 
 

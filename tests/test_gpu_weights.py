@@ -101,7 +101,7 @@ def _assert_selection_equals_sweeps(knobs, wp, weights, run, planner_kw=None, n_
 
 
 # ---- 1. the handle's own weighting reproduces the launch, on all three sweep kernels ------------------------------
-@pytest.mark.parametrize("kernel", ["pairs", "items", "generic"])
+@pytest.mark.parametrize("kernel", ["pairs", "items"])
 def test_own_weighting_is_the_winner_config4(config4, kernel):
     frenet, dyn = config4
     pl = _planner()
@@ -109,7 +109,7 @@ def test_own_weighting_is_the_winner_config4(config4, kernel):
     w = _weightings(scenarios.S1_KNOBS)[:4]
     with runners.fot_env(FOT_SWEEP=kernel):
         res = pl.plan_batch(frenet, 6.0, dynamic_obstacles=dyn[:, 0], cost_weights=w)
-        assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == {"pairs": 4, "items": 1, "generic": 2}[kernel]
+        assert int(pl.engine.lib.fot_last_sweep_kind(pl.engine._h)) == {"pairs": 4, "items": 1}[kernel]
     assert (res.best_idx >= 0).sum() > 100
     _assert_own_weighting_is_the_winner(res, 0)
     assert (res.w_idx[:, 1] != res.best_idx).sum() > 0                          # another weighting picks otherwise
@@ -192,7 +192,7 @@ def test_selection_equals_sweeps_static_wall():
 
 
 def test_selection_equals_sweeps_long_time_grid():
-    """129 samples per trajectory: the candidate-major kernel runs, and the jerk sums take NumPy's split summation."""
+    """129 samples per trajectory: fot_sweep_items runs, and the jerk sums take NumPy's split summation."""
     knobs = dict(scenarios.S1_KNOBS, dt=0.05, min_t=6.0, max_t=6.4, d_road_w=0.9, d_t_s=3.0)
     rng = np.random.default_rng(8)
     n = 16

@@ -43,7 +43,7 @@ dist = scenarios.sample_distribution(rng, base, 20)
 bp = BatchFrenetPlanner(CubicSpline2D(*wp), **knobs)
 fs = np.array([[5.0, 5.0, 0.0, 0.0, 0.0, 0.0]])
 res3 = {}
-for kern in ("pairs", "items", "generic"):
+for kern in ("pairs", "items"):
     os.environ["FOT_SWEEP"] = kern
     bp.engine.reload_options()
     ms = []
