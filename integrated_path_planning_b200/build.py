@@ -10,6 +10,7 @@ ROOT = os.path.dirname(HERE)
 SRC = os.path.join(HERE, "csrc", "fot_api.cu")
 DEPS = [SRC, os.path.join(HERE, "csrc", "fot_kernels.cuh"), os.path.join(HERE, "csrc", "fot_device.cuh"),
         os.path.join(HERE, "csrc", "fot_sweep_items.cuh"), os.path.join(HERE, "csrc", "fot_sweep_pairs.cuh"),
+        os.path.join(HERE, "csrc", "fot_sweep_math.cuh"),
         os.path.join(HERE, "csrc", "fot_predict.cuh"), os.path.join(HERE, "csrc", "fot_frenet.cuh"),
         os.path.join(HERE, "csrc", "fot_rank.cuh"), os.path.join(HERE, "csrc", "fot_weights.cuh"),
         os.path.join(ROOT, "include", "fot.h")]

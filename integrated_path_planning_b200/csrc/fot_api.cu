@@ -385,7 +385,7 @@ static bool item_geometry(const fot_handle* h, const fot_batch_t* b, ItemGeom* g
 
 // Geometry of the pair-per-warp kernel (fot_sweep_pairs): one CTA per query (several for small batches), every warp
 // with a private slice of shared memory for the pair it is working on.  False when the shape is outside its range
-// (time grids beyond 64 samples, lateral grids beyond 96 targets, tables that do not fit): fot_sweep_items then runs.
+// (time grids beyond kPairNT = 56 samples, lateral grids beyond 96 targets, tables that do not fit): fot_sweep_items then runs.
 static bool pair_geometry(const fot_handle* h, const fot_batch_t* b, PairGeom* g, size_t* smem_bytes,
                           bool want_fused_box = false) {
   const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = h->plan.cfg.nx;

@@ -348,4 +348,41 @@ __device__ __forceinline__ void argmin_merge(double& c, int& i, double oc, int o
   if (oc < c || (oc == c && oi < i)) { c = oc; i = oi; }
 }
 
+// 1/x and 1/sqrt(x) to fp64 accuracy from the fp32 MUFU seed and two Newton steps (branch-free; the
+// library versions carry slow paths for denormals and cost three times as many instructions).  Used for
+// quantities that only feed the validity chain (a few ulp are immaterial there); arguments are O(1).
+__device__ __forceinline__ double rcp_nr(double a) {
+  double x = (double)__frcp_rn((float)a);
+  x = fma(x, fma(-a, x, 1.0), x);
+  x = fma(x, fma(-a, x, 1.0), x);
+  return x;
+}
+__device__ __forceinline__ double rsqrt_nr(double a) {
+  double y = (double)rsqrtf((float)a);
+  const double h = 0.5 * a;
+  y = fma(y, fma(-h * y, y, 0.5), y);
+  y = fma(y, fma(-h * y, y, 0.5), y);
+  return y;
+}
+
+// Time powers of one sample, built as the reference's TimeCache does (fp.py:594-598).
+struct TPow {
+  double t, t2, t3, t4, t5;
+};
+__device__ __forceinline__ TPow tpow(int n, double dt) {
+  TPow r;
+  r.t = (double)n * dt;
+  r.t2 = r.t * r.t; r.t3 = r.t2 * r.t; r.t4 = r.t2 * r.t2; r.t5 = r.t4 * r.t;
+  return r;
+}
+
+// Order-preserving float <-> unsigned map for atomicMin / atomicMax on floats.
+__device__ __forceinline__ unsigned f2ord(float f) {
+  const unsigned u = __float_as_uint(f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float ord2f(unsigned u) {
+  return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
+}
+
 }  // namespace fot

@@ -1,6 +1,8 @@
-// fot_kernels.cuh -- what the two sweep kernels (fot_sweep_items.cuh, fot_sweep_pairs.cuh) share (sm_100a, fp64).
+// fot_kernels.cuh -- the launch-level kernels around the sweep (sm_100a, fp64).  The sweep kernels themselves are in
+// fot_sweep_items.cuh and fot_sweep_pairs.cuh, their shared per-candidate arithmetic in fot_sweep_math.cuh.
 //
 //   fot_init_kernel : per launch, zero the histogram and mark every per-candidate category unwritten
+//   fot_prepass : per launch, the cost tables (jerk sums, terminal offsets) and the predicted trajectories' boxes
 //   fot_winner : per query, reduce the sweep's per-CTA partials and regenerate the 15 sequences of the
 //        winning candidate only, in the reference's arithmetic order.
 #pragma once
@@ -41,6 +43,128 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 __device__ __forceinline__ void tma_bulk_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
+}
+
+// Cost pieces that depend on one polynomial profile only (fp.py:703-734): the jerk sums  sum_n s'''(t_n)^2,
+// sum_n d'''(t_n)^2  in NumPy's pairwise-summation order (so that costs are bit-identical to the
+// reference) and the terminal lateral offset d(t_end).  One thread per profile; per query the table holds
+//   [n_T][n_v_max] Js | [n_T][n_d] Jp | [n_T][n_d] d_end | [n_B] Js brake | [n_B] Jp brake | [n_B] d_end brake.
+__device__ __forceinline__ void cost_prepass_body(const Plan& P, const Batch& B, double* __restrict__ tab, unsigned block) {
+  const int n_d = P.cfg.n_d, n_T = P.cfg.n_T, n_B = P.cfg.n_B;
+  const int nTv = n_T * B.n_v_max, nTd = n_T * n_d;
+  const int n_prof = nTv + nTd + 2 * n_B;                // profiles with a sum
+  const int stride = nTv + 2 * nTd + 3 * n_B;
+  const long long g = (long long)block * blockDim.x + threadIdx.x;    // one thread per profile
+  if (g >= (long long)B.n_q * n_prof) return;
+  const int q = (int)(g / n_prof), pr = (int)(g - (long long)q * n_prof);
+  const double* fs = B.frenet + 6 * (size_t)q;
+  const double dt = P.cfg.dt;
+  double* out = tab + (size_t)q * stride;
+  const int n_v = B.n_v[q];
+  if (pr < nTv || (pr >= nTv + nTd && pr < nTv + nTd + n_B)) {             // longitudinal
+    Lon L;
+    int N, slot;
+    if (pr < nTv) {
+      const int jT = pr / B.n_v_max, kv = pr - jT * B.n_v_max;
+      if (kv >= n_v) return;
+      N = P.n_steps[jT] + 1;
+      L = lon_solve(fs, B.v_grid[(size_t)q * B.n_v_max + kv], P.T[jT], P.inv4 + 4 * jT, n_v == 1, N - 1);
+      slot = pr;
+    } else {
+      const int b = pr - nTv - nTd;
+      N = P.cfg.n_total;
+      L = lon_solve(fs, 0.0, P.Tb[b], P.inv4b + 4 * b, true, P.n_steps_b[b]);
+      slot = nTv + 2 * nTd + b;
+    }
+    const double a3 = L.a3, a4 = L.a4;
+    const int hold = L.hold;
+    auto jerk2 = [=](int k) {                            // fp.py:647, :722
+      const double j = k > hold ? 0.0 : 6.0 * a3 + 24.0 * a4 * ((double)k * dt);
+      return j * j;
+    };
+    out[slot] = np_pairwise_sum_flat(jerk2, N);
+  } else {                                               // lateral
+    Lat L;
+    int N, slot_j, slot_d;
+    if (pr < nTv + nTd) {
+      const int li = pr - nTv, jT = li / n_d, id = li - jT * n_d;
+      N = P.n_steps[jT] + 1;
+      L = lat_solve(fs, P.d_grid[id], P.T[jT], P.inv5 + 9 * jT, n_d == 1, N - 1);
+      slot_j = nTv + li; slot_d = nTv + nTd + li;
+    } else {
+      const int b = pr - nTv - nTd - n_B;
+      N = P.cfg.n_total;
+      L = lat_solve(fs, fs[3], P.Tb[b], P.inv5b + 9 * b, true, P.n_steps_b[b]);
+      slot_j = nTv + 2 * nTd + n_B + b; slot_d = nTv + 2 * nTd + 2 * n_B + b;
+    }
+    const double a3 = L.a3, a4 = L.a4, a5 = L.a5;
+    const int hold = L.hold;
+    auto jerk2 = [=](int k) {                            // fp.py:691, :718
+      const double t = (double)k * dt;
+      const double j = k > hold ? 0.0 : 6.0 * a3 + 24.0 * a4 * t + 60.0 * a5 * (t * t);
+      return j * j;
+    };
+    out[slot_j] = np_pairwise_sum_flat(jerk2, N);
+    const TPow te = tpow(min(N - 1, hold), dt);
+    out[slot_d] = L.a0 + L.a1 * te.t + L.a2 * te.t2 + L.a3 * te.t3 + L.a4 * te.t4 + L.a5 * te.t5;     // fp.py:688, :719
+  }
+}
+
+// Boxes of the predicted trajectories, once per launch: one warp per trajectory (q, sample, ped),
+// (xmin, xmax, ymin, ymax) over all its steps rounded outward to fp32.  A NaN anywhere makes the
+// whole box NaN, which fails every overlap test: exactly the reference's prefilter, whose np.min /
+// np.max propagate the NaN and thereby remove that pedestrian from the test (fp.py:1211-1222).
+constexpr int kBoxPerWarp = 4;   // trajectories boxed per warp of fot_prepass: their loads are all in flight together
+__device__ __forceinline__ void aabb_prepass_body(const double2* __restrict__ dyn, float4* __restrict__ box, long long n_traj, int T_obs,
+                                                  unsigned block) {
+  const long long warp = ((long long)block * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  const long long t0 = warp * kBoxPerWarp;
+  if (t0 >= n_traj) return;
+  // both loads of each of the warp's <= 64-step trajectories are issued before the first comparison
+  const bool h0 = lane < T_obs, h1 = lane + 32 < T_obs;
+  double2 o0[kBoxPerWarp], o1[kBoxPerWarp];
+#pragma unroll
+  for (int u = 0; u < kBoxPerWarp; ++u) {
+    const double2* src = dyn + (size_t)min(t0 + u, n_traj - 1) * T_obs;
+    o0[u] = h0 ? src[lane] : make_double2(INFINITY, INFINITY);
+    o1[u] = h1 ? src[lane + 32] : o0[u];
+  }
+#pragma unroll
+  for (int u = 0; u < kBoxPerWarp; ++u) {
+    if (t0 + u >= n_traj) break;
+    const double2* src = dyn + (size_t)(t0 + u) * T_obs;
+    bool bad = (h0 && ((o0[u].x != o0[u].x) || (o0[u].y != o0[u].y))) || (h1 && ((o1[u].x != o1[u].x) || (o1[u].y != o1[u].y)));
+    double xlo = h0 ? fmin(o0[u].x, o1[u].x) : INFINITY, xhi = h0 ? fmax(o0[u].x, o1[u].x) : -INFINITY;
+    double ylo = h0 ? fmin(o0[u].y, o1[u].y) : INFINITY, yhi = h0 ? fmax(o0[u].y, o1[u].y) : -INFINITY;
+    for (int k = lane + 64; k < T_obs; k += 32) {
+      const double2 o = src[k];
+      bad |= (o.x != o.x) || (o.y != o.y);
+      xlo = fmin(xlo, o.x); xhi = fmax(xhi, o.x); ylo = fmin(ylo, o.y); yhi = fmax(yhi, o.y);
+    }
+    // outward rounding to fp32 is monotone, so it commutes with min / max: round first, then reduce the ordered-uint
+    // images with one redux each (four instructions instead of forty shuffles and as many fp64 comparisons)
+    const unsigned rxlo = __reduce_min_sync(0xffffffffu, f2ord(__double2float_rd(xlo)));
+    const unsigned rxhi = __reduce_max_sync(0xffffffffu, f2ord(__double2float_ru(xhi)));
+    const unsigned rylo = __reduce_min_sync(0xffffffffu, f2ord(__double2float_rd(ylo)));
+    const unsigned ryhi = __reduce_max_sync(0xffffffffu, f2ord(__double2float_ru(yhi)));
+    bad = __any_sync(0xffffffffu, bad);
+    if (lane == 0) {
+      const float nanf_ = __int_as_float(0x7fc00000);
+      box[t0 + u] = bad ? make_float4(nanf_, nanf_, nanf_, nanf_) : make_float4(ord2f(rxlo), ord2f(rxhi), ord2f(rylo), ord2f(ryhi));
+    }
+  }
+}
+
+// One launch for both prepasses (they are independent and each too small to fill the GPU for long):
+// blocks [0, n_cost_blocks) build the cost tables, the rest box the predicted trajectories.  (Spreading the two kinds
+// evenly over the grid, so that every SM runs FP64-bound and memory-bound blocks together, measured slower: 0.142 against
+// 0.133 ms.)
+__global__ void __launch_bounds__(256)
+fot_prepass(const Plan P, const Batch B, double* __restrict__ cost_tab, unsigned n_cost_blocks,
+            const double2* __restrict__ dyn, float4* __restrict__ box, long long n_traj, int T_obs) {
+  if (blockIdx.x < n_cost_blocks) cost_prepass_body(P, B, cost_tab, blockIdx.x);
+  else aabb_prepass_body(dyn, box, n_traj, T_obs, blockIdx.x - n_cost_blocks);
 }
 
 // ----------------------------------------------------------------------------------------

@@ -41,9 +41,12 @@
 // DESIGN.md section 7); the winner's sequences are regenerated in reference order by fot_winner.
 // The squared forms assume non-negative limits (a negative limit rejects everything, as in the
 // reference).
+//
+// The upload gate, the boxes of a staged obstacle block, the reference point and the flag idiom are shared with
+// fot_sweep_pairs (fot_sweep_math.cuh); the cost tables and trajectory boxes come from fot_prepass (fot_kernels.cuh).
 #pragma once
 #include <type_traits>
-#include "fot_kernels.cuh"
+#include "fot_sweep_math.cuh"
 
 namespace fot {
 
@@ -60,8 +63,6 @@ __device__ unsigned long long g_phase_clk[16];
 #define FOT_ITEM_MIN_CTAS 2
 #endif
 constexpr int kItemThreads = 320;   // largest block of fot_sweep_items
-constexpr int kRowW = 12;           // item row: rx ry cos sin | kappa s 1/s_dot s_dot | A0 B0 A1 B1
-constexpr unsigned F_DROP = 32u;    // silent drop (singular / non-finite / teleport), fp.py:826-833, :944-956
 
 struct ItemGeom {
   int32_t ppc;               // terminal speeds (pairs) per grid block
@@ -98,105 +99,19 @@ struct ItemGeom {
   unsigned* gate;            // [slice] flags, [kGateSlices] set to 1 by a CTA that gave up waiting; nullptr: no gate
 };
 
-#ifndef FOT_GATE_SLEEP_NS
-#define FOT_GATE_SLEEP_NS 1000
-#endif
-constexpr int kGateSlices = 64;
-constexpr long long kGateTimeoutNs = 4000000000ll;   // a gated CTA gives up after 4 s (the host reports the error)
-
-// 1/x and 1/sqrt(x) to fp64 accuracy from the fp32 MUFU seed and two Newton steps (branch-free; the
-// library versions carry slow paths for denormals and cost three times as many instructions).  Used for
-// quantities that only feed the validity chain (a few ulp are immaterial there); arguments are O(1).
-__device__ __forceinline__ double rcp_nr(double a) {
-  double x = (double)__frcp_rn((float)a);
-  x = fma(x, fma(-a, x, 1.0), x);
-  x = fma(x, fma(-a, x, 1.0), x);
-  return x;
-}
-__device__ __forceinline__ double rsqrt_nr(double a) {
-  double y = (double)rsqrtf((float)a);
-  const double h = 0.5 * a;
-  y = fma(y, fma(-h * y, y, 0.5), y);
-  y = fma(y, fma(-h * y, y, 0.5), y);
-  return y;
-}
-
+// The spline tables in shared memory (spline_smem) or the Plan's own arrays.
 struct SplineView {
   const double *knots, *xa, *xb, *xc, *xd, *ya, *yb, *yc, *yd;
   int nx;
 };
-struct RefFast {
-  double rx, ry, cth, sth, rk, rdk;
-};
-// Reference point at arc length s (cs.py:47-166, :215-288) with heading as a unit vector:
-// cos(atan2(y', x')) = x'/|r'| (cc.py:128-129 takes cos/sin of the yaw).  NaN outside the knots.
-__device__ __forceinline__ RefFast spline_ref_fast(const SplineView& V, double s) {
-  RefFast o;
-  const int nx = V.nx;
-  if (!(s >= V.knots[0] && s <= V.knots[nx - 1])) {     // cs.py:62
-    o.rx = o.ry = o.cth = o.sth = o.rk = o.rdk = qnan();
-    return o;
+// spline_ref_tab over the tables of a SplineView.
+struct SplineViewTab {
+  const SplineView& V;
+  __device__ __forceinline__ double operator()(int k, int i) const {
+    const double* t[9] = {V.knots, V.xa, V.xb, V.xc, V.xd, V.ya, V.yb, V.yc, V.yd};
+    return t[k][i];
   }
-  int lo = 0, hi = nx;                                   // searchsorted(side='right') (cs.py:162)
-  while (lo < hi) {
-    const int mid = (lo + hi) >> 1;
-    if (V.knots[mid] <= s) lo = mid + 1; else hi = mid;
-  }
-  int seg = lo - 1;
-  seg = seg < 0 ? 0 : (seg > nx - 2 ? nx - 2 : seg);     // cs.py:165
-  const double dx = s - V.knots[seg];
-  const double dx2 = dx * dx, dx3 = dx2 * dx;
-  const double xa = V.xa[seg], xb = V.xb[seg], xc = V.xc[seg], xd = V.xd[seg];
-  const double ya = V.ya[seg], yb = V.yb[seg], yc = V.yc[seg], yd = V.yd[seg];
-  o.rx = xa + xb * dx + xc * dx2 + xd * dx3;             // cs.py:73-74
-  o.ry = ya + yb * dx + yc * dx2 + yd * dx3;
-  const double x1 = xb + 2.0 * xc * dx + 3.0 * xd * dx2; // cs.py:100
-  const double y1 = yb + 2.0 * yc * dx + 3.0 * yd * dx2;
-  const double x2 = 2.0 * xc + 6.0 * xd * dx;            // cs.py:125
-  const double y2 = 2.0 * yc + 6.0 * yd * dx;
-  const double x3 = 6.0 * xd, y3 = 6.0 * yd;             // cs.py:149
-  const double D = x1 * x1 + y1 * y1;
-  const double rD = rsqrt_nr(D);
-  o.cth = x1 * rD;
-  o.sth = y1 * rD;
-  const double iD15 = rD * rD * rD;                      // D ** -1.5
-  o.rk = (y2 * x1 - x2 * y1) * iD15;                     // cs.py:246
-  const double a = x1 * y2 - y1 * x2;
-  const double b = x1 * y3 - y1 * x3;
-  const double c = x1 * x2 + y1 * y2;
-  o.rdk = b * iD15 - 3.0 * a * c * (iD15 * rD * rD);     // cs.py:273
-  return o;
-}
-
-// Time powers of one sample, built as the reference's TimeCache does (fp.py:594-598).
-struct TPow {
-  double t, t2, t3, t4, t5;
 };
-__device__ __forceinline__ TPow tpow(int n, double dt) {
-  TPow r;
-  r.t = (double)n * dt;
-  r.t2 = r.t * r.t; r.t3 = r.t2 * r.t; r.t4 = r.t2 * r.t2; r.t5 = r.t4 * r.t;
-  return r;
-}
-
-// Order-preserving float <-> unsigned map for atomicMin / atomicMax on floats.
-__device__ __forceinline__ unsigned f2ord(float f) {
-  const unsigned u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float ord2f(unsigned u) {
-  return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
-}
-
-
-// flag |= bit when a > b / when |a| > b: one DSETP and one predicated LOP3 (the compiler's own
-// `cond ? bit : 0` idiom costs a SEL and a LOP3 per flag)
-__device__ __forceinline__ void flag_gt(unsigned& f, double a, double b, unsigned bit) {
-  asm("{\n .reg .pred p;\n setp.gt.f64 p, %1, %2;\n @p or.b32 %0, %0, %3;\n}" : "+r"(f) : "d"(a), "d"(b), "r"(bit));
-}
-__device__ __forceinline__ void flag_abs_gt(unsigned& f, double a, double b, unsigned bit) {
-  asm("{\n .reg .pred p;\n .reg .f64 t;\n abs.f64 t, %1;\n setp.gt.f64 p, t, %2;\n @p or.b32 %0, %0, %3;\n}" : "+r"(f) : "d"(a), "d"(b), "r"(bit));
-}
 
 // Bit i of the result: candidate 32*w + i of pair `pp` has no validity flag (4 flag bytes per word).
 __device__ __forceinline__ unsigned clean_word(const unsigned* flags_pp, int nw4, int n_dl, int w) {
@@ -269,33 +184,7 @@ fot_sweep_items(const Plan P, const Batch B, const Out O, const ItemGeom G) {
   const double2* stat_q = M > 0 ? reinterpret_cast<const double2*>(B.static_raw) + (size_t)(B.static_per_query ? q : 0) * M : nullptr;
 
   // ---- once per CTA: obstacle block in flight, grids and spline tables in shared memory ----------
-  if (kFused && G.gate) {
-    // this query's slice of the obstacle tensor has been uploaded once the progress word passes it
-    if (tid == 0) {
-      const unsigned* flag = G.gate + (G.gate_q0 + q) / G.gate_per;
-      int abort_ = 0;
-      long long t0 = 0;
-      for (unsigned spins = 0;; ++spins) {
-        unsigned seen;
-#ifdef FOT_GATE_POLL_RELAXED
-        asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(flag) : "memory");
-        if (seen == G.gate_epoch) { asm volatile("fence.acq_rel.sys;" ::: "memory"); break; }
-#else
-        asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(seen) : "l"(flag) : "memory");
-        if (seen == G.gate_epoch) break;
-#endif
-        __nanosleep(spins < 64 ? 100 : FOT_GATE_SLEEP_NS);
-        long long now;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-        if (t0 == 0) t0 = now;
-        if (now - t0 > kGateTimeoutNs) { abort_ = 1; G.gate[kGateSlices] = 1u; break; }
-      }
-      asm volatile("fence.proxy.async.global;" ::: "memory");      // the bulk copy below reads what the upload wrote
-      s_abort = abort_;
-    }
-    __syncthreads();
-    if (s_abort) return;
-  }
+  if (kFused && G.gate && gate_wait(G, q, s_abort)) return;
   if (tid == 0 && G.stage_dyn && state_ok) {
     mbar_init(&s_bar, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -419,7 +308,7 @@ fot_sweep_items(const Plan P, const Batch B, const Out O, const ItemGeom G) {
       V.knots = P.knots; V.xa = P.xa; V.xb = P.xb; V.xc = P.xc; V.xd = P.xd;
       V.ya = P.ya; V.yb = P.yb; V.yc = P.yc; V.yd = P.yd;
     }
-    const RefFast rp = spline_ref_fast(V, s);
+    const RefFast rp = spline_ref_tab(SplineViewTab{V}, V.nx, s);
     i_rx = rp.rx; i_ry = rp.ry; i_cth = rp.cth; i_sth = rp.sth; i_rk = rp.rk; i_rdk = rp.rdk;
     i_isd = fabs(i_sd) > 1e-3 ? rcp_nr(i_sd) : 0.0;                            // fp.py:792 EPS_S_DOT
     // lateral basis at this sample: d_i(t) = A(t) + d_i * B(t) (the quintic's right-hand side is linear
@@ -492,29 +381,9 @@ fot_sweep_items(const Plan P, const Batch B, const Out O, const ItemGeom G) {
   const double rc_d = sqrt(r2_dyn) * (1.0 + 1e-9) + 1e-9 + max_off;
   const double wroad = fmax(P.cfg.max_road_width + 1e-9, fabs(fs[3]));
   if (kFused && !boxes_done) {
-    // first block of the CTA: box every predicted trajectory of the staged obstacle block (what fot_prepass
-    // does for a resident tensor): one warp per trajectory, fp32 rounded outward, NaN trajectory -> NaN box
+    // first block of the CTA: box every predicted trajectory of the staged obstacle block
     mbar_wait(&s_bar, 0u);
-    for (int j = tid >> 5; j < SP; j += bd >> 5) {
-      const double2* src = dynst + (size_t)j * B.T_obs;
-      double xlo = INFINITY, xhi = -INFINITY, ylo = INFINITY, yhi = -INFINITY;
-      bool bad = false;
-      for (int k = lane; k < B.T_obs; k += 32) {
-        const double2 o = src[k];
-        bad |= (o.x != o.x) || (o.y != o.y);
-        xlo = fmin(xlo, o.x); xhi = fmax(xhi, o.x); ylo = fmin(ylo, o.y); yhi = fmax(yhi, o.y);
-      }
-      for (int off = 16; off > 0; off >>= 1) {
-        xlo = fmin(xlo, __shfl_xor_sync(0xffffffffu, xlo, off)); xhi = fmax(xhi, __shfl_xor_sync(0xffffffffu, xhi, off));
-        ylo = fmin(ylo, __shfl_xor_sync(0xffffffffu, ylo, off)); yhi = fmax(yhi, __shfl_xor_sync(0xffffffffu, yhi, off));
-      }
-      bad = __any_sync(0xffffffffu, bad);
-      if (lane == 0) {
-        const float nanf_ = __int_as_float(0x7fc00000);
-        sbox[j] = bad ? make_float4(nanf_, nanf_, nanf_, nanf_)
-                      : make_float4(__double2float_rd(xlo), __double2float_ru(xhi), __double2float_rd(ylo), __double2float_ru(yhi));
-      }
-    }
+    box_staged(dynst, sbox, SP, B.T_obs, tid >> 5, bd >> 5, lane);
     boxes_done = true;
     __syncthreads();
   }
@@ -988,128 +857,6 @@ fot_sweep_items(const Plan P, const Batch B, const Out O, const ItemGeom G) {
     O.part_idx[part] = (my_idx == 0x7fffffff) ? -1 : my_idx;
   }
   if (tid < FOT_N_STATS && s_stats[tid] != 0) atomicAdd(&O.stats[(size_t)q * FOT_N_STATS + tid], s_stats[tid]);
-}
-
-// Cost pieces that depend on one polynomial profile only (fp.py:703-734): the jerk sums  sum_n s'''(t_n)^2,
-// sum_n d'''(t_n)^2  in NumPy's pairwise-summation order (so that costs are bit-identical to the
-// reference) and the terminal lateral offset d(t_end).  One thread per profile; per query the table holds
-//   [n_T][n_v_max] Js | [n_T][n_d] Jp | [n_T][n_d] d_end | [n_B] Js brake | [n_B] Jp brake | [n_B] d_end brake.
-__device__ __forceinline__ void cost_prepass_body(const Plan& P, const Batch& B, double* __restrict__ tab, unsigned block) {
-  const int n_d = P.cfg.n_d, n_T = P.cfg.n_T, n_B = P.cfg.n_B;
-  const int nTv = n_T * B.n_v_max, nTd = n_T * n_d;
-  const int n_prof = nTv + nTd + 2 * n_B;                // profiles with a sum
-  const int stride = nTv + 2 * nTd + 3 * n_B;
-  const long long g = (long long)block * blockDim.x + threadIdx.x;    // one thread per profile
-  if (g >= (long long)B.n_q * n_prof) return;
-  const int q = (int)(g / n_prof), pr = (int)(g - (long long)q * n_prof);
-  const double* fs = B.frenet + 6 * (size_t)q;
-  const double dt = P.cfg.dt;
-  double* out = tab + (size_t)q * stride;
-  const int n_v = B.n_v[q];
-  if (pr < nTv || (pr >= nTv + nTd && pr < nTv + nTd + n_B)) {             // longitudinal
-    Lon L;
-    int N, slot;
-    if (pr < nTv) {
-      const int jT = pr / B.n_v_max, kv = pr - jT * B.n_v_max;
-      if (kv >= n_v) return;
-      N = P.n_steps[jT] + 1;
-      L = lon_solve(fs, B.v_grid[(size_t)q * B.n_v_max + kv], P.T[jT], P.inv4 + 4 * jT, n_v == 1, N - 1);
-      slot = pr;
-    } else {
-      const int b = pr - nTv - nTd;
-      N = P.cfg.n_total;
-      L = lon_solve(fs, 0.0, P.Tb[b], P.inv4b + 4 * b, true, P.n_steps_b[b]);
-      slot = nTv + 2 * nTd + b;
-    }
-    const double a3 = L.a3, a4 = L.a4;
-    const int hold = L.hold;
-    auto jerk2 = [=](int k) {                            // fp.py:647, :722
-      const double j = k > hold ? 0.0 : 6.0 * a3 + 24.0 * a4 * ((double)k * dt);
-      return j * j;
-    };
-    out[slot] = np_pairwise_sum_flat(jerk2, N);
-  } else {                                               // lateral
-    Lat L;
-    int N, slot_j, slot_d;
-    if (pr < nTv + nTd) {
-      const int li = pr - nTv, jT = li / n_d, id = li - jT * n_d;
-      N = P.n_steps[jT] + 1;
-      L = lat_solve(fs, P.d_grid[id], P.T[jT], P.inv5 + 9 * jT, n_d == 1, N - 1);
-      slot_j = nTv + li; slot_d = nTv + nTd + li;
-    } else {
-      const int b = pr - nTv - nTd - n_B;
-      N = P.cfg.n_total;
-      L = lat_solve(fs, fs[3], P.Tb[b], P.inv5b + 9 * b, true, P.n_steps_b[b]);
-      slot_j = nTv + 2 * nTd + n_B + b; slot_d = nTv + 2 * nTd + 2 * n_B + b;
-    }
-    const double a3 = L.a3, a4 = L.a4, a5 = L.a5;
-    const int hold = L.hold;
-    auto jerk2 = [=](int k) {                            // fp.py:691, :718
-      const double t = (double)k * dt;
-      const double j = k > hold ? 0.0 : 6.0 * a3 + 24.0 * a4 * t + 60.0 * a5 * (t * t);
-      return j * j;
-    };
-    out[slot_j] = np_pairwise_sum_flat(jerk2, N);
-    const TPow te = tpow(min(N - 1, hold), dt);
-    out[slot_d] = L.a0 + L.a1 * te.t + L.a2 * te.t2 + L.a3 * te.t3 + L.a4 * te.t4 + L.a5 * te.t5;     // fp.py:688, :719
-  }
-}
-
-// Boxes of the predicted trajectories, once per launch: one warp per trajectory (q, sample, ped),
-// (xmin, xmax, ymin, ymax) over all its steps rounded outward to fp32.  A NaN anywhere makes the
-// whole box NaN, which fails every overlap test: exactly the reference's prefilter, whose np.min /
-// np.max propagate the NaN and thereby remove that pedestrian from the test (fp.py:1211-1222).
-constexpr int kBoxPerWarp = 4;   // trajectories boxed per warp of fot_prepass: their loads are all in flight together
-__device__ __forceinline__ void aabb_prepass_body(const double2* __restrict__ dyn, float4* __restrict__ box, long long n_traj, int T_obs,
-                                                  unsigned block) {
-  const long long warp = ((long long)block * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  const long long t0 = warp * kBoxPerWarp;
-  if (t0 >= n_traj) return;
-  // both loads of each of the warp's <= 64-step trajectories are issued before the first comparison
-  const bool h0 = lane < T_obs, h1 = lane + 32 < T_obs;
-  double2 o0[kBoxPerWarp], o1[kBoxPerWarp];
-#pragma unroll
-  for (int u = 0; u < kBoxPerWarp; ++u) {
-    const double2* src = dyn + (size_t)min(t0 + u, n_traj - 1) * T_obs;
-    o0[u] = h0 ? src[lane] : make_double2(INFINITY, INFINITY);
-    o1[u] = h1 ? src[lane + 32] : o0[u];
-  }
-#pragma unroll
-  for (int u = 0; u < kBoxPerWarp; ++u) {
-    if (t0 + u >= n_traj) break;
-    const double2* src = dyn + (size_t)(t0 + u) * T_obs;
-    bool bad = (h0 && ((o0[u].x != o0[u].x) || (o0[u].y != o0[u].y))) || (h1 && ((o1[u].x != o1[u].x) || (o1[u].y != o1[u].y)));
-    double xlo = h0 ? fmin(o0[u].x, o1[u].x) : INFINITY, xhi = h0 ? fmax(o0[u].x, o1[u].x) : -INFINITY;
-    double ylo = h0 ? fmin(o0[u].y, o1[u].y) : INFINITY, yhi = h0 ? fmax(o0[u].y, o1[u].y) : -INFINITY;
-    for (int k = lane + 64; k < T_obs; k += 32) {
-      const double2 o = src[k];
-      bad |= (o.x != o.x) || (o.y != o.y);
-      xlo = fmin(xlo, o.x); xhi = fmax(xhi, o.x); ylo = fmin(ylo, o.y); yhi = fmax(yhi, o.y);
-    }
-    // outward rounding to fp32 is monotone, so it commutes with min / max: round first, then reduce the ordered-uint
-    // images with one redux each (four instructions instead of forty shuffles and as many fp64 comparisons)
-    const unsigned rxlo = __reduce_min_sync(0xffffffffu, f2ord(__double2float_rd(xlo)));
-    const unsigned rxhi = __reduce_max_sync(0xffffffffu, f2ord(__double2float_ru(xhi)));
-    const unsigned rylo = __reduce_min_sync(0xffffffffu, f2ord(__double2float_rd(ylo)));
-    const unsigned ryhi = __reduce_max_sync(0xffffffffu, f2ord(__double2float_ru(yhi)));
-    bad = __any_sync(0xffffffffu, bad);
-    if (lane == 0) {
-      const float nanf_ = __int_as_float(0x7fc00000);
-      box[t0 + u] = bad ? make_float4(nanf_, nanf_, nanf_, nanf_) : make_float4(ord2f(rxlo), ord2f(rxhi), ord2f(rylo), ord2f(ryhi));
-    }
-  }
-}
-
-// One launch for both prepasses (they are independent and each too small to fill the GPU for long):
-// blocks [0, n_cost_blocks) build the cost tables, the rest box the predicted trajectories.  (Spreading the two kinds
-// evenly over the grid, so that every SM runs FP64-bound and memory-bound blocks together, measured slower: 0.142 against
-// 0.133 ms.)
-__global__ void __launch_bounds__(256)
-fot_prepass(const Plan P, const Batch B, double* __restrict__ cost_tab, unsigned n_cost_blocks,
-            const double2* __restrict__ dyn, float4* __restrict__ box, long long n_traj, int T_obs) {
-  if (blockIdx.x < n_cost_blocks) cost_prepass_body(P, B, cost_tab, blockIdx.x);
-  else aabb_prepass_body(dyn, box, n_traj, T_obs, blockIdx.x - n_cost_blocks);
 }
 
 }  // namespace fot

@@ -30,12 +30,13 @@
 // compile-time constant, why there is one code site per job in the collision loop, and why the batch shape of a planning
 // campaign has an instantiation of its own (kFeat = 0) with every other mode compiled out.
 //
-// Reference citations as in fot_sweep_items.cuh (fp.py = src/planning/frenet_planner.py, cs.py = cubic_spline.py,
+// The upload gate, the boxes of a staged obstacle block, the reference point and the flag idiom are the functions of
+// fot_sweep_math.cuh that fot_sweep_items calls too.  Reference citations as in fot_sweep_items.cuh (fp.py = src/planning/frenet_planner.py, cs.py = cubic_spline.py,
 // cc.py = src/core/coordinate_converter.py).
 #pragma once
 #include <cstddef>
 #include <type_traits>
-#include "fot_sweep_items.cuh"
+#include "fot_sweep_math.cuh"
 
 namespace fot {
 
@@ -101,44 +102,11 @@ struct PairGeom {
   unsigned* gate;
 };
 
-// spline_ref_fast (fot_sweep_items.cuh) over the shared-memory tables of PairShared: compile-time strides.
-__device__ __forceinline__ RefFast spline_ref_smem(const double (*T)[kPairNX], int nx, double s) {
-  RefFast o;
-  if (!(s >= T[0][0] && s <= T[0][nx - 1])) {            // cs.py:62
-    o.rx = o.ry = o.cth = o.sth = o.rk = o.rdk = qnan();
-    return o;
-  }
-  int lo = 0, hi = nx;                                   // searchsorted(side='right') (cs.py:162)
-  while (lo < hi) {
-    const int mid = (lo + hi) >> 1;
-    if (T[0][mid] <= s) lo = mid + 1; else hi = mid;
-  }
-  int seg = lo - 1;
-  seg = seg < 0 ? 0 : (seg > nx - 2 ? nx - 2 : seg);     // cs.py:165
-  const double dx = s - T[0][seg];
-  const double dx2 = dx * dx, dx3 = dx2 * dx;
-  const double xa = T[1][seg], xb = T[2][seg], xc = T[3][seg], xd = T[4][seg];
-  const double ya = T[5][seg], yb = T[6][seg], yc = T[7][seg], yd = T[8][seg];
-  o.rx = xa + xb * dx + xc * dx2 + xd * dx3;             // cs.py:73-74
-  o.ry = ya + yb * dx + yc * dx2 + yd * dx3;
-  const double x1 = xb + 2.0 * xc * dx + 3.0 * xd * dx2; // cs.py:100
-  const double y1 = yb + 2.0 * yc * dx + 3.0 * yd * dx2;
-  const double x2 = 2.0 * xc + 6.0 * xd * dx;            // cs.py:125
-  const double y2 = 2.0 * yc + 6.0 * yd * dx;
-  const double x3 = 6.0 * xd, y3 = 6.0 * yd;             // cs.py:149
-  const double D = x1 * x1 + y1 * y1;
-  const double rD = rsqrt_nr(D);
-  o.cth = x1 * rD;
-  o.sth = y1 * rD;
-  const double iD15 = rD * rD * rD;                      // D ** -1.5
-  o.rk = (y2 * x1 - x2 * y1) * iD15;                     // cs.py:246
-  const double a = x1 * y2 - y1 * x2;
-  const double b = x1 * y3 - y1 * x3;
-  const double c = x1 * x2 + y1 * y2;
-  o.rdk = b * iD15 - 3.0 * a * c * (iD15 * rD * rD);     // cs.py:273
-  return o;
-}
-
+// spline_ref_tab over the shared-memory tables of PairShared: compile-time strides.
+struct SmemSplineTab {
+  const double (*T)[kPairNX];
+  __device__ __forceinline__ double operator()(int k, int i) const { return T[k][i]; }
+};
 // kFused: the variant of the gated host-pointer call (waits for its query's upload slice, boxes the trajectories itself).
 // kFeat: which optional modes this instantiation carries (PAIR_*).  The kernel is bound by instruction fetch (DESIGN.md
 // section 4d), so the code of a mode the batch does not use is compiled out of the instantiation it runs instead of
@@ -199,28 +167,7 @@ fot_sweep_pairs(const Plan P, const Batch B, const Out O_, const PairGeom G) {
   (void)NT;
 
   // ---- once per CTA ---------------------------------------------------------------------------------
-  if (kFused && G.gate) {
-    // this query's slice of the obstacle tensor has been uploaded once the slice flag carries the call's epoch
-    if (tid == 0) {
-      const unsigned* flag = G.gate + (G.gate_q0 + q) / G.gate_per;
-      int abort_ = 0;
-      long long t0 = 0;
-      for (unsigned spins = 0;; ++spins) {
-        unsigned seen;
-        asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(seen) : "l"(flag) : "memory");
-        if (seen == G.gate_epoch) break;
-        __nanosleep(spins < 64 ? 100 : FOT_GATE_SLEEP_NS);
-        long long now;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-        if (t0 == 0) t0 = now;
-        if (now - t0 > kGateTimeoutNs) { abort_ = 1; G.gate[kGateSlices] = 1u; break; }
-      }
-      asm volatile("fence.proxy.async.global;" ::: "memory");      // the bulk copy below reads what the upload wrote
-      s_abort = abort_;
-    }
-    __syncthreads();
-    if (s_abort) return;
-  }
+  if (kFused && G.gate && gate_wait(G, q, s_abort)) return;
   // PAIR_LOOSE: obstacle block read from global memory, boxes from global memory, or an unsorted lateral grid
   const bool stage_dyn = !(kFeat & PAIR_LOOSE) || G.stage_dyn, box_smem = !(kFeat & PAIR_LOOSE) || G.box_smem, d_sorted = !(kFeat & PAIR_LOOSE) || P.d_sorted;
   const int vwords = (kFeat & PAIR_BUDGET) ? G.vwords : 0;
@@ -265,29 +212,9 @@ fot_sweep_pairs(const Plan P, const Batch B, const Out O_, const PairGeom G) {
   // them all silently (empty / non-finite guards fp.py:933-946).
   const bool state_ok = fabs(qc[0]) + fabs(qc[1]) + fabs(qc[2]) + fabs(qc[3]) + fabs(qc[4]) + fabs(qc[5]) < INFINITY;
   if (kFused && G.fused_box && staged) {
-    // box every predicted trajectory of the staged obstacle block (what fot_prepass does for a resident tensor):
-    // one warp per trajectory, fp32 rounded outward, NaN trajectory -> NaN box
+    // box every predicted trajectory of the staged obstacle block
     mbar_wait(&s_bar, 0u);
-    for (int j = wid; j < SP; j += bd >> 5) {
-      const double2* src = dynst + (size_t)j * B.T_obs;
-      double xlo = INFINITY, xhi = -INFINITY, ylo = INFINITY, yhi = -INFINITY;
-      bool bad = false;
-      for (int k = lane; k < B.T_obs; k += 32) {
-        const double2 o = src[k];
-        bad |= (o.x != o.x) || (o.y != o.y);
-        xlo = fmin(xlo, o.x); xhi = fmax(xhi, o.x); ylo = fmin(ylo, o.y); yhi = fmax(yhi, o.y);
-      }
-      for (int off = 16; off > 0; off >>= 1) {
-        xlo = fmin(xlo, __shfl_xor_sync(full, xlo, off)); xhi = fmax(xhi, __shfl_xor_sync(full, xhi, off));
-        ylo = fmin(ylo, __shfl_xor_sync(full, ylo, off)); yhi = fmax(yhi, __shfl_xor_sync(full, yhi, off));
-      }
-      bad = __any_sync(full, bad);
-      if (lane == 0) {
-        const float nanf_ = __int_as_float(0x7fc00000);
-        sbox[j] = bad ? make_float4(nanf_, nanf_, nanf_, nanf_)
-                      : make_float4(__double2float_rd(xlo), __double2float_ru(xhi), __double2float_rd(ylo), __double2float_ru(yhi));
-      }
-    }
+    box_staged(dynst, sbox, SP, B.T_obs, wid, bd >> 5, lane);
     __syncthreads();
   }
 
@@ -421,7 +348,7 @@ fot_sweep_pairs(const Plan P, const Batch B, const Out O_, const PairGeom G) {
         const double s = pc[0] + pc[1] * tp.t + pc[2] * tp.t2 + pc[3] * tp.t3 + pc[4] * tp.t4;             // fp.py:644
         i_sd = held ? 0.0 : pc[1] + 2.0 * pc[2] * tp.t + 3.0 * pc[3] * tp.t2 + 4.0 * pc[4] * tp.t3;       // fp.py:645
         i_sdd = held ? 0.0 : 2.0 * pc[2] + 6.0 * pc[3] * tp.t + 12.0 * pc[4] * tp.t2;                      // fp.py:646
-        const RefFast rp = spline_ref_smem(S.spl, P.cfg.nx, s);
+        const RefFast rp = spline_ref_tab(SmemSplineTab{S.spl}, P.cfg.nx, s);
         i_rx = rp.rx; i_ry = rp.ry; i_cth = rp.cth; i_sth = rp.sth; i_rk = rp.rk; i_rdk = rp.rdk;
         i_isd = fabs(i_sd) > 1e-3 ? rcp_nr(i_sd) : 0.0;                            // fp.py:792 EPS_S_DOT
         {
