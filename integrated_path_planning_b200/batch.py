@@ -6,12 +6,13 @@ during compute; `gather_winners` is the single collective (SURVEY.md section 8e)
 """
 from __future__ import annotations
 
+import dataclasses
 from typing import Optional
 
 import numpy as np
 
 from . import _lib
-from .engine import SweepEngine, SweepResult, speed_grid_batch
+from .engine import SweepEngine, SweepResult, fot_batch, fot_result, query_arrays, winner_fields
 from .frenet_host import BatchCoordinateConverter, ego_to_frenet_many
 from .planner import FrenetPlanner
 
@@ -41,26 +42,22 @@ class BatchFrenetPlanner(FrenetPlanner):
         _lib.COST_WEIGHT_KEYS): also every query's winner under each weighting (`SweepResult.w_*`, `under_weights`),
         with its series unless weight_series is False.  cost_terms: also the five cost terms of every candidate
         (`SweepResult.cost_terms`).  With any of these the batch runs as a device-resident `DeviceBatch`."""
-        fs = np.asarray(frenet_states, dtype=np.float64).reshape(-1, 6)
-        n_q = fs.shape[0]
-        if limits is None:
-            limits = self.resolve_limits(constraint_overrides)
+        q, _ = self._batch_arrays(frenet_states, target_speed, dynamic_obstacles, distribution, static_obstacles,
+                                  constraint_overrides, limits, max_stop_distance)
+        return self._run(q, want_candidates, winner_samples, top_k, rank_series, cost_weights, weight_series, cost_terms)
+
+    def _batch_arrays(self, frenet_states, target_speed, dynamic_obstacles=None, distribution=None,
+                      static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None, **run):
+        """(the checked inputs of `plan_batch`, its remaining keywords)."""
         mode, dyn = _lib.FOT_DYN_NONE, None
         if distribution is not None and np.size(distribution) > 0:
             mode, dyn = _lib.FOT_DYN_DISTRIBUTION, np.asarray(distribution, dtype=np.float64)
         elif dynamic_obstacles is not None and np.size(dynamic_obstacles) > 0:
-            d = np.asarray(dynamic_obstacles, dtype=np.float64)
-            mode, dyn = _lib.FOT_DYN_SINGLE, d.reshape(n_q, 1, *d.shape[1:])
-        per_query = static_obstacles is not None and np.ndim(static_obstacles) == 3
-        if top_k > 0 or cost_weights is not None or cost_terms:
-            db = DeviceBatch(self, fs, target_speed, dyn, mode, limits=limits, max_stop_distance=max_stop_distance,
-                             static_obstacles=static_obstacles, top_k=top_k, rank_series=rank_series,
-                             cost_weights=cost_weights, weight_series=weight_series, cost_terms=cost_terms)
-            db.launch()
-            return db.sweep_result(want_candidates, winner_samples)
-        return self.engine.run_host(fs, target_speed, limits, max_stop_distance, static_obstacles, dyn, mode,
-                                    static_per_query=per_query, want_candidates=want_candidates,
-                                    winner_samples=winner_samples)
+            mode, dyn = _lib.FOT_DYN_SINGLE, np.asarray(dynamic_obstacles, dtype=np.float64)[:, None]
+        if limits is None:
+            limits = self.resolve_limits(constraint_overrides)
+        return query_arrays(frenet_states, target_speed, limits, max_stop_distance, static_obstacles, dyn, mode,
+                            self.d_t_s), run
 
     def plan_batch_from_ego(self, ego, target_speed, last_kappa=0.0, converter: Optional[BatchCoordinateConverter] = None,
                             **kwargs):
@@ -69,26 +66,17 @@ class BatchFrenetPlanner(FrenetPlanner):
         ego q; None: fresh ones on this planner's device, as a first plan() call has).  The nearest-point search runs
         on the device (DESIGN.md section 4e), the rest of the Frenet conversion on the host, then `plan_batch` with
         **kwargs.  Returns (SweepResult, ok): where ok is False the conversion failed and plan() would return None --
-        best_idx -1, best_cost inf, stats zero, winner_len 0."""
+        best_idx -1, best_cost inf, stats zero, winner_len 0 (`SweepResult.blank`)."""
         ego = np.asarray(ego, dtype=np.float64).reshape(-1, 5)
         n_q = ego.shape[0]
+        q, run = self._batch_arrays(np.zeros((n_q, 6)), target_speed, **kwargs)    # checked before the device is used
         if converter is None:
             converter = BatchCoordinateConverter(self.csp, n_q, engine=self.engine)
         kappa = np.broadcast_to(np.asarray(last_kappa, dtype=np.float64), (n_q,))
         frenet, ok = ego_to_frenet_many(converter, np.arange(n_q), ego, kappa)
-        res = self.plan_batch(frenet, target_speed, **kwargs)
-        bad = ~ok
-        res.best_idx[bad], res.best_cost[bad], res.stats[bad], res.winner_len[bad] = -1, np.inf, 0, 0
-        if res.rank_idx is not None:
-            res.rank_idx[bad], res.rank_cost[bad] = -1, np.inf
-            if res.rank_len is not None:
-                res.rank_len[bad] = 0
-        if res.w_idx is not None:
-            res.w_idx[bad], res.w_cost[bad] = -1, np.inf
-            if res.w_len is not None:
-                res.w_len[bad] = 0
-        if res.cost_terms is not None:
-            res.cost_terms[bad] = np.nan
+        q.frenet[:] = frenet
+        res = self._run(q, **run)
+        res.blank(~ok)
         return res, ok
 
 
@@ -110,83 +98,54 @@ class DeviceBatch:
                  max_stop_distance=None, static_obstacles=None, top_k: int = 0, rank_series: bool = True,
                  cost_weights=None, weight_series: bool = True, cost_terms: bool = False):
         import torch
-        eng = planner.engine
-        dev = torch.device("cuda", eng.device)
-        fs = np.ascontiguousarray(frenet_states, dtype=np.float64).reshape(-1, 6)
-        n_q = fs.shape[0]
-        target = np.array(np.broadcast_to(np.asarray(target_speed, np.float64), (n_q,)))
-        lim = planner.resolve_limits(None) if limits is None else limits
-        lim = np.array(np.broadcast_to(np.asarray(lim, np.float64), (n_q, 4)))
-        stop = np.full(n_q, np.nan) if max_stop_distance is None else \
-            np.array(np.broadcast_to(np.asarray(max_stop_distance, np.float64), (n_q,)))
-        v_grid, n_v = speed_grid_batch(target, eng.d_t_s)
-        up = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
-        self.t = {"frenet": up(fs), "target": up(target), "limits": up(lim), "stop": up(stop),
-                  "v_grid": up(v_grid), "n_v": up(n_v)}
-        self.engine, self.n_q = eng, n_q
-        self.n_v_host, self.frenet_host = n_v, fs
-        b = _lib.FotBatch()
-        b.n_q, b.n_v_max = n_q, v_grid.shape[1]
-        b.frenet, b.target_speed, b.limits = self.t["frenet"].data_ptr(), self.t["target"].data_ptr(), self.t["limits"].data_ptr()
-        b.stop_dist, b.v_grid, b.n_v = self.t["stop"].data_ptr(), self.t["v_grid"].data_ptr(), self.t["n_v"].data_ptr()
-        if static_obstacles is not None and np.size(static_obstacles) > 0:
-            st = np.ascontiguousarray(static_obstacles, dtype=np.float64)
-            self.t["static"] = up(st)
-            b.static_obs, b.n_static, b.static_per_query = self.t["static"].data_ptr(), st.shape[-2], int(st.ndim == 3)
-        if dyn_mode != _lib.FOT_DYN_NONE:
-            if isinstance(dyn, np.ndarray):
-                dyn = up(np.ascontiguousarray(dyn, dtype=np.float64))
-            assert dyn.dim() == 5 and dyn.shape[0] == n_q and dyn.shape[-1] == 2 and dyn.dtype == torch.float64
-            self.t["dyn"] = dyn.contiguous()
-            b.dyn, b.S, b.P, b.T_obs, b.dyn_mode = self.t["dyn"].data_ptr(), dyn.shape[1], dyn.shape[2], dyn.shape[3], dyn_mode
-        self.batch = b
-        # the whole winner block in one contiguous buffer (what the sharded sweep gathers with one collective)
-        self.block = WinnerBlock(n_q, eng.n_t_max, device=dev)
-        self.out = self.block.views
-        r = _lib.FotResult()
-        r.best_idx, r.best_cost, r.stats = self.out["best_idx"].data_ptr(), self.out["best_cost"].data_ptr(), self.out["stats"].data_ptr()
-        r.winner_len, r.winner = self.out["winner_len"].data_ptr(), self.out["winner"].data_ptr()
-        self.result = r
+        q = query_arrays(frenet_states, target_speed, planner.resolve_limits(None) if limits is None else limits,
+                         max_stop_distance, static_obstacles, dyn, dyn_mode, planner.d_t_s)
+        n_q = len(q.frenet)
         self.top_k = int(top_k)
         if self.top_k > _lib.FOT_MAX_RANKED:
             raise ValueError(f"top_k must be in [1, {_lib.FOT_MAX_RANKED}]")
         weights, per_query = _weight_table(cost_weights, n_q)
         self.n_w = 0 if weights is None else weights.shape[-2]
-        self.stride = eng.lib.fot_candidate_count(eng._h, int(b.n_v_max), 1)
+        eng = planner.engine
+        dev = torch.device("cuda", eng.device)
+        self.engine, self.n_q = eng, n_q
+        self.n_v_host, self.frenet_host = q.n_v, q.frenet
+        # the inputs on the device; a torch dyn stays where it is
+        self.t = {key: a if isinstance(a, torch.Tensor) else torch.from_numpy(a).to(dev)
+                  for key in ("frenet", "target", "limits", "stop", "v_grid", "n_v", "static", "dyn")
+                  if (a := getattr(q, key)) is not None}
+        self.batch = fot_batch(dataclasses.replace(q, **self.t), torch.Tensor.data_ptr)
+        # the whole winner block in one contiguous buffer (what the sharded sweep gathers with one collective)
+        self.block = WinnerBlock(n_q, eng.n_t_max, device=dev)
+        self.out = dict(self.block.views)
+        self.stride = eng.lib.fot_candidate_count(eng._h, int(self.batch.n_v_max), 1)
+
+        def new(where: dict, key: str, shape, dtype) -> int:
+            where[key] = torch.empty(shape, dtype=dtype, device=dev)
+            return where[key].data_ptr()
+
+        def selections(prefix: str, m: int, series: bool, s):      # s: a FotRanked or FotWeighted
+            s.idx = new(self.out, prefix + "_idx", (n_q, m), torch.int32)
+            s.cost = new(self.out, prefix + "_cost", (n_q, m), torch.float64)
+            if series:
+                s.len = new(self.out, prefix + "_len", (n_q, m), torch.int32)
+                s.series = new(self.out, prefix + "_series", (n_q, m, _lib.FOT_N_SERIES, eng.n_t_max), torch.float64)
+            return s
+
         if self.top_k > 0 or self.n_w > 0:
-            self.t["cand_cat"] = torch.empty((n_q, self.stride), dtype=torch.uint8, device=dev)
-            r.cand_cat, r.cand_stride = self.t["cand_cat"].data_ptr(), self.stride
+            new(self.t, "cand_cat", (n_q, self.stride), torch.uint8)
         if self.top_k > 0:
-            self.t["cand_cost"] = torch.empty((n_q, self.stride), dtype=torch.float64, device=dev)
-            r.cand_cost = self.t["cand_cost"].data_ptr()
-            k = self.top_k
-            self.out = dict(self.out, rank_idx=torch.empty((n_q, k), dtype=torch.int32, device=dev),
-                            rank_cost=torch.empty((n_q, k), dtype=torch.float64, device=dev))
-            rk = _lib.FotRanked()
-            rk.k, rk.idx, rk.cost = k, self.out["rank_idx"].data_ptr(), self.out["rank_cost"].data_ptr()
-            if rank_series:
-                self.out["rank_len"] = torch.empty((n_q, k), dtype=torch.int32, device=dev)
-                self.out["rank_series"] = torch.empty((n_q, k, _lib.FOT_N_SERIES, eng.n_t_max), dtype=torch.float64,
-                                                      device=dev)
-                rk.len, rk.series = self.out["rank_len"].data_ptr(), self.out["rank_series"].data_ptr()
-            self.ranked = rk
+            new(self.t, "cand_cost", (n_q, self.stride), torch.float64)
+            self.ranked = selections("rank", self.top_k, rank_series, _lib.FotRanked(k=self.top_k))
         if self.n_w > 0:
-            n_w = self.n_w
-            self.t["weights"] = up(weights)
-            self.out = dict(self.out, w_idx=torch.empty((n_q, n_w), dtype=torch.int32, device=dev),
-                            w_cost=torch.empty((n_q, n_w), dtype=torch.float64, device=dev))
-            wt = _lib.FotWeighted()
-            wt.n_w, wt.per_query, wt.weights = n_w, per_query, self.t["weights"].data_ptr()
-            wt.idx, wt.cost = self.out["w_idx"].data_ptr(), self.out["w_cost"].data_ptr()
-            if weight_series:
-                self.out["w_len"] = torch.empty((n_q, n_w), dtype=torch.int32, device=dev)
-                self.out["w_series"] = torch.empty((n_q, n_w, _lib.FOT_N_SERIES, eng.n_t_max), dtype=torch.float64,
-                                                   device=dev)
-                wt.len, wt.series = self.out["w_len"].data_ptr(), self.out["w_series"].data_ptr()
-            self.weighted = wt
+            self.t["weights"] = torch.from_numpy(weights).to(dev)
+            self.weighted = selections("w", self.n_w, weight_series,
+                                       _lib.FotWeighted(n_w=self.n_w, per_query=per_query,
+                                                        weights=self.t["weights"].data_ptr()))
         self.cost_terms = bool(cost_terms)
         if self.cost_terms:
-            self.out = dict(self.out, cost_terms=torch.empty((n_q, self.stride, 5), dtype=torch.float64, device=dev))
+            new(self.out, "cost_terms", (n_q, self.stride, 5), torch.float64)
+        self.result = fot_result(dict(self.out, **self.t), torch.Tensor.data_ptr)
 
     def launch(self, stream: Optional[int] = None) -> None:
         """Enqueue prepass + sweep + winner kernels on `stream` (raw cudaStream_t).  None: torch's current stream
@@ -214,20 +173,13 @@ class DeviceBatch:
         """Host copy of the outputs of the last launch, once it has finished (launch() without a stream waits), as a
         SweepResult: the candidate table only with want_candidates, which needs top_k > 0 (or cost_weights, for the
         categories alone); winner_samples = k > 0: the first k samples of each winner series."""
-        h = {k: v.cpu().numpy() for k, v in self.out.items()}
+        res = SweepResult(**{k: v.cpu().numpy() for k, v in self.out.items()})
         if winner_samples and winner_samples > 0:
-            h["winner"] = np.ascontiguousarray(h["winner"][:, :, :min(int(winner_samples), h["winner"].shape[2])])
-        res = SweepResult(best_idx=h["best_idx"], best_cost=h["best_cost"], stats=h["stats"],
-                          winner_len=h["winner_len"], winner=h["winner"], rank_idx=h.get("rank_idx"),
-                          rank_cost=h.get("rank_cost"), rank_len=h.get("rank_len"), rank_series=h.get("rank_series"),
-                          w_idx=h.get("w_idx"), w_cost=h.get("w_cost"), w_len=h.get("w_len"),
-                          w_series=h.get("w_series"), cost_terms=h.get("cost_terms"))
+            res.winner = np.ascontiguousarray(res.winner[:, :, :min(int(winner_samples), res.winner.shape[2])])
         if want_candidates:
             res.cand_cat = self.t["cand_cat"].cpu().numpy()
             res.cand_cost = self.t["cand_cost"].cpu().numpy() if "cand_cost" in self.t else None
-        res.n_cand = self.engine.candidate_counts(self.frenet_host, self.n_v_host)
-        res.kernel_ms = self.engine.last_kernel_ms()
-        return res
+        return self.engine.finish_result(res, self.frenet_host, self.n_v_host)
 
     def launch_to_host(self, host_out: dict, stream: Optional[int] = None, winner_samples: int = 0) -> None:
         """fot_plan_batch_device_to_host: sweep the (device-resident) batch and deliver the winners into the host
@@ -244,10 +196,7 @@ class DeviceBatch:
             raise ValueError("launch_to_host does not return weighted outputs or cost terms; use launch()")
         import ctypes as C
         ptr = lambda a: a.data_ptr() if hasattr(a, "data_ptr") else a.ctypes.data
-        r = _lib.FotResult()
-        r.best_idx, r.best_cost, r.stats = ptr(host_out["best_idx"]), ptr(host_out["best_cost"]), ptr(host_out["stats"])
-        r.winner_len, r.winner = ptr(host_out["winner_len"]), ptr(host_out["winner"])
-        r.winner_samples = int(winner_samples)
+        r = fot_result(host_out, ptr, winner_samples)
         _lib.check(self.engine.lib.fot_plan_batch_device_to_host(self.engine._h, C.byref(self.batch), C.byref(r),
                                                                  C.c_void_p(stream) if stream else None),
                    "fot_plan_batch_device_to_host")
@@ -287,9 +236,7 @@ class WinnerBlock:
     def __init__(self, cap: int, n_t_max: int, device=None, sections=None):
         import torch
         self.cap = int(cap)
-        self.sections = sections or (("best_idx", torch.int32, ()), ("winner_len", torch.int32, ()),
-                                     ("stats", torch.int32, (_lib.FOT_N_STATS,)), ("best_cost", torch.float64, ()),
-                                     ("winner", torch.float64, (_lib.FOT_N_SERIES, int(n_t_max))))
+        self.sections = sections or winner_fields(n_t_max)
         self.offsets, off = {}, 0
         for key, dt, shape in self.sections:
             n = self.cap * int(np.prod(shape, dtype=np.int64)) * torch.empty((), dtype=dt).element_size()
@@ -415,10 +362,7 @@ class PeerGather:
             k = self.step
             self.step += 1
         p = self._slice_ptr(k, self.rank)
-        m = _lib.FotResult()
-        off = self.layout.offsets
-        m.best_idx, m.winner_len, m.stats = p + off["best_idx"][0], p + off["winner_len"][0], p + off["stats"][0]
-        m.best_cost, m.winner = p + off["best_cost"][0], p + off["winner"][0]
+        m = fot_result({key: p + off for key, (off, _) in self.layout.offsets.items()}, int)
         _lib.check(self.lib.fot_set_result_mirror(self.engine._h, C.byref(m), C.c_void_p(self.flags_ptr + 4 * self.rank)),
                    "fot_set_result_mirror")
 

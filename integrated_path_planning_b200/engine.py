@@ -11,8 +11,10 @@ The candidate sweep itself runs only on the GPU (csrc/fot_kernels.cuh) through t
 from __future__ import annotations
 
 import ctypes as C
+import functools
+import itertools
 from dataclasses import dataclass
-from typing import Optional
+from typing import Any, Optional
 
 import numpy as np
 
@@ -25,7 +27,7 @@ BRAKE_T_STEP = 0.5
 
 
 def _ptr(a: Optional[np.ndarray]):
-    return None if a is None else a.ctypes.data_as(C.c_void_p)
+    return None if a is None else a.ctypes.data
 
 
 def horizon_grid(min_t, max_t, dt) -> np.ndarray:
@@ -84,6 +86,92 @@ def time_table(T, dt):
     return n_steps, np.linalg.inv(quartic), np.linalg.inv(quintic)
 
 
+def winner_fields(n_t: int):
+    """The winner block of fot_result_t as (name, torch dtype, per-query shape) with n_t samples per winner series, in
+    the order of `WinnerBlock`'s sections: that order is the byte layout the gathers of the sharded sweep move."""
+    import torch
+    return (("best_idx", torch.int32, ()), ("winner_len", torch.int32, ()), ("stats", torch.int32, (_lib.FOT_N_STATS,)),
+            ("best_cost", torch.float64, ()), ("winner", torch.float64, (_lib.FOT_N_SERIES, int(n_t))))
+
+
+@dataclass
+class QueryArrays:
+    """A batch's inputs as fot_batch_t reads them (`query_arrays` builds and checks them)."""
+    frenet: np.ndarray            # [n_q, 6]
+    target: np.ndarray            # [n_q]
+    limits: np.ndarray            # [n_q, 4]
+    stop: np.ndarray              # [n_q], NaN = none
+    v_grid: np.ndarray            # [n_q, n_v_max]
+    n_v: np.ndarray               # [n_q] int32
+    static: Optional[np.ndarray]  # [M, 2] shared or [n_q, M, 2] per query; None when empty
+    static_per_query: bool
+    dyn: Any                      # [n_q, S, P, T, 2] float64, a NumPy array or a CUDA torch tensor; None for FOT_DYN_NONE
+    dyn_mode: int
+
+
+@functools.lru_cache(maxsize=8)
+def _uniform_speed_grid(target_speed: float, n_q: int, d_t_s: float):
+    return speed_grid_batch(np.full(n_q, target_speed), d_t_s)
+
+
+def query_arrays(frenet, target_speed, limits, stop_dist, static, dyn, dyn_mode, d_t_s) -> QueryArrays:
+    """A batch's inputs as QueryArrays, from target_speed and stop_dist (None: no stop distance) as scalars or [n_q],
+    limits [4] or [n_q,4], and dyn as a NumPy array (converted) or a torch tensor.  Raises ValueError on a static or
+    dyn of any other shape than QueryArrays lists: the C side reads them at the offsets those shapes give."""
+    frenet = np.ascontiguousarray(frenet, dtype=np.float64).reshape(-1, 6)
+    n_q = frenet.shape[0]
+    full = lambda a, shape: np.array(np.broadcast_to(np.asarray(a, dtype=np.float64), shape), order="C")
+    target = full(target_speed, (n_q,))
+    if np.ndim(target_speed) == 0:      # one target speed for the whole batch (the usual case): an earlier call's grid
+        v_grid, n_v = _uniform_speed_grid(float(target_speed), n_q, float(d_t_s))
+    else:
+        v_grid, n_v = speed_grid_batch(target, d_t_s)
+    static = np.ascontiguousarray(static, dtype=np.float64) if static is not None and np.size(static) > 0 else None
+    if static is not None and (static.ndim not in (2, 3) or static.shape[-1] != 2 or
+                               (static.ndim == 3 and static.shape[0] != n_q)):
+        raise ValueError(f"static obstacles must be [M, 2] or [n_q={n_q}, M, 2], got {list(static.shape)}")
+    if dyn_mode == _lib.FOT_DYN_NONE:
+        dyn = None
+    else:
+        if hasattr(dyn, "data_ptr"):                # a torch tensor stays where it is
+            import torch
+            dyn, f64 = dyn.contiguous(), torch.float64
+        else:
+            dyn, f64 = np.ascontiguousarray(dyn, dtype=np.float64), np.float64
+        if dyn.ndim != 5 or dyn.shape[0] != n_q or dyn.shape[-1] != 2 or dyn.dtype != f64:
+            raise ValueError(f"dyn must be float64 [n_q={n_q}, S, P, T, 2], got {dyn.dtype} {list(dyn.shape)}")
+    return QueryArrays(frenet, target, full(limits, (n_q, 4)),
+                       full(np.nan if stop_dist is None else stop_dist, (n_q,)), v_grid, n_v, static,
+                       static is not None and static.ndim == 3, dyn, dyn_mode)
+
+
+def fot_batch(q: QueryArrays, ptr) -> "_lib.FotBatch":
+    """fot_batch_t over the arrays of q (host arrays or their device copies); ptr maps one to its address."""
+    b = _lib.FotBatch()
+    b.n_q, b.n_v_max = len(q.frenet), q.v_grid.shape[1]
+    b.frenet, b.target_speed, b.limits, b.stop_dist = ptr(q.frenet), ptr(q.target), ptr(q.limits), ptr(q.stop)
+    b.v_grid, b.n_v = ptr(q.v_grid), ptr(q.n_v)
+    if q.static is not None:
+        b.static_obs, b.n_static, b.static_per_query = ptr(q.static), q.static.shape[-2], int(q.static_per_query)
+    if q.dyn is not None:
+        b.dyn, b.dyn_mode = ptr(q.dyn), q.dyn_mode
+        b.S, b.P, b.T_obs = q.dyn.shape[1], q.dyn.shape[2], q.dyn.shape[3]
+    return b
+
+
+def fot_result(arrays, ptr, winner_samples: int = 0) -> "_lib.FotResult":
+    """fot_result_t over the winner-block fields of arrays and, where not None, its cand_cat / cand_cost (addresses: ptr)."""
+    r = _lib.FotResult()
+    for name, _, _ in winner_fields(0):
+        setattr(r, name, ptr(arrays[name]))
+    if arrays.get("cand_cat") is not None:
+        r.cand_cat, r.cand_stride = ptr(arrays["cand_cat"]), arrays["cand_cat"].shape[1]
+    if arrays.get("cand_cost") is not None:
+        r.cand_cost = ptr(arrays["cand_cost"])
+    r.winner_samples = int(winner_samples)
+    return r
+
+
 @dataclass
 class SweepResult:
     """Host copy of fot_result_t for n_q queries."""
@@ -119,46 +207,46 @@ class SweepResult:
     def alternatives(self, q: int = 0):
         """The ranked alternatives of query q, best first: a list of {"index", "cost", "series"}, where series holds
         the 15 sequences truncated to their kept length (None when the series were not requested)."""
-        out = []
-        for r in range(self.rank_idx.shape[1]):
-            i = int(self.rank_idx[q, r])
-            if i < 0:
-                break
-            series = None
-            if self.rank_series is not None:
-                n = int(self.rank_len[q, r])
-                series = {name: self.rank_series[q, r, j, :n].copy() for j, name in enumerate(SERIES)}
-            out.append({"index": i, "cost": np.float64(self.rank_cost[q, r]), "series": series})
-        return out
+        entries = (self._entry("rank", q, r) for r in range(self.rank_idx.shape[1]))
+        return list(itertools.takewhile(lambda e: e is not None, entries))
 
     def under_weights(self, q: int = 0):
         """The winner of query q under each weighting, in weighting order: {"index", "cost", "series"} (series: the 15
         sequences truncated to their kept length, or None when they were not requested), or None where no candidate
         is feasible under that weighting."""
-        out = []
-        for w in range(self.w_idx.shape[1]):
-            i = int(self.w_idx[q, w])
-            if i < 0:
-                out.append(None)
-                continue
-            series = None
-            if self.w_series is not None:
-                n = int(self.w_len[q, w])
-                series = {name: self.w_series[q, w, j, :n].copy() for j, name in enumerate(SERIES)}
-            out.append({"index": i, "cost": np.float64(self.w_cost[q, w]), "series": series})
-        return out
+        return [self._entry("w", q, w) for w in range(self.w_idx.shape[1])]
+
+    def _entry(self, block: str, q: int, j: int):
+        """Entry j of query q of the ranked ("rank") or weighted ("w") outputs, or None where its index is -1."""
+        i = int(getattr(self, block + "_idx")[q, j])
+        if i < 0:
+            return None
+        series, lens = getattr(self, block + "_series"), getattr(self, block + "_len")
+        if series is not None:
+            n = int(lens[q, j])
+            series = {name: series[q, j, s, :n].copy() for s, name in enumerate(SERIES)}
+        return {"index": i, "cost": np.float64(getattr(self, block + "_cost")[q, j]), "series": series}
+
+    def blank(self, rows) -> None:
+        """Queries `rows` (indices or a mask) as plan() returning None leaves them: index -1, cost inf, stats and kept
+        lengths 0 in the winner, ranked and weighted outputs, cost terms NaN; the series and candidate table stay."""
+        for name, value in (("best_idx", -1), ("best_cost", np.inf), ("stats", 0), ("winner_len", 0), ("rank_idx", -1),
+                            ("rank_cost", np.inf), ("rank_len", 0), ("w_idx", -1), ("w_cost", np.inf), ("w_len", 0),
+                            ("cost_terms", np.nan)):
+            a = getattr(self, name)
+            if a is not None:
+                a[rows] = value
 
 
 class SweepEngine:
     """Owns one fot handle (one device).  Built from the planner's constructor knobs."""
 
     def __init__(self, reference_path, *, max_speed, dt, d_road_w, max_road_width, robot_radius,
-                 obstacle_radius, min_t, max_t, d_t_s, k_j, k_t, k_d, k_s_dot, k_lat, k_lon,
+                 obstacle_radius, min_t, max_t, k_j, k_t, k_d, k_s_dot, k_lat, k_lon,
                  chance_epsilon=0.0, collision_margin_inflation=1.0, footprint=None, device=0):
         self.lib = _lib.load()
         self.device = int(device)
         self.dt = dt
-        self.d_t_s = d_t_s
         sp = spline_tables(reference_path)
 
         T = horizon_grid(min_t, max_t, dt)
@@ -212,7 +300,6 @@ class SweepEngine:
         self.T, self.d_grid, self.Tb = self._keep["T"], self._keep["d_grid"], self._keep["Tb"]
         self.n_steps, self.n_steps_b, self.n_total = self._keep["n_steps"], self._keep["n_steps_b"], n_total
         self._pinned = {}
-        self._grid_cache = None
         self._near_bufs = None                             # nearest_s: pinned / device staging, grown on demand
         self._near_stream = None                           # nearest_s: its stream
         self._h = C.c_void_p()
@@ -241,55 +328,20 @@ class SweepEngine:
         has_brake = (frenet[:, 1] > 0.1) & (self.n_B > 0)
         return per_T * n_v.astype(np.int64) * self.n_d + has_brake * self.n_B * self.n_total
 
-    def run_host(self, frenet, target_speed, limits, stop_dist=None, static=None, dyn=None,
-                 dyn_mode=_lib.FOT_DYN_NONE, static_per_query=False, want_candidates=False,
-                 winner_samples: int = 0) -> SweepResult:
-        """One fot_plan_batch_host call.  Shapes: frenet [n_q,6], target_speed [n_q], limits [n_q,4],
-        stop_dist [n_q] (NaN = none), static [M,2] or [n_q,M,2], dyn [n_q,S,P,T,2].
-        winner_samples = k > 0: only the first k samples of each winner series come back (`winner` is
-        [n_q,15,k]); `fetch_winners` reads full series of the last call from the device."""
-        f64c = lambda a: np.ascontiguousarray(a, dtype=np.float64)
-        frenet = f64c(frenet).reshape(-1, 6)
-        n_q = frenet.shape[0]
-        target = f64c(np.broadcast_to(np.asarray(target_speed, dtype=np.float64), (n_q,)))
-        limits = f64c(np.broadcast_to(np.asarray(limits, dtype=np.float64), (n_q, 4)))
-        stop = f64c(np.full(n_q, np.nan) if stop_dist is None else np.broadcast_to(np.asarray(stop_dist, dtype=np.float64), (n_q,)))
-        # one target speed for the whole batch (the usual case): the grid of the previous call with the same target
-        key = (float(target_speed), n_q) if np.ndim(target_speed) == 0 else None
-        if key is not None and self._grid_cache is not None and self._grid_cache[0] == key:
-            v_grid, n_v = self._grid_cache[1]
-        else:
-            v_grid, n_v = speed_grid_batch(target, self.d_t_s)
-            self._grid_cache = (key, (v_grid, n_v)) if key is not None else None
-        b = _lib.FotBatch()
-        b.n_q, b.n_v_max = n_q, v_grid.shape[1]
-        b.frenet, b.target_speed, b.limits, b.stop_dist = _ptr(frenet), _ptr(target), _ptr(limits), _ptr(stop)
-        b.v_grid, b.n_v = _ptr(v_grid), _ptr(n_v)
-        keep = [frenet, target, limits, stop, v_grid, n_v]
-        if static is not None and np.size(static) > 0:
-            static = f64c(static)
-            b.n_static = static.shape[-2]
-            b.static_per_query = int(bool(static_per_query))
-            b.static_obs = _ptr(static)
-            keep.append(static)
-        if dyn_mode != _lib.FOT_DYN_NONE:
-            dyn = f64c(dyn)
-            if dyn.ndim != 5 or dyn.shape[0] != n_q or dyn.shape[-1] != 2:
-                raise ValueError(f"dyn must be [n_q,S,P,T,2], got {dyn.shape}")
-            b.S, b.P, b.T_obs = dyn.shape[1], dyn.shape[2], dyn.shape[3]
-            b.dyn, b.dyn_mode = _ptr(dyn), dyn_mode
-            keep.append(dyn)
+    def run_host(self, q: QueryArrays, want_candidates=False, winner_samples: int = 0) -> SweepResult:
+        """One fot_plan_batch_host call on the host arrays of q.  winner_samples = k > 0: only the first k samples
+        of each winner series come back (`winner` is [n_q,15,k]); `fetch_winners` reads full series of the last
+        call from the device."""
         k_head = min(int(winner_samples), self.n_t_max) if winner_samples and winner_samples > 0 else 0
-        res = self._result_buffers(n_q, want_candidates, int(b.n_v_max), k_head)
-        r = _lib.FotResult()
-        r.winner_samples = k_head
-        r.best_idx, r.best_cost, r.stats = _ptr(res.best_idx), _ptr(res.best_cost), _ptr(res.stats)
-        r.winner_len, r.winner = _ptr(res.winner_len), _ptr(res.winner)
-        if want_candidates:
-            r.cand_cat, r.cand_cost, r.cand_stride = _ptr(res.cand_cat), _ptr(res.cand_cost), res.cand_cat.shape[1]
+        res = self._result_buffers(len(q.frenet), want_candidates, q.v_grid.shape[1], k_head)
+        b, r = fot_batch(q, _ptr), fot_result(vars(res), _ptr, k_head)
         _lib.check(self.lib.fot_plan_batch_host(self._h, C.byref(b), C.byref(r)), "fot_plan_batch_host")
+        return self.finish_result(res, q.frenet, q.n_v)
+
+    def finish_result(self, res: SweepResult, frenet: np.ndarray, n_v: np.ndarray) -> SweepResult:
+        """res with the candidates generated per query and the device time of the last launch filled in."""
         res.n_cand = self.candidate_counts(frenet, n_v)
-        res.kernel_ms = float(self.lib.fot_last_kernel_ms(self._h))
+        res.kernel_ms = self.last_kernel_ms()
         return res
 
     def fetch_winners(self, q0: int, n: int) -> np.ndarray:
@@ -312,9 +364,7 @@ class SweepEngine:
         cached = self._pinned.get(key)
         if cached is None:
             pin = lambda shape, dt: torch.empty(shape, dtype=dt, pin_memory=True).numpy()
-            cached = dict(best_idx=pin((n_q,), torch.int32), best_cost=pin((n_q,), torch.float64),
-                          stats=pin((n_q, _lib.FOT_N_STATS), torch.int32), winner_len=pin((n_q,), torch.int32),
-                          winner=pin((n_q, _lib.FOT_N_SERIES, k_head or self.n_t_max), torch.float64))
+            cached = {name: pin((n_q, *shape), dt) for name, dt, shape in winner_fields(k_head or self.n_t_max)}
             if want_candidates:
                 cached["cand_cat"] = pin((n_q, stride), torch.uint8)
                 cached["cand_cost"] = pin((n_q, stride), torch.float64)

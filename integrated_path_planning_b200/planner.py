@@ -19,7 +19,7 @@ from typing import Dict, List, Optional
 import numpy as np
 
 from . import _lib
-from .engine import SweepEngine, SweepResult
+from .engine import QueryArrays, SweepEngine, SweepResult, query_arrays
 from .frenet_host import CoordinateConverter, ego_to_frenet
 from .types import FrenetPath, FrenetState, SERIES
 
@@ -127,7 +127,7 @@ class FrenetPlanner:
             self._engine = SweepEngine(
                 self.csp, max_speed=self.max_speed, dt=self.dt, d_road_w=self.d_road_w,
                 max_road_width=self.max_road_width, robot_radius=self.robot_radius,
-                obstacle_radius=self.obstacle_radius, min_t=self.min_t, max_t=self.max_t, d_t_s=self.d_t_s,
+                obstacle_radius=self.obstacle_radius, min_t=self.min_t, max_t=self.max_t,
                 k_j=self.k_j, k_t=self.k_t, k_d=self.k_d, k_s_dot=self.k_s_dot, k_lat=self.k_lat,
                 k_lon=self.k_lon, chance_epsilon=self.chance_epsilon,
                 collision_margin_inflation=self.collision_margin_inflation, footprint=self.footprint,
@@ -244,24 +244,29 @@ class FrenetPlanner:
         static = None
         if static_obstacles is not None and len(static_obstacles) > 0:
             static = np.asarray(static_obstacles, dtype=np.float64).reshape(-1, 2)
-        stop = np.nan if max_stop_distance is None else float(max_stop_distance)
-        frenet = np.asarray(frenet_state, dtype=np.float64).reshape(1, 6)
-        limits = self.resolve_limits(constraint_overrides)
-        if top_k > 0 or cost_weights is not None:
-            from .batch import DeviceBatch           # batch.py builds on this module
-            db = DeviceBatch(self, frenet, float(target_speed), dyn, mode, limits=limits, max_stop_distance=stop,
-                             static_obstacles=static, top_k=top_k, cost_weights=cost_weights)
-            db.launch()
-            res = db.sweep_result(want_candidates)
-        else:
-            res = self.engine.run_host(frenet, float(target_speed), limits, stop, static, dyn, mode,
-                                       want_candidates=want_candidates)
+        q = query_arrays(np.reshape(frenet_state, (1, 6)), float(target_speed), self.resolve_limits(constraint_overrides),
+                         max_stop_distance, static, dyn, mode, self.d_t_s)
+        res = self._run(q, want_candidates, top_k=top_k, cost_weights=cost_weights)
         self.last_result = res
         stats = {key: int(res.stats[0, _lib.STAT_KEYS.index(key)]) for key in _REF_STAT_ORDER}
         if max_stop_distance is not None:
             stats["stop_distance_error"] = int(res.stats[0, _lib.STAT_KEYS.index("stop_distance_error")])
         self.last_check_stats = stats
         return res
+
+    def _run(self, q: QueryArrays, want_candidates: bool = False, winner_samples: int = 0, top_k: int = 0,
+             rank_series: bool = True, cost_weights=None, weight_series: bool = True,
+             cost_terms: bool = False) -> SweepResult:
+        """Sweep the batch q: as a device-resident `DeviceBatch` when it asks for ranked alternatives, cost weightings
+        or cost terms (outputs only the device-side calls produce), otherwise through the host-pointer call."""
+        if top_k > 0 or cost_weights is not None or cost_terms:
+            from .batch import DeviceBatch           # batch.py builds on this module
+            db = DeviceBatch(self, q.frenet, q.target, q.dyn, q.dyn_mode, limits=q.limits, max_stop_distance=q.stop,
+                             static_obstacles=q.static, top_k=top_k, rank_series=rank_series,
+                             cost_weights=cost_weights, weight_series=weight_series, cost_terms=cost_terms)
+            db.launch()
+            return db.sweep_result(want_candidates, winner_samples)
+        return self.engine.run_host(q, want_candidates, winner_samples)
 
     def _feed_back_curvature(self, path: FrenetPath) -> FrenetPath:
         """The ego curvature the next call starts from (frenet_planner.py:301-302)."""
