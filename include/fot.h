@@ -36,7 +36,8 @@ extern "C" {
 #define FOT_ABI_MINOR 1     /* additions within a version that change no existing struct, entry point or behaviour, so a
                                caller built against an earlier minor of the same version keeps working; 0 at each new
                                version.  Version 8: 1: + fot_weighted_t, fot_select_weighted, fot_cost_terms (winners
-                               under many cost weightings, the five cost terms per candidate) */
+                               under many cost weightings, the five cost terms per candidate); + fot_route_t,
+                               fot_add_route, fot_set_routes (every query on its own reference path) */
 #define FOT_MAX_CIRCLES 8
 #define FOT_MAX_RANKED 32
 #define FOT_N_STATS 8    /* ok, max_speed, max_accel, max_curvature, max_lat_accel, road_bound, collision, stop_distance */
@@ -276,8 +277,9 @@ float fot_last_kernel_ms(const fot_handle_t* h);
 int fot_last_sweep_kind(const fot_handle_t* h);
 
 /* fot_sweep_pairs is compiled per set of optional modes (1 static obstacles, 2 footprint circles, 4 violation budget,
- * 8 per-candidate outputs, 16 unstaged obstacle block / unsorted lateral grid; DESIGN.md section 4d) and the smallest
- * instantiated superset of what a batch needs runs: the set of the last launch, or -1 if another kernel ran. */
+ * 8 per-candidate outputs, 16 unstaged obstacle block / unsorted lateral grid, 32 per-query routes; DESIGN.md sections
+ * 4d, 4h) and the smallest instantiated superset of what a batch needs runs: the set of the last launch, or -1 if
+ * another kernel ran. */
 int fot_last_pair_features(const fot_handle_t* h);
 
 /* Device time of the three stages of the `back`-th most recent launch on this handle (0 = the
@@ -289,6 +291,29 @@ int fot_launch_stage_ms(const fot_handle_t* h, int back, float ms[3]);
  * FP64/FP32 figure).  kind: 0 = FP64 FMA, 1 = FP32 FMA, 2 = packed FP32x2 FMA.
  * Writes achieved TFLOP/s (2 flops per FMA). */
 int fot_probe_fma_tflops(int device, int kind, double* tflops_out);
+
+/* ---- routes: every query on its own reference path (DESIGN.md section 4h) ------------------------------------------
+ * A handle plans on the path given to fot_create (route 0) and on any number of further paths registered with
+ * fot_add_route.  Only the path is per query: grids, dt, radii, cost weights and footprint stay the handle's.  A query
+ * on route r gives, bit for bit, what a handle created with route r's path gives for it. */
+typedef struct fot_route {   /* one more reference path: CubicSpline1D coefficients as in fot_tables_t, HOST pointers */
+  int32_t nx;                /* >= 2 knots */
+  const double* knots;       /* [nx] */
+  const double *xa, *xb, *xc, *xd, *ya, *yb, *yc, *yd;   /* [nx], [nx-1], [nx], [nx-1] */
+} fot_route_t;
+/* Copies a path to the handle's device; *route_id = 1, 2, ...  Route 0 is the path of fot_create.
+   Not while a call on this handle is in flight (it may reallocate the route tables). */
+int fot_add_route(fot_handle_t* h, const fot_route_t* route, int32_t* route_id);
+/* DEVICE pointer: route[i] is the route of query i (point i) of every following fot_plan_batch_device,
+   fot_plan_batch_device_to_host, fot_plan_batch_host, fot_rank_candidates, fot_select_weighted and
+   fot_nearest_s_device call on this handle; the array must cover that call's n_q (n) and stay valid until the call
+   has finished.  It is device memory for fot_plan_batch_host too.  NULL: every query on route 0, i.e. the behaviour
+   without routes.  A route id outside [0, n_routes) plans nothing for that query (best_idx -1, best_cost +inf, stats
+   zero, no ranked or weighted entry, its cand_cat entries left unwritten; the search gives s_out NaN, status 1) and no
+   route table is read for it.
+   Kernel choice and shared memory of a launch with a binding follow the LONGEST registered route: fot_sweep_pairs when
+   it has at most 48 knots, else fot_sweep_items, which keeps the tables in shared memory up to 128 knots. */
+int fot_set_routes(fot_handle_t* h, const int32_t* route);
 
 /* ---- next row (SURVEY.md section 8f, rank 1): the predictor's post-processing on the device ---------
  * Builds the obstacle tensor fot_batch_t.dyn consumes, so that batched roll-outs never upload it.

@@ -85,6 +85,14 @@ class FotWeighted(C.Structure):
     ]
 
 
+class FotRoute(C.Structure):
+    _fields_ = [
+        ("nx", C.c_int32), ("knots", c_double_p),
+        ("xa", c_double_p), ("xb", c_double_p), ("xc", c_double_p), ("xd", c_double_p),
+        ("ya", c_double_p), ("yb", c_double_p), ("yc", c_double_p), ("yd", c_double_p),
+    ]
+
+
 # every symbol include/fot.h declares: (name, restype, argtypes)
 SYMBOLS = (
     ("fot_abi_version", C.c_int, ()),
@@ -127,6 +135,8 @@ SYMBOLS = (
                                             C.c_void_p, C.c_double, c_double_p, C.c_int, C.c_void_p)),
     ("fot_nearest_s_device", C.c_int, (C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p)),
+    ("fot_add_route", C.c_int, (C.c_void_p, C.POINTER(FotRoute), C.POINTER(C.c_int32))),
+    ("fot_set_routes", C.c_int, (C.c_void_p, C.c_void_p)),
 )
 
 _lib = None

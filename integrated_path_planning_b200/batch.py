@@ -12,8 +12,8 @@ from typing import Optional
 import numpy as np
 
 from . import _lib
-from .engine import SweepEngine, SweepResult, fot_batch, fot_result, query_arrays, winner_fields
-from .frenet_host import BatchCoordinateConverter, ego_to_frenet_many
+from .engine import SweepEngine, SweepResult, fot_batch, fot_result, query_arrays, route_array, winner_fields
+from .frenet_host import BatchCoordinateConverter, RoutedCoordinateConverter, ego_to_frenet_many
 from .planner import FrenetPlanner
 
 
@@ -32,7 +32,7 @@ class BatchFrenetPlanner(FrenetPlanner):
                    static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None,
                    want_candidates: bool = False, winner_samples: int = 0, top_k: int = 0,
                    rank_series: bool = True, cost_weights=None, weight_series: bool = True,
-                   cost_terms: bool = False) -> SweepResult:
+                   cost_terms: bool = False, route=None) -> SweepResult:
         """frenet_states [n_q,6]; target_speed scalar or [n_q]; dynamic_obstacles [n_q,P,T,2] or
         distribution [n_q,S,P,T,2]; static_obstacles [M,2] (shared) or [n_q,M,2]; limits [n_q,4]
         overrides constraint_overrides; max_stop_distance scalar / [n_q] (NaN = none); winner_samples = k > 0
@@ -41,13 +41,16 @@ class BatchFrenetPlanner(FrenetPlanner):
         with their series unless rank_series is False.  cost_weights [n_w,6] (every query) or [n_q,n_w,6] (columns
         _lib.COST_WEIGHT_KEYS): also every query's winner under each weighting (`SweepResult.w_*`, `under_weights`),
         with its series unless weight_series is False.  cost_terms: also the five cost terms of every candidate
-        (`SweepResult.cost_terms`).  With any of these the batch runs as a device-resident `DeviceBatch`."""
+        (`SweepResult.cost_terms`).  With any of these the batch runs as a device-resident `DeviceBatch`.  route: the
+        reference path of every query, an id into `routes` (`add_route`), one for all queries or [n_q]; None: route 0.
+        A routed query gives what a planner built on its route gives."""
         q, _ = self._batch_arrays(frenet_states, target_speed, dynamic_obstacles, distribution, static_obstacles,
-                                  constraint_overrides, limits, max_stop_distance)
+                                  constraint_overrides, limits, max_stop_distance, route=route)
         return self._run(q, want_candidates, winner_samples, top_k, rank_series, cost_weights, weight_series, cost_terms)
 
     def _batch_arrays(self, frenet_states, target_speed, dynamic_obstacles=None, distribution=None,
-                      static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None, **run):
+                      static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None, route=None,
+                      **run):
         """(the checked inputs of `plan_batch`, its remaining keywords)."""
         mode, dyn = _lib.FOT_DYN_NONE, None
         if distribution is not None and np.size(distribution) > 0:
@@ -56,22 +59,34 @@ class BatchFrenetPlanner(FrenetPlanner):
             mode, dyn = _lib.FOT_DYN_SINGLE, np.asarray(dynamic_obstacles, dtype=np.float64)[:, None]
         if limits is None:
             limits = self.resolve_limits(constraint_overrides)
-        return query_arrays(frenet_states, target_speed, limits, max_stop_distance, static_obstacles, dyn, mode,
-                            self.d_t_s), run
+        q = query_arrays(frenet_states, target_speed, limits, max_stop_distance, static_obstacles, dyn, mode, self.d_t_s)
+        q.route = route_array(route, len(q.frenet), len(self.routes))
+        return q, run
 
     def plan_batch_from_ego(self, ego, target_speed, last_kappa=0.0, converter: Optional[BatchCoordinateConverter] = None,
                             **kwargs):
         """plan() for n_q ego states at once: ego [n_q,5] (x, y, yaw, v, a), last_kappa scalar or [n_q] (the ego
         curvature plan() keeps between calls), `converter` the n_q nearest-point caches to use and update (row q for
-        ego q; None: fresh ones on this planner's device, as a first plan() call has).  The nearest-point search runs
-        on the device (DESIGN.md section 4e), the rest of the Frenet conversion on the host, then `plan_batch` with
-        **kwargs.  Returns (SweepResult, ok): where ok is False the conversion failed and plan() would return None --
+        ego q; None: fresh ones on this planner's device, as a first plan() call has, each on the query's route when
+        **kwargs has `route`).  The nearest-point search runs on the device (DESIGN.md section 4e), the rest of the
+        Frenet conversion on the host, then `plan_batch` with **kwargs.  Returns (SweepResult, ok): where ok is False the conversion failed and plan() would return None --
         best_idx -1, best_cost inf, stats zero, winner_len 0 (`SweepResult.blank`)."""
         ego = np.asarray(ego, dtype=np.float64).reshape(-1, 5)
         n_q = ego.shape[0]
         q, run = self._batch_arrays(np.zeros((n_q, 6)), target_speed, **kwargs)    # checked before the device is used
-        if converter is None:
+        if converter is None and q.route is not None:
+            converter = RoutedCoordinateConverter(self.routes, q.route, engine=self.engine)
+        elif converter is None:
             converter = BatchCoordinateConverter(self.csp, n_q, engine=self.engine)
+        else:
+            # the converter's rows must search the paths the queries plan on: a row converted on one path and planned
+            # on another would be a wrong Frenet state, not an error
+            want = np.zeros(n_q, dtype=np.int64) if q.route is None else q.route.astype(np.int64)
+            have = converter.route[:n_q] if isinstance(converter, RoutedCoordinateConverter) else np.zeros(n_q, np.int64)
+            if not np.array_equal(have, want):
+                raise ValueError("converter routes differ from the queries' route: pass a RoutedCoordinateConverter "
+                                 "over this planner's routes with the same route array (rows on route 0 only: a "
+                                 "BatchCoordinateConverter)")
         kappa = np.broadcast_to(np.asarray(last_kappa, dtype=np.float64), (n_q,))
         frenet, ok = ego_to_frenet_many(converter, np.arange(n_q), ego, kappa)
         q.frenet[:] = frenet
@@ -96,11 +111,12 @@ class DeviceBatch:
 
     def __init__(self, planner: FrenetPlanner, frenet_states, target_speed, dyn, dyn_mode, limits=None,
                  max_stop_distance=None, static_obstacles=None, top_k: int = 0, rank_series: bool = True,
-                 cost_weights=None, weight_series: bool = True, cost_terms: bool = False):
+                 cost_weights=None, weight_series: bool = True, cost_terms: bool = False, route=None):
         import torch
         q = query_arrays(frenet_states, target_speed, planner.resolve_limits(None) if limits is None else limits,
                          max_stop_distance, static_obstacles, dyn, dyn_mode, planner.d_t_s)
         n_q = len(q.frenet)
+        route = route_array(route, n_q, len(planner.routes))
         self.top_k = int(top_k)
         if self.top_k > _lib.FOT_MAX_RANKED:
             raise ValueError(f"top_k must be in [1, {_lib.FOT_MAX_RANKED}]")
@@ -114,6 +130,8 @@ class DeviceBatch:
         self.t = {key: a if isinstance(a, torch.Tensor) else torch.from_numpy(a).to(dev)
                   for key in ("frenet", "target", "limits", "stop", "v_grid", "n_v", "static", "dyn")
                   if (a := getattr(q, key)) is not None}
+        if route is not None:
+            self.t["route"] = torch.from_numpy(route).to(dev)
         self.batch = fot_batch(dataclasses.replace(q, **self.t), torch.Tensor.data_ptr)
         # the whole winner block in one contiguous buffer (what the sharded sweep gathers with one collective)
         self.block = WinnerBlock(n_q, eng.n_t_max, device=dev)
@@ -159,15 +177,20 @@ class DeviceBatch:
             return
         self._enqueue(stream)
 
+    def _route_ptr(self):
+        r = self.t.get("route")
+        return None if r is None else r.data_ptr()
+
     def _enqueue(self, stream) -> None:
-        self.engine.run_device(self.batch, self.result, stream)
-        if self.top_k > 0:
-            r = self.result
-            self.engine.rank_device(self.batch, r.cand_cat, r.cand_cost, r.cand_stride, self.ranked, stream)
-        if self.n_w > 0:
-            self.engine.select_weighted_device(self.batch, self.result.cand_cat, self.stride, self.weighted, stream)
-        if self.cost_terms:
-            self.engine.cost_terms_device(self.batch, self.stride, self.out["cost_terms"].data_ptr(), stream)
+        with self.engine.routes_bound(self._route_ptr()):
+            self.engine.run_device(self.batch, self.result, stream)
+            if self.top_k > 0:
+                r = self.result
+                self.engine.rank_device(self.batch, r.cand_cat, r.cand_cost, r.cand_stride, self.ranked, stream)
+            if self.n_w > 0:
+                self.engine.select_weighted_device(self.batch, self.result.cand_cat, self.stride, self.weighted, stream)
+            if self.cost_terms:
+                self.engine.cost_terms_device(self.batch, self.stride, self.out["cost_terms"].data_ptr(), stream)
 
     def sweep_result(self, want_candidates: bool = False, winner_samples: int = 0) -> SweepResult:
         """Host copy of the outputs of the last launch, once it has finished (launch() without a stream waits), as a
@@ -197,9 +220,10 @@ class DeviceBatch:
         import ctypes as C
         ptr = lambda a: a.data_ptr() if hasattr(a, "data_ptr") else a.ctypes.data
         r = fot_result(host_out, ptr, winner_samples)
-        _lib.check(self.engine.lib.fot_plan_batch_device_to_host(self.engine._h, C.byref(self.batch), C.byref(r),
-                                                                 C.c_void_p(stream) if stream else None),
-                   "fot_plan_batch_device_to_host")
+        with self.engine.routes_bound(self._route_ptr()):
+            _lib.check(self.engine.lib.fot_plan_batch_device_to_host(self.engine._h, C.byref(self.batch), C.byref(r),
+                                                                     C.c_void_p(stream) if stream else None),
+                       "fot_plan_batch_device_to_host")
 
     def dense_evals(self) -> int:
         """Densely credited point-vs-obstacle tests of this batch (SURVEY.md section 8d)."""

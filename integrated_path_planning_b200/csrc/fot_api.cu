@@ -107,9 +107,12 @@ std::set<fot_handle*> g_live;     // handles alive in this process (fot_reload_o
 
 // The instantiations of fot_sweep_pairs that exist (mode sets, PAIR_*), smallest first: the campaign shape, + static
 // obstacles, + per-candidate outputs, + both, the unstaged obstacle block (large sample sets), the violation budget
-// (chance-constrained planning), static obstacles + footprint (the corridor scenarios), everything.
+// (chance-constrained planning), static obstacles + footprint (the corridor scenarios), everything; then the routed
+// counterparts (PAIR_ROUTES, per-query reference paths) of the campaign shape, + static obstacles, + per-candidate outputs
+// (top_k, cost weights) and everything.
 #define FOT_PAIR_INSTANCES(X) X(0) X(PAIR_STATIC) X(PAIR_OUTPUTS) X(PAIR_STATIC | PAIR_OUTPUTS) X(PAIR_LOOSE) X(PAIR_BUDGET) \
-  X(PAIR_STATIC | PAIR_FOOTPRINT) X(PAIR_ALL)
+  X(PAIR_STATIC | PAIR_FOOTPRINT) X(PAIR_ALL) X(PAIR_ROUTES) X(PAIR_ROUTES | PAIR_STATIC) X(PAIR_ROUTES | PAIR_OUTPUTS)     \
+  X(PAIR_ROUTES | PAIR_ALL)
 #define FOT_PAIR_LIST(f) (f),
 static const int kPairInstances[] = {FOT_PAIR_INSTANCES(FOT_PAIR_LIST)};
 static const int kPairInstanceCount = (int)(sizeof(kPairInstances) / sizeof(kPairInstances[0]));
@@ -118,7 +121,9 @@ static PairKernel pair_kernel(bool fused, int feat) {
   switch (feat) {
 #define FOT_PAIR_CASE(f) case (f): return fused ? fot_sweep_pairs<true, (f)> : fot_sweep_pairs<false, (f)>;
     FOT_PAIR_INSTANCES(FOT_PAIR_CASE)
-    default: return fused ? fot_sweep_pairs<true, PAIR_ALL> : fot_sweep_pairs<false, PAIR_ALL>;
+    default:
+      if (feat & PAIR_ROUTES) return fused ? fot_sweep_pairs<true, PAIR_ROUTES | PAIR_ALL> : fot_sweep_pairs<false, PAIR_ROUTES | PAIR_ALL>;
+      return fused ? fot_sweep_pairs<true, PAIR_ALL> : fot_sweep_pairs<false, PAIR_ALL>;
   }
 }
 
@@ -150,6 +155,13 @@ struct fot_handle {
   unsigned mirror_seq = 0;
   const double* last_winner_d = nullptr;   // full winner series of the last host-result call (device, in out_d)
   int last_winner_nq = 0;
+  // routes (fot_add_route): host copies of the device tables of Routes, route 0 = the path of fot_create
+  std::vector<double> rt_tab;        // every route's nine tables, nx doubles each
+  std::vector<int32_t> rt_nx{0};     // [0] number of routes, [1 + r] knots of route r
+  std::vector<int32_t> rt_off;       // [r] offset of route r in rt_tab
+  int max_nx = 0;                    // most knots of any route: kernel choice and shared memory of a routed launch
+  void* routes_dev = nullptr;        // rt_tab | rt_nx | rt_off on the device
+  const int32_t* route_ids = nullptr;   // fot_set_routes: per-query route ids (device), null = no binding
   Buf stage_h, stage_d, out_d, dyn_d, stat_d;   // host-API staging
   fot_handle() { stage_h.host = true; gate_h.host = true; }
 };
@@ -219,6 +231,12 @@ extern "C" int fot_create(const fot_config_t* cfg, const fot_tables_t* tb, int d
   P.xa = D + oxa; P.xb = D + oxb; P.xc = D + oxc; P.xd = D + oxd;
   P.ya = D + oya; P.yb = D + oyb; P.yc = D + oyc; P.yd = D + oyd;
   P.n_steps = I; P.n_steps_b = I + nT;
+  {
+    const fot_route_t r0{nx, tb->knots, tb->xa, tb->xb, tb->xc, tb->xd, tb->ya, tb->yb, tb->yc, tb->yd};
+    int32_t id = 0;
+    const int rc = fot_add_route(h, &r0, &id);
+    if (rc != FOT_OK) return rc;
+  }
 
   CK(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&h->stream2, cudaStreamNonBlocking));
@@ -243,6 +261,8 @@ extern "C" int fot_create(const fot_config_t* cfg, const fot_tables_t* tb, int d
   h->smem_optin -= 2048;   // leave room for the kernels' static shared memory
   CK(cudaFuncSetAttribute(fot_sweep_items<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
   CK(cudaFuncSetAttribute(fot_sweep_items<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
+  CK(cudaFuncSetAttribute(fot_sweep_items<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
+  CK(cudaFuncSetAttribute(fot_sweep_items<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
   for (int i = 0; i < kPairInstanceCount; ++i)
     for (int f = 0; f < 2; ++f)
       CK(cudaFuncSetAttribute(pair_kernel(f != 0, kPairInstances[i]), cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_optin));
@@ -268,6 +288,7 @@ extern "C" int fot_destroy(fot_handle_t* h) {
                  &h->out_d, &h->dyn_d, &h->stat_d})
     b->release();
   if (h->tables_dev) cudaFree(h->tables_dev);
+  if (h->routes_dev) cudaFree(h->routes_dev);
   for (auto ev : h->ring) if (ev) cudaEventDestroy(ev);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
@@ -291,11 +312,26 @@ extern "C" int fot_candidate_count(const fot_handle_t* h, int n_v, int has_brake
   return h->plan.cfg.n_T * n_v * h->plan.cfg.n_d + (has_brake ? h->plan.cfg.n_B : 0);
 }
 
+// Knots of the path(s) a launch sweeps: with a route binding the longest route's (fot_set_routes), else the handle's path.
+static int sweep_nx(const fot_handle* h) { return h->route_ids ? h->max_nx : h->plan.cfg.nx; }
+
+// The Routes of a launch whose first query is query q_off of the bound route array (all null without a binding).
+static Routes routes_of(const fot_handle* h, size_t q_off) {
+  Routes R{};
+  if (!h->route_ids) return R;
+  const size_t n_routes = h->rt_off.size();
+  R.id = h->route_ids + q_off;
+  R.tab = (const double*)h->routes_dev;
+  R.nx = (const int32_t*)(R.tab + h->rt_tab.size());
+  R.off = R.nx + 1 + n_routes;
+  return R;
+}
+
 // Geometry of the sample-major kernel (fot_sweep_items).  Returns false, with the limit that was exceeded in
 // fot_last_error, when the batch's shape is outside what that kernel covers: then no sweep kernel takes it.
 static bool item_geometry(const fot_handle* h, const fot_batch_t* b, ItemGeom* g, size_t* smem_bytes,
                           bool want_fused_box = false) {
-  const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = h->plan.cfg.nx;
+  const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = sweep_nx(h);
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
   const long long SPl = has_dyn ? (long long)b->S * b->P : 0;
   char why[160];
@@ -388,7 +424,7 @@ static bool item_geometry(const fot_handle* h, const fot_batch_t* b, ItemGeom* g
 // (time grids beyond kPairNT = 56 samples, lateral grids beyond 96 targets, tables that do not fit): fot_sweep_items then runs.
 static bool pair_geometry(const fot_handle* h, const fot_batch_t* b, PairGeom* g, size_t* smem_bytes,
                           bool want_fused_box = false) {
-  const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = h->plan.cfg.nx;
+  const int NT = h->plan.n_t_max, nd = h->plan.cfg.n_d, nB = h->plan.cfg.n_B, nx = sweep_nx(h);
   const bool has_dyn = b->dyn_mode != FOT_DYN_NONE;
   const long long SPl = has_dyn ? (long long)b->S * b->P : 0;
   if (NT > kPairNT || nd > kPairND || b->n_v_max > kPairNV || nx > kPairNX || h->plan.cfg.n_T > kPairNH || SPl > (1 << 20) || b->n_static > (1 << 20)) return false;
@@ -553,6 +589,7 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
   B.static_raw = b->n_static > 0 ? b->static_obs : nullptr;
   B.dyn_box = dyn_box;
   B.cost_tab = cost_tab;
+  B.rt = routes_of(h, q_off);
   Out O{};
   O.best_idx = r->best_idx; O.best_cost = r->best_cost; O.stats = r->stats; O.winner_len = r->winner_len;
   O.winner = r->winner; O.cand_cat = r->cand_cat; O.cand_cost = r->cand_cost; O.cand_stride = r->cand_stride;
@@ -593,13 +630,17 @@ static int launch_all(fot_handle* h, const fot_batch_t* b, const fot_result_t* r
     if (!h->plan.d_sorted) need |= PAIR_LOOSE;
     need |= h->opt.pair_feat;
     if (!h->opt.pair_simple) need = PAIR_ALL;
-    int feat = PAIR_ALL;
+    if (B.rt.id) need |= PAIR_ROUTES;
+    int feat = PAIR_ALL | (need & PAIR_ROUTES);
     for (int i = 0; i < kPairInstanceCount; ++i)
       if ((kPairInstances[i] & need) == need) { feat = kPairInstances[i]; break; }
     pair_kernel(pg.fused_box != 0, feat)<<<(unsigned)n_part, kPairThreads, s.smem, st>>>(h->plan, B, O, pg);
     h->last_pair_feat = feat;
-  } else if (ig.fused_box) fot_sweep_items<true><<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
-  else fot_sweep_items<false><<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
+  } else {
+    auto items = B.rt.id ? (ig.fused_box ? fot_sweep_items<true, true> : fot_sweep_items<false, true>)
+                         : (ig.fused_box ? fot_sweep_items<true> : fot_sweep_items<false>);
+    items<<<(unsigned)n_part, ig.threads, s.smem, st>>>(h->plan, B, O, ig);
+  }
   h->last_sweep_kind = s.kind;
   CK(cudaEventRecord(ring[2], st));
   fot_winner<<<b->n_q, 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, O, ig.ctas_per_query);
@@ -642,6 +683,7 @@ extern "C" int fot_rank_candidates(fot_handle_t* h, const fot_batch_t* b, const 
     Batch B{};
     B.n_q = b->n_q; B.n_v_max = b->n_v_max;
     B.frenet = b->frenet; B.v_grid = b->v_grid; B.n_v = b->n_v;
+    B.rt = routes_of(h, 0);
     fot_rank_series<<<(unsigned)((size_t)b->n_q * out->k), 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, R);
   }
   CK(cudaGetLastError());
@@ -654,6 +696,7 @@ static int weighted_pieces(fot_handle* h, const fot_batch_t* b, cudaStream_t st,
   *B = Batch{};
   B->n_q = b->n_q; B->n_v_max = b->n_v_max;
   B->frenet = b->frenet; B->target = b->target_speed; B->v_grid = b->v_grid; B->n_v = b->n_v;
+  B->rt = routes_of(h, 0);
   const long long n_prof = (long long)b->n_q * piece_profiles(h->plan.cfg, b->n_v_max);
   if ((n_prof + 255) / 256 > 0x7fffffffll) return fail(FOT_ERR_ARG, "batch too large for one launch");
   CK(h->w_pieces.reserve((size_t)b->n_q * piece_stride(h->plan.cfg, b->n_v_max) * sizeof(double)));
@@ -1082,6 +1125,50 @@ extern "C" int fot_set_result_mirror(fot_handle_t* h, const fot_result_t* mirror
   return FOT_OK;
 }
 
+// ---- routes: per-query reference paths (DESIGN.md section 4h) ------------------------------------------------------
+extern "C" int fot_add_route(fot_handle_t* h, const fot_route_t* route, int32_t* route_id) {
+  if (!h || !route || !route_id) return fail(FOT_ERR_ARG, "fot_add_route: null argument");
+  const int nx = route->nx;
+  if (nx < 2) return fail(FOT_ERR_ARG, "fot_add_route: a route needs at least 2 knots");
+  const double* tabs[9] = {route->knots, route->xa, route->xb, route->xc, route->xd, route->ya, route->yb, route->yc, route->yd};
+  for (const double* t : tabs)
+    if (!t) return fail(FOT_ERR_ARG, "fot_add_route: null spline table");
+  if (h->rt_tab.size() + 9 * (size_t)nx > 0x7fffffffull) return fail(FOT_ERR_TOO_LARGE, "fot_add_route: route tables beyond 2^31 doubles");
+  // host copies first; the device blob is rebuilt from them (a new route is rare, and never on the planning path)
+  std::vector<double> tab = h->rt_tab;
+  const size_t off = tab.size();
+  for (int k = 0; k < 9; ++k) {
+    const int n = (k == 2 || k == 4 || k == 6 || k == 8) ? nx - 1 : nx;     // b and d have nx - 1 entries
+    tab.insert(tab.end(), tabs[k], tabs[k] + n);
+    if (n < nx) tab.push_back(0.0);
+  }
+  std::vector<int32_t> nxs = h->rt_nx, offs = h->rt_off;
+  nxs.push_back(nx);
+  nxs[0] = (int32_t)(nxs.size() - 1);
+  offs.push_back((int32_t)off);
+  const size_t dbytes = tab.size() * sizeof(double), ibytes = (nxs.size() + offs.size()) * sizeof(int32_t);
+  CK(cudaSetDevice(h->device));
+  void* dev = nullptr;
+  CK(cudaMalloc(&dev, dbytes + ibytes));
+  cudaError_t e = cudaMemcpy(dev, tab.data(), dbytes, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy((char*)dev + dbytes, nxs.data(), nxs.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess)
+    e = cudaMemcpy((char*)dev + dbytes + nxs.size() * sizeof(int32_t), offs.data(), offs.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) { cudaFree(dev); return fail(FOT_ERR_CUDA, "fot_add_route: upload", e); }
+  if (h->routes_dev) cudaFree(h->routes_dev);
+  h->routes_dev = dev;
+  h->rt_tab.swap(tab); h->rt_nx.swap(nxs); h->rt_off.swap(offs);
+  h->max_nx = std::max(h->max_nx, nx);
+  *route_id = h->rt_nx[0] - 1;
+  return FOT_OK;
+}
+
+extern "C" int fot_set_routes(fot_handle_t* h, const int32_t* route) {
+  if (!h) return fail(FOT_ERR_ARG, "fot_set_routes: null handle");
+  h->route_ids = route;
+  return FOT_OK;
+}
+
 extern "C" int fot_peer_alloc(int device, size_t bytes, void** ptr, unsigned char handle[64]) {
   if (!ptr || !handle || bytes == 0) return fail(FOT_ERR_ARG, "fot_peer_alloc: bad argument");
   static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
@@ -1284,7 +1371,9 @@ extern "C" int fot_nearest_s_device(fot_handle_t* h, void* stream, int n, const 
     CK(cudaStreamWaitEvent(st, h->ev_join, 0));
   }
   const int threads = 256, per_block = threads / 32;
-  fot_nearest_s<<<(unsigned)((n + per_block - 1) / per_block), threads, 0, st>>>(h->plan, n, x, y, prev_s, s_out, status);
+  const unsigned blocks = (unsigned)((n + per_block - 1) / per_block);
+  if (h->route_ids) fot_nearest_s_routed<<<blocks, threads, 0, st>>>(h->plan, routes_of(h, 0), n, x, y, prev_s, s_out, status);
+  else fot_nearest_s<<<blocks, threads, 0, st>>>(h->plan, n, x, y, prev_s, s_out, status);
   CK(cudaGetLastError());
   if (!stream) CK(cudaStreamSynchronize(st));
   return FOT_OK;

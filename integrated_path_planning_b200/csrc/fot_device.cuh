@@ -24,6 +24,16 @@ struct Plan {
   double d_min, d_max;     // extreme lateral targets
 };
 
+// Per-query reference paths (fot_add_route / fot_set_routes; DESIGN.md section 4h).  All null: every query plans on the
+// Plan's own path.  Route r's nine spline tables lie at tab + off[r], each nx[1 + r] doubles long (knots | x: a b c d |
+// y: a b c d; the b and d tables use nx - 1 of them); nx[0] is the number of routes.  Route 0 is the Plan's path.
+struct Routes {
+  const int32_t* id;     // [n_q] route of query q (already offset to the launch's first query)
+  const int32_t* nx;     // [1 + n_routes]
+  const int32_t* off;    // [n_routes]
+  const double* tab;
+};
+
 // One batch, device pointers.
 struct Batch {
   int32_t n_q, n_v_max;
@@ -36,10 +46,27 @@ struct Batch {
   const double* static_raw;   // [n_q or 1][M][2] or null
   const float4* dyn_box;      // [n_q][S*P] trajectory boxes (xmin, xmax, ymin, ymax) from fot_aabb_prepass
   const double* cost_tab;     // [n_q][n_T*(n_v_max + 2 n_d) + 3 n_B] jerk sums / terminal offsets from fot_cost_prepass
-  // Unused.  Out and the geometry follow Batch in the sweep kernels' parameters; without these 32 bytes ptxas schedules
-  // fot_sweep_pairs differently, and the sweep of bench.py ran 1.2 % slower (1.597 against 1.578 ms; B200, 1000 W).
-  const void* pad_[4];
+  // Per-query routes, null unless the handle has a route binding.  These 32 bytes were padding before routes existed and
+  // are kept in any case: Out and the geometry follow Batch in the sweep kernels' parameters, and without them ptxas
+  // schedules fot_sweep_pairs differently -- the sweep of bench.py ran 1.2 % slower (1.597 against 1.578 ms; B200, 1000 W).
+  Routes rt;
 };
+
+// V = P with the spline tables and knot count of query q's route.  Without routes V is P.  False for a route id outside
+// [0, n_routes): that query plans nothing, and no table is read for it.
+__device__ __forceinline__ bool route_plan(const Plan& P, const Routes& R, int q, Plan& V) {
+  V = P;
+  if (!R.id) return true;
+  const int r = R.id[q];
+  if (r < 0 || r >= R.nx[0]) return false;
+  const int nx = R.nx[1 + r];
+  const double* t = R.tab + R.off[r];
+  V.cfg.nx = nx;
+  V.knots = t;
+  V.xa = t + nx;     V.xb = t + 2 * nx; V.xc = t + 3 * nx; V.xd = t + 4 * nx;
+  V.ya = t + 5 * nx; V.yb = t + 6 * nx; V.yc = t + 7 * nx; V.yd = t + 8 * nx;
+  return true;
+}
 
 struct Out {
   int32_t* best_idx; double* best_cost; int32_t* stats; int32_t* winner_len; double* winner;

@@ -118,13 +118,24 @@ __device__ __forceinline__ double near_argmin(const Plan& P, double x, double y,
   return b_k == n - 1 ? hi : (double)b_k * step + lo;
 }
 
-// One warp per query.  x, y, prev_s (NaN: no cache) [n]; s_out, status [n].  prev_s is read, never written.
-__global__ void __launch_bounds__(256) fot_nearest_s(const Plan P, int n, const double* __restrict__ xs,
-                                                     const double* __restrict__ ys, const double* __restrict__ prev_s,
-                                                     double* __restrict__ s_out, int32_t* __restrict__ status) {
+// One warp per query.  x, y, prev_s (NaN: no cache) [n]; s_out, status [n].  prev_s is read, never written.  kRoutes:
+// point q is searched on its own route (R; a bad route id gives status 1).  A template parameter, so that the
+// unrouted kernel keeps its code and registers.
+template <bool kRoutes>
+__device__ __forceinline__ void nearest_s_body(const Plan& P_, const Routes& R, int n, const double* __restrict__ xs,
+                                               const double* __restrict__ ys, const double* __restrict__ prev_s,
+                                               double* __restrict__ s_out, int32_t* __restrict__ status) {
   const int q = (int)((blockIdx.x * (unsigned)blockDim.x + threadIdx.x) >> 5);
   const int lane = threadIdx.x & 31;
   if (q >= n) return;                                  // whole warps leave together
+  Plan PR_;
+  if constexpr (kRoutes) {
+    if (!route_plan(P_, R, q, PR_)) {
+      if (lane == 0) { s_out[q] = qnan(); status[q] = 1; }
+      return;
+    }
+  }
+  const Plan& P = kRoutes ? PR_ : P_;
   const double x = xs[q], y = ys[q], prev = prev_s[q];
   const double end = P.knots[P.cfg.nx - 1];            // reference_path.s[-1]
   bool sure = isfinite(x) && isfinite(y) && (isfinite(prev) || isnan(prev)) && end > 0.0;
@@ -172,6 +183,16 @@ __global__ void __launch_bounds__(256) fot_nearest_s(const Plan P, int n, const 
     s_out[q] = sure ? best : qnan();
     status[q] = sure ? 0 : 1;
   }
+}
+__global__ void __launch_bounds__(256) fot_nearest_s(const Plan P, int n, const double* __restrict__ xs,
+                                                     const double* __restrict__ ys, const double* __restrict__ prev_s,
+                                                     double* __restrict__ s_out, int32_t* __restrict__ status) {
+  nearest_s_body<false>(P, Routes{}, n, xs, ys, prev_s, s_out, status);
+}
+__global__ void __launch_bounds__(256) fot_nearest_s_routed(const Plan P, const Routes R, int n, const double* __restrict__ xs,
+                                                            const double* __restrict__ ys, const double* __restrict__ prev_s,
+                                                            double* __restrict__ s_out, int32_t* __restrict__ status) {
+  nearest_s_body<true>(P, R, n, xs, ys, prev_s, s_out, status);
 }
 
 }  // namespace fot

@@ -253,6 +253,8 @@ fot_winner(const Plan P, const Batch B, const Out O, int parts_per_query) {
   double* W = O.winner + (size_t)q * FOT_N_SERIES * NT;
   double* MW = O.m_winner ? O.m_winner + (size_t)q * FOT_N_SERIES * NT : nullptr;       // mirror (peer memory), see Out
   if (O.m_stats && tid < FOT_N_STATS) O.m_stats[(size_t)q * FOT_N_STATS + tid] = O.stats[(size_t)q * FOT_N_STATS + tid];   // final since the sweep
+  Plan V;                                                // the query's route (the sweep left no partial for a bad id)
+  if (!route_plan(P, B.rt, q, V)) i = 0x7fffffff;
   if (i == 0x7fffffff) {
     if (tid == 0) {
       O.best_idx[q] = -1; O.best_cost[q] = INFINITY; O.winner_len[q] = 0;
@@ -260,7 +262,7 @@ fot_winner(const Plan P, const Batch B, const Out O, int parts_per_query) {
     }
     return;
   }
-  const int len = regenerate(P, B, q, i, tt, W, MW, &s_first_nan);
+  const int len = regenerate(V, B, q, i, tt, W, MW, &s_first_nan);
   if (tid == 0) {
     O.best_idx[q] = i;
     O.best_cost[q] = c;

@@ -70,11 +70,13 @@ fot_rank_series(const Plan P, const Batch B, const Ranked R) {
   const int i = R.idx[slot];
   if (i < 0) return;
   const int q = (int)(slot / R.k);
+  Plan V;                                              // the query's route (a bad id never ranks a candidate)
+  if (!route_plan(P, B.rt, q, V)) return;
   if (threadIdx.x == 0) s_first_nan = 0x7fffffff;
   for (int n = threadIdx.x; n < NT; n += blockDim.x) tt_fill(tt, n, P.cfg.dt);
   __syncthreads();
-  const int len = R.series ? regenerate<true>(P, B, q, i, tt, R.series + slot * FOT_N_SERIES * NT, nullptr, &s_first_nan)
-                           : regenerate<false>(P, B, q, i, tt, nullptr, nullptr, &s_first_nan);
+  const int len = R.series ? regenerate<true>(V, B, q, i, tt, R.series + slot * FOT_N_SERIES * NT, nullptr, &s_first_nan)
+                           : regenerate<false>(V, B, q, i, tt, nullptr, nullptr, &s_first_nan);
   if (threadIdx.x == 0) R.len[slot] = len;
 }
 

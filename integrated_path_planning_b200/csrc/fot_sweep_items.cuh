@@ -130,9 +130,9 @@ __device__ __forceinline__ unsigned clean_word(const unsigned* flags_pp, int nw4
 }
 
 // kFused: the variant of the gated host-pointer call (waits for its query's upload slice, boxes the trajectories
-// itself).  A template parameter rather than a run-time branch: the resident path keeps exactly the code (and the
-// register allocation) it is tuned for.
-template <bool kFused>
+// itself).  kRoutes: every query on its own reference path (Batch::rt, DESIGN.md section 4h).  Template parameters
+// rather than run-time branches: the resident path keeps exactly the code (and the register allocation) it is tuned for.
+template <bool kFused, bool kRoutes = false>
 __global__ void __launch_bounds__(kItemThreads, FOT_ITEM_MIN_CTAS)
 fot_sweep_items(const Plan P, const Batch B, const Out O, const ItemGeom G) {
   extern __shared__ __align__(16) unsigned char smb[];
@@ -184,6 +184,8 @@ fot_sweep_items(const Plan P, const Batch B, const Out O, const ItemGeom G) {
   const double2* stat_q = M > 0 ? reinterpret_cast<const double2*>(B.static_raw) + (size_t)(B.static_per_query ? q : 0) * M : nullptr;
 
   // ---- once per CTA: obstacle block in flight, grids and spline tables in shared memory ----------
+  Plan PR_;                                               // kRoutes: the query's route (route_plan, below)
+  const Plan& PS = kRoutes ? PR_ : P;                    // spline tables and knot count of this query
   if (kFused && G.gate && gate_wait(G, q, s_abort)) return;
   if (tid == 0 && G.stage_dyn && state_ok) {
     mbar_init(&s_bar, 1);
@@ -194,15 +196,26 @@ fot_sweep_items(const Plan P, const Batch B, const Out O, const ItemGeom G) {
   }
   if (tid < FOT_N_STATS) s_stats[tid] = 0;
   for (int i = tid; i < n_d; i += bd) dgrid[i] = P.d_grid[i];
+  if constexpr (kRoutes) {
+    // the route's id is read behind the bulk copy; a bad id plans nothing (the copy must have landed before the CTA
+    // exits; thread 0 initialised the barrier and waits on it)
+    if (!route_plan(P, B.rt, q, PR_)) {
+      if (tid == 0) {
+        if (G.stage_dyn && state_ok) mbar_wait(&s_bar, 0u);
+        O.part_cost[part] = INFINITY; O.part_idx[part] = -1;
+      }
+      return;
+    }
+  }
   if (G.spline_smem) {
-    const int nx = P.cfg.nx;
+    const int nx = PS.cfg.nx;
     for (int i = tid; i < nx; i += bd) {
-      spl[i] = P.knots[i];
-      spl[nx + i] = P.xa[i];      spl[3 * nx + i] = P.xc[i];
-      spl[5 * nx + i] = P.ya[i];  spl[7 * nx + i] = P.yc[i];
+      spl[i] = PS.knots[i];
+      spl[nx + i] = PS.xa[i];      spl[3 * nx + i] = PS.xc[i];
+      spl[5 * nx + i] = PS.ya[i];  spl[7 * nx + i] = PS.yc[i];
       if (i < nx - 1) {
-        spl[2 * nx + i] = P.xb[i]; spl[4 * nx + i] = P.xd[i];
-        spl[6 * nx + i] = P.yb[i]; spl[8 * nx + i] = P.yd[i];
+        spl[2 * nx + i] = PS.xb[i]; spl[4 * nx + i] = PS.xd[i];
+        spl[6 * nx + i] = PS.yb[i]; spl[8 * nx + i] = PS.yd[i];
       }
     }
   }
@@ -299,14 +312,14 @@ fot_sweep_items(const Plan P, const Batch B, const Out O, const ItemGeom G) {
     i_sd = held ? 0.0 : L.a1 + 2.0 * L.a2 * tp.t + 3.0 * L.a3 * tp.t2 + 4.0 * L.a4 * tp.t3;      // fp.py:645
     i_sdd = held ? 0.0 : 2.0 * L.a2 + 6.0 * L.a3 * tp.t + 12.0 * L.a4 * tp.t2;                    // fp.py:646
     SplineView V;
-    V.nx = P.cfg.nx;
+    V.nx = PS.cfg.nx;
     if (G.spline_smem) {
       const int nx = V.nx;
       V.knots = spl; V.xa = spl + nx; V.xb = spl + 2 * nx; V.xc = spl + 3 * nx; V.xd = spl + 4 * nx;
       V.ya = spl + 5 * nx; V.yb = spl + 6 * nx; V.yc = spl + 7 * nx; V.yd = spl + 8 * nx;
     } else {
-      V.knots = P.knots; V.xa = P.xa; V.xb = P.xb; V.xc = P.xc; V.xd = P.xd;
-      V.ya = P.ya; V.yb = P.yb; V.yc = P.yc; V.yd = P.yd;
+      V.knots = PS.knots; V.xa = PS.xa; V.xb = PS.xb; V.xc = PS.xc; V.xd = PS.xd;
+      V.ya = PS.ya; V.yb = PS.yb; V.yc = PS.yc; V.yd = PS.yd;
     }
     const RefFast rp = spline_ref_tab(SplineViewTab{V}, V.nx, s);
     i_rx = rp.rx; i_ry = rp.ry; i_cth = rp.cth; i_sth = rp.sth; i_rk = rp.rk; i_rdk = rp.rdk;

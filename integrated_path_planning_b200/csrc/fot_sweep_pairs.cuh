@@ -112,8 +112,11 @@ struct SmemSplineTab {
 // section 4d), so the code of a mode the batch does not use is compiled out of the instantiation it runs instead of
 // being branched over: 0 is the shape of a planning campaign (no static obstacles, one collision circle, no violation
 // budget, sorted lateral grid, staged obstacle block, no per-candidate outputs); the host picks the smallest
-// instantiated superset of what the batch needs (fot_api.cu, kPairInstances).
-enum : int { PAIR_STATIC = 1, PAIR_FOOTPRINT = 2, PAIR_BUDGET = 4, PAIR_OUTPUTS = 8, PAIR_LOOSE = 16, PAIR_ALL = 31 };
+// instantiated superset of what the batch needs (fot_api.cu, kPairInstances).  PAIR_ROUTES: every query on its own
+// reference path (Batch::rt, DESIGN.md section 4h) -- the CTA copies that route's tables and keeps its knot count in a
+// register; PAIR_ALL is every mode but this one.
+enum : int { PAIR_STATIC = 1, PAIR_FOOTPRINT = 2, PAIR_BUDGET = 4, PAIR_OUTPUTS = 8, PAIR_LOOSE = 16, PAIR_ALL = 31,
+             PAIR_ROUTES = 32 };
 template <bool kFused, int kFeat>
 __global__ void __launch_bounds__(kPairThreads, FOT_PAIR_MIN_CTAS)
 fot_sweep_pairs(const Plan P, const Batch B, const Out O_, const PairGeom G) {
@@ -167,6 +170,8 @@ fot_sweep_pairs(const Plan P, const Batch B, const Out O_, const PairGeom G) {
   (void)NT;
 
   // ---- once per CTA ---------------------------------------------------------------------------------
+  Plan PR_;                                                 // PAIR_ROUTES: the query's route (route_plan, below)
+  const Plan& PS = (kFeat & PAIR_ROUTES) ? PR_ : P;        // spline tables and knot count of this query
   if (kFused && G.gate && gate_wait(G, q, s_abort)) return;
   // PAIR_LOOSE: obstacle block read from global memory, boxes from global memory, or an unsorted lateral grid
   const bool stage_dyn = !(kFeat & PAIR_LOOSE) || G.stage_dyn, box_smem = !(kFeat & PAIR_LOOSE) || G.box_smem, d_sorted = !(kFeat & PAIR_LOOSE) || P.d_sorted;
@@ -193,15 +198,26 @@ fot_sweep_pairs(const Plan P, const Batch B, const Out O_, const PairGeom G) {
   else if (tid == 10) qc[10] = B.target[q];
   else if (tid == 11) qc[11] = B.stop_dist[q];
   for (int i = tid; i < B.n_v_max; i += bd) qc[12 + i] = B.v_grid[(size_t)q * B.n_v_max + i];
+  if constexpr ((kFeat & PAIR_ROUTES) != 0) {
+    // the route's id is read beside the other per-query loads, behind the bulk copy; a bad id plans nothing (the
+    // copy must have landed before the CTA exits; thread 0 initialised the barrier and waits on it)
+    if (!route_plan(P, B.rt, q, PR_)) {
+      if (tid == 0) {
+        if (staged) mbar_wait(&s_bar, 0u);
+        O.part_cost[part] = INFINITY; O.part_idx[part] = -1;
+      }
+      return;
+    }
+  }
   {
-    const int nx = P.cfg.nx;
+    const int nx = PS.cfg.nx;
     for (int i = tid; i < nx; i += bd) {
-      S.spl[0][i] = P.knots[i];
-      S.spl[1][i] = P.xa[i];  S.spl[3][i] = P.xc[i];
-      S.spl[5][i] = P.ya[i];  S.spl[7][i] = P.yc[i];
+      S.spl[0][i] = PS.knots[i];
+      S.spl[1][i] = PS.xa[i];  S.spl[3][i] = PS.xc[i];
+      S.spl[5][i] = PS.ya[i];  S.spl[7][i] = PS.yc[i];
       if (i < nx - 1) {
-        S.spl[2][i] = P.xb[i]; S.spl[4][i] = P.xd[i];
-        S.spl[6][i] = P.yb[i]; S.spl[8][i] = P.yd[i];
+        S.spl[2][i] = PS.xb[i]; S.spl[4][i] = PS.xd[i];
+        S.spl[6][i] = PS.yb[i]; S.spl[8][i] = PS.yd[i];
       }
     }
   }
@@ -348,7 +364,7 @@ fot_sweep_pairs(const Plan P, const Batch B, const Out O_, const PairGeom G) {
         const double s = pc[0] + pc[1] * tp.t + pc[2] * tp.t2 + pc[3] * tp.t3 + pc[4] * tp.t4;             // fp.py:644
         i_sd = held ? 0.0 : pc[1] + 2.0 * pc[2] * tp.t + 3.0 * pc[3] * tp.t2 + 4.0 * pc[4] * tp.t3;       // fp.py:645
         i_sdd = held ? 0.0 : 2.0 * pc[2] + 6.0 * pc[3] * tp.t + 12.0 * pc[4] * tp.t2;                      // fp.py:646
-        const RefFast rp = spline_ref_tab(SmemSplineTab{S.spl}, P.cfg.nx, s);
+        const RefFast rp = spline_ref_tab(SmemSplineTab{S.spl}, PS.cfg.nx, s);
         i_rx = rp.rx; i_ry = rp.ry; i_cth = rp.cth; i_sth = rp.sth; i_rk = rp.rk; i_rdk = rp.rdk;
         i_isd = fabs(i_sd) > 1e-3 ? rcp_nr(i_sd) : 0.0;                            // fp.py:792 EPS_S_DOT
         {

@@ -10,6 +10,7 @@ The candidate sweep itself runs only on the GPU (csrc/fot_kernels.cuh) through t
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import functools
 import itertools
@@ -107,6 +108,25 @@ class QueryArrays:
     static_per_query: bool
     dyn: Any                      # [n_q, S, P, T, 2] float64, a NumPy array or a CUDA torch tensor; None for FOT_DYN_NONE
     dyn_mode: int
+    route: Optional[np.ndarray] = None   # [n_q] int32 route of every query (`route_array`); None: every query on route 0
+
+
+def route_array(route, n_q: int, n_routes: int) -> Optional[np.ndarray]:
+    """The per-query route ids of a batch as a contiguous int32 [n_q] array, from None (every query on route 0: returns
+    None), one integer for every query, or [n_q] integers.  Raises ValueError on a non-integer value, a wrong shape or an
+    id outside [0, n_routes): checked on the host, before anything reaches the device."""
+    if route is None:
+        return None
+    a = np.asarray(route)
+    if a.dtype == np.bool_ or not np.issubdtype(a.dtype, np.integer):
+        raise ValueError(f"route must be integers, got {a.dtype}")
+    if a.ndim == 0:
+        a = np.full(n_q, a)
+    elif a.shape != (n_q,):
+        raise ValueError(f"route must be a scalar or [n_q={n_q}], got {list(a.shape)}")
+    if a.size and (a.min() < 0 or a.max() >= n_routes):
+        raise ValueError(f"route ids must be in [0, {n_routes}), got {int(a.min())}..{int(a.max())}")
+    return np.ascontiguousarray(a, dtype=np.int32)
 
 
 @functools.lru_cache(maxsize=8)
@@ -306,6 +326,31 @@ class SweepEngine:
         _lib.check(self.lib.fot_create(C.byref(cfg), C.byref(tb), self.device, C.byref(self._h)), "fot_create")
         self.n_t_max = self.lib.fot_n_t_max(self._h)
 
+    def add_route(self, path) -> int:
+        """Registers one more reference path (a CubicSpline2D or the reference's spline object) on the device: its id
+        (1, 2, ...) is what the route arrays of the batch calls name.  Route 0 is the path of the constructor."""
+        sp = spline_tables(path)
+        self._keep.setdefault("routes", []).append(sp)      # host tables stay alive with the engine
+        r = _lib.FotRoute(nx=len(sp["knots"]))
+        for name, _ in _lib.FotRoute._fields_[1:]:
+            setattr(r, name, sp[name].ctypes.data_as(_lib.c_double_p))
+        rid = C.c_int32()
+        _lib.check(self.lib.fot_add_route(self._h, C.byref(r), C.byref(rid)), "fot_add_route")
+        return int(rid.value)
+
+    @contextlib.contextmanager
+    def routes_bound(self, route_ptr: Optional[int]):
+        """The calls inside the block plan query q on the route in route_ptr[q] (a device int32 array; fot_set_routes);
+        the binding is cleared on leaving, so none outlives the block.  None: no binding."""
+        if route_ptr is None:
+            yield
+            return
+        _lib.check(self.lib.fot_set_routes(self._h, C.c_void_p(route_ptr)), "fot_set_routes")
+        try:
+            yield
+        finally:
+            self.lib.fot_set_routes(self._h, None)
+
     def close(self):
         if getattr(self, "_h", None):
             self.lib.fot_destroy(self._h)
@@ -335,8 +380,17 @@ class SweepEngine:
         k_head = min(int(winner_samples), self.n_t_max) if winner_samples and winner_samples > 0 else 0
         res = self._result_buffers(len(q.frenet), want_candidates, q.v_grid.shape[1], k_head)
         b, r = fot_batch(q, _ptr), fot_result(vars(res), _ptr, k_head)
-        _lib.check(self.lib.fot_plan_batch_host(self._h, C.byref(b), C.byref(r)), "fot_plan_batch_host")
+        route_d = self._device_route(q.route)                # the route array is device memory for this call too
+        with self.routes_bound(None if route_d is None else route_d.data_ptr()):
+            _lib.check(self.lib.fot_plan_batch_host(self._h, C.byref(b), C.byref(r)), "fot_plan_batch_host")
         return self.finish_result(res, q.frenet, q.n_v)
+
+    def _device_route(self, route: Optional[np.ndarray]):
+        """A route array (`route_array`) as an int32 tensor on this engine's device, or None."""
+        if route is None:
+            return None
+        import torch
+        return torch.from_numpy(np.ascontiguousarray(route, dtype=np.int32)).to(torch.device("cuda", self.device))
 
     def finish_result(self, res: SweepResult, frenet: np.ndarray, n_v: np.ndarray) -> SweepResult:
         """res with the candidates generated per query and the device time of the last launch filled in."""
@@ -400,10 +454,11 @@ class SweepEngine:
         _lib.check(self.lib.fot_cost_terms(self._h, C.byref(batch), int(cand_stride), C.c_void_p(terms),
                                            C.c_void_p(stream) if stream else None), "fot_cost_terms")
 
-    def nearest_s(self, x, y, prev_s):
-        """fot_nearest_s_device for m points on this engine's path: returns (s [m], status [m] int32), status 0 where
-        s is the reference's best_s, 1 where the host has to recompute it.  One upload of x | y | prev_s, one
-        download of s | status, one synchronise; prev_s (NaN = no cache) is not modified."""
+    def nearest_s(self, x, y, prev_s, route=None):
+        """fot_nearest_s_device for m points on this engine's path (route: [m] route ids, point k on route[k]): returns
+        (s [m], status [m] int32), status 0 where s is the reference's best_s, 1 where the host has to recompute it.
+        One upload of x | y | prev_s, one download of s | status, one synchronise; prev_s (NaN = no cache) is not
+        modified."""
         import torch
         m = len(x)
         if m == 0:
@@ -426,11 +481,14 @@ class SweepEngine:
         stream = self._near_stream
         with torch.cuda.stream(stream):
             d_in[:3 * m].copy_(h_in[:3 * m], non_blocking=True)
+            route_d = None if route is None else \
+                torch.from_numpy(np.ascontiguousarray(route, dtype=np.int32)).to(d_in.device, non_blocking=False)
             p_in, p_out = d_in.data_ptr(), d_out.data_ptr()
-            _lib.check(self.lib.fot_nearest_s_device(self._h, C.c_void_p(stream.cuda_stream), m, C.c_void_p(p_in),
-                                                     C.c_void_p(p_in + 8 * m), C.c_void_p(p_in + 16 * m),
-                                                     C.c_void_p(p_out), C.c_void_p(p_out + 8 * m)),
-                       "fot_nearest_s_device")
+            with self.routes_bound(None if route_d is None else route_d.data_ptr()):
+                _lib.check(self.lib.fot_nearest_s_device(self._h, C.c_void_p(stream.cuda_stream), m, C.c_void_p(p_in),
+                                                         C.c_void_p(p_in + 8 * m), C.c_void_p(p_in + 16 * m),
+                                                         C.c_void_p(p_out), C.c_void_p(p_out + 8 * m)),
+                           "fot_nearest_s_device")
             h_out[:12 * m].copy_(d_out[:12 * m], non_blocking=True)
         stream.synchronize()
         raw = h_out.numpy()

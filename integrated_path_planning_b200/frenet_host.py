@@ -334,7 +334,10 @@ class BatchCoordinateConverter:
         `valid` (False where the reference raises)."""
         x = np.asarray(x, dtype=np.float64)
         y = np.asarray(y, dtype=np.float64)
-        rs = self.nearest_s(idx, x, y)
+        return self._points_at(self.nearest_s(idx, x, y), x, y)
+
+    def _points_at(self, rs, x, y):
+        """The rest of `reference_points` once the nearest arc lengths rs of the points (x, y) are known."""
         rx, ry = (np.array(v, dtype=np.float64) for v in self.one._xy_many(rs))
         valid = np.ones(len(rs), dtype=bool)
         for r in np.nonzero(np.isnan(rx) | np.isnan(ry))[0]:              # coordinate_converter.py:289-296
@@ -375,6 +378,65 @@ class BatchCoordinateConverter:
             rate = b / _pow(d, 1.5) - 3.0 * a * c / _pow(d, 2.5)
         nan = np.where(inside, 0.0, np.nan)
         return yaw + nan, kappa + nan, rate + nan
+
+
+class RoutedCoordinateConverter:
+    """`BatchCoordinateConverter` for rows on different reference paths: row q searches `paths[route[q]]`.  One device
+    search covers every row whatever its route (the engine's routes must be `paths`, in order); the rows it cannot
+    certify, and the rest of the conversion, go through the converter of their own route.  Caches, results and the
+    device_rows / host_rows counts are those of one BatchCoordinateConverter per route."""
+
+    def __init__(self, paths, route, engine=None):
+        from .engine import route_array
+        r = np.asarray(route)
+        if r.ndim != 1:
+            raise ValueError(f"route must be [n], got {list(r.shape)}")
+        self.route = route_array(r, len(r), len(paths)).astype(np.int64)     # integers in [0, len(paths)), else ValueError
+        n = len(self.route)
+        self.parts = [BatchCoordinateConverter(p, n) for p in paths]
+        self.prev_s = np.full(n, np.nan)
+        for part in self.parts:                            # one cache: row q is only ever touched by its own route's part
+            part.prev_s = self.prev_s
+        self.engine = engine
+        self.device_rows = 0
+        self.host_rows = 0
+
+    def _by_route(self, idx):
+        """(route, positions in idx of its rows) for every route that idx touches."""
+        r = self.route[idx]
+        return [(k, np.nonzero(r == k)[0]) for k in np.unique(r)]
+
+    def nearest_s(self, idx, x, y):
+        idx = np.asarray(idx, dtype=np.int64)
+        x = np.asarray(x, dtype=np.float64)
+        y = np.asarray(y, dtype=np.float64)
+        best = np.zeros(len(idx))
+        if self.engine is None:
+            for k, sel in self._by_route(idx):
+                best[sel] = self.parts[k]._nearest_s_host(idx[sel], x[sel], y[sel])
+            return best
+        best, status = self.engine.nearest_s(x, y, self.prev_s[idx], route=self.route[idx])
+        sure = status == 0
+        self.prev_s[idx[sure]] = best[sure]
+        redo = np.nonzero(~sure)[0]
+        for k, sel in self._by_route(idx[redo]):          # their caches still hold the values from before this call
+            rows = redo[sel]
+            best[rows] = self.parts[k]._nearest_s_host(idx[rows], x[rows], y[rows])
+        self.device_rows += len(idx) - len(redo)
+        self.host_rows += len(redo)
+        return best
+
+    def reference_points(self, idx, x, y):
+        """BatchCoordinateConverter.reference_points, each row on its own route."""
+        idx = np.asarray(idx, dtype=np.int64)
+        x = np.asarray(x, dtype=np.float64)
+        y = np.asarray(y, dtype=np.float64)
+        rs = self.nearest_s(idx, x, y)
+        out = [np.empty(len(idx)) for _ in range(6)] + [np.zeros(len(idx), dtype=bool)]
+        for k, sel in self._by_route(idx):
+            for a, v in zip(out, self.parts[k]._points_at(rs[sel], x[sel], y[sel])):
+                a[sel] = v
+        return tuple(out)
 
 
 def _pow(base, exponent: float):

@@ -20,6 +20,7 @@ import numpy as np
 
 from . import _lib
 from .engine import QueryArrays, SweepEngine, SweepResult, query_arrays
+from .spline import spline_tables
 from .frenet_host import CoordinateConverter, ego_to_frenet
 from .types import FrenetPath, FrenetState, SERIES
 
@@ -89,6 +90,7 @@ class FrenetPlanner:
                  obstacle_radius: float = 0.3, min_t: float = MIN_T, max_t: float = MAX_T,
                  d_t_s: float = D_T_S, n_s_sample: int = N_S_SAMPLE, **kwargs):
         self.csp = reference_path
+        self.routes = [reference_path]           # route r of the batch calls (add_route); route 0 is this path
         self.max_speed = max_speed
         self.max_accel = max_accel
         self.max_curvature = max_curvature
@@ -132,7 +134,20 @@ class FrenetPlanner:
                 k_lon=self.k_lon, chance_epsilon=self.chance_epsilon,
                 collision_margin_inflation=self.collision_margin_inflation, footprint=self.footprint,
                 device=self.device)
+            for path in self.routes[1:]:
+                self._engine.add_route(path)
         return self._engine
+
+    def add_route(self, reference_path) -> int:
+        """One more reference path (a CubicSpline2D or the reference's spline object) for the batch calls, which take a
+        `route` per query; returns its id, the index into `routes`.  Everything but the path -- grids, limits, weights,
+        radii, footprint -- stays this planner's.  plan() keeps planning on the constructor's path (route 0)."""
+        spline_tables(reference_path)            # a path without numeric coefficients is refused here, on the host
+        self.routes.append(reference_path)
+        if self._engine is not None:
+            rid = self._engine.add_route(reference_path)
+            assert rid == len(self.routes) - 1, (rid, len(self.routes))
+        return len(self.routes) - 1
 
     def resolve_limits(self, constraint_overrides) -> np.ndarray:
         """[max_speed, max_accel, max_curvature, max_lat_accel] after overrides (frenet_planner.py:921-930)."""
@@ -263,7 +278,8 @@ class FrenetPlanner:
             from .batch import DeviceBatch           # batch.py builds on this module
             db = DeviceBatch(self, q.frenet, q.target, q.dyn, q.dyn_mode, limits=q.limits, max_stop_distance=q.stop,
                              static_obstacles=q.static, top_k=top_k, rank_series=rank_series,
-                             cost_weights=cost_weights, weight_series=weight_series, cost_terms=cost_terms)
+                             cost_weights=cost_weights, weight_series=weight_series, cost_terms=cost_terms,
+                             route=q.route)
             db.launch()
             return db.sweep_result(want_candidates, winner_samples)
         return self.engine.run_host(q, want_candidates, winner_samples)

@@ -18,7 +18,8 @@ src/pedestrian/observer.py:52-86; src/simulation/replay_source.py:31-111), so th
 reference's trajectories (tests/test_gpu_rollout.py, golden roll-outs recorded from the unmodified
 reference by tests/golden/make_golden_rollout.py).  Pedestrian ground truth stays outside (replay), as in
 the reference's own pysocialforce-free source; static obstacles and the ego footprint (single circle or the
-multi-circle cover) are shared by the simulations of a batch.
+multi-circle cover) are shared by the simulations of a batch.  The reference path may differ: with `routes`, each
+simulation drives its own (DESIGN.md section 4h), so that a campaign over several scenarios' roads is one lock-step.
 """
 from __future__ import annotations
 
@@ -30,7 +31,8 @@ import numpy as np
 
 from . import _lib
 from .batch import BatchFrenetPlanner, DeviceBatch
-from .frenet_host import BatchCoordinateConverter, ego_to_frenet_many
+from .engine import route_array
+from .frenet_host import BatchCoordinateConverter, RoutedCoordinateConverter, ego_to_frenet_many
 from .prediction import DevicePredictionPostprocessor, safety_metrics
 from .spline import CubicSpline2D
 
@@ -183,7 +185,11 @@ class _StateMachines:
 class BatchedClosedLoop:
     """N closed-loop simulations of the reference's planning stack, advanced in lock-step.
 
-    waypoints_x / waypoints_y : the reference path (shared)
+    waypoints_x / waypoints_y : the reference path (route 0)
+    routes       : [(wx, wy), ...] further reference paths, routes 1, 2, ...; None: none
+    route        : [N] route of each simulation (an integer for all; None: route 0).  Planning, the nearest-point
+                   caches and the goal check (`s[-1] - s_now < 2.0`) follow each simulation's own path; a simulation
+                   gives what a loop over its path alone gives.
     knobs        : SimulationConfig fields by name (dt, obs_len, ego_*, planner and state-machine knobs)
     ped_tracks   : [N, T_frames, P, 2] replayed pedestrian positions, one frame per dt
     ego0         : [N, 5] initial (x, y, yaw, v, a)
@@ -199,7 +205,8 @@ class BatchedClosedLoop:
     """
 
     def __init__(self, waypoints_x, waypoints_y, knobs: Dict[str, float], ped_tracks: np.ndarray, ego0: np.ndarray,
-                 device: int = 0, static_obstacles=None, record: bool = False, sampler=None, cost_weights=None):
+                 device: int = 0, static_obstacles=None, record: bool = False, sampler=None, cost_weights=None,
+                 routes=None, route=None):
         k = {key: (None if (isinstance(v, float) and math.isnan(v)) else v) for key, v in knobs.items()}
         self.k = k
         self.dt = float(k["dt"])
@@ -210,6 +217,8 @@ class BatchedClosedLoop:
         self.n, self.n_frames, self.P, _ = self.tracks.shape
         self.ego = np.array(ego0, dtype=np.float64).reshape(self.n, 5).copy()
         self.spline = CubicSpline2D(list(waypoints_x), list(waypoints_y))
+        self.paths = [self.spline] + [CubicSpline2D(list(wx), list(wy)) for wx, wy in (routes or [])]
+        self.route = route_array(route, self.n, len(self.paths))            # None: every simulation on route 0
         self.ego_radius, self.ped_radius = _knob(k, "ego_radius", 1.0), _knob(k, "ped_radius", 0.3)
         self.footprint = footprint_from_knobs(k)
         self.planner = BatchFrenetPlanner(
@@ -220,6 +229,8 @@ class BatchedClosedLoop:
             max_t=_knob(k, "max_t", 5.0), d_t_s=_knob(k, "d_t_s", 5.0 / 3.6), k_j=k["k_j"], k_t=k["k_t"], k_d=k["k_d"],
             k_s_dot=k["k_s_dot"], k_lat=k["k_lat"], k_lon=k["k_lon"], chance_epsilon=_knob(k, "chance_epsilon", 0.0),
             collision_margin_inflation=_knob(k, "collision_margin_inflation", 1.0), footprint=self.footprint, device=device)
+        for path in self.paths[1:]:
+            self.planner.add_route(path)
         self.device = device
         # [N, 6] weighting of each simulation's cost (columns _lib.COST_WEIGHT_KEYS): every planning attempt selects
         # under it from the same sweep (fot_select_weighted) instead of under the knobs above; None: the knobs
@@ -238,8 +249,14 @@ class BatchedClosedLoop:
         # per-simulation planner state: ego curvature cache and the two nearest-point caches (the planner's
         # converter and the simulator's own goal-check converter are separate objects in the reference)
         self.last_kappa = np.zeros(self.n)
-        self.plan_conv = BatchCoordinateConverter(self.spline, self.n, engine=self.planner.engine)
-        self.goal_conv = BatchCoordinateConverter(self.spline, self.n, engine=self.planner.engine)
+        if self.route is None:
+            self.plan_conv = BatchCoordinateConverter(self.spline, self.n, engine=self.planner.engine)
+            self.goal_conv = BatchCoordinateConverter(self.spline, self.n, engine=self.planner.engine)
+            self.path_end = None
+        else:
+            self.plan_conv = RoutedCoordinateConverter(self.paths, self.route, engine=self.planner.engine)
+            self.goal_conv = RoutedCoordinateConverter(self.paths, self.route, engine=self.planner.engine)
+            self.path_end = np.array([p.s[-1] for p in self.paths], dtype=np.float64)[self.route]   # s[-1] of each simulation's path
         # replayed pedestrians (replay_source.py:31-111): forward-difference velocities, shared clock
         vel = np.zeros_like(self.tracks)
         if self.n_frames >= 2:
@@ -291,7 +308,7 @@ class BatchedClosedLoop:
         batch = DeviceBatch(self.planner, frenet, target, dyn_dev.index_select(0, sel), mode,
                             limits=limits, max_stop_distance=msd,
                             static_obstacles=self.static_points if len(self.static_points) else None,
-                            cost_weights=weights)
+                            cost_weights=weights, route=None if self.route is None else self.route[np.asarray(idx)])
         batch.launch(None)
         if weights is None:
             o_idx, o_len, o_cost, o_win = (batch.out[key] for key in ("best_idx", "winner_len", "best_cost", "winner"))
@@ -417,7 +434,8 @@ class BatchedClosedLoop:
         alive = idx[~collided[idx]]
         if len(alive):
             s_now = self.goal_conv.nearest_s(alive, self.ego[alive, 0], self.ego[alive, 1])
-            done = alive[self.spline.s[-1] - s_now < 2.0]
+            end = self.spline.s[-1] if self.path_end is None else self.path_end[alive]
+            done = alive[end - s_now < 2.0]
             self.active[done], self.reason[done] = False, "goal"
         if self.record:
             md, ttc = m2["min_distance"].cpu().numpy(), m2["ttc"].cpu().numpy()
