@@ -37,7 +37,9 @@ extern "C" {
                                caller built against an earlier minor of the same version keeps working; 0 at each new
                                version.  Version 8: 1: + fot_weighted_t, fot_select_weighted, fot_cost_terms (winners
                                under many cost weightings, the five cost terms per candidate); + fot_route_t,
-                               fot_add_route, fot_set_routes (every query on its own reference path) */
+                               fot_add_route, fot_set_routes (every query on its own reference path); then, still under
+                               minor 1, + fot_assessed_t, fot_assess_trajectories: fot_abi_minor() does not tell whether
+                               a library has them, a caller looks the symbol up (DESIGN.md section 4i) */
 #define FOT_MAX_CIRCLES 8
 #define FOT_MAX_RANKED 32
 #define FOT_N_STATS 8    /* ok, max_speed, max_accel, max_curvature, max_lat_accel, road_bound, collision, stop_distance */
@@ -314,6 +316,52 @@ int fot_add_route(fot_handle_t* h, const fot_route_t* route, int32_t* route_id);
    Kernel choice and shared memory of a launch with a binding follow the LONGEST registered route: fot_sweep_pairs when
    it has at most 48 knots, else fot_sweep_items, which keeps the tables in shared memory up to 128 knots. */
 int fot_set_routes(fot_handle_t* h, const int32_t* route);
+
+/* ---- trajectory assessment (DESIGN.md section 4i) -------------------------------------------------------------------
+ * How close m trajectories per query come to an obstacle field, and how many of its samples they collide with, in the
+ * reference's collision geometry (collision_geometry / hits_static / hits_dynamic, frenet_planner.py:1126-1233).  The
+ * trajectories are series blocks [n_q][m][FOT_N_SERIES][n_t] -- the layout of fot_result_t.winner, fot_ranked_t.series
+ * and fot_weighted_t.series, with n_t = fot_n_t_max -- of which samples [0, len[q][j]) of rows t, x, y and yaw are read
+ * (len is clipped to [0, n_t]).  The field is the dyn / S / P / T_obs / static_obs / n_static / static_per_query part of
+ * a fot_batch_t of the same n_q queries (dyn_mode FOT_DYN_NONE: no dynamic obstacles; any S is accepted).
+ *   circle centres  (x, y), or (x, y) + offset * (cos yaw, sin yaw) for each footprint circle of the handle
+ *   time index      k = clip(rint(t / dt), 0, T_obs - 1) with the handle's dt (a NaN t gives 0)
+ *   distance        d2 = dx*dx + dy*dy, unfused; a NaN d2 is neither a minimum nor a hit
+ *   NaN rule        a pedestrian trajectory with a NaN at any step is ignored entirely (the reference's box prefilter)
+ * Outputs per (q, j), for the n_r threshold pairs r2[i] = (r2_dyn, r2_static) of squared centre distances:
+ *   dyn_min    [n_q][m]       sqrt of the smallest d2 to any dynamic obstacle sample, +inf if there is none
+ *   dyn_at     [n_q][m][4]    (n, circle, s, p) of that minimum; ties go to the first entry in C order of an
+ *                             [len, n_circ, S, P] array (np.argmin); -1 if there is none
+ *   static_min [n_q][m], static_at [n_q][m][3]   the same for the static points, in order (n, circle, point)
+ *   dyn_hits   [n_q][m][n_r]  obstacle samples s in [0, S) where some sample, circle and pedestrian has d2 <= r2_dyn
+ *   first_hit  [n_q][m][n_r]  first trajectory sample n with a dynamic (d2 <= r2_dyn) or static (d2 <= r2_static) hit, -1
+ *   static_hit [n_q][m][n_r]  1 if some static point lies within r2_static, else 0
+ * With the handle's own pair -- (collide_r2_single, collide_r2) for a single-sample field, (collide_r2, collide_r2) for a
+ * distribution -- a trajectory is collision-free in the planner's sense iff static_hit == 0 and
+ * dyn_hits <= floor(chance_epsilon * S) (dyn_hits == 0 for a single sample).  A slot with len 0 (padded ranks, queries
+ * without a winner) gives +inf, -1 and 0.  Footprint centres use CUDA cos / sin: with circles, distances may differ
+ * from NumPy's by a few ulp (DESIGN.md 4b, 4i); with the single centre circle they are bit-identical. */
+#define FOT_MAX_ASSESSED 256   /* trajectories per query */
+#define FOT_MAX_RADII 16       /* threshold pairs */
+#define FOT_MAX_ASSESS_NT 320  /* series row length */
+typedef struct fot_assessed {
+  int32_t m;                /* 1 .. FOT_MAX_ASSESSED */
+  int32_t n_t;              /* row length of the series block, 1 .. FOT_MAX_ASSESS_NT */
+  int32_t n_r;              /* 1 .. FOT_MAX_RADII */
+  const double*  series;    /* [n_q][m][FOT_N_SERIES][n_t] */
+  const int32_t* len;       /* [n_q][m] samples to assess */
+  const double*  r2;        /* [n_r][2] (r2_dyn, r2_static) */
+  double*  dyn_min;         /* [n_q][m] */
+  int32_t* dyn_at;          /* [n_q][m][4] */
+  double*  static_min;      /* [n_q][m] */
+  int32_t* static_at;       /* [n_q][m][3] */
+  int32_t* dyn_hits;        /* [n_q][m][n_r] */
+  int32_t* first_hit;       /* [n_q][m][n_r] */
+  int32_t* static_hit;      /* [n_q][m][n_r] */
+} fot_assessed_t;
+/* Assess the trajectories of `a` against the field `obstacles` (its query arrays are not read).  DEVICE pointers;
+   stream-ordered on `stream` behind the launch that wrote the series (NULL: the handle's stream, synchronised). */
+int fot_assess_trajectories(fot_handle_t* h, const fot_batch_t* obstacles, const fot_assessed_t* a, void* stream);
 
 /* ---- next row (SURVEY.md section 8f, rank 1): the predictor's post-processing on the device ---------
  * Builds the obstacle tensor fot_batch_t.dyn consumes, so that batched roll-outs never upload it.

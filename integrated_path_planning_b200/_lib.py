@@ -16,6 +16,9 @@ FOT_ABI_MINOR = 1
 FOT_MAX_CIRCLES = 8
 FOT_MAX_RANKED = 32
 FOT_MAX_WEIGHT_SETS = 256
+FOT_MAX_ASSESSED = 256
+FOT_MAX_RADII = 16
+FOT_MAX_ASSESS_NT = 320
 FOT_N_STATS = 8
 FOT_N_SERIES = 15
 FOT_DYN_NONE, FOT_DYN_SINGLE, FOT_DYN_DISTRIBUTION = 0, 1, 2
@@ -85,6 +88,15 @@ class FotWeighted(C.Structure):
     ]
 
 
+class FotAssessed(C.Structure):
+    _fields_ = [
+        ("m", C.c_int32), ("n_t", C.c_int32), ("n_r", C.c_int32),
+        ("series", C.c_void_p), ("len", C.c_void_p), ("r2", C.c_void_p),
+        ("dyn_min", C.c_void_p), ("dyn_at", C.c_void_p), ("static_min", C.c_void_p), ("static_at", C.c_void_p),
+        ("dyn_hits", C.c_void_p), ("first_hit", C.c_void_p), ("static_hit", C.c_void_p),
+    ]
+
+
 class FotRoute(C.Structure):
     _fields_ = [
         ("nx", C.c_int32), ("knots", c_double_p),
@@ -137,6 +149,7 @@ SYMBOLS = (
                                        C.c_void_p)),
     ("fot_add_route", C.c_int, (C.c_void_p, C.POINTER(FotRoute), C.POINTER(C.c_int32))),
     ("fot_set_routes", C.c_int, (C.c_void_p, C.c_void_p)),
+    ("fot_assess_trajectories", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotAssessed), C.c_void_p)),
 )
 
 _lib = None

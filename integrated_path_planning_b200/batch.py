@@ -12,7 +12,8 @@ from typing import Optional
 import numpy as np
 
 from . import _lib
-from .engine import SweepEngine, SweepResult, fot_batch, fot_result, query_arrays, route_array, winner_fields
+from .engine import (ASSESS_FIELDS, SweepEngine, SweepResult, assess_radii, fot_batch, fot_result, query_arrays, route_array,
+                     winner_fields)
 from .frenet_host import BatchCoordinateConverter, RoutedCoordinateConverter, ego_to_frenet_many
 from .planner import FrenetPlanner
 
@@ -32,7 +33,8 @@ class BatchFrenetPlanner(FrenetPlanner):
                    static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None,
                    want_candidates: bool = False, winner_samples: int = 0, top_k: int = 0,
                    rank_series: bool = True, cost_weights=None, weight_series: bool = True,
-                   cost_terms: bool = False, route=None) -> SweepResult:
+                   cost_terms: bool = False, route=None, assess: bool = False, assess_obstacles=None,
+                   assess_r2=None) -> SweepResult:
         """frenet_states [n_q,6]; target_speed scalar or [n_q]; dynamic_obstacles [n_q,P,T,2] or
         distribution [n_q,S,P,T,2]; static_obstacles [M,2] (shared) or [n_q,M,2]; limits [n_q,4]
         overrides constraint_overrides; max_stop_distance scalar / [n_q] (NaN = none); winner_samples = k > 0
@@ -43,10 +45,14 @@ class BatchFrenetPlanner(FrenetPlanner):
         with its series unless weight_series is False.  cost_terms: also the five cost terms of every candidate
         (`SweepResult.cost_terms`).  With any of these the batch runs as a device-resident `DeviceBatch`.  route: the
         reference path of every query, an id into `routes` (`add_route`), one for all queries or [n_q]; None: route 0.
-        A routed query gives what a planner built on its route gives."""
+        A routed query gives what a planner built on its route gives.  assess: also the closest approach and collision
+        counts of the winner (and of the ranked alternatives with top_k > 0) against the batch's own obstacle field, or
+        against assess_obstacles [n_q, S, P, T, 2], under the threshold pairs assess_r2 (`DeviceBatch`;
+        `SweepResult.assessed`, `assessment`)."""
         q, _ = self._batch_arrays(frenet_states, target_speed, dynamic_obstacles, distribution, static_obstacles,
                                   constraint_overrides, limits, max_stop_distance, route=route)
-        return self._run(q, want_candidates, winner_samples, top_k, rank_series, cost_weights, weight_series, cost_terms)
+        return self._run(q, want_candidates, winner_samples, top_k, rank_series, cost_weights, weight_series, cost_terms,
+                         assess, assess_obstacles, assess_r2)
 
     def _batch_arrays(self, frenet_states, target_speed, dynamic_obstacles=None, distribution=None,
                       static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None, route=None,
@@ -107,11 +113,20 @@ class DeviceBatch:
     launch also writes the per-candidate categories (shared with top_k) and selects each query's winner under every
     weighting (fot_select_weighted) into out["w_idx"] / out["w_cost"] [n_q, n_w] and, with weight_series,
     out["w_len"] [n_q, n_w] and out["w_series"] [n_q, n_w, 15, n_t_max].  cost_terms: out["cost_terms"]
-    [n_q, stride, 5] = (Jp, Jd, Js, Jv, Jt) of every candidate (fot_cost_terms)."""
+    [n_q, stride, 5] = (Jp, Jd, Js, Jv, Jt) of every candidate (fot_cost_terms).
+
+    assess: every launch also assesses its winners -- or, with top_k > 0 and rank_series, its ranked alternatives, of
+    which rank 0 is the winner -- against an obstacle field (fot_assess_trajectories, DESIGN.md section 4i) into
+    out["a_<name>"] for the names of engine.ASSESS_FIELDS, [n_q, m, ...] with m = 1 or top_k.  The field is the batch's
+    own (dyn and static obstacles), or assess_obstacles [n_q, S, P, T, 2] (a NumPy array or a CUDA tensor, read as S
+    samples of P pedestrians) with the batch's static obstacles.  assess_r2: threshold pairs (r2_dyn, r2_static), one
+    or [n_r, 2]; None: the handle's own pair for that field (`SweepEngine.own_radii`), under which a trajectory is
+    collision-free iff static_hit == 0 and dyn_hits <= floor(chance_epsilon * S)."""
 
     def __init__(self, planner: FrenetPlanner, frenet_states, target_speed, dyn, dyn_mode, limits=None,
                  max_stop_distance=None, static_obstacles=None, top_k: int = 0, rank_series: bool = True,
-                 cost_weights=None, weight_series: bool = True, cost_terms: bool = False, route=None):
+                 cost_weights=None, weight_series: bool = True, cost_terms: bool = False, route=None,
+                 assess: bool = False, assess_obstacles=None, assess_r2=None):
         import torch
         q = query_arrays(frenet_states, target_speed, planner.resolve_limits(None) if limits is None else limits,
                          max_stop_distance, static_obstacles, dyn, dyn_mode, planner.d_t_s)
@@ -121,6 +136,10 @@ class DeviceBatch:
         if self.top_k > _lib.FOT_MAX_RANKED:
             raise ValueError(f"top_k must be in [1, {_lib.FOT_MAX_RANKED}]")
         weights, per_query = _weight_table(cost_weights, n_q)
+        self.assess = bool(assess)
+        a_obs, a_mode = _assess_field(assess_obstacles, n_q) if self.assess else (None, None)
+        a_mode = q.dyn_mode if a_obs is None else a_mode
+        a_r2 = assess_radii(assess_r2) if self.assess and assess_r2 is not None else None
         self.n_w = 0 if weights is None else weights.shape[-2]
         eng = planner.engine
         dev = torch.device("cuda", eng.device)
@@ -163,6 +182,24 @@ class DeviceBatch:
         self.cost_terms = bool(cost_terms)
         if self.cost_terms:
             new(self.out, "cost_terms", (n_q, self.stride, 5), torch.float64)
+        if self.assess:
+            self.assess_field = _lib.FotBatch.from_buffer_copy(self.batch)
+            if a_obs is not None:
+                self.t["a_dyn"] = a_obs.to(dev).contiguous() if isinstance(a_obs, torch.Tensor) else torch.from_numpy(a_obs).to(dev)
+                f = self.assess_field
+                f.dyn, f.dyn_mode = self.t["a_dyn"].data_ptr(), _lib.FOT_DYN_DISTRIBUTION
+                f.S, f.P, f.T_obs = a_obs.shape[1], a_obs.shape[2], a_obs.shape[3]
+            r2 = eng.own_radii(a_mode) if a_r2 is None else a_r2
+            self.t["a_r2"] = torch.from_numpy(r2).to(dev)
+            ranked = self.top_k > 0 and rank_series
+            m, n_r = (self.top_k if ranked else 1), r2.shape[0]
+            a = _lib.FotAssessed(m=m, n_t=eng.n_t_max, n_r=n_r, r2=self.t["a_r2"].data_ptr())
+            a.series = self.out["rank_series" if ranked else "winner"].data_ptr()
+            a.len = self.out["rank_len" if ranked else "winner_len"].data_ptr()
+            for name, dt, shape in ASSESS_FIELDS:
+                setattr(a, name, new(self.out, "a_" + name, (n_q, m, *(n_r if d == "r" else d for d in shape)),
+                                     getattr(torch, dt)))
+            self.assessed = a
         self.result = fot_result(dict(self.out, **self.t), torch.Tensor.data_ptr)
 
     def launch(self, stream: Optional[int] = None) -> None:
@@ -191,12 +228,17 @@ class DeviceBatch:
                 self.engine.select_weighted_device(self.batch, self.result.cand_cat, self.stride, self.weighted, stream)
             if self.cost_terms:
                 self.engine.cost_terms_device(self.batch, self.stride, self.out["cost_terms"].data_ptr(), stream)
+            if self.assess:
+                self.engine.assess_device(self.assess_field, self.assessed, stream)
 
     def sweep_result(self, want_candidates: bool = False, winner_samples: int = 0) -> SweepResult:
         """Host copy of the outputs of the last launch, once it has finished (launch() without a stream waits), as a
         SweepResult: the candidate table only with want_candidates, which needs top_k > 0 (or cost_weights, for the
         categories alone); winner_samples = k > 0: the first k samples of each winner series."""
-        res = SweepResult(**{k: v.cpu().numpy() for k, v in self.out.items()})
+        host = {k: v.cpu().numpy() for k, v in self.out.items()}
+        assessed = {name: host.pop("a_" + name) for name, _, _ in ASSESS_FIELDS} if self.assess else None
+        res = SweepResult(**host)
+        res.assessed = assessed
         if winner_samples and winner_samples > 0:
             res.winner = np.ascontiguousarray(res.winner[:, :, :min(int(winner_samples), res.winner.shape[2])])
         if want_candidates:
@@ -211,10 +253,12 @@ class DeviceBatch:
         the raw cudaStream_t on which the batch's inputs become ready (None: they are ready).  `winner_samples = k > 0`:
         only the first k samples of every winner series come back (`host_out["winner"]` is [n_q, 15, k]) -- what a
         closed-loop caller consumes (integrated_simulator.py:663), 240 B instead of 6.1 KB per query at k = 2.
-        Ranked and weighted outputs do not come back through this call: a batch with top_k > 0, cost_weights or
-        cost_terms raises ValueError."""
+        Ranked, weighted and assessed outputs do not come back through this call: a batch with top_k > 0,
+        cost_weights, cost_terms or assess raises ValueError."""
         if self.top_k > 0:
             raise ValueError("launch_to_host does not return ranked outputs; use launch() with top_k > 0")
+        if self.assess:
+            raise ValueError("launch_to_host does not return assessments; use launch() with assess=True")
         if self.n_w > 0 or self.cost_terms:
             raise ValueError("launch_to_host does not return weighted outputs or cost terms; use launch()")
         import ctypes as C
@@ -231,6 +275,22 @@ class DeviceBatch:
         n_circ = max(1, self.engine.n_circles)
         per_point = self.batch.S * self.batch.P + self.batch.n_static
         return int(pts.sum()) * n_circ * int(per_point)
+
+
+def _assess_field(obstacles, n_q: int):
+    """(assess_obstacles as a float64 [n_q, S, P, T, 2] NumPy array or torch tensor, or None; the dyn mode the handle's
+    own threshold pair is taken for).  Raises ValueError on any other shape or dtype."""
+    if obstacles is None:
+        return None, None
+    if hasattr(obstacles, "data_ptr"):
+        import torch
+        a, f64 = obstacles, torch.float64
+    else:
+        a, f64 = np.ascontiguousarray(obstacles, dtype=np.float64), np.float64
+    if a.ndim != 5 or a.shape[0] != n_q or a.shape[-1] != 2 or a.dtype != f64 or min(a.shape) < 1:
+        raise ValueError(f"assess_obstacles must be float64 [n_q={n_q}, S, P, T, 2] with S, P, T >= 1, "
+                         f"got {a.dtype} {list(a.shape)}")
+    return a, _lib.FOT_DYN_DISTRIBUTION
 
 
 def _weight_table(cost_weights, n_q: int):

@@ -19,6 +19,7 @@
 #include "fot_frenet.cuh"
 #include "fot_rank.cuh"
 #include "fot_weights.cuh"
+#include "fot_assess.cuh"
 
 using namespace fot;
 
@@ -686,6 +687,47 @@ extern "C" int fot_rank_candidates(fot_handle_t* h, const fot_batch_t* b, const 
     B.rt = routes_of(h, 0);
     fot_rank_series<<<(unsigned)((size_t)b->n_q * out->k), 128, (size_t)kTT * h->plan.n_t_max * sizeof(double), st>>>(h->plan, B, R);
   }
+  CK(cudaGetLastError());
+  if (!stream) CK(cudaStreamSynchronize(st));
+  return FOT_OK;
+}
+
+extern "C" int fot_assess_trajectories(fot_handle_t* h, const fot_batch_t* b, const fot_assessed_t* a, void* stream) {
+  if (!h || !b || !a) return fail(FOT_ERR_ARG, "fot_assess_trajectories: null argument");
+  if (b->n_q < 1) return fail(FOT_ERR_ARG, "fot_assess_trajectories: n_q must be >= 1");
+  if (a->m < 1 || a->m > FOT_MAX_ASSESSED) return fail(FOT_ERR_ARG, "fot_assess_trajectories: m must be in [1, FOT_MAX_ASSESSED]");
+  if (a->n_t < 1 || a->n_t > FOT_MAX_ASSESS_NT)
+    return fail(FOT_ERR_ARG, "fot_assess_trajectories: n_t must be in [1, FOT_MAX_ASSESS_NT]");
+  if (a->n_r < 1 || a->n_r > FOT_MAX_RADII) return fail(FOT_ERR_ARG, "fot_assess_trajectories: n_r must be in [1, FOT_MAX_RADII]");
+  if (!a->series || !a->len) return fail(FOT_ERR_ARG, "fot_assess_trajectories: null series or len");
+  if (!a->r2) return fail(FOT_ERR_ARG, "fot_assess_trajectories: null r2");
+  if (!a->dyn_min || !a->dyn_at || !a->static_min || !a->static_at || !a->dyn_hits || !a->first_hit || !a->static_hit)
+    return fail(FOT_ERR_ARG, "fot_assess_trajectories: null output array");
+  if (b->n_static < 0 || b->S < 0 || b->P < 0 || b->T_obs < 0)
+    return fail(FOT_ERR_ARG, "fot_assess_trajectories: negative obstacle shape");
+  if (b->n_static > 0 && !b->static_obs) return fail(FOT_ERR_ARG, "fot_assess_trajectories: static obstacles missing");
+  if (b->dyn_mode != FOT_DYN_NONE && b->dyn_mode != FOT_DYN_SINGLE && b->dyn_mode != FOT_DYN_DISTRIBUTION)
+    return fail(FOT_ERR_ARG, "fot_assess_trajectories: bad dyn_mode");
+  const bool has_dyn = b->dyn_mode != FOT_DYN_NONE && (long long)b->S * b->P * b->T_obs > 0;
+  if (has_dyn && !b->dyn) return fail(FOT_ERR_ARG, "fot_assess_trajectories: dynamic obstacles missing");
+  if ((size_t)b->n_q * a->m * a->n_r > 0x7fffffffull) return fail(FOT_ERR_ARG, "fot_assess_trajectories: batch too large");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  // one sample per thread; a whole trajectory always fits (n_t <= FOT_MAX_ASSESS_NT <= kAssessMaxThreads)
+  const int samples = (int)std::min<long long>((long long)a->m * a->n_t, kAssessMaxThreads);
+  const int threads = std::max(64, (std::max(samples, a->n_t) + 31) / 32 * 32);
+  const size_t smem = (size_t)threads * assess_smem_per_thread(std::max(h->plan.cfg.n_circles, 1));
+  // the kernel's static arrays (7.3 KB) count against the 48 KB a launch gets without opting in
+  if (smem > 32 * 1024) CK(cudaFuncSetAttribute(fot_assess, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  Batch B{};
+  B.n_q = b->n_q;
+  B.n_static = b->n_static; B.static_per_query = b->static_per_query;
+  B.S = has_dyn ? b->S : 0; B.P = has_dyn ? b->P : 0; B.T_obs = has_dyn ? b->T_obs : 0; B.dyn_mode = b->dyn_mode;
+  B.dyn_raw = has_dyn ? b->dyn : nullptr;
+  B.static_raw = b->n_static > 0 ? b->static_obs : nullptr;
+  const Assess A{a->m, a->n_t, a->n_r, a->series, a->len, a->r2, a->dyn_min, a->dyn_at, a->static_min, a->static_at,
+                 a->dyn_hits, a->first_hit, a->static_hit};
+  fot_assess<<<(unsigned)b->n_q, threads, smem, st>>>(h->plan, B, A);
   CK(cudaGetLastError());
   if (!stream) CK(cudaStreamSynchronize(st));
   return FOT_OK;

@@ -370,9 +370,17 @@ __device__ __forceinline__ double wrap_angle(double a) {
   return atan2(s, c);
 }
 
-// Lexicographic (cost, index) minimum: first strict minimum in generation order (fp.py:1254-1257).
-__device__ __forceinline__ void argmin_merge(double& c, int& i, double oc, int oi) {
+// Lexicographic (cost, index) minimum: first strict minimum in generation order (fp.py:1254-1257).  A NaN value never
+// replaces the running minimum.  I: int for candidate indices, long long for the flat indices of fot_assess.
+template <class I>
+__device__ __forceinline__ void argmin_merge(double& c, I& i, double oc, I oi) {
   if (oc < c || (oc == c && oi < i)) { c = oc; i = oi; }
+}
+
+// Centre of one footprint circle: the path point moved `off` along the heading (hx, hy) = (cos yaw, sin yaw)
+// (footprint.py:44-45, fp.py:1152-1160).
+__device__ __forceinline__ double2 footprint_centre(double x, double y, double hx, double hy, double off) {
+  return make_double2(x + off * hx, y + off * hy);
 }
 
 // 1/x and 1/sqrt(x) to fp64 accuracy from the fp32 MUFU seed and two Newton steps (branch-free; the

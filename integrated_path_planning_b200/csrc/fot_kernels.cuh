@@ -110,6 +110,11 @@ __device__ __forceinline__ void cost_prepass_body(const Plan& P, const Batch& B,
   }
 }
 
+// The NaN rule of the box prepass below for one step (a NaN x or y): fot_assess, which reads every step of a trajectory
+// itself, applies it with this function.  The prepass keeps its expression written out: calling this function there
+// changes the instructions ptxas schedules for fot_prepass.
+__device__ __forceinline__ bool nan_step(double2 o) { return (o.x != o.x) || (o.y != o.y); }
+
 // Boxes of the predicted trajectories, once per launch: one warp per trajectory (q, sample, ped),
 // (xmin, xmax, ymin, ymax) over all its steps rounded outward to fp32.  A NaN anywhere makes the
 // whole box NaN, which fails every overlap test: exactly the reference's prefilter, whose np.min /

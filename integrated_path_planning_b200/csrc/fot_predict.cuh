@@ -253,8 +253,8 @@ __global__ void fot_safety_kernel(const double* __restrict__ ego, const double* 
     const double ax = px - x, ay = py - y;                                     // :373-374, one row or a [k,2] matrix
     const bool ahead = (np_ == 1 ? fma(ay, hy, ax * hx) : fma(ax, hx, ay * hy)) > 0.0;
     for (int c = 0; c < (n_circ > 0 ? n_circ : 1); ++c) {
-      const double cx = n_circ > 0 ? x + offsets.v[c] * hx : x, cy = n_circ > 0 ? y + offsets.v[c] * hy : y;   // footprint.py:45
-      const double rx = px - cx, ry = py - cy;
+      const double2 cc = n_circ > 0 ? footprint_centre(x, y, hx, hy, offsets.v[c]) : make_double2(x, y);   // footprint.py:45
+      const double rx = px - cc.x, ry = py - cc.y;
       const double dist = sqrt(rx * rx + ry * ry);                             // :337-339
       dmin = nan_min(dmin, dist);
       if (ahead) dmin_ahead = nan_min(dmin_ahead, dist);

@@ -179,6 +179,44 @@ def fot_batch(q: QueryArrays, ptr) -> "_lib.FotBatch":
     return b
 
 
+# outputs of fot_assess_trajectories per (query, trajectory): (key, dtype name, trailing shape; "r" = n_r)
+ASSESS_FIELDS = (("dyn_min", "float64", ()), ("dyn_at", "int32", (4,)), ("static_min", "float64", ()),
+                 ("static_at", "int32", (3,)), ("dyn_hits", "int32", ("r",)), ("first_hit", "int32", ("r",)),
+                 ("static_hit", "int32", ("r",)))
+
+
+def assess_radii(r2) -> np.ndarray:
+    """Threshold pairs (r2_dyn, r2_static) of fot_assess_trajectories as a contiguous float64 [n_r, 2] array, from one
+    pair or [n_r, 2].  Raises ValueError on any other shape or n_r outside [1, FOT_MAX_RADII]."""
+    a = np.ascontiguousarray(r2, dtype=np.float64)
+    if a.ndim == 1:
+        a = a.reshape(1, -1)
+    if a.ndim != 2 or a.shape[1] != 2 or not 1 <= a.shape[0] <= _lib.FOT_MAX_RADII:
+        raise ValueError(f"r2 must be one (r2_dyn, r2_static) pair or [n_r, 2] with n_r in [1, {_lib.FOT_MAX_RADII}], "
+                         f"got {list(np.shape(r2))}")
+    return a
+
+
+def pack_paths(paths, n_t: Optional[int] = None):
+    """A list of m FrenetPath-like objects (attributes named as types.SERIES) as the series block of one query:
+    (series [m, 15, n_t] float64, NaN past each path's end; len [m] int32 = the samples of x).  n_t defaults to the
+    longest path (at least 1).  Raises ValueError for m outside [1, FOT_MAX_ASSESSED] or a path longer than n_t or
+    FOT_MAX_ASSESS_NT."""
+    paths = list(paths)
+    if not 1 <= len(paths) <= _lib.FOT_MAX_ASSESSED:
+        raise ValueError(f"assess takes 1 to {_lib.FOT_MAX_ASSESSED} paths, got {len(paths)}")
+    lens = np.array([len(getattr(p, "x")) for p in paths], dtype=np.int32)
+    n_t = max(1, int(lens.max())) if n_t is None else int(n_t)
+    if int(lens.max()) > n_t or n_t > _lib.FOT_MAX_ASSESS_NT:
+        raise ValueError(f"paths of up to {_lib.FOT_MAX_ASSESS_NT} samples can be assessed, got {int(lens.max())}")
+    series = np.full((len(paths), _lib.FOT_N_SERIES, n_t), np.nan)
+    for j, p in enumerate(paths):
+        for r, name in enumerate(SERIES):
+            v = np.asarray(getattr(p, name, ()), dtype=np.float64).reshape(-1)[:lens[j]]
+            series[j, r, :v.size] = v
+    return series, lens
+
+
 def fot_result(arrays, ptr, winner_samples: int = 0) -> "_lib.FotResult":
     """fot_result_t over the winner-block fields of arrays and, where not None, its cand_cat / cand_cost (addresses: ptr)."""
     r = _lib.FotResult()
@@ -216,6 +254,10 @@ class SweepResult:
     w_len: Optional[np.ndarray] = None        # [n_q, n_w] int32, or None without series
     w_series: Optional[np.ndarray] = None     # [n_q, n_w, 15, n_t_max], or None
     cost_terms: Optional[np.ndarray] = None   # [n_q, stride, 5] (Jp, Jd, Js, Jv, Jt), NaN past the candidates
+    # trajectory assessment (assess=True; include/fot.h fot_assessed_t): {name: array} for the names of ASSESS_FIELDS,
+    # [n_q, m], [n_q, m, 4], [n_q, m, 3] or [n_q, m, n_r]; column 0 the winner, or with ranked series column j rank j.
+    # A plain attribute, not a field: None unless the batch was assessed.
+    assessed = None
 
     def series(self, q: int = 0):
         """The 15 winner sequences of query q truncated to their kept length, or None."""
@@ -236,6 +278,14 @@ class SweepResult:
         is feasible under that weighting."""
         return [self._entry("w", q, w) for w in range(self.w_idx.shape[1])]
 
+    def assessment(self, q: int = 0):
+        """The assessment of query q (a batch run with assess=True): {name: array} for the names of ASSESS_FIELDS, each
+        with a leading dimension of one column per assessed trajectory -- column 0 the winner, or with ranked series
+        column j rank j.  Blank columns (no winner, padded ranks) hold +inf, -1 and 0."""
+        if self.assessed is None:
+            raise ValueError("this result has no assessment: run the batch with assess=True")
+        return {name: self.assessed[name][q].copy() for name, _, _ in ASSESS_FIELDS}
+
     def _entry(self, block: str, q: int, j: int):
         """Entry j of query q of the ranked ("rank") or weighted ("w") outputs, or None where its index is -1."""
         i = int(getattr(self, block + "_idx")[q, j])
@@ -249,13 +299,18 @@ class SweepResult:
 
     def blank(self, rows) -> None:
         """Queries `rows` (indices or a mask) as plan() returning None leaves them: index -1, cost inf, stats and kept
-        lengths 0 in the winner, ranked and weighted outputs, cost terms NaN; the series and candidate table stay."""
+        lengths 0 in the winner, ranked and weighted outputs, cost terms NaN, assessments blank (+inf, -1, 0); the
+        series and candidate table stay."""
         for name, value in (("best_idx", -1), ("best_cost", np.inf), ("stats", 0), ("winner_len", 0), ("rank_idx", -1),
                             ("rank_cost", np.inf), ("rank_len", 0), ("w_idx", -1), ("w_cost", np.inf), ("w_len", 0),
                             ("cost_terms", np.nan)):
             a = getattr(self, name)
             if a is not None:
                 a[rows] = value
+        for name, value in (("dyn_min", np.inf), ("dyn_at", -1), ("static_min", np.inf), ("static_at", -1),
+                            ("dyn_hits", 0), ("first_hit", -1), ("static_hit", 0)):
+            if self.assessed is not None:
+                self.assessed[name][rows] = value
 
 
 class SweepEngine:
@@ -291,6 +346,7 @@ class SweepEngine:
         dyn_radius = inflated_radius * collision_margin_inflation
         sq_rubicon = inflated_radius ** 2
         sq_rubicon_dyn = dyn_radius ** 2
+        self.collide_r2, self.collide_r2_single, self.chance_epsilon = sq_rubicon, sq_rubicon_dyn, float(chance_epsilon)
 
         cfg = _lib.FotConfig()
         cfg.dt, cfg.max_speed, cfg.max_road_width = dt, max_speed, max_road_width
@@ -453,6 +509,18 @@ class SweepEngine:
         """fot_cost_terms: (Jp, Jd, Js, Jv, Jt) of every candidate of `batch` into terms [n_q, cand_stride, 5]."""
         _lib.check(self.lib.fot_cost_terms(self._h, C.byref(batch), int(cand_stride), C.c_void_p(terms),
                                            C.c_void_p(stream) if stream else None), "fot_cost_terms")
+
+    def own_radii(self, dyn_mode: int) -> np.ndarray:
+        """This handle's own threshold pair [1, 2] for a field of dyn_mode: (collide_r2_single, collide_r2) for a single
+        sample, (collide_r2, collide_r2) otherwise -- under it fot_assess_trajectories reproduces the collision verdict."""
+        r2d = self.collide_r2_single if dyn_mode == _lib.FOT_DYN_SINGLE else self.collide_r2
+        return np.array([[r2d, self.collide_r2]], dtype=np.float64)
+
+    def assess_device(self, obstacles: "_lib.FotBatch", assessed: "_lib.FotAssessed", stream=None) -> None:
+        """fot_assess_trajectories: the trajectories of `assessed` against the field of `obstacles` (device pointers),
+        stream-ordered behind the launch that wrote their series."""
+        _lib.check(self.lib.fot_assess_trajectories(self._h, C.byref(obstacles), C.byref(assessed),
+                                                    C.c_void_p(stream) if stream else None), "fot_assess_trajectories")
 
     def nearest_s(self, x, y, prev_s, route=None):
         """fot_nearest_s_device for m points on this engine's path (route: [m] route ids, point k on route[k]): returns

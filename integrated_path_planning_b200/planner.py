@@ -19,7 +19,7 @@ from typing import Dict, List, Optional
 import numpy as np
 
 from . import _lib
-from .engine import QueryArrays, SweepEngine, SweepResult, query_arrays
+from .engine import ASSESS_FIELDS, QueryArrays, SweepEngine, SweepResult, assess_radii, pack_paths, query_arrays
 from .spline import spline_tables
 from .frenet_host import CoordinateConverter, ego_to_frenet
 from .types import FrenetPath, FrenetState, SERIES
@@ -217,6 +217,54 @@ class FrenetPlanner:
             self._feed_back_curvature(_frenet_path(own, res.best_cost[0]))
         return [None if e is None else _frenet_path(e["series"], e["cost"]) for e in res.under_weights(0)]
 
+    def assess(self, paths, static_obstacles, dynamic_obstacles=None, dynamic_obstacles_distribution=None,
+               r2=None) -> Dict[str, np.ndarray]:
+        """How close each of `paths` (FrenetPath objects: this planner's, plan_alternatives', or the reference
+        planner's) comes to an obstacle field given as plan() takes it, on the device (fot_assess_trajectories,
+        DESIGN.md section 4i).  Returns {name: array with one row per path} for the names of engine.ASSESS_FIELDS --
+        dyn_min, dyn_at (n, circle, s, p), static_min, static_at (n, circle, point), and dyn_hits, first_hit,
+        static_hit per threshold pair -- plus "collision_free" [m] bool under the planner's own pair.  r2: threshold
+        pairs (r2_dyn, r2_static), one or [n_r, 2]; None: the planner's own pair for the field, under which
+        collision_free is the verdict plan() gives the same positions (static_hit == 0 and dyn_hits <=
+        floor(chance_epsilon * S)).  Only t, x, y and yaw of the paths are read."""
+        import ctypes as C
+        import torch
+        series, lens = pack_paths(paths)
+        user_r2 = None if r2 is None else assess_radii(r2)
+        mode, dyn = classify_dynamic(dynamic_obstacles, dynamic_obstacles_distribution)
+        static = None
+        if static_obstacles is not None and len(static_obstacles) > 0:
+            static = np.asarray(static_obstacles, dtype=np.float64).reshape(-1, 2)
+        eng = self.engine
+        own = eng.own_radii(mode)
+        r2 = own if user_r2 is None else np.concatenate([own, user_r2])     # row 0: the verdict's own pair
+        dev = torch.device("cuda", eng.device)
+        t = {"series": torch.from_numpy(series).to(dev), "len": torch.from_numpy(lens).to(dev),
+             "r2": torch.from_numpy(np.ascontiguousarray(r2)).to(dev)}
+        b = _lib.FotBatch(n_q=1)
+        if static is not None:
+            t["static"] = torch.from_numpy(np.ascontiguousarray(static)).to(dev)
+            b.static_obs, b.n_static = t["static"].data_ptr(), static.shape[0]
+        if dyn is not None:
+            t["dyn"] = torch.from_numpy(np.ascontiguousarray(dyn)).to(dev)
+            b.dyn, b.dyn_mode = t["dyn"].data_ptr(), mode
+            b.S, b.P, b.T_obs = dyn.shape[1], dyn.shape[2], dyn.shape[3]
+        m, n_r = len(lens), r2.shape[0]
+        a = _lib.FotAssessed(m=m, n_t=series.shape[-1], n_r=n_r, series=t["series"].data_ptr(), len=t["len"].data_ptr(),
+                             r2=t["r2"].data_ptr())
+        out = {}
+        for name, dt, shape in ASSESS_FIELDS:
+            out[name] = torch.empty((m, *(n_r if d == "r" else d for d in shape)), dtype=getattr(torch, dt), device=dev)
+            setattr(a, name, out[name].data_ptr())
+        eng.assess_device(b, a)                       # the handle's stream, synchronised
+        res = {name: v.cpu().numpy() for name, v in out.items()}
+        allowed = int(np.floor(self.chance_epsilon * b.S)) if mode == _lib.FOT_DYN_DISTRIBUTION else 0
+        res["collision_free"] = (res["static_hit"][:, 0] == 0) & (res["dyn_hits"][:, 0] <= allowed)
+        if user_r2 is not None:                       # the caller's pairs only
+            for name in ("dyn_hits", "first_hit", "static_hit"):
+                res[name] = res[name][:, 1:]
+        return res
+
     def cost_weight_table(self, weights) -> np.ndarray:
         """[n_w, 6] float64 weightings (columns _lib.COST_WEIGHT_KEYS) from an [n_w, 6] array or a list of dicts keyed
         by those names; a key a dict leaves out takes this planner's own value.  Raises ValueError on anything else
@@ -271,15 +319,16 @@ class FrenetPlanner:
 
     def _run(self, q: QueryArrays, want_candidates: bool = False, winner_samples: int = 0, top_k: int = 0,
              rank_series: bool = True, cost_weights=None, weight_series: bool = True,
-             cost_terms: bool = False) -> SweepResult:
-        """Sweep the batch q: as a device-resident `DeviceBatch` when it asks for ranked alternatives, cost weightings
-        or cost terms (outputs only the device-side calls produce), otherwise through the host-pointer call."""
-        if top_k > 0 or cost_weights is not None or cost_terms:
+             cost_terms: bool = False, assess: bool = False, assess_obstacles=None, assess_r2=None) -> SweepResult:
+        """Sweep the batch q: as a device-resident `DeviceBatch` when it asks for ranked alternatives, cost weightings,
+        cost terms or an assessment (outputs only the device-side calls produce), otherwise through the host-pointer
+        call."""
+        if top_k > 0 or cost_weights is not None or cost_terms or assess:
             from .batch import DeviceBatch           # batch.py builds on this module
             db = DeviceBatch(self, q.frenet, q.target, q.dyn, q.dyn_mode, limits=q.limits, max_stop_distance=q.stop,
                              static_obstacles=q.static, top_k=top_k, rank_series=rank_series,
                              cost_weights=cost_weights, weight_series=weight_series, cost_terms=cost_terms,
-                             route=q.route)
+                             route=q.route, assess=assess, assess_obstacles=assess_obstacles, assess_r2=assess_r2)
             db.launch()
             return db.sweep_result(want_candidates, winner_samples)
         return self.engine.run_host(q, want_candidates, winner_samples)

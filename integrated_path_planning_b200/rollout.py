@@ -202,11 +202,18 @@ class BatchedClosedLoop:
                    against the whole sample set under the chance constraint knobs["chance_epsilon"]
                    (integrated_simulator.py:457-460, :582; frenet_planner.py:1076-1124), else against the
                    representative sample.
+    assess       : also assess every step's executed plan (fot_assess_trajectories, DESIGN.md section 4i) against the
+                   whole sample set with its t = 0 column when there is a sampler -- even when planning used the
+                   representative sample -- else against the tensor planned against, under the planner's own radius
+                   pair; run() then also returns plan_min_distance (closest approach to any predicted sample) and
+                   plan_hit_fraction (dyn_hits / S: the share of the S samples the plan collides with), [N, steps],
+                   NaN where no plan was executed (none found, or a winner of fewer than 2 samples, which the ego
+                   does not follow).  Nothing else changes.
     """
 
     def __init__(self, waypoints_x, waypoints_y, knobs: Dict[str, float], ped_tracks: np.ndarray, ego0: np.ndarray,
                  device: int = 0, static_obstacles=None, record: bool = False, sampler=None, cost_weights=None,
-                 routes=None, route=None):
+                 routes=None, route=None, assess: bool = False):
         k = {key: (None if (isinstance(v, float) and math.isnan(v)) else v) for key, v in knobs.items()}
         self.k = k
         self.dt = float(k["dt"])
@@ -240,6 +247,10 @@ class BatchedClosedLoop:
             if self.cost_weights.shape != (self.n, len(_lib.COST_WEIGHT_KEYS)):
                 raise ValueError(f"cost_weights must be [{self.n}, {len(_lib.COST_WEIGHT_KEYS)}], "
                                  f"got {list(self.cost_weights.shape)}")
+        self.assess = bool(assess)
+        if self.assess and self.cost_weights is not None:
+            raise ValueError("assess=True assesses the planner's own winner; it does not take cost_weights")
+        self.last_assessment = None                     # (plan_min_distance, plan_hit_fraction) of the last step's idx
         self.post = DevicePredictionPostprocessor(pred_len=int(_knob(k, "pred_len", 12)), sgan_dt=SGAN_DT, sim_dt=self.dt,
                                                   plan_horizon=_knob(k, "max_t", 5.0), device=device)
         self.sampler = sampler
@@ -296,7 +307,7 @@ class BatchedClosedLoop:
             self._ped_step()
 
     # -- one planning attempt for the simulations `idx` -------------------------------------------
-    def _plan(self, idx, target, limits, msd, dyn_dev, mode=_lib.FOT_DYN_SINGLE):
+    def _plan(self, idx, target, limits, msd, dyn_dev, mode=_lib.FOT_DYN_SINGLE, assess_dev=None):
         import torch
         t0 = time.perf_counter()
         # ok False = conversion failure: plan() returns None (frenet_planner.py:346-374)
@@ -308,7 +319,8 @@ class BatchedClosedLoop:
         batch = DeviceBatch(self.planner, frenet, target, dyn_dev.index_select(0, sel), mode,
                             limits=limits, max_stop_distance=msd,
                             static_obstacles=self.static_points if len(self.static_points) else None,
-                            cost_weights=weights, route=None if self.route is None else self.route[np.asarray(idx)])
+                            cost_weights=weights, route=None if self.route is None else self.route[np.asarray(idx)],
+                            assess=self.assess, assess_obstacles=None if assess_dev is None else assess_dev.index_select(0, sel))
         batch.launch(None)
         if weights is None:
             o_idx, o_len, o_cost, o_win = (batch.out[key] for key in ("best_idx", "winner_len", "best_cost", "winner"))
@@ -318,6 +330,11 @@ class BatchedClosedLoop:
         wlen = o_len.cpu().numpy()
         win = o_win[:, 9:15, :2].cpu().numpy()                         # x y yaw c v a, first two samples
         found = ok & (best >= 0)
+        if self.assess:                                                # the winner's closest approach and hit share
+            S = (dyn_dev if assess_dev is None else assess_dev).shape[1]
+            a_min = batch.out["a_dyn_min"][:, 0].cpu().numpy()
+            a_frac = batch.out["a_dyn_hits"][:, 0, 0].cpu().numpy() / S
+            self._last_assess = (np.where(found, a_min, np.nan), np.where(found, a_frac, np.nan))
         self._last_full = (o_win.cpu().numpy(), o_cost.cpu().numpy()) if self.record else None
         self.timers["frenet_host"] += t1 - t0
         self.timers["sweep"] += time.perf_counter() - t1
@@ -334,7 +351,7 @@ class BatchedClosedLoop:
         # prediction (integrated_simulator.py:424-527): CV from the observer's last two float32 samples, or the
         # current positions alone while the observer is still filling
         ready = len(self.hist) >= self.obs_len
-        mode, dist_dense, best_dense = _lib.FOT_DYN_SINGLE, None, None
+        mode, dist_dense, best_dense, assess_dev = _lib.FOT_DYN_SINGLE, None, None, None
         if ready and self.sampler is not None:
             # sample sets from the generator stand-in; everything behind it on the device
             import torch
@@ -359,6 +376,8 @@ class BatchedClosedLoop:
                 if self.distribution_aware:
                     dyn = self.post.prepend_current(dense, pos, pick=None, conditional=False)
                     mode = _lib.FOT_DYN_DISTRIBUTION
+                elif self.assess:                                      # the whole sample set, t = 0 column included
+                    assess_dev = self.post.prepend_current(dense, pos, pick=None, conditional=False)
         elif ready:
             stale = max(ts - self.hist_t[-1], 0.0)
             dyn = self.post.predict_cv(self.hist[-1], self.hist[-2], stale, pos, obs_float32=True)
@@ -384,7 +403,9 @@ class BatchedClosedLoop:
         # planning cycle with escalation retries (:529-653)
         state_before = self.fsm.state[idx].copy()
         target, limits, msd = self.fsm.planner_config(idx)
-        found, wlen, win = self._plan(idx, target, limits, msd, dyn, mode)
+        found, wlen, win = self._plan(idx, target, limits, msd, dyn, mode, assess_dev)
+        if self.assess:
+            a_min, a_frac = self._last_assess
         if self.record:
             full_w, full_c = (a.copy() for a in self._last_full)
         self.fsm.update(idx, found, clearance[idx], ahead[idx], self.ego[idx, 3])
@@ -398,8 +419,10 @@ class BatchedClosedLoop:
             calls[retry] += 1
             sub = idx[retry]
             t2, l2, m2 = self.fsm.planner_config(sub)
-            f2, w2, win2 = self._plan(sub, t2, l2, m2, dyn, mode)
+            f2, w2, win2 = self._plan(sub, t2, l2, m2, dyn, mode, assess_dev)
             found[retry], wlen[retry], win[retry] = f2, w2, win2
+            if self.assess:
+                a_min[retry], a_frac[retry] = self._last_assess
             if self.record:
                 full_w[retry], full_c[retry] = self._last_full
             failed = retry[~f2]
@@ -410,6 +433,8 @@ class BatchedClosedLoop:
 
         # ego update (:655-676) or adaptive emergency stop (:749-802)
         follow = found & (wlen >= 2)
+        if self.assess:                                                # a winner shorter than 2 samples is not executed
+            a_min[~follow], a_frac[~follow] = np.nan, np.nan
         f_idx = idx[follow]
         self.ego[f_idx] = win[follow][:, [0, 1, 2, 4, 5], 1]          # x y yaw v a of the winner's second sample
         self.last_kappa[f_idx] = win[follow][:, 3, 1]                  # frenet_planner.py:301-302
@@ -449,6 +474,8 @@ class BatchedClosedLoop:
                     "dist": None if rec["dist"] is None else rec["dist"][i],
                     "ped_pos": pos[i].copy(), "ped_vel": vel[i].copy(), "pred": None if rec["pred"] is None else rec["pred"][i],
                     "path": full_w[j][:, :n_w].copy() if found[j] else None, "cost": float(full_c[j]) if found[j] else float("inf")})
+        if self.assess:
+            self.last_assessment = (a_min, a_frac)
         self.time += dt
         self.timers["total"] += time.perf_counter() - t_step
         return idx, found, calls
@@ -502,7 +529,8 @@ class BatchedClosedLoop:
         return path
 
     def run(self, n_steps: Optional[int] = None):
-        """IntegratedSimulator.run (:842-892) for every simulation; returns per-simulation histories."""
+        """IntegratedSimulator.run (:842-892) for every simulation; returns per-simulation histories (with assess=True
+        also plan_min_distance and plan_hit_fraction)."""
         if n_steps is None:
             n_steps = int(self.k["total_time"] / self.dt)
         ego_hist = np.full((self.n, n_steps, 5), np.nan)
@@ -510,6 +538,8 @@ class BatchedClosedLoop:
         found_hist = np.zeros((self.n, n_steps), dtype=bool)
         calls_hist = np.zeros((self.n, n_steps), dtype=np.int64)
         steps = np.zeros(self.n, dtype=np.int64)
+        if self.assess:
+            min_hist, frac_hist = np.full((self.n, n_steps), np.nan), np.full((self.n, n_steps), np.nan)
         for s in range(n_steps):
             if not self.active.any():
                 break
@@ -519,5 +549,10 @@ class BatchedClosedLoop:
             found_hist[idx, s] = found
             calls_hist[idx, s] = calls
             steps[idx] += 1
-        return {"ego": ego_hist, "fsm": fsm_hist, "found": found_hist, "calls": calls_hist, "steps": steps,
-                "reason": self.reason.copy()}
+            if self.assess:
+                min_hist[idx, s], frac_hist[idx, s] = self.last_assessment
+        out = {"ego": ego_hist, "fsm": fsm_hist, "found": found_hist, "calls": calls_hist, "steps": steps,
+               "reason": self.reason.copy()}
+        if self.assess:
+            out["plan_min_distance"], out["plan_hit_fraction"] = min_hist, frac_hist
+        return out
