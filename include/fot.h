@@ -38,8 +38,9 @@ extern "C" {
                                version.  Version 8: 1: + fot_weighted_t, fot_select_weighted, fot_cost_terms (winners
                                under many cost weightings, the five cost terms per candidate); + fot_route_t,
                                fot_add_route, fot_set_routes (every query on its own reference path); then, still under
-                               minor 1, + fot_assessed_t, fot_assess_trajectories: fot_abi_minor() does not tell whether
-                               a library has them, a caller looks the symbol up (DESIGN.md section 4i) */
+                               minor 1, + fot_assessed_t, fot_assess_trajectories, then fot_assess_candidates:
+                               fot_abi_minor() does not tell whether a library has them, a caller looks the symbol up
+                               (DESIGN.md sections 4i, 4j) */
 #define FOT_MAX_CIRCLES 8
 #define FOT_MAX_RANKED 32
 #define FOT_N_STATS 8    /* ok, max_speed, max_accel, max_curvature, max_lat_accel, road_bound, collision, stop_distance */
@@ -362,6 +363,33 @@ typedef struct fot_assessed {
 /* Assess the trajectories of `a` against the field `obstacles` (its query arrays are not read).  DEVICE pointers;
    stream-ordered on `stream` behind the launch that wrote the series (NULL: the handle's stream, synchronised). */
 int fot_assess_trajectories(fot_handle_t* h, const fot_batch_t* obstacles, const fot_assessed_t* a, void* stream);
+
+/* ---- candidate assessment (DESIGN.md section 4j) --------------------------------------------------------------------
+ * The assessment above for EVERY generated candidate of every query, including those the sweep rejects, without a
+ * sweep and without writing a series anywhere: each candidate is regenerated on chip and reduced there.
+ *   candidates  those query q generates, in generation order -- the grid, then the brake ladder when the query
+ *               generates it (initial s_d > 0.1): the columns of cand_cat and fot_cost_terms.  Column i of
+ *               [n_q][cand_stride] is candidate i; columns past the query's candidates (fot_candidate_count) are blank.
+ *   samples     [0, keep) with keep the reference's kept length (fp.py:826-833, :866): N when no x is NaN, else the
+ *               first NaN index when it is >= 2, else 0; a finite q = 1 - kappa_ref * d <= 0.05 at any sample makes x[0]
+ *               NaN and so keep 0.  keep == 0 gives a blank column: +inf, -1 and 0.
+ *   series      t, x, y and yaw of a candidate are the values fot_rank_candidates / fot_winner write for it, bit for bit
+ *               (the same time table, profile, spline and Frenet-to-Cartesian functions, yaw = wrap_angle).
+ * Everything else -- circle centres, time index, unfused d2, the NaN rule, the (d2, flat index) tie order, the threshold
+ * pairs and the outputs -- is fot_assess_trajectories', so column i equals what fot_assess_trajectories returns for
+ * candidate i's series with len = keep.  Under the handle's own pair a candidate of category FOT_CAT_OK, FOT_CAT_COLL or
+ * FOT_CAT_STOP is collision-free iff its category is not FOT_CAT_COLL.  The query's route follows fot_set_routes; a route
+ * id out of range gives blank columns and reads no route table.
+ *   queries  frenet, target_speed, v_grid, n_v, n_v_max and n_q of a fot_batch_t (what fot_cost_terms reads)
+ *   field    the dyn / S / P / T_obs / dyn_mode / static_obs / n_static / static_per_query part of a fot_batch_t of the
+ *            same n_q queries, as for fot_assess_trajectories: the planning field or another one
+ *   out      a fot_assessed_t with m == cand_stride (FOT_MAX_ASSESSED does not bound it here), series and len NULL,
+ *            n_t ignored; its outputs are [n_q][cand_stride][...]
+ *   keep     [n_q][cand_stride] kept samples per column (0 for blank columns), or NULL
+ * DEVICE pointers; asynchronous on `stream` (NULL: the handle's stream, synchronised).  Declared under FOT_ABI_MINOR 1:
+ * a caller looks the symbol up. */
+int fot_assess_candidates(fot_handle_t* h, const fot_batch_t* queries, const fot_batch_t* field, int cand_stride,
+                          const fot_assessed_t* out, int32_t* keep, void* stream);
 
 /* ---- next row (SURVEY.md section 8f, rank 1): the predictor's post-processing on the device ---------
  * Builds the obstacle tensor fot_batch_t.dyn consumes, so that batched roll-outs never upload it.

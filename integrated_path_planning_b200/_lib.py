@@ -150,6 +150,8 @@ SYMBOLS = (
     ("fot_add_route", C.c_int, (C.c_void_p, C.POINTER(FotRoute), C.POINTER(C.c_int32))),
     ("fot_set_routes", C.c_int, (C.c_void_p, C.c_void_p)),
     ("fot_assess_trajectories", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotAssessed), C.c_void_p)),
+    ("fot_assess_candidates", C.c_int, (C.c_void_p, C.POINTER(FotBatch), C.POINTER(FotBatch), C.c_int,
+                                        C.POINTER(FotAssessed), C.c_void_p, C.c_void_p)),
 )
 
 _lib = None

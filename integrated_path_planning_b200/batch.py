@@ -34,7 +34,7 @@ class BatchFrenetPlanner(FrenetPlanner):
                    want_candidates: bool = False, winner_samples: int = 0, top_k: int = 0,
                    rank_series: bool = True, cost_weights=None, weight_series: bool = True,
                    cost_terms: bool = False, route=None, assess: bool = False, assess_obstacles=None,
-                   assess_r2=None) -> SweepResult:
+                   assess_r2=None, assess_candidates: bool = False) -> SweepResult:
         """frenet_states [n_q,6]; target_speed scalar or [n_q]; dynamic_obstacles [n_q,P,T,2] or
         distribution [n_q,S,P,T,2]; static_obstacles [M,2] (shared) or [n_q,M,2]; limits [n_q,4]
         overrides constraint_overrides; max_stop_distance scalar / [n_q] (NaN = none); winner_samples = k > 0
@@ -48,11 +48,13 @@ class BatchFrenetPlanner(FrenetPlanner):
         A routed query gives what a planner built on its route gives.  assess: also the closest approach and collision
         counts of the winner (and of the ranked alternatives with top_k > 0) against the batch's own obstacle field, or
         against assess_obstacles [n_q, S, P, T, 2], under the threshold pairs assess_r2 (`DeviceBatch`;
-        `SweepResult.assessed`, `assessment`)."""
+        `SweepResult.assessed`, `assessment`).  assess_candidates: the same assessment for every generated candidate,
+        the rejected ones included, against the same field and pairs (`SweepResult.cand_assessed`,
+        `candidate_assessment`; with want_candidates the table's categories and costs come along)."""
         q, _ = self._batch_arrays(frenet_states, target_speed, dynamic_obstacles, distribution, static_obstacles,
                                   constraint_overrides, limits, max_stop_distance, route=route)
         return self._run(q, want_candidates, winner_samples, top_k, rank_series, cost_weights, weight_series, cost_terms,
-                         assess, assess_obstacles, assess_r2)
+                         assess, assess_obstacles, assess_r2, assess_candidates)
 
     def _batch_arrays(self, frenet_states, target_speed, dynamic_obstacles=None, distribution=None,
                       static_obstacles=None, constraint_overrides=None, limits=None, max_stop_distance=None, route=None,
@@ -121,12 +123,19 @@ class DeviceBatch:
     own (dyn and static obstacles), or assess_obstacles [n_q, S, P, T, 2] (a NumPy array or a CUDA tensor, read as S
     samples of P pedestrians) with the batch's static obstacles.  assess_r2: threshold pairs (r2_dyn, r2_static), one
     or [n_r, 2]; None: the handle's own pair for that field (`SweepEngine.own_radii`), under which a trajectory is
-    collision-free iff static_hit == 0 and dyn_hits <= floor(chance_epsilon * S)."""
+    collision-free iff static_hit == 0 and dyn_hits <= floor(chance_epsilon * S).
+
+    assess_candidates: every launch also assesses every generated candidate of every query -- regenerated on the
+    device, never stored (fot_assess_candidates, DESIGN.md section 4j) -- against the same field and threshold pairs
+    into out["ca_<name>"] [n_q, stride, ...] for the names of engine.ASSESS_FIELDS and out["ca_keep"] [n_q, stride],
+    column i candidate i in generation order.  candidate_table: also write the per-candidate categories and costs
+    (for `sweep_result(want_candidates=True)` without top_k)."""
 
     def __init__(self, planner: FrenetPlanner, frenet_states, target_speed, dyn, dyn_mode, limits=None,
                  max_stop_distance=None, static_obstacles=None, top_k: int = 0, rank_series: bool = True,
                  cost_weights=None, weight_series: bool = True, cost_terms: bool = False, route=None,
-                 assess: bool = False, assess_obstacles=None, assess_r2=None):
+                 assess: bool = False, assess_obstacles=None, assess_r2=None, assess_candidates: bool = False,
+                 candidate_table: bool = False):
         import torch
         q = query_arrays(frenet_states, target_speed, planner.resolve_limits(None) if limits is None else limits,
                          max_stop_distance, static_obstacles, dyn, dyn_mode, planner.d_t_s)
@@ -137,9 +146,11 @@ class DeviceBatch:
             raise ValueError(f"top_k must be in [1, {_lib.FOT_MAX_RANKED}]")
         weights, per_query = _weight_table(cost_weights, n_q)
         self.assess = bool(assess)
-        a_obs, a_mode = _assess_field(assess_obstacles, n_q) if self.assess else (None, None)
+        self.assess_candidates = bool(assess_candidates)
+        any_assess = self.assess or self.assess_candidates
+        a_obs, a_mode = _assess_field(assess_obstacles, n_q) if any_assess else (None, None)
         a_mode = q.dyn_mode if a_obs is None else a_mode
-        a_r2 = assess_radii(assess_r2) if self.assess and assess_r2 is not None else None
+        a_r2 = assess_radii(assess_r2) if any_assess and assess_r2 is not None else None
         self.n_w = 0 if weights is None else weights.shape[-2]
         eng = planner.engine
         dev = torch.device("cuda", eng.device)
@@ -169,9 +180,9 @@ class DeviceBatch:
                 s.series = new(self.out, prefix + "_series", (n_q, m, _lib.FOT_N_SERIES, eng.n_t_max), torch.float64)
             return s
 
-        if self.top_k > 0 or self.n_w > 0:
+        if self.top_k > 0 or self.n_w > 0 or candidate_table:
             new(self.t, "cand_cat", (n_q, self.stride), torch.uint8)
-        if self.top_k > 0:
+        if self.top_k > 0 or candidate_table:
             new(self.t, "cand_cost", (n_q, self.stride), torch.float64)
             self.ranked = selections("rank", self.top_k, rank_series, _lib.FotRanked(k=self.top_k))
         if self.n_w > 0:
@@ -182,7 +193,7 @@ class DeviceBatch:
         self.cost_terms = bool(cost_terms)
         if self.cost_terms:
             new(self.out, "cost_terms", (n_q, self.stride, 5), torch.float64)
-        if self.assess:
+        if any_assess:
             self.assess_field = _lib.FotBatch.from_buffer_copy(self.batch)
             if a_obs is not None:
                 self.t["a_dyn"] = a_obs.to(dev).contiguous() if isinstance(a_obs, torch.Tensor) else torch.from_numpy(a_obs).to(dev)
@@ -191,6 +202,7 @@ class DeviceBatch:
                 f.S, f.P, f.T_obs = a_obs.shape[1], a_obs.shape[2], a_obs.shape[3]
             r2 = eng.own_radii(a_mode) if a_r2 is None else a_r2
             self.t["a_r2"] = torch.from_numpy(r2).to(dev)
+        if self.assess:
             ranked = self.top_k > 0 and rank_series
             m, n_r = (self.top_k if ranked else 1), r2.shape[0]
             a = _lib.FotAssessed(m=m, n_t=eng.n_t_max, n_r=n_r, r2=self.t["a_r2"].data_ptr())
@@ -200,6 +212,14 @@ class DeviceBatch:
                 setattr(a, name, new(self.out, "a_" + name, (n_q, m, *(n_r if d == "r" else d for d in shape)),
                                      getattr(torch, dt)))
             self.assessed = a
+        if self.assess_candidates:
+            n_r = self.t["a_r2"].shape[0]
+            a = _lib.FotAssessed(m=self.stride, n_t=0, n_r=n_r, r2=self.t["a_r2"].data_ptr())
+            for name, dt, shape in ASSESS_FIELDS:
+                setattr(a, name, new(self.out, "ca_" + name, (n_q, self.stride, *(n_r if d == "r" else d for d in shape)),
+                                     getattr(torch, dt)))
+            new(self.out, "ca_keep", (n_q, self.stride), torch.int32)
+            self.cand_assessed = a
         self.result = fot_result(dict(self.out, **self.t), torch.Tensor.data_ptr)
 
     def launch(self, stream: Optional[int] = None) -> None:
@@ -230,6 +250,9 @@ class DeviceBatch:
                 self.engine.cost_terms_device(self.batch, self.stride, self.out["cost_terms"].data_ptr(), stream)
             if self.assess:
                 self.engine.assess_device(self.assess_field, self.assessed, stream)
+            if self.assess_candidates:
+                self.engine.assess_candidates_device(self.batch, self.assess_field, self.stride, self.cand_assessed,
+                                                     self.out["ca_keep"].data_ptr(), stream)
 
     def sweep_result(self, want_candidates: bool = False, winner_samples: int = 0) -> SweepResult:
         """Host copy of the outputs of the last launch, once it has finished (launch() without a stream waits), as a
@@ -237,8 +260,11 @@ class DeviceBatch:
         categories alone); winner_samples = k > 0: the first k samples of each winner series."""
         host = {k: v.cpu().numpy() for k, v in self.out.items()}
         assessed = {name: host.pop("a_" + name) for name, _, _ in ASSESS_FIELDS} if self.assess else None
+        cand_assessed = {name: host.pop("ca_" + name) for name in (*(f[0] for f in ASSESS_FIELDS), "keep")} \
+            if self.assess_candidates else None
         res = SweepResult(**host)
         res.assessed = assessed
+        res.cand_assessed = cand_assessed
         if winner_samples and winner_samples > 0:
             res.winner = np.ascontiguousarray(res.winner[:, :, :min(int(winner_samples), res.winner.shape[2])])
         if want_candidates:
@@ -254,11 +280,13 @@ class DeviceBatch:
         only the first k samples of every winner series come back (`host_out["winner"]` is [n_q, 15, k]) -- what a
         closed-loop caller consumes (integrated_simulator.py:663), 240 B instead of 6.1 KB per query at k = 2.
         Ranked, weighted and assessed outputs do not come back through this call: a batch with top_k > 0,
-        cost_weights, cost_terms or assess raises ValueError."""
+        cost_weights, cost_terms, assess or assess_candidates raises ValueError."""
         if self.top_k > 0:
             raise ValueError("launch_to_host does not return ranked outputs; use launch() with top_k > 0")
         if self.assess:
             raise ValueError("launch_to_host does not return assessments; use launch() with assess=True")
+        if self.assess_candidates:
+            raise ValueError("launch_to_host does not return candidate assessments; use launch() with assess_candidates=True")
         if self.n_w > 0 or self.cost_terms:
             raise ValueError("launch_to_host does not return weighted outputs or cost terms; use launch()")
         import ctypes as C

@@ -13,7 +13,7 @@ DEPS = [SRC, os.path.join(HERE, "csrc", "fot_kernels.cuh"), os.path.join(HERE, "
         os.path.join(HERE, "csrc", "fot_sweep_math.cuh"),
         os.path.join(HERE, "csrc", "fot_predict.cuh"), os.path.join(HERE, "csrc", "fot_frenet.cuh"),
         os.path.join(HERE, "csrc", "fot_rank.cuh"), os.path.join(HERE, "csrc", "fot_weights.cuh"),
-        os.path.join(HERE, "csrc", "fot_assess.cuh"),
+        os.path.join(HERE, "csrc", "fot_assess.cuh"), os.path.join(HERE, "csrc", "fot_assess_cand.cuh"),
         os.path.join(ROOT, "include", "fot.h")]
 OUT = os.path.join(HERE, "libfot.so")
 

@@ -20,6 +20,7 @@
 #include "fot_rank.cuh"
 #include "fot_weights.cuh"
 #include "fot_assess.cuh"
+#include "fot_assess_cand.cuh"
 
 using namespace fot;
 
@@ -149,6 +150,7 @@ struct fot_handle {
   int sms = 148;                     // SM count of the device (block-per-CTA grouping, host chunk sizes)
   Buf part_cost, part_idx, dyn_box, cost_tab;   // device scratch
   Buf w_pieces;                      // cost pieces of fot_select_weighted / fot_cost_terms (fot_weights.cuh)
+  Buf ca_nan;                        // NaN bits of the pedestrian trajectories of fot_assess_candidates (fot_assess_cand.cuh)
   int last_pair_feat = -1;           // mode set (PAIR_*) of the fot_sweep_pairs instantiation of the last launch
   int last_sweep_kind = 0;           // 4: fot_sweep_pairs, 1: fot_sweep_items
   fot_result_t mirror{};             // fot_set_result_mirror: second destination of the winner block (all null: none)
@@ -285,8 +287,8 @@ extern "C" int fot_destroy(fot_handle_t* h) {
   { std::lock_guard<std::mutex> lk(g_live_mu); g_live.erase(h); }
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();          // every stream of the handle (compute, priority, copy) is idle before its buffers go
-  for (Buf* b : {&h->gate_d, &h->gate_h, &h->part_cost, &h->part_idx, &h->dyn_box, &h->cost_tab, &h->w_pieces, &h->stage_h, &h->stage_d,
-                 &h->out_d, &h->dyn_d, &h->stat_d})
+  for (Buf* b : {&h->gate_d, &h->gate_h, &h->part_cost, &h->part_idx, &h->dyn_box, &h->cost_tab, &h->w_pieces, &h->ca_nan, &h->stage_h,
+                 &h->stage_d, &h->out_d, &h->dyn_d, &h->stat_d})
     b->release();
   if (h->tables_dev) cudaFree(h->tables_dev);
   if (h->routes_dev) cudaFree(h->routes_dev);
@@ -728,6 +730,72 @@ extern "C" int fot_assess_trajectories(fot_handle_t* h, const fot_batch_t* b, co
   const Assess A{a->m, a->n_t, a->n_r, a->series, a->len, a->r2, a->dyn_min, a->dyn_at, a->static_min, a->static_at,
                  a->dyn_hits, a->first_hit, a->static_hit};
   fot_assess<<<(unsigned)b->n_q, threads, smem, st>>>(h->plan, B, A);
+  CK(cudaGetLastError());
+  if (!stream) CK(cudaStreamSynchronize(st));
+  return FOT_OK;
+}
+
+extern "C" int fot_assess_candidates(fot_handle_t* h, const fot_batch_t* b, const fot_batch_t* f, int cand_stride,
+                                     const fot_assessed_t* a, int32_t* keep, void* stream) {
+  if (!h || !b || !f || !a) return fail(FOT_ERR_ARG, "fot_assess_candidates: null argument");
+  if (b->n_q < 1 || b->n_v_max < 1) return fail(FOT_ERR_ARG, "fot_assess_candidates: n_q and n_v_max must be >= 1");
+  if (a->series || a->len) return fail(FOT_ERR_ARG, "fot_assess_candidates: series and len must be null (candidates are regenerated)");
+  if (a->m != cand_stride) return fail(FOT_ERR_ARG, "fot_assess_candidates: m must equal cand_stride");
+  if (a->n_r < 1 || a->n_r > FOT_MAX_RADII) return fail(FOT_ERR_ARG, "fot_assess_candidates: n_r must be in [1, FOT_MAX_RADII]");
+  if (!a->r2) return fail(FOT_ERR_ARG, "fot_assess_candidates: null r2");
+  if (!a->dyn_min || !a->dyn_at || !a->static_min || !a->static_at || !a->dyn_hits || !a->first_hit || !a->static_hit)
+    return fail(FOT_ERR_ARG, "fot_assess_candidates: null output array");
+  if (!b->frenet || !b->target_speed || !b->v_grid || !b->n_v) return fail(FOT_ERR_ARG, "fot_assess_candidates: null query array");
+  if (f->n_static < 0 || f->S < 0 || f->P < 0 || f->T_obs < 0)
+    return fail(FOT_ERR_ARG, "fot_assess_candidates: negative obstacle shape");
+  if (f->n_static > 0 && !f->static_obs) return fail(FOT_ERR_ARG, "fot_assess_candidates: static obstacles missing");
+  if (f->dyn_mode != FOT_DYN_NONE && f->dyn_mode != FOT_DYN_SINGLE && f->dyn_mode != FOT_DYN_DISTRIBUTION)
+    return fail(FOT_ERR_ARG, "fot_assess_candidates: bad dyn_mode");
+  const bool has_dyn = f->dyn_mode != FOT_DYN_NONE && (long long)f->S * f->P * f->T_obs > 0;
+  if (has_dyn && !f->dyn) return fail(FOT_ERR_ARG, "fot_assess_candidates: dynamic obstacles missing");
+  if ((size_t)b->n_q * cand_stride * a->n_r > 0x7fffffffull) return fail(FOT_ERR_ARG, "fot_assess_candidates: batch too large");
+  const int n_max = fot_candidate_count(h, b->n_v_max, 1);
+  if (cand_stride < n_max) return fail(FOT_ERR_ARG, "fot_assess_candidates: cand_stride too small");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  Batch B{};
+  B.n_q = b->n_q; B.n_v_max = b->n_v_max;
+  B.frenet = b->frenet; B.target = b->target_speed; B.v_grid = b->v_grid; B.n_v = b->n_v;
+  B.n_static = f->n_static; B.static_per_query = f->static_per_query;
+  B.S = has_dyn ? f->S : 0; B.P = has_dyn ? f->P : 0; B.T_obs = has_dyn ? f->T_obs : 0; B.dyn_mode = f->dyn_mode;
+  B.dyn_raw = has_dyn ? f->dyn : nullptr;
+  B.static_raw = f->n_static > 0 ? f->static_obs : nullptr;
+  B.rt = routes_of(h, 0);
+  AssessCand C{};
+  C.A = Assess{a->m, 0, a->n_r, nullptr, nullptr, a->r2, a->dyn_min, a->dyn_at, a->static_min, a->static_at,
+               a->dyn_hits, a->first_hit, a->static_hit};
+  C.keep = keep;
+  const long long SP = (long long)B.S * B.P;
+  if (has_dyn) {
+    // one bit per pedestrian trajectory: a NaN at any step (the NaN rule), once per launch
+    C.nan_words = (int32_t)((SP + 31) / 32);
+    const long long n_words = (long long)b->n_q * C.nan_words;
+    if ((n_words * 32 + 255) / 256 > 0x7fffffffll) return fail(FOT_ERR_ARG, "fot_assess_candidates: field too large for one launch");
+    CK(h->ca_nan.reserve((size_t)n_words * sizeof(unsigned)));
+    C.nan_bits = (const unsigned*)h->ca_nan.p;
+    fot_assess_cand_nan<<<(unsigned)((n_words * 32 + 255) / 256), 256, 0, st>>>((const double2*)f->dyn, SP, B.T_obs, n_words,
+                                                                             C.nan_words, (unsigned*)h->ca_nan.p);
+  }
+  C.sc = has_dyn ? std::min(B.S, kCandPass) : 0;
+  // CTAs per query: one once the batch fills the GPU several times over; a small batch (one plan() call of 66 563
+  // candidates) is dealt to many
+  const long long per_cta = kCandThreads;
+  long long cpq = ((long long)h->sms * 4 + b->n_q - 1) / b->n_q;
+  cpq = std::max<long long>(1, std::min<long long>(cpq, (n_max + per_cta - 1) / per_cta));
+  C.cpq = (int32_t)cpq;
+  if ((long long)b->n_q * cpq > 0x7fffffffll) return fail(FOT_ERR_ARG, "fot_assess_candidates: batch too large for one launch");
+  const size_t stage_bytes = (size_t)SP * B.T_obs * sizeof(double2);
+  const bool stage = has_dyn && stage_bytes <= kCandStageMax;
+  const size_t smem = assess_cand_smem(h->plan.n_t_max, a->n_r, C.sc, stage ? stage_bytes : 0);
+  if (smem > (size_t)h->smem_optin) return fail(FOT_ERR_TOO_LARGE, "fot_assess_candidates: shared memory");
+  auto kern = stage ? fot_assess_cand<true> : fot_assess_cand<false>;
+  if (smem > 32 * 1024) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<(unsigned)(b->n_q * cpq), kCandThreads, smem, st>>>(h->plan, B, C);
   CK(cudaGetLastError());
   if (!stream) CK(cudaStreamSynchronize(st));
   return FOT_OK;

@@ -258,6 +258,10 @@ class SweepResult:
     # [n_q, m], [n_q, m, 4], [n_q, m, 3] or [n_q, m, n_r]; column 0 the winner, or with ranked series column j rank j.
     # A plain attribute, not a field: None unless the batch was assessed.
     assessed = None
+    # candidate assessment (assess_candidates=True; include/fot.h fot_assess_candidates): the same names plus "keep",
+    # [n_q, stride, ...], column i candidate i in generation order, blank past the query's candidates.  A plain
+    # attribute: None unless the batch asked for it.
+    cand_assessed = None
 
     def series(self, q: int = 0):
         """The 15 winner sequences of query q truncated to their kept length, or None."""
@@ -286,6 +290,20 @@ class SweepResult:
             raise ValueError("this result has no assessment: run the batch with assess=True")
         return {name: self.assessed[name][q].copy() for name, _, _ in ASSESS_FIELDS}
 
+    def candidate_assessment(self, q: int = 0):
+        """The assessment of every candidate of query q (a batch run with assess_candidates=True): {name: array} for
+        the names of ASSESS_FIELDS and "keep" (samples assessed), one row per candidate in generation order, trimmed to
+        the query's n_cand candidates; with "cand_cat" and "cand_cost" too when the candidate table was requested.
+        Rows with keep 0 (emptied candidates, failed conversions) hold +inf, -1 and 0."""
+        if self.cand_assessed is None:
+            raise ValueError("this result has no candidate assessment: run the batch with assess_candidates=True")
+        n = int(self.n_cand[q]) if self.n_cand is not None else self.cand_assessed["keep"].shape[1]
+        out = {name: self.cand_assessed[name][q, :n].copy() for name in (*(f[0] for f in ASSESS_FIELDS), "keep")}
+        for name in ("cand_cat", "cand_cost"):
+            if getattr(self, name) is not None:
+                out[name] = getattr(self, name)[q, :n].copy()
+        return out
+
     def _entry(self, block: str, q: int, j: int):
         """Entry j of query q of the ranked ("rank") or weighted ("w") outputs, or None where its index is -1."""
         i = int(getattr(self, block + "_idx")[q, j])
@@ -299,8 +317,8 @@ class SweepResult:
 
     def blank(self, rows) -> None:
         """Queries `rows` (indices or a mask) as plan() returning None leaves them: index -1, cost inf, stats and kept
-        lengths 0 in the winner, ranked and weighted outputs, cost terms NaN, assessments blank (+inf, -1, 0); the
-        series and candidate table stay."""
+        lengths 0 in the winner, ranked and weighted outputs, cost terms NaN, assessments and candidate assessments
+        blank (+inf, -1, 0, keep 0); the series and candidate table stay."""
         for name, value in (("best_idx", -1), ("best_cost", np.inf), ("stats", 0), ("winner_len", 0), ("rank_idx", -1),
                             ("rank_cost", np.inf), ("rank_len", 0), ("w_idx", -1), ("w_cost", np.inf), ("w_len", 0),
                             ("cost_terms", np.nan)):
@@ -308,9 +326,11 @@ class SweepResult:
             if a is not None:
                 a[rows] = value
         for name, value in (("dyn_min", np.inf), ("dyn_at", -1), ("static_min", np.inf), ("static_at", -1),
-                            ("dyn_hits", 0), ("first_hit", -1), ("static_hit", 0)):
-            if self.assessed is not None:
+                            ("dyn_hits", 0), ("first_hit", -1), ("static_hit", 0), ("keep", 0)):
+            if self.assessed is not None and name in self.assessed:
                 self.assessed[name][rows] = value
+            if self.cand_assessed is not None:
+                self.cand_assessed[name][rows] = value
 
 
 class SweepEngine:
@@ -521,6 +541,15 @@ class SweepEngine:
         stream-ordered behind the launch that wrote their series."""
         _lib.check(self.lib.fot_assess_trajectories(self._h, C.byref(obstacles), C.byref(assessed),
                                                     C.c_void_p(stream) if stream else None), "fot_assess_trajectories")
+
+    def assess_candidates_device(self, queries: "_lib.FotBatch", field: "_lib.FotBatch", cand_stride: int,
+                                 assessed: "_lib.FotAssessed", keep: Optional[int] = None, stream=None) -> None:
+        """fot_assess_candidates: every generated candidate of `queries` (device pointers) regenerated on the device and
+        assessed against the field of `field` into the [n_q, cand_stride, ...] outputs of `assessed` (series and len
+        null) and keep [n_q, cand_stride] (or None).  Needs no sweep."""
+        _lib.check(self.lib.fot_assess_candidates(self._h, C.byref(queries), C.byref(field), int(cand_stride),
+                                                  C.byref(assessed), C.c_void_p(keep) if keep else None,
+                                                  C.c_void_p(stream) if stream else None), "fot_assess_candidates")
 
     def nearest_s(self, x, y, prev_s, route=None):
         """fot_nearest_s_device for m points on this engine's path (route: [m] route ids, point k on route[k]): returns

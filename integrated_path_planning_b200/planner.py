@@ -265,6 +265,39 @@ class FrenetPlanner:
                 res[name] = res[name][:, 1:]
         return res
 
+    def candidate_assessment(self, ego_state, static_obstacles, dynamic_obstacles=None,
+                             target_speed: float = TARGET_SPEED, constraint_overrides: Optional[Dict[str, float]] = None,
+                             dynamic_obstacles_distribution=None, max_stop_distance: Optional[float] = None,
+                             assess_obstacles=None, r2=None) -> Optional[Dict[str, np.ndarray]]:
+        """Every candidate plan() generates from the current ego state, the rejected ones included, with how close it
+        comes to an obstacle field (fot_assess_candidates, DESIGN.md section 4j): {name: array with one row per
+        candidate, in generation order} -- "cand_cat" (the sweep's category, _lib.CAT_*), "cand_cost", "keep" (samples
+        assessed; 0 for an emptied candidate, whose row is blank: +inf, -1, 0) and the names of engine.ASSESS_FIELDS.
+        The field is plan()'s own, or assess_obstacles [S, P, T, 2] (read as S samples, with plan()'s static points).
+        r2: threshold pairs (r2_dyn, r2_static), one or [n_r, 2]; None: the planner's own pair for the field, under
+        which a candidate of category OK, COLL or STOP is collision-free iff it is not COLL.  None where plan() returns
+        None before sweeping (the ego state does not convert).  Side effects are plan()'s, from the winner of the same
+        launch: last_check_stats, last_result, the nearest-point cache and the curvature fed back."""
+        user_r2 = None if r2 is None else assess_radii(r2)               # checked before the device is used
+        field = None
+        if assess_obstacles is not None:
+            field = np.asarray(assess_obstacles, dtype=np.float64)
+            if field.ndim != 4 or field.shape[-1] != 2:
+                raise ValueError(f"assess_obstacles must be [S, P, T, 2], got {list(field.shape)}")
+            field = field[None]
+        self.last_check_stats = None
+        self.last_result = None
+        fs = self._cartesian_to_frenet_state(ego_state)
+        if fs is None:
+            return None
+        res = self._sweep(fs.to_array(), static_obstacles, dynamic_obstacles, target_speed, constraint_overrides,
+                          dynamic_obstacles_distribution, max_stop_distance, want_candidates=True,
+                          assess_candidates=True, assess_obstacles=field, assess_r2=user_r2)
+        own = res.series(0)
+        if own is not None:
+            self._feed_back_curvature(_frenet_path(own, res.best_cost[0]))
+        return res.candidate_assessment(0)
+
     def cost_weight_table(self, weights) -> np.ndarray:
         """[n_w, 6] float64 weightings (columns _lib.COST_WEIGHT_KEYS) from an [n_w, 6] array or a list of dicts keyed
         by those names; a key a dict leaves out takes this planner's own value.  Raises ValueError on anything else
@@ -300,7 +333,7 @@ class FrenetPlanner:
 
     def _sweep(self, frenet_state, static_obstacles, dynamic_obstacles, target_speed, constraint_overrides,
                dynamic_obstacles_distribution, max_stop_distance, want_candidates: bool = False,
-               top_k: int = 0, cost_weights=None) -> SweepResult:
+               top_k: int = 0, cost_weights=None, **assess) -> SweepResult:
         """One query through the sweep (ranked when top_k > 0, selected under each weighting of cost_weights [n_w, 6]
         when given); sets last_result and last_check_stats."""
         mode, dyn = classify_dynamic(dynamic_obstacles, dynamic_obstacles_distribution)
@@ -309,7 +342,7 @@ class FrenetPlanner:
             static = np.asarray(static_obstacles, dtype=np.float64).reshape(-1, 2)
         q = query_arrays(np.reshape(frenet_state, (1, 6)), float(target_speed), self.resolve_limits(constraint_overrides),
                          max_stop_distance, static, dyn, mode, self.d_t_s)
-        res = self._run(q, want_candidates, top_k=top_k, cost_weights=cost_weights)
+        res = self._run(q, want_candidates, top_k=top_k, cost_weights=cost_weights, **assess)
         self.last_result = res
         stats = {key: int(res.stats[0, _lib.STAT_KEYS.index(key)]) for key in _REF_STAT_ORDER}
         if max_stop_distance is not None:
@@ -319,16 +352,19 @@ class FrenetPlanner:
 
     def _run(self, q: QueryArrays, want_candidates: bool = False, winner_samples: int = 0, top_k: int = 0,
              rank_series: bool = True, cost_weights=None, weight_series: bool = True,
-             cost_terms: bool = False, assess: bool = False, assess_obstacles=None, assess_r2=None) -> SweepResult:
+             cost_terms: bool = False, assess: bool = False, assess_obstacles=None, assess_r2=None,
+             assess_candidates: bool = False) -> SweepResult:
         """Sweep the batch q: as a device-resident `DeviceBatch` when it asks for ranked alternatives, cost weightings,
         cost terms or an assessment (outputs only the device-side calls produce), otherwise through the host-pointer
         call."""
-        if top_k > 0 or cost_weights is not None or cost_terms or assess:
+        if top_k > 0 or cost_weights is not None or cost_terms or assess or assess_candidates:
             from .batch import DeviceBatch           # batch.py builds on this module
             db = DeviceBatch(self, q.frenet, q.target, q.dyn, q.dyn_mode, limits=q.limits, max_stop_distance=q.stop,
                              static_obstacles=q.static, top_k=top_k, rank_series=rank_series,
                              cost_weights=cost_weights, weight_series=weight_series, cost_terms=cost_terms,
-                             route=q.route, assess=assess, assess_obstacles=assess_obstacles, assess_r2=assess_r2)
+                             route=q.route, assess=assess, assess_obstacles=assess_obstacles, assess_r2=assess_r2,
+                             assess_candidates=assess_candidates,
+                             candidate_table=assess_candidates and want_candidates)
             db.launch()
             return db.sweep_result(want_candidates, winner_samples)
         return self.engine.run_host(q, want_candidates, winner_samples)
